@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (one rank per GPU under torchrun for N>1)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py ... --dump-outputs DIR                    (also write the last timed step's outputs, see dump_outputs)
 
 A "step" = one pass of the hot path over one batch: mapped reads (SoA) -> per-base depth of every
 contig -> per-contig statistics (the work of reference metacov/pileup.py:9-26 driven by the loop at
@@ -163,8 +164,7 @@ def run_reference(args):
     """--impl reference: the CPU implementation of the path on the host cores (the reference itself needs
     pysam/htslib, absent from this image, so this is the C port of oracle/, kind 'port').  Same workload as the GPU
     arm at the same N (N x the named shape); built with the oracle-side generator, so this process never loads the
-    product library.  A step = the whole workload; the number of timed steps is bounded so that the run ends within
-    a few minutes."""
+    product library.  A step = the whole workload; --warmup untimed steps, then exactly --steps timed ones."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -177,36 +177,67 @@ def run_reference(args):
     regions = (tid, np.zeros_like(tid), w.contig_len)
     times = []
     aligned = 0
-    budget_s, t_begin = 150.0, time.perf_counter()
-    steps_done = 0
     for k in range(args.warmup + args.steps):
         t0 = time.perf_counter()
         d, off, info = cport.depth(batch, w.contig_len, mode="par", threads=cores)
-        cport.region_stats(d, off, w.contig_len, *regions, threads=cores)
+        st = cport.region_stats(d, off, w.contig_len, *regions, threads=cores)
         dt = time.perf_counter() - t0
         aligned = info["aligned_bases"]
         if k >= args.warmup:
             times.append(dt)
-            steps_done += 1
-            if time.perf_counter() - t_begin > budget_s and steps_done >= 2:
-                break
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, st, w.contig_len, lambda c: d[off[c]:off[c] + w.contig_len[c]])
     ms = 1e3 * float(np.mean(times))
     value = aligned / (ms / 1e3)
     py_rate, py_n = python_port_rate(batch, w.contig_len, 1)
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
-        "steps": steps_done, "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True,
+        "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "int32", "data": "synthetic",
         "config": {"workload": workload_label(args.workload, args.gpus, w), "scale": args.scale},
         "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": "port",
-                         "sample": "the whole %s workload per step (C port oracle/coverage.c, contig-parallel pthreads); %d of the %d "
-                                   "requested steps timed (time budget %d s)" % (args.workload, steps_done, args.steps, int(budget_s)),
+                         "sample": "the whole %s workload per step (C port oracle/coverage.c, contig-parallel pthreads), %d timed "
+                                   "steps" % (args.workload, args.steps),
                          "python_port_value": py_rate,
                          "python_port_sample": "first contig (%d reads) through the reference-structured Python loop, 1 core" % py_n},
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
     emit(args.real_stdout, line)
+
+
+DUMP_STATS_FIELDS = ("sum", "sumsq", "iq_sum", "n_ge1", "n_geN", "min", "max", "med_lo", "med_hi", "flags")
+DUMP_MAX_REGIONS = 100_000           # 10 float64 fields: at most 8 MB of statistics
+DUMP_MAX_DEPTH = 12 * 2 ** 20        # float32 depth values: at most 48 MB
+
+
+def dump_outputs(out_dir, records, lengths, depth_of, tid_base=0):
+    """--dump-outputs: what the timed path handed its caller in the last step, as DIR/<name>.npy.
+    `records` are the statistics records, `depth_of(c)` the depth of local contig c (length lengths[c]).
+
+    stats_<field>.npy   per-region statistics records (float64), one entry per region in region order; above
+                        DUMP_MAX_REGIONS regions a seeded sample, whose region indices are in stats_index.npy
+    depth.npy           per-base depth (float32) of a seeded sample of whole contigs, concatenated
+    depth_contigs.npy   the global contig ids of that sample, in the order their depth is concatenated (float64)
+    With the same arguments the workload is the same, so two builds give files that compare entry by entry.
+    With --gpus N > 1 rank 0 writes the file: the records are the gathered ones of all regions, the depth sample is
+    drawn from rank 0's own contig range only (the reference arm draws from all contigs), so depth samples of the two
+    arms at N > 1 are matched through depth_contigs.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    g = len(records)
+    idx = np.arange(g) if g <= DUMP_MAX_REGIONS else np.sort(np.random.default_rng(0).choice(g, DUMP_MAX_REGIONS, replace=False))
+    if g > DUMP_MAX_REGIONS:
+        np.save(os.path.join(out_dir, "stats_index.npy"), idx.astype(np.float64))
+    for f in DUMP_STATS_FIELDS:
+        np.save(os.path.join(out_dir, "stats_%s.npy" % f), records[f][idx].astype(np.float64))
+    contigs, room = [], DUMP_MAX_DEPTH
+    for c in np.random.default_rng(1).permutation(len(lengths)):
+        if lengths[c] <= room:
+            contigs.append(int(c))
+            room -= int(lengths[c])
+    depth = [depth_of(c) for c in contigs]
+    np.save(os.path.join(out_dir, "depth.npy"), np.concatenate(depth).astype(np.float32) if depth else np.zeros(0, np.float32))
+    np.save(os.path.join(out_dir, "depth_contigs.npy"), np.asarray(contigs, dtype=np.float64) + tid_base)
 
 
 def batch_bytes(b):
@@ -259,7 +290,7 @@ def strong_scaling_c4(args, sharding, synth, dist, torch, world, rank, local, de
     al = torch.tensor([info["aligned_bases"]], dtype=torch.int64, device=dev)
     if world > 1:
         dist.all_reduce(al)
-    steps = max(5, min(args.steps, 20))
+    steps = args.steps
     barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
@@ -437,10 +468,12 @@ def run_ours(args):
     l0 = eng.launch_count()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
-    run_steps(args.steps, lambda: depth_dev(dbatch))
+    last = run_steps(args.steps, lambda: depth_dev(dbatch))
     ev1.record()
     barrier()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, np.array(last), lengths, eng.copy_depth, c0)
     ms_total = ev0.elapsed_time(ev1)
     t_t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:
@@ -785,7 +818,7 @@ def _main(real_stdout):
                     help="depth formulation of the device-resident step: fused sorted path (default, what sorted BAM input takes) "
                          "or the any-order push path (clear + atomics + decoupled look-back scan)")
     ap.add_argument("--scale", type=float, default=1.0, help="fraction of the named workload per GPU")
-    ap.add_argument("--e2e-steps", type=int, default=0, help="steps of the e2e legs (0: as many as --steps, at least 5)")
+    ap.add_argument("--e2e-steps", type=int, default=0, help="steps of the e2e legs (0: as many as --steps)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-bam", action="store_true", help="skip the from-the-BAM-file leg of e2e")
     ap.add_argument("--bam-reads", type=int, default=2_000_000, help="reads written to the synthetic BAM of the from-file leg")
@@ -794,10 +827,12 @@ def _main(real_stdout):
     ap.add_argument("--strong-scale", type=float, default=1.0, help="fraction of config C4 (1 B reads) used by the strong-scaling block")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--breakdown", action="store_true", help="print a host-side time breakdown of one step to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the statistics records and a sample of the depth of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
     args.real_stdout = real_stdout
     if args.e2e_steps <= 0:
-        args.e2e_steps = max(5, args.steps)
+        args.e2e_steps = args.steps
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -205,8 +205,9 @@ def reg2bin(beg, end):
 
 
 def write_bam(path, references, lengths, tid, pos, flag, mapq, cig_off, cig, l_seq=None, isize=None,
-              names=None, seqs=None, text=None, with_index=True):
-    """Write a BAM (and a BAI that carries only the metadata pseudo-bins) from SoA arrays."""
+              names=None, seqs=None, text=None, with_index=True, aux=None):
+    """Write a BAM (and a BAI that carries only the metadata pseudo-bins) from SoA arrays.
+    ``aux``: optional per-record bytes of encoded optional fields (SAM spec 4.2.4), appended after the qualities."""
     n = len(tid)
     if text is None:
         text = "@HD\tVN:1.4\tSO:coordinate\n" + "".join(
@@ -235,7 +236,7 @@ def write_bam(path, references, lengths, tid, pos, flag, mapq, cig_off, cig, l_s
         body = struct.pack("<iiBBHHHiiii", int(tid[i]), int(pos[i]), len(name), int(mapq[i]),
                            reg2bin(max(int(pos[i]), 0), max(end, 1)) if tid[i] >= 0 else 4680,
                            len(ops), int(flag[i]), ls, -1, -1, int(isize[i]) if isize is not None else 0)
-        body += name + ops.tobytes() + packed + qual
+        body += name + ops.tobytes() + packed + qual + (aux[i] if aux is not None else b"")
         parts.append(struct.pack("<i", len(body)) + body)
     with open(path, "wb") as fh:
         fh.write(bgzf_compress(b"".join(parts)))

@@ -6,7 +6,6 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden")
-REF_DATA = "/root/reference/tests/data"
 
 
 def load_soa(name):
@@ -14,6 +13,24 @@ def load_soa(name):
     z = np.load(os.path.join(GOLD, name), allow_pickle=False)
     batch = ReadBatch(z["tid"], z["pos"], z["flag"], z["mapq"], z["cig_off"].astype(np.uint32), z["cig"])
     return z, batch
+
+
+def write_fixture_bam(path):
+    """The reference's fixture BAM (tests/data/bbmap.sorted.bam, 4 112 reads on ref1 / ref2), rebuilt by the oracle's
+    writer from the columns decoded from it (golden/fixture_soa.npz): names, sequences, insert sizes.  Qualities are
+    0xff and the optional fields (AM:C, XT:A, RG:Z, of varying length) are SYNTHETIC stand-ins, not the fixture's:
+    they only give every record an optional-field block for the readers to step over.  The BAI carries only the
+    metadata pseudo-bins.  Writes path + ".bai" too."""
+    from oracle import bamio
+    z = np.load(os.path.join(GOLD, "fixture_soa.npz"), allow_pickle=False)
+    so = z["seq_off"]
+    n = len(z["tid"])
+    aux = [b"AMC" + bytes([int(z["mapq"][i])]) + b"XTA" + (b"U" if z["mapq"][i] else b"R") +
+           b"RGZ" + b"lane%d\0" % (i % 11 * 7) for i in range(n)]
+    bamio.write_bam(path, [str(x) for x in z["references"]], z["lengths"].tolist(), z["tid"], z["pos"], z["flag"],
+                    z["mapq"], z["cig_off"], z["cig"], l_seq=z["l_seq"], isize=z["isize"], names=[str(x) for x in z["names"]],
+                    seqs=[z["seq"][so[i]:so[i + 1]] for i in range(n)], aux=aux)
+    return path
 
 
 def load_json(name):

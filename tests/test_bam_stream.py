@@ -7,7 +7,7 @@ import os
 import numpy as np
 import pytest
 
-from helpers import REF_DATA, load_soa
+from helpers import load_soa, write_fixture_bam
 from oracle import bamio, cport
 
 
@@ -23,9 +23,7 @@ def _write_synth_bam(tmp_path, scale=0.004, seed=None):
 
 def test_stream_batches_are_the_file(tmp_path):
     from metacov_b200.alignmentfile import BamStream
-    paths = [_write_synth_bam(tmp_path)[0]]
-    if os.path.exists(os.path.join(REF_DATA, "bbmap.sorted.bam")):          # (the reference tree exists in the build container only)
-        paths.append(os.path.join(REF_DATA, "bbmap.sorted.bam"))
+    paths = [_write_synth_bam(tmp_path)[0], write_fixture_bam(str(tmp_path / "bbmap.sorted.bam"))]
     for path in paths:
         hdr, recs = bamio.read_bam(path)
         for batch_reads in (997, 1 << 20):

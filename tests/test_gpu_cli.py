@@ -8,8 +8,8 @@ import numpy as np
 import pytest
 from click.testing import CliRunner
 
-from helpers import load_json, load_soa
-from oracle import bamio, cport
+from helpers import load_json, load_soa, write_fixture_bam
+from oracle import cport
 from test_dropin_surface import BLAST7
 
 pytestmark = pytest.mark.gpu
@@ -17,15 +17,8 @@ pytestmark = pytest.mark.gpu
 
 @pytest.fixture(scope="module")
 def fixture_bam(tmp_path_factory):
-    """The reference fixture re-encoded from tests/golden/fixture_soa.npz (the GPU box has no /root/reference)."""
-    z, b = load_soa("fixture_soa.npz")
-    d = tmp_path_factory.mktemp("bam")
-    path = str(d / "fixture.bam")
-    so = z["seq_off"]
-    seqs = [z["seq"][so[i]:so[i + 1]] for i in range(len(b.tid))]
-    bamio.write_bam(path, [str(x) for x in z["references"]], z["lengths"].tolist(), b.tid, b.pos, b.flag, b.mapq,
-                    b.cig_off, b.cig, isize=z["isize"], names=[str(x) for x in z["names"]], seqs=seqs)
-    return path
+    """The reference fixture rebuilt from tests/golden/fixture_soa.npz (helpers.write_fixture_bam)."""
+    return write_fixture_bam(str(tmp_path_factory.mktemp("bam") / "fixture.bam"))
 
 
 def test_classic_api_matches_golden(fixture_bam):

@@ -1,12 +1,11 @@
 """Host-side logic of the product package, CPU only: float finishing of `classic`, the BAM
 reader, the synthetic generator, region parsing."""
 import io
-import os
 
 import numpy as np
 import pytest
 
-from helpers import REF_DATA, load_soa
+from helpers import load_soa, write_fixture_bam
 from oracle import bamio, classic as oc
 
 
@@ -71,11 +70,10 @@ def test_native_bam_reader_roundtrip(tmp_path):
         AlignmentFile(str(bad))
 
 
-@pytest.mark.skipif(not os.path.exists(REF_DATA), reason="reference fixtures not present on this box")
-def test_native_bam_reader_on_reference_fixture():
+def test_native_bam_reader_on_reference_fixture(tmp_path):
     from metacov_b200 import AlignmentFile
     z, b = load_soa("fixture_soa.npz")
-    with AlignmentFile(os.path.join(REF_DATA, "bbmap.sorted.bam")) as af:
+    with AlignmentFile(write_fixture_bam(str(tmp_path / "bbmap.sorted.bam"))) as af:
         assert af.references == ("ref1", "ref2") and af.lengths == (425, 575)
         assert (af.mapped, af.unmapped) == (3979, 133)
         s = af.soa()

@@ -6,7 +6,7 @@ import os
 import numpy as np
 import pytest
 
-from helpers import REF_DATA, assert_classic_equal, fake_bam, load_json, load_soa, regions_of
+from helpers import assert_classic_equal, fake_bam, load_json, load_soa, regions_of, write_fixture_bam
 from oracle import bamio, classic as oc, cport
 from oracle.pysam_boundary import FakeAlignmentFile, PileupFilter, plp_columns
 
@@ -107,13 +107,13 @@ def test_isize_known_answers_appendix_b():
     assert cnt.tolist() == [1996, 1983, 60, 73]
 
 
-@pytest.mark.skipif(not os.path.exists(REF_DATA), reason="reference fixtures not present on this box")
-def test_bam_reader_on_reference_fixture():
-    hdr, recs = bamio.read_bam(os.path.join(REF_DATA, "bbmap.sorted.bam"))
+def test_bam_reader_on_reference_fixture(tmp_path):
+    path = write_fixture_bam(str(tmp_path / "bbmap.sorted.bam"))
+    hdr, recs = bamio.read_bam(path)
     z, b = load_soa("fixture_soa.npz")
     assert hdr.references == ("ref1", "ref2") and hdr.lengths == (425, 575)
     assert np.array_equal(recs.tid, b.tid) and np.array_equal(recs.cig, b.cig)
-    per_ref, n_no_coor = bamio.read_bai_stats(os.path.join(REF_DATA, "bbmap.sorted.bam.bai"))
+    per_ref, n_no_coor = bamio.read_bai_stats(path + ".bai")
     assert per_ref == [(1694, 38), (2285, 91)] and n_no_coor == 4
 
 
