@@ -48,7 +48,7 @@ def build(force=False, verbose=False):
     if not force and not _stale():
         return LIB
     nvcc = _nvcc()
-    extra = os.environ.get("MCOV_NVCC_EXTRA", "").split()      # tuning hook, e.g. -DMCOV_TILE_MIN_CTAS=5
+    extra = os.environ.get("MCOV_NVCC_EXTRA", "").split()      # tuning hook, e.g. -DMCOV_TT_STAGES=4
     os.makedirs(BUILD_DIR, exist_ok=True)
     objs = []
     for src in CUDA_SOURCES + CXX_SOURCES:

@@ -90,20 +90,6 @@ __device__ __forceinline__ void st_release_u64(unsigned long long* p, unsigned l
   asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" :: "l"(p), "l"(v) : "memory");
 }
 
-// cp.async (LDGSTS): global -> shared copies that hold no register while in flight; out-of-range
-// copies (valid = false) write zeros.
-__device__ __forceinline__ void cp_async_16(void* smem, const void* gmem, bool valid) {
-  const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" :: "r"(s), "l"(gmem), "r"(valid ? 16 : 0) : "memory");
-}
-__device__ __forceinline__ void cp_async_4(void* smem, const void* gmem, bool valid) {
-  const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" :: "r"(s), "l"(gmem), "r"(valid ? 4 : 0) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" :: "n"(N) : "memory"); }
-
 // Programmatic dependent launch (sm_90+): a kernel launched with the programmatic-stream-serialization
 // attribute may start while its predecessor in the stream drains; pdl_wait() blocks until the predecessor
 // has completed and its writes are visible (a no-op for a normal launch), pdl_launch_dependents() lets the

@@ -51,19 +51,18 @@ enum PassState { kIdle = 0, kAccumulating = 1, kDepthReady = 2, kStreaming = 3 }
 
 // kernel ids for the optional per-kernel CUDA-event timing (mcov_profile_*)
 enum KernelId {
-  kKExpand = 0, kKScan, kKFusedPrep, kKTileFirst, kKScanCounts, kKFarScatter, kKFusedTile,
-  kKInitStats, kKRegionStats, kKWindowSums, kKIsizeHist, kKGroupCount, kKSortedStats, kKClear, kKRegionStatsSmall, kKCapReplay, kKUnpack, kKKmerHist, kKRegionStatsWarp,
-  kKExpPrep, kKExpEntries, kKExpRegion, kKExpRevsum, kKRegionHist, kKHistFinish, kKRunCount, kKRunOffsets, kKRunWrite, kKRunEnds, kKBgzfInflate, kKBamGuess, kKBamWalkCount, kKBamWalkWrite, kKDeltaUnpack, kKStreamAcc, kKFusedPrepTma, kKFusedTileTma, kKStatsStream, kKStatsSplitFinish, kKBlockUnpack, kKBamNamesSeq,
+  kKExpand = 0, kKScan, kKFusedPrep, kKScanCounts, kKFarScatter,
+  kKWindowSums, kKIsizeHist, kKGroupCount, kKSortedStats, kKClear, kKRegionStatsSmall, kKCapReplay, kKUnpack, kKKmerHist, kKRegionStatsWarp,
+  kKExpPrep, kKExpEntries, kKExpRegion, kKExpRevsum, kKRegionHist, kKHistFinish, kKRunCount, kKRunOffsets, kKRunWrite, kKRunEnds, kKBgzfInflate, kKBamGuess, kKBamWalkCount, kKBamWalkWrite, kKDeltaUnpack, kKStreamAcc, kKFusedPrepTma, kKFusedTileTma, kKStatsStream, kKBlockUnpack, kKBamNamesSeq,
   kKernelCount
 };
 
 struct ProfRec { int id; cudaEvent_t a, b; };
 
-// cached chunk table of the last region set (mcov_region_stats_run)
+// cached task table of the last region set (mcov_region_stats_run)
 struct RegionPlan {
   bool valid = false;
-  int64_t g = 0, n_tasks = 0, n_small = 0;
-  int32_t n_multi = 0;
+  int64_t g = 0, n_small = 0;
   int32_t ss_grid = 0, n_split = 0;      // balanced stream over the large regions (k_stats_stream.cuh): CTAs, split regions
   int64_t n_contigs_epoch = -1;
   std::vector<int32_t> tid, start, end, rlen, rpad;
@@ -138,7 +137,7 @@ struct mcov_ctx {
   } bam;
 
   // fused (sorted) path scratch
-  mcov::DevBuf d_end_slot, d_start_slot, d_far_list, d_tile_cnt, d_tile_off, d_far_sorted;
+  mcov::DevBuf d_start_slot, d_far_list, d_tile_cnt, d_tile_off, d_far_sorted;
 
   // stats scratch
   mcov::DevBuf d_ss_pieces, d_ss_cta, d_ss_split, d_ss_pool;
@@ -150,7 +149,7 @@ struct mcov_ctx {
   int64_t stream_tile_lo = 0;         // tiles below this one hold final depth
   int64_t stream_reads = 0;           // distinct reads pushed so far
   bool stream_started = false;        // (count_del = 0 streams: the difference array has been cleared)
-  mcov::DevBuf d_tasks, d_rlen, d_rchunks, d_rhist, d_pool, d_done, d_out, d_win_slot, d_win_n, d_win_out, d_htasks, d_tile_heavy, d_run_tasks, d_run_counts, d_run_out;
+  mcov::DevBuf d_tasks, d_rlen, d_done, d_out, d_win_slot, d_win_n, d_win_out, d_htasks, d_tile_heavy, d_run_tasks, d_run_counts, d_run_out;
   int64_t n_runs = -1;               // records held in d_run_out ([tid | start | end | depth] x n_runs), -1 = none
   mcov::PinBuf h_pin;
   // pipelined statistics (mcov_region_stats_submit / collect): two pinned slots

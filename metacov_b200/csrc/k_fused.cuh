@@ -19,9 +19,10 @@
 //                  the start of tile T.
 //   k_far_scatter  bucket the far ends by tile (counting sort); list the tiles that hold
 //                  very many reads (scheduled first by the tile kernel).
-//   k_fused_tile   persistent CTAs drawing tiles of kTile slots by ticket (heavy tiles
-//                  first): +1/-1 of the tile's reads
-//                  go to SHARED-memory counters (starts and ends kept apart),
+//   k_fused_tile_tma (k_tile_tma.cuh)  persistent CTAs drawing tiles of kTile slots by
+//                  ticket (heavy tiles first); a producer warp stages each tile's records
+//                  with TMA bulk copies, and the consumer warps send +1/-1 of the tile's reads
+//                  to SHARED-memory counters (starts and ends kept apart),
 //                  the ends of near reads that started before the tile are
 //                  found by walking back at most max_span slots in the sorted
 //                  order -- and because kNearSpan = kTile every near read that
@@ -482,7 +483,7 @@ struct PrepWarp {
 // kernels): a warp-uniform FAST PATH takes the overwhelmingly common case -- all 128 reads of the
 // warp (and the read before them, pvT/pvP on lane 0) lie in one valid contig at non-negative
 // positions -- where the contig's constants live in uniform registers and nothing is 64-bit.  Near
-// reads need no per-tile aggregate (see k_fused_tile), so the only cross-thread work is the tile
+// reads need no per-tile aggregate (see the file header), so the only cross-thread work is the tile
 // border detection.  Any other warp iteration takes prep_general.
 __device__ __forceinline__ void prep_emit(const FusedArgs& f, const int64_t i0, const PrepReads& R, const int32_t pvT,
                                           const int32_t pvP, const int lane, PrepWarp& W) {
@@ -612,289 +613,6 @@ __global__ void k_far_scatter(FusedArgs f) {
     uint32_t base = T > 0 ? f.tile_cnt[T - 1] : 0u;
     uint32_t p = atomicAdd(f.tile_cursor + T, 1u);
     f.far_sorted[base + p] = (uint32_t)(e - (T << kTileShift));
-  }
-}
-
-struct TileMeta {
-  uint32_t r0, r1, jmin;   // own reads [r0,r1); walk-back candidates [jmin,r0)
-};
-
-__device__ __forceinline__ TileMeta load_tile_meta(const FusedArgs& f, int64_t tile) {
-  TileMeta m;
-  m.r0 = m.r1 = m.jmin = 0;
-  if (tile < f.n_tiles) {
-    m.r0 = f.tile_first[tile]; m.r1 = f.tile_first[tile + 1];
-    m.jmin = tile > 0 ? f.tile_first[tile - 1] : 0u;
-  }
-  return m;
-}
-
-#ifndef MCOV_TILE_MIN_CTAS
-#define MCOV_TILE_MIN_CTAS (20480 / kTile)   /* 1280 resident threads per SM at <= 51 registers */
-#endif
-constexpr int kPreOwn = 4;     // own records staged per thread: one aligned 16-byte copy
-
-// Stage the records of a tile in shared memory with cp.async (no registers are held while the
-// copy is in flight): four own records per thread from the 16-byte aligned index below r0 and one
-// walk-back candidate.  Every thread later reads back only what it copied itself, so
-// cp.async.wait_group is all the synchronisation this needs.  Out-of-range copies write zeros.
-__device__ __forceinline__ void stage_recs(const FusedArgs& f, const TileMeta& m, uint4* s_own, uint32_t* s_back) {
-  const uint32_t j = (m.r0 & ~3u) + 4u * threadIdx.x;
-  cp_async_16(s_own + threadIdx.x, f.rec + j, j < m.r1);             // the buffer is padded past n
-  const bool vb = m.r0 > m.jmin + threadIdx.x;                        // jb = r0 - 1 - tid >= jmin
-  cp_async_4(s_back + threadIdx.x, f.rec + (vb ? m.r0 - 1u - threadIdx.x : 0u), vb);
-  cp_async_commit();
-}
-
-// Per-slot counters of a tile.  PACKED (the normal case): ONE 32-bit word per slot, starts in the
-// low half and ends in the high half, which halves the shared-memory traffic of the scan and of
-// the clear; valid while fewer than 65 536 reads touch the tile.  Otherwise two 32-bit arrays.
-template <bool PACKED>
-__device__ __forceinline__ void count_start(int* s_cnt, int* s_end, uint32_t slot) { atomicAdd(&s_cnt[slot], 1); }
-template <bool PACKED>
-__device__ __forceinline__ void count_end(int* s_cnt, int* s_end, uint32_t slot) {
-  if (PACKED) atomicAdd(&s_cnt[slot], 0x10000); else atomicAdd(&s_end[slot], 1);
-}
-
-// +1 at the start of an own read, +1 in the end counters if it ends inside the tile (a far
-// read's code kRecFar lies beyond any in-tile end)
-template <bool PACKED>
-__device__ __forceinline__ void tile_own(int* s_cnt, int* s_end, uint32_t r) {
-  const uint32_t code = r >> kTileShift;
-  if (code) {
-    const uint32_t local = r & (kTile - 1);
-    count_start<PACKED>(s_cnt, s_end, local);
-    const uint32_t el = local + code;
-    if (el < (uint32_t)kTile) count_end<PACKED>(s_cnt, s_end, el);
-  }
-}
-
-struct TileCtx {            // what one tile's body needs (all warp-uniform except the thread ids)
-  int64_t tile;
-  TileMeta m;
-  uint32_t reach;
-  bool has_far;
-  int par;
-};
-
-// One tile: scatter the +1s into shared memory, block-scan, store the depth.  Returns through
-// mx / cap the running maxima.  Barrier protocol: see k_fused_tile.
-template <bool PACKED>
-__device__ __forceinline__ void tile_body(const FusedArgs& f, const TileCtx& c, int* s_cnt, int* s_end, const uint4* s_own,
-                                          const uint32_t* s_back, int* s_warp, int* s_open, int& mx, int& cap) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const TileMeta& m_cur = c.m;
-  const int64_t tile = c.tile;
-  const int par = c.par;
-  const int64_t base = tile << kTileShift;
-  // reads that start in this tile (tile_first ranges: every record in [r0,r1) belongs here)
-  {
-    uint4 own = s_own[threadIdx.x];
-    const uint32_t j = (m_cur.r0 & ~3u) + 4u * threadIdx.x;   // own.x is record j; valid records: [r0, r1)
-    if (j < m_cur.r0 || j + 4u > m_cur.r1) {
-      if (j + 0u < m_cur.r0 || j + 0u >= m_cur.r1) own.x = 0u;
-      if (j + 1u < m_cur.r0 || j + 1u >= m_cur.r1) own.y = 0u;
-      if (j + 2u < m_cur.r0 || j + 2u >= m_cur.r1) own.z = 0u;
-      if (j + 3u < m_cur.r0 || j + 3u >= m_cur.r1) own.w = 0u;
-    }
-    tile_own<PACKED>(s_cnt, s_end, own.x);
-    tile_own<PACKED>(s_cnt, s_end, own.y);
-    tile_own<PACKED>(s_cnt, s_end, own.z);
-    tile_own<PACKED>(s_cnt, s_end, own.w);
-  }
-  for (uint32_t j = (m_cur.r0 & ~3u) + kPreOwn * kFusedThreads + threadIdx.x; j < m_cur.r1; j += kFusedThreads)
-    tile_own<PACKED>(s_cnt, s_end, f.rec[j]);              // dense tiles: the rest straight from global
-  // near reads that started before the tile and end inside it: walk back while the start is
-  // within max_span of the tile (sorted order => monotone distance).  reach <= kNearSpan = kTile,
-  // so every candidate started in the previous tile: exactly the records [jmin, r0).
-  // Each hit is a read that covers the last slot before the tile, and all of them end in this
-  // tile: their number is the near depth entering the tile.
-  {
-    uint32_t r = s_back[threadIdx.x];
-    int64_t j = (int64_t)m_cur.r0 - 1 - threadIdx.x;
-    int open = 0;
-    while (j >= (int64_t)m_cur.jmin) {
-      const uint32_t d = (uint32_t)kTile - (r & (kTile - 1));     // distance behind the tile start (>= 1)
-      if (d > c.reach) break;
-      const uint32_t code = r >> kTileShift;
-      if (code >= d && code <= kNearSpan) { count_end<PACKED>(s_cnt, s_end, code - d); ++open; }
-      j -= kFusedThreads;
-      if (j >= (int64_t)m_cur.jmin) r = f.rec[j];
-    }
-    open = __reduce_add_sync(0xffffffffu, open);
-    if (lane == 0 && open) atomicAdd(&s_open[par], open);
-  }
-  // far reads: ends bucketed for this tile, and how many of them are open at the tile border
-  int carry = 0;
-  if (c.has_far) {
-    carry = tile > 0 ? f.tile_agg[tile - 1] : 0;
-    const uint32_t k0 = tile > 0 ? f.tile_cnt[tile - 1] : 0u, k1 = f.tile_cnt[tile];
-    for (uint32_t k = k0 + threadIdx.x; k < k1; k += kFusedThreads)
-      count_end<PACKED>(s_cnt, s_end, f.far_sorted[k] & (kTile - 1));
-  }
-  __syncthreads();
-
-  // block scan of (starts - ends), warp-striped like k_scan_inplace.  cap[p] = depth[p-1] +
-  // starts[p] is folded into one value per vector, relative to the vector's incoming depth.
-  const int4* vs = reinterpret_cast<const int4*>(s_cnt);
-  const int4* ve = reinterpret_cast<const int4*>(s_end);
-  int4 v[kTileVec];
-  int run[kTileVec], capv[kTileVec];
-#pragma unroll
-  for (int j = 0; j < kTileVec; ++j) {
-    int idx = (warp * kTileVec + j) * 32 + lane;
-    int4 st = vs[idx], en;
-    if (PACKED) {
-      en = make_int4((int)((unsigned)st.x >> 16), (int)((unsigned)st.y >> 16), (int)((unsigned)st.z >> 16), (int)((unsigned)st.w >> 16));
-      st = make_int4(st.x & 0xffff, st.y & 0xffff, st.z & 0xffff, st.w & 0xffff);
-    } else {
-      en = ve[idx];
-    }
-    v[j].x = st.x - en.x;
-    v[j].y = v[j].x + st.y - en.y;
-    v[j].z = v[j].y + st.z - en.z;
-    v[j].w = v[j].z + st.w - en.w;
-    capv[j] = max(max(st.x, v[j].x + st.y), max(v[j].y + st.z, v[j].z + st.w));
-    run[j] = v[j].w;
-  }
-  int acc = 0;
-#pragma unroll
-  for (int j = 0; j < kTileVec; ++j) {
-    int x = run[j];
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      int y = __shfl_up_sync(0xffffffffu, x, o);
-      if (lane >= o) x += y;
-    }
-    int total = __shfl_sync(0xffffffffu, x, 31);
-    run[j] = x - run[j] + acc;
-    acc += total;
-  }
-  if (lane == 31) s_warp[warp] = acc;
-  __syncthreads();                                     // also: every warp has read the counters
-  {
-    // clear the counters for the next tile now; the barrier at the end of the body publishes it
-    int4* z0 = reinterpret_cast<int4*>(s_cnt);
-    int4* z1 = reinterpret_cast<int4*>(s_end);
-    for (int k = threadIdx.x; k < kTile / 4; k += kFusedThreads) { z0[k] = make_int4(0, 0, 0, 0); if (!PACKED) z1[k] = make_int4(0, 0, 0, 0); }
-  }
-  int off = carry + s_open[par];                       // far reads open at the border + near reads open at the border
-  if (threadIdx.x == 0) s_open[par ^ 1] = 0;           // the other buffer: last read before the previous end-of-body barrier
-#pragma unroll
-  for (int k = 0; k < kFusedThreads / 32; ++k) off += (k < warp) ? s_warp[k] : 0;
-  int4* out = reinterpret_cast<int4*>(f.depth + base);
-  const int64_t n_vec = (f.n_slots - base) >> 2;
-  int cap_t = 0;
-#pragma unroll
-  for (int j = 0; j < kTileVec; ++j) {
-    int idx = (warp * kTileVec + j) * 32 + lane;
-    int o = off + run[j];
-    cap_t = max(cap_t, o + capv[j]);
-    v[j].x += o; v[j].y += o; v[j].z += o; v[j].w += o;
-    mx = max(mx, max(max(v[j].x, v[j].y), max(v[j].z, v[j].w)));
-    if (idx < n_vec) st_stream_int4(out + idx, v[j]);
-  }
-  cap = max(cap, cap_t);
-  // htslib's cap could fire somewhere in this tile (rare): remember the tile for the exact replay
-  if (f.max_depth > 0 && cap_t > f.max_depth) atomicMax(f.tile_cap + tile, cap_t);
-  __syncthreads();                                     // counters cleared; s_warp is rewritten by the next tile
-}
-
-// Persistent, software-pipelined: while tile k is accumulated in shared memory, scanned and
-// stored, the records of tile k+1 are being copied into shared memory (cp.async) and the
-// metadata of tile k+2 is in flight.
-__global__ void __launch_bounds__(kFusedThreads, MCOV_TILE_MIN_CTAS)
-k_fused_tile(const __grid_constant__ FusedArgs f) {
-  __shared__ __align__(16) int s_cnt[kTile];            // packed: starts | ends << 16; unpacked: starts
-  __shared__ __align__(16) int s_end[kTile];            // unpacked tiles only
-  __shared__ __align__(16) uint4 s_own[2][kFusedThreads];
-  __shared__ uint32_t s_back[2][kFusedThreads];
-  __shared__ int s_warp[kFusedThreads / 32];
-  __shared__ int s_warp2[kFusedThreads / 32];
-  __shared__ int s_open[2];                             // near reads open at the tile border (double-buffered)
-  PassCounters* pc = f.e.pc;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  {                                                     // (before the dependency wait: touches nothing global)
-    int4* z0 = reinterpret_cast<int4*>(s_cnt);
-    int4* z1 = reinterpret_cast<int4*>(s_end);
-    for (int k = threadIdx.x; k < kTile / 4; k += kFusedThreads) { z0[k] = make_int4(0, 0, 0, 0); z1[k] = make_int4(0, 0, 0, 0); }
-    if (threadIdx.x < 2) s_open[threadIdx.x] = 0;
-  }
-  pdl_wait();                                           // records, tile_first and the far tables are complete
-  pdl_launch_dependents();
-  // Tile order.  Work per tile is proportional to the reads in it, and skewed abundance makes that
-  // vary 100-fold, so tiles are handed out through TICKETS instead of a fixed stride: tickets
-  // [0, n_heavy) are the heavy tiles listed by k_far_scatter (largest jobs first), tickets
-  // [n_heavy, n_heavy + n_tiles) all tiles in position order (heavy ones are skipped there).  A CTA's
-  // first four tickets are b, b+G, b+2G, b+3G; after that one atomicAdd per tile, issued four tiles ahead
-  // so that the software pipeline below (records of the next tile, metadata of the one after) never
-  // waits for it.  The depth does not depend on the order: every tile is self-contained.
-  __shared__ unsigned s_tk[2];
-  const uint32_t n_heavy = pc->n_heavy;
-  auto resolve = [&](unsigned tk, TileMeta& m) -> int64_t {   // ticket -> tile id; -1: nothing to do; n_tiles: past the end
-    m.r0 = m.r1 = m.jmin = 0;
-    int64_t T;
-    if (tk < n_heavy) {
-      T = f.tile_heavy[tk];
-    } else {
-      T = (int64_t)(tk - n_heavy);
-      if (T >= f.n_tiles) return f.n_tiles;
-    }
-    m = load_tile_meta(f, T);
-    if (tk >= n_heavy && n_heavy != 0 && m.r1 - m.r0 >= f.heavy_min) { m.r0 = m.r1 = m.jmin = 0; return -1; }
-    return T;
-  };
-  const unsigned G = gridDim.x;
-  TileCtx c;
-  c.reach = pc->max_span;                               // written by k_fused_prep
-  c.has_far = pc->n_far != 0;                           // else the far tables are all zero and are not read
-  c.par = 0;
-  c.tile = resolve(blockIdx.x, c.m);
-  TileMeta m_next;
-  int64_t t_next = resolve(blockIdx.x + G, m_next);
-  unsigned tk_nn = blockIdx.x + 2u * G;                 // ticket of the tile after next
-  unsigned tk_hold = blockIdx.x + 3u * G;               // thread 0: the ticket after that (drawn one iteration ago)
-  stage_recs(f, c.m, s_own[0], s_back[0]);
-  int mx = 0, cap = 0;
-  __syncthreads();
-
-#pragma unroll 1
-  for (unsigned it = 0; c.tile < f.n_tiles; ++it, c.par ^= 1) {
-    unsigned tk_new = 0;
-    if (threadIdx.x == 0) tk_new = 4u * G + atomicAdd(&pc->ticket2, 1u);   // not looked at before the end of this iteration
-    // the following tiles first: these copies / loads stay in flight during the whole body
-    stage_recs(f, m_next, s_own[c.par ^ 1], s_back[c.par ^ 1]);   // empty ranges for "nothing to do" / past the end
-    TileMeta m_nn;
-    const int64_t t_nn = resolve(tk_nn, m_nn);
-    cp_async_wait<1>();                                           // this tile's records have landed
-    if (c.tile >= 0) {
-      // every +1 of the tile comes from an own record, a walk-back candidate or a far end: fewer
-      // than 65 536 of them keep both halves of the packed counters from overflowing
-      uint32_t touching = c.m.r1 - c.m.jmin;
-      if (c.has_far) touching += f.tile_cnt[c.tile] - (c.tile > 0 ? f.tile_cnt[c.tile - 1] : 0u);
-      if (threadIdx.x == 0) s_tk[it & 1] = tk_hold;               // (published by the barriers of the body)
-      if (touching < 65536u) tile_body<true>(f, c, s_cnt, s_end, s_own[c.par], s_back[c.par], s_warp, s_open, mx, cap);
-      else tile_body<false>(f, c, s_cnt, s_end, s_own[c.par], s_back[c.par], s_warp, s_open, mx, cap);
-    } else {                                                      // a heavy tile met again in position order: done already
-      if (threadIdx.x == 0) { s_tk[it & 1] = tk_hold; s_open[c.par ^ 1] = 0; }
-      __syncthreads();
-    }
-    tk_nn = s_tk[it & 1];
-    tk_hold = tk_new;
-    c.tile = t_next; c.m = m_next;
-    t_next = t_nn; m_next = m_nn;
-  }
-  cp_async_wait<0>();
-
-  mx = warp_max(mx);
-  cap = warp_max(cap);
-  if (lane == 0) { s_warp[warp] = mx; s_warp2[warp] = cap; }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    int m = 0, c2 = 0;
-    for (int k = 0; k < kFusedThreads / 32; ++k) { m = max(m, s_warp[k]); c2 = max(c2, s_warp2[k]); }
-    if (m > 0) atomicMax(&pc->max_depth_seen, m);
-    if (c2 > 0) atomicMax(&pc->cap_metric, c2);
   }
 }
 

@@ -8,7 +8,7 @@
 //
 // Decoupled look-back (one pass, 4 B read + 4 B write per slot = 8*(L+C)
 // algorithmic bytes).  Tile = 512 threads x 32 slots (64 KB), warp-striped
-// L1-bypassing 128-bit loads/stores, tile id = blockIdx.x.
+// L1-bypassing 128-bit loads/stores, tile id drawn as a ticket.
 //
 // Measured on B200, C2 (50 M slots; profiles/r01_o_scan_sweep.txt, r01_p_scan_variants.txt):
 //   150.5 us  256 thr x 16 slots, atomic ticket for the tile id (first version)
@@ -20,7 +20,6 @@
 // aggregates, and neither a wider window nor prefetching shortens that wait.  The fused path
 // (k_fused.cuh) exists because its tiles need no predecessor at all.
 #pragma once
-#include <cooperative_groups.h>
 #include "common.cuh"
 
 namespace mcov {
@@ -30,9 +29,6 @@ namespace mcov {
 #endif
 #ifndef MCOV_SCAN_THREADS
 #define MCOV_SCAN_THREADS 512
-#endif
-#ifndef MCOV_SCAN_TICKET
-#define MCOV_SCAN_TICKET 1                                    // 0: tile id = blockIdx.x (relies on in-order CTA dispatch)
 #endif
 constexpr int kScanThreads = MCOV_SCAN_THREADS;
 constexpr int kScanVec = MCOV_SCAN_VEC;                       // int4 per thread
@@ -81,13 +77,9 @@ k_scan_inplace(int32_t* __restrict__ data, int64_t n_slots, unsigned long long* 
   // scan between prep and tile, nothing measurable on the 3 052 tiles of the push path).
   __shared__ unsigned s_tile;
   pdl_wait();
-#if MCOV_SCAN_TICKET
   if (threadIdx.x == 0) s_tile = atomicAdd(reinterpret_cast<unsigned*>(status + gridDim.x), 1u);
   __syncthreads();
   const int64_t tile = s_tile;
-#else
-  const int64_t tile = blockIdx.x;
-#endif
   pdl_launch_dependents();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t base = tile * kScanTile;
@@ -167,66 +159,6 @@ k_scan_inplace(int32_t* __restrict__ data, int64_t n_slots, unsigned long long* 
     if (m > 0) atomicMax(&pc->max_depth_seen, m);
     if (p2 > 0) atomicMax(&pc->cap_metric, p2);
   }
-}
-
-// A short array (the per-tile counters of a C2-sized batch: 2 x 24 416 ints) scanned in place by ONE THREAD-BLOCK CLUSTER of
-// eight CTAs: each CTA scans an eighth (every thread at most two 128-bit vectors, kept in registers), the CTA totals are
-// exchanged through DISTRIBUTED SHARED MEMORY (cluster.map_shared_rank) behind one cluster barrier, and every CTA adds
-// the totals of the ranks below it.  No status words, no spinning on a predecessor -- and still SLOWER than the three
-// look-back tiles of k_scan_inplace on this array (10.7 us against 8.7 us by CUDA events on B200: the cluster launch and
-// its two barriers cost more than the spin), so it is an opt-in variant (MCOV_SCAN_CLUSTER), kept as the measured answer
-// to "would a cluster with DSMEM do better here".  n is a multiple of 4 and at most kScanSmallMax.
-constexpr int kScanSmallThreads = 1024;
-constexpr int kScanSmallCluster = 8;
-constexpr int kScanSmallRows = 2;                                            // vectors per thread
-constexpr int64_t kScanSmallMax = (int64_t)kScanSmallCluster * kScanSmallThreads * kScanSmallRows * 4;    // 65 536 ints
-__global__ void __cluster_dims__(kScanSmallCluster, 1, 1) __launch_bounds__(kScanSmallThreads)
-k_scan_small(int32_t* __restrict__ data, int64_t n) {
-  namespace cg = cooperative_groups;
-  cg::cluster_group cluster = cg::this_cluster();
-  __shared__ int s_warp[kScanSmallThreads / 32];
-  __shared__ int s_total;                                                     // this CTA's sum, read by the ranks above it
-  pdl_wait();
-  pdl_launch_dependents();
-  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
-  const int rank = (int)cluster.block_rank();
-  const int nvec = (int)(n >> 2);
-  const int per_cta = (nvec + kScanSmallCluster - 1) / kScanSmallCluster;     // <= kScanSmallThreads * kScanSmallRows
-  const int c0 = min(rank * per_cta, nvec), c1 = min(c0 + per_cta, nvec);
-  int4* v = reinterpret_cast<int4*>(data);
-  int4 x[kScanSmallRows];
-#pragma unroll
-  for (int r = 0; r < kScanSmallRows; ++r) {
-    const int k = c0 + r * kScanSmallThreads + t;
-    x[r] = k < c1 ? __ldcg(v + k) : make_int4(0, 0, 0, 0);
-    x[r].y += x[r].x; x[r].z += x[r].y; x[r].w += x[r].z;
-  }
-  int carry = 0;                                                              // sum of the rows before (this CTA)
-#pragma unroll
-  for (int r = 0; r < kScanSmallRows; ++r) {
-    int inc = x[r].w;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += y; }
-    if (lane == 31) s_warp[warp] = inc;
-    __syncthreads();
-    int before = carry, total = 0;
-#pragma unroll
-    for (int w = 0; w < kScanSmallThreads / 32; ++w) { const int sw = s_warp[w]; if (w < warp) before += sw; total += sw; }
-    const int off = before + (inc - x[r].w);
-    x[r].x += off; x[r].y += off; x[r].z += off; x[r].w += off;
-    carry += total;
-    __syncthreads();                                                          // (s_warp is rewritten by the next row)
-  }
-  if (t == 0) s_total = carry;
-  cluster.sync();
-  int base = 0;
-  for (int q = 0; q < rank; ++q) base += *cluster.map_shared_rank(&s_total, q);
-#pragma unroll
-  for (int r = 0; r < kScanSmallRows; ++r) {
-    const int k = c0 + r * kScanSmallThreads + t;
-    if (k < c1) { x[r].x += base; x[r].y += base; x[r].z += base; x[r].w += base; v[k] = x[r]; }
-  }
-  cluster.sync();                                                             // no CTA leaves while its s_total may still be read
 }
 
 }  // namespace mcov

@@ -14,10 +14,11 @@
 // the last bin, is flagged kStatOverflow and is finished exactly by the GPU
 // radix-sort path (stats_sort.cu).
 //
-// Work unit = one chunk of one region; regions are arbitrary [start,end) slices
-// and may overlap (reference cli.py:85-95 with tests/data/regions.blast7).  A
-// region made of several chunks merges its partial histogram into a global
-// per-region histogram; the last chunk to finish walks it.
+// Regions are arbitrary [start,end) slices and may overlap (reference
+// cli.py:85-95 with tests/data/regions.blast7).  Regions longer than
+// kSmallRegion slots go through the balanced stream of k_stats_stream.cuh; the
+// others get one warp each (k_region_stats_warp), with one CTA each as the
+// retry path (k_region_stats_small).
 //
 // HBM bytes per launch (algorithmic): 4 * sum(region lengths) + 64 * G.
 #pragma once
@@ -31,8 +32,8 @@ constexpr int kStatValid = 1;      // mcov_region_stats.flags bit0
 constexpr int kStatOverflow = 2;   // bit1
 
 struct StatTask {
-  int64_t slot;     // first slot of the chunk inside the depth array
-  int32_t n;        // slots in this chunk
+  int64_t slot;     // first slot of the region inside the depth array
+  int32_t n;        // slots of the region inside its contig
   int32_t region;   // region index
 };
 
@@ -41,11 +42,7 @@ struct StatArgs {
   const StatTask* tasks;
   const int32_t* region_len;      // slots of the region inside its contig
   const int32_t* region_pad;      // positions of the region beyond the contig end: depth 0 there
-  const int32_t* region_chunks;   // chunks per region
-  const int32_t* region_hist;     // index into hist_pool (multi-chunk regions) or -1
-  uint32_t* hist_pool;            // [n_multi][kHistBins], zeroed
-  uint32_t* region_done;          // per-region arrival counter, zeroed
-  mcov_region_stats* out;         // device; every record is fully written by exactly one CTA
+  mcov_region_stats* out;         // device; every record is fully written by exactly one warp or CTA
   int32_t breadth_n;
 };
 
@@ -164,112 +161,12 @@ __device__ __forceinline__ void hist_partial(uint32_t* s_hist, const int4& q, in
   }
 }
 
-struct RegionScratch {          // per multi-chunk region; zero between runs (the last chunk resets it)
-  uint32_t done;                // chunks that have merged their histogram
+struct RegionScratch {          // per split region of k_stats_stream; zero between runs (the CTA that walks the region resets it)
+  uint32_t done;                // pieces that have merged their histogram
   uint32_t max_bin;             // highest non-empty bin
   uint32_t min_bin_inv;         // kHistBins-1 - lowest non-empty bin
   uint32_t pad;
 };
-
-// One CTA per chunk.  The streaming loop feeds the counting histogram and tracks the range of bins
-// it touched; everything after it (merge, walk) is limited to that range, which for real depth
-// profiles is a few dozen bins -- so a chunk costs little more than its stream and regions can be
-// cut finely enough to keep every SM busy to the end.  Multi-chunk regions merge their bin range
-// into a global per-region histogram; the last chunk to arrive pulls the merged range back, leaves
-// the global copy zeroed for the next run, and finishes the region.
-__global__ void __launch_bounds__(kStatThreads, 4)
-k_region_stats(StatArgs a) {
-  __shared__ __align__(16) uint32_t s_hist[kHistBins];
-  __shared__ unsigned long long s_u64[6 * (kStatThreads / 32)];
-  __shared__ int s_i32[4 * (kStatThreads / 32)];
-  __shared__ int s_med[2];
-  __shared__ int s_last;
-
-  const StatTask task = a.tasks[blockIdx.x];            // (the plan is older than the previous kernel)
-  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
-  const int g = task.region;
-  const int n_chunks = a.region_chunks[g];
-  const int pad = a.region_pad[g];
-  const long long n_region = (long long)a.region_len[g] + pad;
-  {
-    uint4* h4 = reinterpret_cast<uint4*>(s_hist);
-    for (int k = t; k < kHistBins / 4; k += kStatThreads) h4[k] = make_uint4(0, 0, 0, 0);
-  }
-  pdl_wait();                                           // the depth (k_fused_tile / k_scan_inplace) is complete
-  __syncthreads();
-
-  // ---- stream the chunk: aligned int4 window covering [slot, slot+n) ----
-  const int64_t s0 = task.slot, s1 = task.slot + task.n;
-  const int64_t a0 = s0 & ~(int64_t)3;
-  const int64_t nvec = ((s1 - a0) + 3) >> 2;
-  const int4* vp = reinterpret_cast<const int4*>(a.depth + a0);
-  const int head = (int)(s0 - a0);                      // elements to skip in the first vector
-  const int tail = (int)((a0 + (nvec << 2)) - s1);      // elements to skip in the last vector
-  const int64_t jf0 = head ? 1 : 0, jf1 = nvec - (tail ? 1 : 0);   // full vectors [jf0, jf1)
-  int lo = kHistBins, hi = -1;
-  // four independent 128-bit loads in flight per thread
-  for (int64_t j = jf0 + t; j < jf1; j += 4 * kStatThreads) {
-    int4 q0 = __ldcs(vp + j), q1, q2, q3;
-    const bool v1 = j + kStatThreads < jf1, v2 = j + 2 * kStatThreads < jf1, v3 = j + 3 * kStatThreads < jf1;
-    if (v1) q1 = __ldcs(vp + j + kStatThreads);
-    if (v2) q2 = __ldcs(vp + j + 2 * kStatThreads);
-    if (v3) q3 = __ldcs(vp + j + 3 * kStatThreads);
-    hist_vec(s_hist, q0, lo, hi);
-    if (v1) hist_vec(s_hist, q1, lo, hi);
-    if (v2) hist_vec(s_hist, q2, lo, hi);
-    if (v3) hist_vec(s_hist, q3, lo, hi);
-  }
-  if (nvec > 0) {
-    if (nvec == 1) { if (t == 0 && (head || tail)) hist_partial(s_hist, __ldcs(vp), head, 4 - tail, lo, hi); }
-    else {
-      if (t == 0 && head) hist_partial(s_hist, __ldcs(vp), head, 4, lo, hi);
-      if (t == 32 && tail) hist_partial(s_hist, __ldcs(vp + nvec - 1), 0, 4 - tail, lo, hi);
-    }
-  }
-  // bin range of the chunk
-  lo = warp_min(lo); hi = warp_max(hi);
-  if (lane == 0) { s_i32[warp] = lo; s_i32[kStatThreads / 32 + warp] = hi; }
-  __syncthreads();                                      // also: the histogram is complete
-  lo = kHistBins; hi = -1;
-#pragma unroll
-  for (int k = 0; k < kStatThreads / 32; ++k) { lo = min(lo, s_i32[k]); hi = max(hi, s_i32[kStatThreads / 32 + k]); }
-  mcov_region_stats* out = a.out + g;                   // (hist_walk rewrites s_i32 only after its own barriers)
-
-  if (n_chunks > 1) {
-    // ---- multi-chunk region: merge the touched bins into the region's global histogram ----
-    uint32_t* gh = a.hist_pool + (int64_t)a.region_hist[g] * kHistBins;
-    RegionScratch* rs = reinterpret_cast<RegionScratch*>(a.region_done) + a.region_hist[g];
-    for (int b = lo + t; b <= hi; b += kStatThreads) {
-      uint32_t c = s_hist[b];
-      if (c) atomicAdd(gh + b, c);
-    }
-    __syncthreads();
-    if (t == 0) {
-      if (hi >= lo) { atomicMax(&rs->max_bin, (uint32_t)hi); atomicMax(&rs->min_bin_inv, (uint32_t)(kHistBins - 1 - lo)); }
-      __threadfence();                                  // the CTA's merges (ordered by the barrier) before the arrival
-      unsigned prev = atomicAdd(&rs->done, 1u);
-      s_last = (prev == (unsigned)(n_chunks - 1));
-    }
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
-    // last chunk of the region: pull the merged range, leave the global copy clean for the next run
-    lo = kHistBins - 1 - (int)*((volatile uint32_t*)&rs->min_bin_inv);
-    hi = (int)*((volatile uint32_t*)&rs->max_bin);
-    for (int b = lo + t; b <= hi; b += kStatThreads) { s_hist[b] = __ldcg(gh + b); gh[b] = 0u; }
-    __syncthreads();
-    if (t == 0) { rs->done = 0u; rs->max_bin = 0u; rs->min_bin_inv = 0u; }
-  }
-  if (pad > 0) {                       // zeros beyond the contig end join the multiset (untouched bins are 0)
-    if (t == 0) s_hist[0] += (uint32_t)pad;
-    if (hi < 0) hi = 0;
-    lo = 0;
-    __syncthreads();
-  }
-  if (hi < lo) { lo = 0; hi = 0; }     // empty region: hist_walk over one (empty) bin
-  WalkOut w = hist_walk<kStatThreads>(s_hist, n_region, a.breadth_n, lo, hi, s_u64, s_i32, s_med);
-  if (t == 0) write_stats(out, w);
-}
 
 // ---- small regions (<= kSmallRegion slots): one 256-thread CTA per region ---------------------------
 // Hundreds of thousands of short contigs (config C3) make the fixed cost of clearing and walking
@@ -356,12 +253,12 @@ __device__ __forceinline__ int min4(const int4 q) { return min(min(q.x, q.y), mi
 __device__ __forceinline__ int max4(const int4 q) { return max(max(q.x, q.y), max(q.z, q.w)); }
 
 __global__ void __launch_bounds__(kWarpsPerCta * 32)
-k_region_stats_warp(StatArgs a, int64_t task0, int64_t n_tasks, uint32_t* __restrict__ retry) {
+k_region_stats_warp(StatArgs a, int64_t n_tasks, uint32_t* __restrict__ retry) {
   __shared__ __align__(16) uint32_t s_win[kWarpsPerCta][kWarpBins];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t wi = (int64_t)blockIdx.x * kWarpsPerCta + warp;
   if (wi >= n_tasks) return;
-  const StatTask task = a.tasks[task0 + wi];
+  const StatTask task = a.tasks[wi];
   const int g = task.region;
   const int pad = a.region_pad[g];
   const long long n = (long long)a.region_len[g] + pad;
@@ -433,7 +330,7 @@ k_region_stats_warp(StatArgs a, int64_t task0, int64_t n_tasks, uint32_t* __rest
   if (hi < lo) hi = lo;
   const int nb = hi - lo + 1;
   if (nb > kWarpBins || hi >= kHistBins - 1 || vlo < 0) {       // does not fit (or leaves the bin range): retry path
-    if (lane == 0) { uint32_t k = atomicAdd(retry, 1u); retry[1 + k] = (uint32_t)(task0 + wi); }
+    if (lane == 0) { uint32_t k = atomicAdd(retry, 1u); retry[1 + k] = (uint32_t)wi; }
     return;
   }
   if (pad > 0 && lane == 0) atomicAdd(&win[0], (uint32_t)pad);      // pad > 0 => wlo == 0

@@ -1,21 +1,20 @@
 // k_stats_stream.cuh -- region statistics as ONE balanced stream over the depth (large regions).
 //
-// k_region_stats (k_stats.cuh) gives every region (or 64 k-slot chunk) its own CTA.  On config C2
-// that is 1 000 equal CTAs on 592 resident slots = 1.69 waves: the second wave runs two thirds
-// empty, each CTA starts with a cold pipeline and ends with a clear / walk during which it loads
-// nothing -- 0.58 of the HBM peak, top stall long_scoreboard (60 %).  Here the concatenation of
-// all large regions is cut into EQUAL slices, one per persistent CTA (2 per SM), whatever the
-// region boundaries are:
+// One CTA per region (or per chunk of a region) leaves the machine badly balanced: on config C2,
+// 1 000 equal CTAs on 592 resident slots = 1.69 waves, each CTA starting with a cold pipeline and
+// ending with a clear / walk during which it loads nothing (DESIGN.md 3.3).  Here the
+// concatenation of all large regions is cut into EQUAL slices, one per persistent CTA (2 per SM),
+// whatever the region boundaries are:
 //   * a producer warp streams the CTA's slice through a ring of 16 KB shared-memory stages with
 //     TMA bulk copies behind mbarriers -- it runs ahead across region boundaries, so the stream
 //     never stops while the consumers finish a region;
 //   * 8 consumer warps feed the exact counting histogram (8192 one-value bins, ATOMS.POPC.INC)
 //     from shared memory;
 //   * a region that lies wholly inside a slice is walked and written by its CTA; a region cut by
-//     a slice border adds its touched bins to a per-split-region histogram in global memory
-//     (fire-and-forget reductions, nobody waits) and k_stats_split_finish walks those (at most one
-//     per slice border) once the stream kernel is done.
-// Records are identical to k_region_stats: same hist_walk.
+//     a slice border (at most one per border) adds its touched bins to a per-split-region
+//     histogram in global memory (fire-and-forget reductions, nobody waits), and the CTA whose
+//     piece of it arrives last pulls the merged bin range back and walks the region.
+// The walk is hist_walk (k_stats.cuh), the same as for the small regions.
 #pragma once
 #include "k_stats.cuh"
 
@@ -55,7 +54,6 @@ struct SsArgs {
   uint32_t* split_hist;             // [n_split][kHistBins], zero between runs
   RegionScratch* split_scratch;     // [n_split] arrival counter + bin range of the merged histogram, zero between runs
   const int32_t* split_pieces;      // [n_split] pieces of the split region: the CTA that merges the last one walks the region
-                                    // (nullptr: k_stats_split_finish does, the tuning hook MCOV_SPLIT_FINISH_KERNEL)
   mcov_region_stats* out;
   int32_t breadth_n;
 };
@@ -170,36 +168,32 @@ k_stats_stream(const __grid_constant__ SsArgs a) {
         const uint32_t c = s_hist[b];
         if (c) atomicAdd(gh + b, c);
       }
-      if (a.split_pieces) named_bar_sync<1, kSsConsumers>();             // the CTA's merges are issued before its arrival
+      named_bar_sync<1, kSsConsumers>();                                 // the CTA's merges are issued before its arrival
       if (t == 0) {
         if (d.pad > 0) { atomicAdd(gh, (uint32_t)d.pad); lo = 0; if (hi < 0) hi = 0; }
         if (hi >= lo) {
           atomicMax(&rs->max_bin, (uint32_t)hi);
           atomicMax(&rs->min_bin_inv, (uint32_t)(kHistBins - 1 - lo));
         }
-        if (a.split_pieces) {
-          __threadfence();
-          const unsigned prev = atomicAdd(&rs->done, 1u);
-          s_last = prev == (unsigned)(a.split_pieces[d.split] - 1) ? 1 : 0;
-        }
+        __threadfence();
+        const unsigned prev = atomicAdd(&rs->done, 1u);
+        s_last = prev == (unsigned)(a.split_pieces[d.split] - 1) ? 1 : 0;
       }
       if (hi < lo) { lo = 0; hi = -1; }
-      if (a.split_pieces) {
+      named_bar_sync<1, kSsConsumers>();
+      if (s_last) {
+        // the last piece of the region has arrived here: pull the merged bin range (it contains this piece's), leave the
+        // global copy zeroed for the next run, walk
+        __threadfence();
+        int mlo = kHistBins - 1 - (int)*((volatile uint32_t*)&rs->min_bin_inv), mhi = (int)*((volatile uint32_t*)&rs->max_bin);
+        if (mhi < mlo) { mlo = 0; mhi = 0; }
+        for (int b = mlo + t; b <= mhi; b += kSsConsumers) { s_hist[b] = __ldcg(gh + b); gh[b] = 0u; }
         named_bar_sync<1, kSsConsumers>();
-        if (s_last) {
-          // the last piece of the region has arrived here: pull the merged bin range (it contains this piece's), leave the
-          // global copy zeroed for the next run, walk -- what k_stats_split_finish did in a launch of its own
-          __threadfence();
-          int mlo = kHistBins - 1 - (int)*((volatile uint32_t*)&rs->min_bin_inv), mhi = (int)*((volatile uint32_t*)&rs->max_bin);
-          if (mhi < mlo) { mlo = 0; mhi = 0; }
-          for (int b = mlo + t; b <= mhi; b += kSsConsumers) { s_hist[b] = __ldcg(gh + b); gh[b] = 0u; }
-          named_bar_sync<1, kSsConsumers>();
-          if (t == 0) { rs->done = 0u; rs->max_bin = 0u; rs->min_bin_inv = 0u; }
-          const long long n_region = (long long)a.region_len[d.region] + a.region_pad[d.region];
-          const WalkOut w = hist_walk<kSsConsumers, true>(s_hist, n_region, a.breadth_n, mlo, mhi, s_u64, s_i32, s_med);
-          if (t == 0) write_stats(a.out + d.region, w);
-          lo = mlo; hi = mhi;                                            // (the range to clear below)
-        }
+        if (t == 0) { rs->done = 0u; rs->max_bin = 0u; rs->min_bin_inv = 0u; }
+        const long long n_region = (long long)a.region_len[d.region] + a.region_pad[d.region];
+        const WalkOut w = hist_walk<kSsConsumers, true>(s_hist, n_region, a.breadth_n, mlo, mhi, s_u64, s_i32, s_med);
+        if (t == 0) write_stats(a.out + d.region, w);
+        lo = mlo; hi = mhi;                                              // (the range to clear below)
       }
     }
     named_bar_sync<1, kSsConsumers>();                                  // walk / merge have read the bins
@@ -207,29 +201,6 @@ k_stats_stream(const __grid_constant__ SsArgs a) {
     lo = kHistBins; hi = -1;
     named_bar_sync<1, kSsConsumers>();
   }
-}
-
-// One CTA per split region: pull the merged bin range, leave the global copy zeroed for the next run, walk.
-__global__ void __launch_bounds__(kSsConsumers)
-k_stats_split_finish(SsArgs a, const int32_t* __restrict__ split_region) {
-  __shared__ __align__(16) uint32_t s_hist[kHistBins];
-  __shared__ unsigned long long s_u64[6 * (kSsConsumers / 32)];
-  __shared__ int s_i32[4 * (kSsConsumers / 32)];
-  __shared__ int s_med[2];
-  pdl_wait();
-  pdl_launch_dependents();
-  const int sp = blockIdx.x, t = threadIdx.x;
-  const int g = split_region[sp];
-  RegionScratch* rs = a.split_scratch + sp;
-  uint32_t* gh = a.split_hist + (int64_t)sp * kHistBins;
-  int lo = kHistBins - 1 - (int)rs->min_bin_inv, hi = (int)rs->max_bin;
-  if (hi < lo) { lo = 0; hi = 0; }
-  for (int b = lo + t; b <= hi; b += kSsConsumers) { s_hist[b] = __ldcg(gh + b); gh[b] = 0u; }
-  __syncthreads();
-  if (t == 0) { rs->done = 0u; rs->max_bin = 0u; rs->min_bin_inv = 0u; }
-  const long long n_region = (long long)a.region_len[g] + a.region_pad[g];
-  const WalkOut w = hist_walk<kSsConsumers>(s_hist, n_region, a.breadth_n, lo, hi, s_u64, s_i32, s_med);
-  if (t == 0) write_stats(a.out + g, w);
 }
 
 }  // namespace mcov

@@ -2,21 +2,22 @@
 // tiles' records through a ring of shared-memory stages with TMA bulk copies behind mbarriers,
 // four consumer warps turn them into depth.
 //
-// Same arithmetic as k_fused_tile (k_fused.cuh): a tile's +1 / +1 go to packed start|end counters in
-// shared memory, the ends of near reads that started before the tile are found by walking back in
-// the sorted order (their number IS the depth entering the tile), far ends come from the buckets,
-// block scan, 128-bit streaming stores.  What moved:
+// A tile's +1 / +1 go to packed start|end counters in shared memory, the ends of near reads that
+// started before the tile are found by walking back in the sorted order (their number IS the depth
+// entering the tile, see k_fused.cuh), far ends come from the buckets, block scan, 128-bit streaming
+// stores.  How the work is split:
 //   * everything that is latency and bookkeeping -- drawing tickets, resolving them to tiles,
 //     loading tile_first, staging records -- is done by ONE thread of a separate warp, several
 //     tiles ahead of the consumers, instead of by every thread of the CTA in front of every tile
-//     (k_fused_tile spent ~70 % of its 54 M warp instructions outside the scan itself);
+//     (done that way, ~70 % of the tile kernel's 54 M warp instructions lay outside the scan);
 //   * records arrive by cp.async.bulk (one copy per tile: walk-back candidates and own records are
 //     contiguous in the sorted order), consumers read them from shared memory;
-//   * two barriers per tile instead of three (a thread clears exactly the counter vectors it has
-//     just read), over the four consumer warps only;
+//   * two barriers per tile (a thread clears exactly the counter vectors it has just read), over
+//     the four consumer warps only;
 //   * tiles touched by >= 32 768 reads take two 32-bit passes (starts, then ends) over the same
 //     8 KB of counters instead of a second counter array, so a CTA needs 8 KB + the ring.
-// Tile order: tickets, heavy tiles first, exactly as in k_fused_tile.  A pass may be restricted to
+// Tile order: tickets, heavy tiles (listed by k_far_scatter) first, then all tiles in position order.
+// The depth does not depend on the order: every tile is self-contained.  A pass may be restricted to
 // the tile range [tile_lo, tile_hi) (streaming: successive batches of a sorted file).
 #pragma once
 #include "k_fused.cuh"
@@ -32,32 +33,13 @@ namespace mcov {
 #ifndef MCOV_TT_CTAS
 #define MCOV_TT_CTAS 8
 #endif
-#ifndef MCOV_TT_BLOCKED
-#define MCOV_TT_BLOCKED 0
-#endif
 #ifndef MCOV_TT_BATCH
 #define MCOV_TT_BATCH 4               // records a thread of a dense tile fetches from global memory before it scatters them
 #endif
 constexpr int kTtStages = MCOV_TT_STAGES;
-// Counter layout.  BLOCKED: a thread owns 16 CONSECUTIVE slots (four vectors), so the block scan needs one warp
-// scan per thread instead of one per vector (4 x 10 shuffle/add instructions -> 10).  Consecutive lanes then read
-// vectors 64 bytes apart, which would be a 4-way bank conflict; the counters are therefore stored with the
-// vector index XOR-swizzled by bits 3..5 (slot ^ ((slot >> 3) & 0x1C)), which makes those reads conflict-free and
-// costs the scatter two instructions per atomic.  MEASURED on B200 (C2): 88 us against 64 us for the warp-striped
-// layout -- the four 128-bit stores of a thread then lie 64 bytes apart across lanes, every store instruction
-// fills only half of each 32-byte sector it touches, and that costs far more than the 30 instructions saved.
-// Kept as a compile-time variant (it would need a swizzled TMA tensor store to pay off); default off.
-constexpr bool kTtBlocked = MCOV_TT_BLOCKED != 0;
-__device__ __forceinline__ uint32_t tt_phys(uint32_t slot) { return kTtBlocked ? (slot ^ ((slot >> 3) & 0x1Cu)) : slot; }
 constexpr int kTtStageRecs = MCOV_TT_STAGE_RECS;             // records staged per tile (walk-back candidates + own)
 constexpr int kTtThreads = kFusedThreads + 32;               // 4 consumer warps + the producer warp
 static_assert(kTtStageRecs % 4 == 0, "stage = whole 16-byte vectors");
-
-// logical vector (four slots) number j of a thread, and where the counters of that vector live
-__device__ __forceinline__ int tt_vec(int warp, int lane, int j) {
-  return kTtBlocked ? (warp * 128 + lane * kTileVec + j) : ((warp * kTileVec + j) * 32 + lane);
-}
-__device__ __forceinline__ int tt_vec_phys(int v) { return kTtBlocked ? (v ^ ((v >> 3) & 7)) : v; }
 
 struct TtMeta {
   int64_t tile;           // < 0: no more tiles
@@ -96,7 +78,7 @@ template <int WHAT, bool ALL_STAGED>
 __device__ __forceinline__ int tt_scatter(const FusedArgs& f, const TtMeta& m, const uint32_t* s_rec, int* s_cnt, uint32_t reach,
                                           bool has_far) {
   const int t = threadIdx.x;
-  if (WHAT == 0 && ALL_STAGED && !kTtBlocked) {
+  if (WHAT == 0 && ALL_STAGED) {
     // the common case, branch-free: both atomics of every record are issued; an end beyond the tile goes to the spare
     // counter behind the tile, a record that does not count here (code 0: filtered, or far) to the lane's own spare
     // counter (spares are never read and never cleared)
@@ -130,14 +112,14 @@ __device__ __forceinline__ int tt_scatter(const FusedArgs& f, const TtMeta& m, c
         const uint32_t code = r[u] >> kTileShift;
         if (code) {
           const uint32_t local = r[u] & (kTile - 1);
-          if (WHAT != 2) atomicAdd(&s_cnt[tt_phys(local)], 1);
+          if (WHAT != 2) atomicAdd(&s_cnt[local], 1);
           const uint32_t el = local + code;
-          if (WHAT != 1 && el < (uint32_t)kTile) atomicAdd(&s_cnt[tt_phys(el)], WHAT == 0 ? 0x10000 : 1);
+          if (WHAT != 1 && el < (uint32_t)kTile) atomicAdd(&s_cnt[el], WHAT == 0 ? 0x10000 : 1);
         }
       }
     }
   }
-  // near reads that started before the tile and end inside it (see k_fused_tile): walk back while the
+  // near reads that started before the tile and end inside it (see k_fused.cuh): walk back while the
   // start is within `reach` slots of the tile; every hit covers the last slot before the tile
   int open = 0;
   if (WHAT != 1) {
@@ -146,11 +128,11 @@ __device__ __forceinline__ int tt_scatter(const FusedArgs& f, const TtMeta& m, c
       const uint32_t d = (uint32_t)kTile - (r & (kTile - 1));
       if (d > reach) break;
       const uint32_t code = r >> kTileShift;
-      if (code >= d && code <= kNearSpan) { atomicAdd(&s_cnt[tt_phys(code - d)], WHAT == 0 ? 0x10000 : 1); ++open; }
+      if (code >= d && code <= kNearSpan) { atomicAdd(&s_cnt[code - d], WHAT == 0 ? 0x10000 : 1); ++open; }
     }
     if (has_far) {
       const uint32_t k0 = m.tile > 0 ? f.tile_cnt[m.tile - 1] : 0u, k1 = f.tile_cnt[m.tile];
-      for (uint32_t k = k0 + t; k < k1; k += kFusedThreads) atomicAdd(&s_cnt[tt_phys(f.far_sorted[k] & (kTile - 1))], WHAT == 0 ? 0x10000 : 1);
+      for (uint32_t k = k0 + t; k < k1; k += kFusedThreads) atomicAdd(&s_cnt[f.far_sorted[k] & (kTile - 1)], WHAT == 0 ? 0x10000 : 1);
     }
   }
   return open;
@@ -257,7 +239,9 @@ k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
     // with one two-way dot product per slot)
     const bool packed = m.touching < 32768u;
     // v[j] = prefix sums of (starts - ends) inside vector j; capv[j] = max over its slots of (prefix before the slot +
-    // starts of the slot): cap[p] = depth[p-1] + starts[p] relative to the vector's incoming depth
+    // starts of the slot): cap[p] = depth[p-1] + starts[p] relative to the vector's incoming depth.
+    // Vectors are warp-striped, so a warp's 128-bit depth stores are contiguous; a blocked layout (one warp scan per
+    // thread instead of four) half-fills every store's sectors and measured slower (DESIGN.md 3.1).
     int4 v[kTileVec];
     int capv[kTileVec];
     if (packed) {
@@ -269,7 +253,7 @@ k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
       const int4* vs = reinterpret_cast<const int4*>(s_cnt);
 #pragma unroll
       for (int j = 0; j < kTileVec; ++j) {
-        const int idx = tt_vec_phys(tt_vec(warp, lane, j));
+        const int idx = (warp * kTileVec + j) * 32 + lane;
         const int4 c = vs[idx];
         reinterpret_cast<int4*>(s_cnt)[idx] = make_int4(0, 0, 0, 0);      // cleared by the thread that read it
         // starts - ends of a packed counter, accumulated: ONE instruction (IDP.2A: lo * 1 + hi * -1 + acc)
@@ -287,7 +271,7 @@ k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
       named_bar_sync<1, kFusedThreads>();
 #pragma unroll
       for (int j = 0; j < kTileVec; ++j) {
-        const int idx = tt_vec_phys(tt_vec(warp, lane, j));
+        const int idx = (warp * kTileVec + j) * 32 + lane;
         st[j] = reinterpret_cast<const int4*>(s_cnt)[idx];
         reinterpret_cast<int4*>(s_cnt)[idx] = make_int4(0, 0, 0, 0);
       }
@@ -298,7 +282,7 @@ k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
       named_bar_sync<1, kFusedThreads>();
 #pragma unroll
       for (int j = 0; j < kTileVec; ++j) {
-        const int idx = tt_vec_phys(tt_vec(warp, lane, j));
+        const int idx = (warp * kTileVec + j) * 32 + lane;
         en[j] = reinterpret_cast<const int4*>(s_cnt)[idx];
         reinterpret_cast<int4*>(s_cnt)[idx] = make_int4(0, 0, 0, 0);
         v[j].x = st[j].x - en[j].x;
@@ -314,7 +298,7 @@ k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
 #pragma unroll
     for (int j = 0; j < kTileVec; ++j) run[j] = v[j].w;
     int acc = 0;
-    if (!kTtBlocked && packed) {
+    if (packed) {
       // the totals of two rows share one scan: |partial sums| < 32 768 in a packed tile, so two signed 16-bit
       // halves add independently modulo a borrow that the unpacking undoes (lo = sign-extended low half,
       // hi = (x - lo) >> 16)
@@ -328,18 +312,6 @@ k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
       const int T1 = (t01 - T0) >> 16, T3 = (t23 - T2) >> 16;
       run[0] = e0; run[1] = e1 + T0; run[2] = e2 + T0 + T1; run[3] = e3 + T0 + T1 + T2;
       acc = T0 + T1 + T2 + T3;
-    } else if (kTtBlocked) {
-      // the thread's four vectors are consecutive: one warp scan over the threads' totals
-      const int t0 = run[0], t1 = t0 + run[1], t2 = t1 + run[2], t3 = t2 + run[3];
-      int x = t3;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const int y = __shfl_up_sync(0xffffffffu, x, o);
-        if (lane >= o) x += y;
-      }
-      acc = __shfl_sync(0xffffffffu, x, 31);
-      const int ex = x - t3;
-      run[0] = ex; run[1] = ex + t0; run[2] = ex + t1; run[3] = ex + t2;
     } else {
 #pragma unroll
       for (int j = 0; j < kTileVec; ++j) {
@@ -368,7 +340,7 @@ k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
     int cap_t = 0;
 #pragma unroll
     for (int j = 0; j < kTileVec; ++j) {
-      const int idx = tt_vec(warp, lane, j);
+      const int idx = (warp * kTileVec + j) * 32 + lane;
       const int o = off + run[j];
       cap_t = max(cap_t, o + capv[j]);
       v[j].x += o; v[j].y += o; v[j].z += o; v[j].w += o;

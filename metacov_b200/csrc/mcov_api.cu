@@ -233,14 +233,13 @@ int fused_depth_sorted(mcov_ctx* ctx, const ExpandArgs& a, int64_t tile_lo = -1,
     const int64_t groups = (n + kPrepPer - 1) / kPrepPer;
     // short-read hot path: SoA chunks staged by TMA bulk copies behind mbarriers (k_prep_tma.cuh); needs 32-bit
     // offsets and 16-byte aligned columns.  Anything else takes the per-thread loads of k_fused_prep.
-    static const bool no_tma = std::getenv("MCOV_PREP_LEGACY") != nullptr;     // tuning hook
     // Long CIGARs (config C5: ~2 700 ops per read) are reduced by whole warps straight from global memory in either
     // kernel, and there the 8 x 4 warps per SM of k_fused_prep keep more loads in flight than the staged kernel's 3 x 8
     // consumer warps (B200, C5 at 1 M reads: 2.4 ms against 4.6 ms): more than kPrepLongOps ops per read on average
     // take k_fused_prep.
     constexpr int64_t kPrepLongOps = 16;
     const bool long_cigars = a.n_cig >= 0 && a.n_cig > kPrepLongOps * n;
-    const bool tma = !off64 && !no_tma && !long_cigars && al(a.tid, 16) && al(a.pos, 16) && al(a.cig_off, 16) && al(a.flag, 16) &&
+    const bool tma = !off64 && !long_cigars && al(a.tid, 16) && al(a.pos, 16) && al(a.cig_off, 16) && al(a.flag, 16) &&
                      al(a.mapq, 16) && al(a.cig, 16);
     if (tma) {
       const int64_t n_chunks = (n + kPtChunk - 1) / kPtChunk;
@@ -255,29 +254,16 @@ int fused_depth_sorted(mcov_ctx* ctx, const ExpandArgs& a, int64_t tile_lo = -1,
   // prep -> scan_counts -> far_scatter -> tile (-> statistics) are chained with programmatic dependent
   // launches: each kernel's CTAs are in place before its predecessor has drained
   const bool pdl = ctx->n_slots <= kPdlMaxSlots;
-  // (measured on C2, 48 840 counters: look-back kernel 8.7 us by events; ONE CTA of 1 024 threads 45 us -- a single SM's
-  //  dependent L2 round trips; an 8-CTA cluster exchanging totals through distributed shared memory 10.7 us -- the cluster
-  //  launch and its two barriers cost more than the look-back's spin.  The cluster variant stays behind MCOV_SCAN_CLUSTER.)
-  static const bool scan_cluster = std::getenv("MCOV_SCAN_CLUSTER") != nullptr;             // tuning hook
-  if (scan_len <= kScanSmallMax && scan_cluster)
-    MCOV_LAUNCH(ctx, kKScanCounts, CU(launch_pdl(pdl, k_scan_small, dim3(kScanSmallCluster), dim3(kScanSmallThreads), 0, s, f.tile_agg, scan_len)));
-  else
-    MCOV_LAUNCH(ctx, kKScanCounts, CU(launch_pdl(pdl, k_scan_inplace<false>, dim3((unsigned)scan_tiles), dim3(kScanThreads), 0, s,
-        f.tile_agg, scan_len, reinterpret_cast<unsigned long long*>(z + o_st), pc_of(ctx))));
+  // (the look-back scan beat one CTA and an 8-CTA cluster on these counters: DESIGN.md 3.1)
+  MCOV_LAUNCH(ctx, kKScanCounts, CU(launch_pdl(pdl, k_scan_inplace<false>, dim3((unsigned)scan_tiles), dim3(kScanThreads), 0, s,
+      f.tile_agg, scan_len, reinterpret_cast<unsigned long long*>(z + o_st), pc_of(ctx))));
   MCOV_LAUNCH(ctx, kKFarScatter, CU(launch_pdl(pdl, k_far_scatter, dim3(ctx->n_sm * 2), dim3(256), 0, s, f)));
   ctx->fused_blob.assign(reinterpret_cast<const unsigned char*>(&f), reinterpret_cast<const unsigned char*>(&f) + sizeof(f));
-  {
-    static const bool tile_legacy = std::getenv("MCOV_TILE_LEGACY") != nullptr;     // tuning hook
-    if (f.tile_hi <= f.tile_lo) {
-      // (a streamed batch that does not reach a new tile: everything it holds is carried into the next one)
-    } else if (tile_legacy && !f.streaming) {
-      const unsigned grid = (unsigned)std::min<int64_t>(n_tiles, (int64_t)ctx->n_sm * MCOV_TILE_MIN_CTAS);   // persistent
-      MCOV_LAUNCH(ctx, kKFusedTile, CU(launch_pdl(pdl, k_fused_tile, dim3(grid), dim3(kFusedThreads), 0, s, f)));
-    } else {
-      // warp-specialised: producer warp + TMA record ring + 4 consumer warps (k_tile_tma.cuh); persistent
-      const unsigned grid = (unsigned)std::min<int64_t>(f.tile_hi - f.tile_lo, (int64_t)ctx->n_sm * MCOV_TT_CTAS);
-      MCOV_LAUNCH(ctx, kKFusedTileTma, CU(launch_pdl(pdl, k_fused_tile_tma, dim3(std::max(grid, 1u)), dim3(kTtThreads), 0, s, f)));
-    }
+  // (a streamed batch that does not reach a new tile launches no tile kernel: everything it holds is carried into the next one)
+  if (f.tile_hi > f.tile_lo) {
+    // warp-specialised: producer warp + TMA record ring + 4 consumer warps (k_tile_tma.cuh); persistent
+    const unsigned grid = (unsigned)std::min<int64_t>(f.tile_hi - f.tile_lo, (int64_t)ctx->n_sm * MCOV_TT_CTAS);
+    MCOV_LAUNCH(ctx, kKFusedTileTma, CU(launch_pdl(pdl, k_fused_tile_tma, dim3(std::max(grid, 1u)), dim3(kTtThreads), 0, s, f)));
   }
   // htslib's max_depth cap: replayed on the device, in stream order, where the tile kernel found that
   // it can fire (k_cap_replay returns after one load otherwise) -- every consumer of the depth that
@@ -391,9 +377,8 @@ int block_stage(mcov_ctx* ctx, const void* block, int64_t bytes, ExpandArgs& a, 
   // The unpack kernel needs the block's copy and nothing else -- it writes the columns of THIS staging set, which no kernel
   // of the previous pass reads -- so it runs on a stream of its own and fills whatever the previous pass leaves idle (the
   // tails of its kernels, the gaps between them) instead of queueing behind it.  (Per-kernel timing keeps it on the main
-  // stream: the event pairs are recorded there.  MCOV_UNPACK_INLINE: the same without timing, for A/B.)
-  static const bool unpack_inline = std::getenv("MCOV_UNPACK_INLINE") != nullptr;
-  if (ctx->profiling || unpack_inline) {
+  // stream: the event pairs are recorded there.)
+  if (ctx->profiling) {
     CU(cudaStreamWaitEvent(ctx->stream, ctx->copied, 0));
     MCOV_LAUNCH(ctx, kKBlockUnpack, (k_block_expand<<<(unsigned)n_chunks, kBlkThreads, 0, ctx->stream>>>(b)));
   } else {
@@ -424,14 +409,10 @@ int configure_kernels(mcov_ctx* ctx) {
   CU(cudaFuncSetAttribute(k_block_expand, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
   CU(cudaFuncSetAttribute(k_fused_prep<false>, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
   CU(cudaFuncSetAttribute(k_scan_inplace<false>, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
-  CU(cudaFuncSetAttribute(k_scan_small, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
   CU(cudaFuncSetAttribute(k_far_scatter, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
   CU(cudaFuncSetAttribute(k_fused_tile_tma, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
-  CU(cudaFuncSetAttribute(k_fused_tile, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
   CU(cudaFuncSetAttribute(k_cap_replay, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
   CU(cudaFuncSetAttribute(k_stats_stream, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
-  CU(cudaFuncSetAttribute(k_stats_split_finish, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
-  CU(cudaFuncSetAttribute(k_region_stats, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
   CU(cudaFuncSetAttribute(k_region_stats_warp, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
   CU(cudaFuncSetAttribute(k_region_stats_small, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
   return MCOV_OK;
@@ -499,9 +480,9 @@ void mcov_destroy(mcov_ctx* ctx) {
     if (s.consumed) cudaEventDestroy(s.consumed);
     s.tid.release(); s.pos.release(); s.flag.release(); s.mapq.release(); s.cig_off.release(); s.cig.release(); s.raw.release();
   }
-  DevBuf* bufs[] = {&ctx->d_len, &ctx->d_off, &ctx->depth_own, &ctx->d_pc, &ctx->d_status, &ctx->d_end_slot,
+  DevBuf* bufs[] = {&ctx->d_len, &ctx->d_off, &ctx->depth_own, &ctx->d_pc, &ctx->d_status,
                     &ctx->d_start_slot, &ctx->d_far_list, &ctx->d_tile_cnt, &ctx->d_tile_off, &ctx->d_far_sorted,
-                    &ctx->d_tasks, &ctx->d_rlen, &ctx->d_rchunks, &ctx->d_rhist, &ctx->d_pool, &ctx->d_done,
+                    &ctx->d_tasks, &ctx->d_rlen, &ctx->d_done,
                     &ctx->d_cap_scratch, &ctx->d_flag_lut, &ctx->d_stream_acc, &ctx->d_ss_pieces, &ctx->d_ss_cta, &ctx->d_ss_split, &ctx->d_ss_pool,
                     &ctx->d_out, &ctx->d_win_slot, &ctx->d_win_n, &ctx->d_win_out, &ctx->d_htasks, &ctx->d_tile_heavy, &ctx->d_run_tasks, &ctx->d_run_counts, &ctx->d_run_out};
   for (DevBuf* b : bufs) b->release();
@@ -1070,12 +1051,12 @@ int mcov_pass_info_get(mcov_ctx* ctx, mcov_pass_info* out) {
 }
 
 static const char* kKernelNames[kKernelCount] = {
-    "k_expand", "k_scan_inplace", "k_fused_prep", "k_tile_first", "k_scan_counts", "k_far_scatter", "k_fused_tile",
-    "k_init_region_stats", "k_region_stats", "k_window_sums", "k_isize_hist", "k_group_count", "k_sorted_stats",
+    "k_expand", "k_scan_inplace", "k_fused_prep", "k_scan_counts", "k_far_scatter",
+    "k_window_sums", "k_isize_hist", "k_group_count", "k_sorted_stats",
     "memset_depth", "k_region_stats_small", "k_cap_replay", "k_unpack_reads", "k_kmer_hist", "k_region_stats_warp",
     "k_exp_prep", "k_exp_entries", "k_exp_region", "k_exp_revsum", "k_region_hist", "k_hist_finish", "k_run_count", "k_run_offsets", "k_run_write", "k_run_ends",
     "k_bgzf_inflate", "k_bam_guess", "k_bam_walk_count", "k_bam_walk_write", "k_delta_unpack", "k_stream_accumulate",
-    "k_fused_prep_tma", "k_fused_tile_tma", "k_stats_stream", "k_stats_split_finish", "k_block_unpack", "k_bam_names_seq"};
+    "k_fused_prep_tma", "k_fused_tile_tma", "k_stats_stream", "k_block_unpack", "k_bam_names_seq"};
 
 int mcov_copy_to_host(mcov_ctx* ctx, const void* dev, void* host, int64_t n_bytes) {
   if (!ctx) return MCOV_ERR_ARG;
@@ -1141,13 +1122,13 @@ int mcov_copy_depth(mcov_ctx* ctx, int32_t tid, int32_t start, int32_t end, int3
   return MCOV_OK;
 }
 
-// Build (or reuse) the chunk table of a region set and enqueue the statistics kernel writing g
+// Build (or reuse) the plan of a region set and enqueue the statistics kernels writing g
 // records to d_out (device memory).
 static int stats_launch(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int32_t* start, const int32_t* end,
                         int32_t breadth_n, mcov_region_stats* d_out) {
   cudaStream_t s = ctx->stream;
   RegionPlan& rp = ctx->plan;
-  // The chunk table of a region set is cached on the device: a caller that asks for the same
+  // The plan of a region set is cached on the device: a caller that asks for the same
   // regions again (cli.py loops, benchmarks) pays for it once.
   const bool same = rp.valid && rp.g == g && rp.n_contigs_epoch == ctx->contig_epoch && g > 0 &&
                     std::memcmp(rp.tid.data(), tid, (size_t)g * 4) == 0 &&
@@ -1155,167 +1136,107 @@ static int stats_launch(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int3
                     std::memcmp(rp.end.data(), end, (size_t)g * 4) == 0;
   if (!same && g > 0) {
     rp.valid = false;
-    // A region may reach past its contig: the reference's vector is end-start long whatever the
-    // contig length (pileup.py:10-11) and stays 0 there, so those positions count as depth 0.
-    int64_t total = 0;
     for (int64_t i = 0; i < g; ++i) {
       if (tid[i] < 0 || tid[i] >= ctx->n_contigs || start[i] < 0 || end[i] < start[i])
         return fail(ctx, MCOV_ERR_ARG, "mcov_region_stats_run: need 0 <= start <= end and a valid tid");
-      int64_t len = ctx->len[tid[i]];
-      total += std::max<int64_t>(0, std::min<int64_t>(end[i], len) - std::min<int64_t>(start[i], len));
     }
-    // Chunk length.  Splitting a region is not free: a short CTA spends most of its life in the
-    // latency chain around the stream (clear, first loads, merge atomics, arrival counter) -- measured
-    // on C2 (1 000 regions of 50 kb): 52 us with one chunk per region, 62 / 73 / 87 us with chunks of
-    // 32 k / 16 k / 8 k slots.  So chunks are as long as possible (64 k slots) and only shrink when
-    // the work would otherwise leave the machine underfilled (~1.5 waves of 4 CTAs/SM).
-    int64_t chunk_max = (total / ((int64_t)ctx->n_sm * 6) + 4095) / 4096 * 4096;
-    chunk_max = std::max<int64_t>(8192, std::min<int64_t>(65536, chunk_max));
-    if (const char* ov = std::getenv("MCOV_STAT_CHUNK")) {          // tuning hook
-      int64_t v = std::atoll(ov);
-      if (v >= 4096) chunk_max = (v + 3) & ~(int64_t)3;
-    }
-    std::vector<StatTask> tasks, small;
-    tasks.reserve((size_t)(total / chunk_max + 1024));
+    // A region may reach past its contig: the reference's vector is end-start long whatever the
+    // contig length (pileup.py:10-11) and stays 0 there, so those positions count as depth 0.
+    // A region is LARGE (k_stats_stream) when more than kSmallRegion of its slots lie inside the
+    // contig, SMALL (k_region_stats_warp) when it has fewer but at least one slot or one padding
+    // position; a region with neither is in no list.
+    std::vector<StatTask> small;
     rp.rlen.assign((size_t)g, 0); rp.rpad.assign((size_t)g, 0);
-    std::vector<int32_t> rchunks((size_t)g), rhist((size_t)g);
-    int32_t n_multi = 0;
     for (int64_t i = 0; i < g; ++i) {
       int64_t len = ctx->len[tid[i]];
       int64_t cs = std::min<int64_t>(start[i], len), ce = std::min<int64_t>(end[i], len);
       int64_t n = ce - cs;
       int32_t pad = (int32_t)((int64_t)end[i] - start[i] - n);
-      int32_t nch = (int32_t)((n + chunk_max - 1) / chunk_max);
-      if (nch == 0 && pad > 0) nch = 1;             // nothing but zeros: one empty chunk finishes it
-      if (nch == 1 && n <= kSmallRegion) {          // short region: the range-limited kernel
+      rp.rlen[i] = (int32_t)n; rp.rpad[i] = pad;
+      if (n <= kSmallRegion && n + pad > 0) {
         StatTask t;
         t.slot = ctx->off[tid[i]] + cs; t.n = (int32_t)n; t.region = (int32_t)i;
         small.push_back(t);
-        rp.rlen[i] = (int32_t)n; rp.rpad[i] = pad; rchunks[i] = 1; rhist[i] = -1;
-        continue;
-      }
-      int64_t per = nch > 0 ? (((n + nch - 1) / nch + 3) & ~(int64_t)3) : 0;     // even split, 16-byte multiple
-      rp.rlen[i] = (int32_t)n; rp.rpad[i] = pad; rchunks[i] = nch;
-      rhist[i] = nch > 1 ? n_multi++ : -1;
-      int64_t slot = ctx->off[tid[i]] + cs;
-      for (int32_t k = 0; k < nch; ++k) {
-        StatTask t;
-        t.slot = slot + (int64_t)k * per;
-        t.n = (int32_t)std::max<int64_t>(0, std::min<int64_t>(per, n - (int64_t)k * per));
-        t.region = (int32_t)i;
-        tasks.push_back(t);
       }
     }
     // The balanced stream over the large regions (k_stats_stream.cuh): their concatenation cut into equal slices,
     // one per persistent CTA; a region cut by a slice border becomes a "split" region with a global histogram.
-    {
-      int64_t total_big = 0;
-      for (int64_t i = 0; i < g; ++i) if (rchunks[i] >= 1 && !(rchunks[i] == 1 && rp.rlen[i] <= kSmallRegion)) total_big += rp.rlen[i];
-      std::vector<SsPiece> pieces;
-      std::vector<int32_t> cta_start, split_region, split_npieces;
-      int32_t grid = (int32_t)std::min<int64_t>((int64_t)ctx->n_sm * MCOV_SS_CTAS, std::max<int64_t>(1, total_big / 16384));
-      const int64_t W = std::max<int64_t>(4, ((total_big + grid - 1) / grid + 3) & ~(int64_t)3);
-      int64_t room = W;
-      cta_start.push_back(0);
-      for (int64_t i = 0; i < g && total_big > 0; ++i) {
-        if (rchunks[i] < 1 || (rchunks[i] == 1 && rp.rlen[i] <= kSmallRegion)) continue;
-        int64_t rem = rp.rlen[i];
-        int64_t slot = ctx->off[tid[i]] + std::min<int64_t>(start[i], ctx->len[tid[i]]);
-        const size_t first_piece = pieces.size();
-        while (rem > 0) {
-          const int64_t take = std::min(rem, room);
-          SsPiece pc;
-          pc.slot = slot; pc.n = (int32_t)take; pc.region = (int32_t)i; pc.pad = pieces.size() == first_piece ? rp.rpad[i] : 0; pc.split = -1;
-          pieces.push_back(pc);
-          rem -= take; slot += take; room -= take;
-          if (room == 0) { cta_start.push_back((int32_t)pieces.size()); room = W; }
-        }
-        if (pieces.size() - first_piece > 1) {
-          const int32_t id = (int32_t)split_region.size();
-          split_region.push_back((int32_t)i);
-          split_npieces.push_back((int32_t)(pieces.size() - first_piece));
-          for (size_t k = first_piece; k < pieces.size(); ++k) pieces[k].split = id;
-        }
+    int64_t total_big = 0;
+    for (int64_t i = 0; i < g; ++i) if (rp.rlen[i] > kSmallRegion) total_big += rp.rlen[i];
+    std::vector<SsPiece> pieces;
+    std::vector<int32_t> cta_start, split_npieces;
+    const int32_t grid = (int32_t)std::min<int64_t>((int64_t)ctx->n_sm * MCOV_SS_CTAS, std::max<int64_t>(1, total_big / 16384));
+    const int64_t W = std::max<int64_t>(4, ((total_big + grid - 1) / grid + 3) & ~(int64_t)3);
+    int64_t room = W;
+    cta_start.push_back(0);
+    for (int64_t i = 0; i < g && total_big > 0; ++i) {
+      if (rp.rlen[i] <= kSmallRegion) continue;
+      int64_t rem = rp.rlen[i];
+      int64_t slot = ctx->off[tid[i]] + std::min<int64_t>(start[i], ctx->len[tid[i]]);
+      const size_t first_piece = pieces.size();
+      while (rem > 0) {
+        const int64_t take = std::min(rem, room);
+        SsPiece pc;
+        pc.slot = slot; pc.n = (int32_t)take; pc.region = (int32_t)i; pc.pad = pieces.size() == first_piece ? rp.rpad[i] : 0; pc.split = -1;
+        pieces.push_back(pc);
+        rem -= take; slot += take; room -= take;
+        if (room == 0) { cta_start.push_back((int32_t)pieces.size()); room = W; }
       }
-      if (cta_start.back() != (int32_t)pieces.size()) cta_start.push_back((int32_t)pieces.size());
-      rp.ss_grid = total_big > 0 ? (int32_t)cta_start.size() - 1 : 0;
-      rp.n_split = (int32_t)split_region.size();
-      if (rp.ss_grid > 0) {
-        CU(ctx->d_ss_pieces.ensure(pieces.size() * sizeof(SsPiece)));
-        CU(ctx->d_ss_cta.ensure(cta_start.size() * 4));
-        CU(ctx->d_ss_split.ensure(std::max<size_t>(split_region.size(), 1) * 8));      // [region of the split | its pieces]
-        CU(ctx->d_ss_pool.ensure((size_t)std::max(rp.n_split, 1) * (sizeof(RegionScratch) + (size_t)kHistBins * 4)));
-        CU(cudaMemcpyAsync(ctx->d_ss_pieces.p, pieces.data(), pieces.size() * sizeof(SsPiece), cudaMemcpyHostToDevice, s));
-        CU(cudaMemcpyAsync(ctx->d_ss_cta.p, cta_start.data(), cta_start.size() * 4, cudaMemcpyHostToDevice, s));
-        if (rp.n_split) {
-          CU(cudaMemcpyAsync(ctx->d_ss_split.p, split_region.data(), split_region.size() * 4, cudaMemcpyHostToDevice, s));
-          CU(cudaMemcpyAsync(ctx->d_ss_split.as<int32_t>() + split_region.size(), split_npieces.data(), split_npieces.size() * 4,
-                             cudaMemcpyHostToDevice, s));
-          CU(cudaMemsetAsync(ctx->d_ss_pool.p, 0, (size_t)rp.n_split * (sizeof(RegionScratch) + (size_t)kHistBins * 4), s));
-        }
-        CU(cudaStreamSynchronize(s));                 // the host vectors above go out of scope
+      if (pieces.size() - first_piece > 1) {
+        const int32_t id = (int32_t)split_npieces.size();
+        split_npieces.push_back((int32_t)(pieces.size() - first_piece));
+        for (size_t k = first_piece; k < pieces.size(); ++k) pieces[k].split = id;
       }
     }
-    // Largest jobs first, and -- for the warp-per-region kernel, where a CTA of 8 warps lives as long as its
-    // largest region -- neighbours of similar size: with the log-normal contig lengths of config C3 an
-    // unsorted CTA keeps its slots for about twice the mean of its regions.
+    if (cta_start.back() != (int32_t)pieces.size()) cta_start.push_back((int32_t)pieces.size());
+    rp.ss_grid = total_big > 0 ? (int32_t)cta_start.size() - 1 : 0;
+    rp.n_split = (int32_t)split_npieces.size();
+    if (rp.ss_grid > 0) {
+      CU(ctx->d_ss_pieces.ensure(pieces.size() * sizeof(SsPiece)));
+      CU(ctx->d_ss_cta.ensure(cta_start.size() * 4));
+      CU(ctx->d_ss_split.ensure(std::max<size_t>(split_npieces.size(), 1) * 4));      // pieces of each split region
+      CU(ctx->d_ss_pool.ensure((size_t)std::max(rp.n_split, 1) * (sizeof(RegionScratch) + (size_t)kHistBins * 4)));
+      CU(cudaMemcpyAsync(ctx->d_ss_pieces.p, pieces.data(), pieces.size() * sizeof(SsPiece), cudaMemcpyHostToDevice, s));
+      CU(cudaMemcpyAsync(ctx->d_ss_cta.p, cta_start.data(), cta_start.size() * 4, cudaMemcpyHostToDevice, s));
+      if (rp.n_split) {
+        CU(cudaMemcpyAsync(ctx->d_ss_split.p, split_npieces.data(), split_npieces.size() * 4, cudaMemcpyHostToDevice, s));
+        CU(cudaMemsetAsync(ctx->d_ss_pool.p, 0, (size_t)rp.n_split * (sizeof(RegionScratch) + (size_t)kHistBins * 4), s));
+      }
+    }
+    // Largest regions first, and neighbours of similar size: a CTA of 8 warps lives as long as its largest
+    // region, and with the log-normal contig lengths of config C3 an unsorted CTA keeps its slots for about
+    // twice the mean of its regions.
     auto by_size = [](const StatTask& x, const StatTask& y) { return x.n > y.n; };
-    if (!std::is_sorted(tasks.begin(), tasks.end(), by_size)) std::stable_sort(tasks.begin(), tasks.end(), by_size);
     if (!std::is_sorted(small.begin(), small.end(), by_size)) std::stable_sort(small.begin(), small.end(), by_size);
-    rp.n_tasks = (int64_t)tasks.size();
     rp.n_small = (int64_t)small.size();
-    rp.n_multi = n_multi;
-    tasks.insert(tasks.end(), small.begin(), small.end());     // [chunk tasks | small-region tasks]
     CU(ctx->d_out.ensure((size_t)g * sizeof(mcov_region_stats)));
-    CU(ctx->d_tasks.ensure(std::max<size_t>(tasks.size(), 1) * sizeof(StatTask)));
-    CU(ctx->d_rlen.ensure((size_t)g * 8)); CU(ctx->d_rchunks.ensure((size_t)g * 4)); CU(ctx->d_rhist.ensure((size_t)g * 4));
-    CU(ctx->d_pool.ensure((size_t)std::max(n_multi, 1) * (sizeof(RegionScratch) + (size_t)kHistBins * 4) + 16));
+    CU(ctx->d_tasks.ensure(std::max<size_t>(small.size(), 1) * sizeof(StatTask)));
+    CU(ctx->d_rlen.ensure((size_t)g * 8));
     int32_t* d_rlen = ctx->d_rlen.as<int32_t>();
-    if (!tasks.empty()) CU(cudaMemcpyAsync(ctx->d_tasks.p, tasks.data(), tasks.size() * sizeof(StatTask), cudaMemcpyHostToDevice, s));
+    if (!small.empty()) CU(cudaMemcpyAsync(ctx->d_tasks.p, small.data(), small.size() * sizeof(StatTask), cudaMemcpyHostToDevice, s));
     CU(cudaMemcpyAsync(d_rlen, rp.rlen.data(), (size_t)g * 4, cudaMemcpyHostToDevice, s));
     CU(cudaMemcpyAsync(d_rlen + g, rp.rpad.data(), (size_t)g * 4, cudaMemcpyHostToDevice, s));
-    CU(cudaMemcpyAsync(ctx->d_rchunks.p, rchunks.data(), (size_t)g * 4, cudaMemcpyHostToDevice, s));
-    CU(cudaMemcpyAsync(ctx->d_rhist.p, rhist.data(), (size_t)g * 4, cudaMemcpyHostToDevice, s));
-    // [RegionScratch per multi-chunk region | hist_pool]: zeroed here once; every run leaves it zeroed
-    if (n_multi) CU(cudaMemsetAsync(ctx->d_pool.p, 0, (size_t)n_multi * (sizeof(RegionScratch) + (size_t)kHistBins * 4), s));
     CU(cudaStreamSynchronize(s));                   // the host vectors above go out of scope
     rp.tid.assign(tid, tid + g); rp.start.assign(start, start + g); rp.end.assign(end, end + g);
     rp.g = g; rp.n_contigs_epoch = ctx->contig_epoch; rp.valid = true;
   }
   if (g > 0) {
-    const size_t done_bytes = (size_t)rp.n_multi * sizeof(RegionScratch);
-    static const bool stats_legacy = std::getenv("MCOV_STATS_LEGACY") != nullptr;     // tuning hook
-    if (rp.ss_grid > 0 && !stats_legacy) {
+    if (rp.ss_grid > 0) {
       SsArgs a;
       int32_t* d_rlen = ctx->d_rlen.as<int32_t>();
       a.depth = ctx->depth; a.pieces = ctx->d_ss_pieces.as<SsPiece>(); a.cta_piece_start = ctx->d_ss_cta.as<int32_t>();
       a.region_len = d_rlen; a.region_pad = d_rlen + g;
       a.split_scratch = ctx->d_ss_pool.as<RegionScratch>();
       a.split_hist = reinterpret_cast<uint32_t*>(ctx->d_ss_pool.as<char>() + (size_t)rp.n_split * sizeof(RegionScratch));
+      a.split_pieces = ctx->d_ss_split.as<int32_t>();
       a.out = d_out; a.breadth_n = breadth_n;
-      static const bool finish_kernel = std::getenv("MCOV_SPLIT_FINISH_KERNEL") != nullptr;   // tuning hook: split regions walked by a second launch
-      a.split_pieces = (rp.n_split && !finish_kernel) ? ctx->d_ss_split.as<int32_t>() + rp.n_split : nullptr;
       const bool pdl = ctx->n_slots <= kPdlMaxSlots;
       MCOV_LAUNCH(ctx, kKStatsStream, CU(launch_pdl(pdl, k_stats_stream, dim3((unsigned)rp.ss_grid), dim3(kSsThreads), (size_t)kSsSmemBytes, s, a)));
-      if (rp.n_split && finish_kernel)
-        MCOV_LAUNCH(ctx, kKStatsSplitFinish, CU(launch_pdl(pdl, k_stats_split_finish, dim3((unsigned)rp.n_split), dim3(kSsConsumers), 0, s, a,
-                                                     (const int32_t*)ctx->d_ss_split.as<int32_t>())));
-    } else if (rp.n_tasks) {
-      StatArgs a;
-      int32_t* d_rlen = ctx->d_rlen.as<int32_t>();
-      a.depth = ctx->depth; a.tasks = ctx->d_tasks.as<StatTask>(); a.region_len = d_rlen; a.region_pad = d_rlen + g;
-      a.region_chunks = ctx->d_rchunks.as<int32_t>(); a.region_hist = ctx->d_rhist.as<int32_t>();
-      a.region_done = ctx->d_pool.as<uint32_t>();
-      a.hist_pool = reinterpret_cast<uint32_t*>(ctx->d_pool.as<char>() + done_bytes);
-      a.out = d_out; a.breadth_n = breadth_n;
-      MCOV_LAUNCH(ctx, kKRegionStats, CU(launch_pdl(ctx->n_slots <= kPdlMaxSlots, k_region_stats, dim3((unsigned)rp.n_tasks), dim3(kStatThreads), 0, s, a)));
     }
     if (rp.n_small) {
       StatArgs a;
       int32_t* d_rlen = ctx->d_rlen.as<int32_t>();
       a.depth = ctx->depth; a.tasks = ctx->d_tasks.as<StatTask>(); a.region_len = d_rlen; a.region_pad = d_rlen + g;
-      a.region_chunks = ctx->d_rchunks.as<int32_t>(); a.region_hist = ctx->d_rhist.as<int32_t>();
-      a.region_done = nullptr; a.hist_pool = nullptr;
       a.out = d_out; a.breadth_n = breadth_n;
       // one warp per region first; regions whose depth range does not fit a warp's window are
       // collected in a retry list (device side) and finished by the CTA-per-region kernel
@@ -1323,7 +1244,7 @@ static int stats_launch(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int3
       uint32_t* retry = ctx->d_done.as<uint32_t>();
       CU(cudaMemsetAsync(retry, 0, 4, s));
       const unsigned wgrid = (unsigned)((rp.n_small + kWarpsPerCta - 1) / kWarpsPerCta);
-      MCOV_LAUNCH(ctx, kKRegionStatsWarp, (k_region_stats_warp<<<wgrid, kWarpsPerCta * 32, 0, s>>>(a, rp.n_tasks, rp.n_small, retry)));
+      MCOV_LAUNCH(ctx, kKRegionStatsWarp, (k_region_stats_warp<<<wgrid, kWarpsPerCta * 32, 0, s>>>(a, rp.n_small, retry)));
       CU(cudaGetLastError());
       const unsigned rgrid = (unsigned)std::min<int64_t>(rp.n_small, (int64_t)ctx->n_sm * 6);
       MCOV_LAUNCH(ctx, kKRegionStatsSmall, (k_region_stats_small<<<rgrid, kSmallThreads, 0, s>>>(a, retry)));

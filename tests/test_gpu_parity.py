@@ -497,8 +497,9 @@ def test_full_size_c2_bit_exact_and_properties():
 
 
 def test_dense_tile_takes_unpacked_counters():
-    """A tile touched by >= 65 536 reads leaves the packed (16+16 bit) counters of k_fused_tile for the
-    two-array path; depth stays bit-exact either way (cap disabled: 70 000 reads start at one position)."""
+    """A tile touched by >= 32 768 reads leaves the packed (16+16 bit) counters of k_fused_tile_tma for two
+    32-bit passes (starts, then ends); depth stays bit-exact either way (cap disabled: 70 000 reads start at
+    one position)."""
     from metacov_b200 import ReadBatch
     rng = np.random.default_rng(21)
     lengths = np.array([9000, 4000], np.int32)
