@@ -94,16 +94,79 @@ int ensure_depth(mcov_ctx* ctx) {
   return MCOV_OK;
 }
 
-int wait_pending_copy(mcov_ctx* ctx);
+// A transport block is copied without the call waiting for the copy (the host goes on to enqueue the statistics and
+// to prepare the next batch while the link is busy); the copy is waited for at the start of the NEXT staging call,
+// in mcov_sync and in mcov_destroy -- the block must stay unchanged until then.
+int wait_pending_copy(mcov_ctx* ctx) {
+  if (!ctx->copy_pending) return MCOV_OK;
+  ctx->copy_pending = false;
+  CU(cudaEventSynchronize(ctx->copied));
+  return MCOV_OK;
+}
+
+// The next of the two staging sets, once the kernels of the pass that last read it are done.
+int acquire_stage(mcov_ctx* ctx, ReadStage** out) {
+  int rc = wait_pending_copy(ctx);
+  if (rc) return rc;
+  ReadStage& s = ctx->stage[ctx->stage_next];
+  ctx->stage_next ^= 1;
+  if (s.in_flight) { CU(cudaEventSynchronize(s.consumed)); s.in_flight = false; }
+  *out = &s;
+  return MCOV_OK;
+}
+
+// Entries of the 32-bit CIGAR offsets of n reads as the device rebuilds them: scanned in place, so a multiple of 4.
+int64_t off_len_of(int64_t n) { return (n + 1 + 3) & ~(int64_t)3; }
+
+// Size a staging set's columns for n reads of n_cig ops in all (32-bit offsets).
+int stage_columns(mcov_ctx* ctx, ReadStage& st, int64_t n, int64_t n_cig) {
+  const size_t n1 = (size_t)std::max<int64_t>(n, 1);
+  CU(st.tid.ensure(n1 * 4)); CU(st.pos.ensure(n1 * 4)); CU(st.flag.ensure(n1 * 2)); CU(st.mapq.ensure(n1));
+  CU(st.cig_off.ensure((size_t)off_len_of(n) * 4)); CU(st.cig.ensure((size_t)n_cig * 4 + 16));
+  return MCOV_OK;
+}
+
+// The context's half of a pass's ExpandArgs: contig table, filter, depth store and pass counters.
+void context_args(mcov_ctx* ctx, ExpandArgs& a) {
+  a.contig_off = ctx->d_off.as<int64_t>(); a.contig_len = ctx->d_len.as<int32_t>(); a.n_contigs = ctx->n_contigs;
+  a.filt = ctx->filt; a.delta = ctx->depth; a.pc = pc_of(ctx);
+}
+
+// The ExpandArgs of a batch held in the columns of a staging set (stage_columns).
+ExpandArgs columns_of(mcov_ctx* ctx, const ReadStage& st, int64_t n, int64_t n_cig) {
+  ExpandArgs a;
+  std::memset(&a, 0, sizeof(a));
+  a.n = n; a.n_cig = n_cig;
+  a.tid = st.tid.as<int32_t>(); a.pos = st.pos.as<int32_t>(); a.flag = st.flag.as<uint16_t>();
+  a.mapq = st.mapq.as<uint8_t>(); a.cig_off = st.cig_off.as<uint32_t>(); a.cig = st.cig.as<uint32_t>();
+  context_args(ctx, a);
+  a.cig_aligned16 = 1;
+  return a;
+}
+
+bool aligned(const void* p, uintptr_t m) { return (reinterpret_cast<uintptr_t>(p) & (m - 1)) == 0; }
+
+// The columns allow the vector loads of the prep and expand kernels (k_fused.cuh).
+int vec_ok(const ExpandArgs& a) {
+  return (aligned(a.tid, 16) && aligned(a.pos, 16) && aligned(a.cig_off64 ? (const void*)a.cig_off64 : (const void*)a.cig_off, 16) &&
+          aligned(a.flag, 8) && aligned(a.mapq, 4)) ? 1 : 0;
+}
 
 // Stage host SoA into device memory on the copy stream (double-buffered), or
 // pass device pointers through.  On return `a` holds device pointers and the
-// compute stream has been made to wait for the copies.
+// compute stream has been made to wait for the copies.  An empty batch stages
+// nothing: `a` then holds only the pass counters.
 int stage_reads(mcov_ctx* ctx, int64_t n, const int32_t* tid, const int32_t* pos, const uint16_t* flag,
                 const uint8_t* mapq, const void* cig_off, bool off64, const uint32_t* cig, int mem_kind,
                 ExpandArgs& a, ReadStage** used) {
   *used = nullptr;
-  { int wrc = wait_pending_copy(ctx); if (wrc) return wrc; }
+  if (n == 0) {
+    std::memset(&a, 0, sizeof(a));
+    a.pc = pc_of(ctx);
+    return MCOV_OK;
+  }
+  ReadStage* s = nullptr;
+  { int rc = mem_kind == MCOV_MEM_HOST ? acquire_stage(ctx, &s) : wait_pending_copy(ctx); if (rc) return rc; }
   a.n = n;
   a.n_cig = -1;
   a.cig_off = nullptr; a.cig_off64 = nullptr;
@@ -123,46 +186,28 @@ int stage_reads(mcov_ctx* ctx, int64_t n, const int32_t* tid, const int32_t* pos
       a.n_cig = ctx->ncig_val;
     }
   } else if (mem_kind == MCOV_MEM_HOST) {
-    ReadStage& s = ctx->stage[ctx->stage_next];
-    ctx->stage_next ^= 1;
-    if (s.in_flight) { CU(cudaEventSynchronize(s.consumed)); s.in_flight = false; }
     const uint64_t n_cig = off64 ? static_cast<const uint64_t*>(cig_off)[n] : static_cast<const uint32_t*>(cig_off)[n];
     a.n_cig = (int64_t)n_cig;
-    CU(s.tid.ensure(n * 4)); CU(s.pos.ensure(n * 4)); CU(s.flag.ensure(n * 2)); CU(s.mapq.ensure(n));
-    CU(s.cig_off.ensure((n + 1) * ow)); CU(s.cig.ensure((size_t)n_cig * 4 + 16));
+    CU(s->tid.ensure(n * 4)); CU(s->pos.ensure(n * 4)); CU(s->flag.ensure(n * 2)); CU(s->mapq.ensure(n));
+    CU(s->cig_off.ensure((n + 1) * ow)); CU(s->cig.ensure((size_t)n_cig * 4 + 16));
     cudaStream_t cs = ctx->copy_stream;
-    CU(cudaMemcpyAsync(s.tid.p, tid, n * 4, cudaMemcpyHostToDevice, cs));
-    CU(cudaMemcpyAsync(s.pos.p, pos, n * 4, cudaMemcpyHostToDevice, cs));
-    CU(cudaMemcpyAsync(s.flag.p, flag, n * 2, cudaMemcpyHostToDevice, cs));
-    CU(cudaMemcpyAsync(s.mapq.p, mapq, n, cudaMemcpyHostToDevice, cs));
-    CU(cudaMemcpyAsync(s.cig_off.p, cig_off, (n + 1) * ow, cudaMemcpyHostToDevice, cs));
-    if (n_cig) CU(cudaMemcpyAsync(s.cig.p, cig, (size_t)n_cig * 4, cudaMemcpyHostToDevice, cs));
+    CU(cudaMemcpyAsync(s->tid.p, tid, n * 4, cudaMemcpyHostToDevice, cs));
+    CU(cudaMemcpyAsync(s->pos.p, pos, n * 4, cudaMemcpyHostToDevice, cs));
+    CU(cudaMemcpyAsync(s->flag.p, flag, n * 2, cudaMemcpyHostToDevice, cs));
+    CU(cudaMemcpyAsync(s->mapq.p, mapq, n, cudaMemcpyHostToDevice, cs));
+    CU(cudaMemcpyAsync(s->cig_off.p, cig_off, (n + 1) * ow, cudaMemcpyHostToDevice, cs));
+    if (n_cig) CU(cudaMemcpyAsync(s->cig.p, cig, (size_t)n_cig * 4, cudaMemcpyHostToDevice, cs));
     CU(cudaEventRecord(ctx->copied, cs));
     CU(cudaStreamWaitEvent(ctx->stream, ctx->copied, 0));
-    a.tid = s.tid.as<int32_t>(); a.pos = s.pos.as<int32_t>(); a.flag = s.flag.as<uint16_t>();
-    a.mapq = s.mapq.as<uint8_t>(); a.cig = s.cig.as<uint32_t>();
-    if (off64) a.cig_off64 = s.cig_off.as<uint64_t>(); else a.cig_off = s.cig_off.as<uint32_t>();
-    *used = &s;
+    a.tid = s->tid.as<int32_t>(); a.pos = s->pos.as<int32_t>(); a.flag = s->flag.as<uint16_t>();
+    a.mapq = s->mapq.as<uint8_t>(); a.cig = s->cig.as<uint32_t>();
+    if (off64) a.cig_off64 = s->cig_off.as<uint64_t>(); else a.cig_off = s->cig_off.as<uint32_t>();
+    *used = s;
   } else {
     return fail(ctx, MCOV_ERR_ARG, "mem_kind must be MCOV_MEM_HOST or MCOV_MEM_DEVICE");
   }
-  a.contig_off = ctx->d_off.as<int64_t>();
-  a.contig_len = ctx->d_len.as<int32_t>();
-  a.n_contigs = ctx->n_contigs;
-  a.filt = ctx->filt;
-  a.delta = ctx->depth;
-  a.pc = pc_of(ctx);
-  a.cig_aligned16 = ((reinterpret_cast<uintptr_t>(a.cig) & 15u) == 0) ? 1 : 0;
-  return MCOV_OK;
-}
-
-// A transport block is copied without the call waiting for the copy (the host goes on to enqueue the statistics and
-// to prepare the next batch while the link is busy); the copy is waited for at the start of the NEXT staging call,
-// in mcov_sync and in mcov_destroy -- the block must stay unchanged until then.
-int wait_pending_copy(mcov_ctx* ctx) {
-  if (!ctx->copy_pending) return MCOV_OK;
-  ctx->copy_pending = false;
-  CU(cudaEventSynchronize(ctx->copied));
+  context_args(ctx, a);
+  a.cig_aligned16 = aligned(a.cig, 16) ? 1 : 0;
   return MCOV_OK;
 }
 
@@ -225,10 +270,8 @@ int fused_depth_sorted(mcov_ctx* ctx, const ExpandArgs& a, int64_t tile_lo = -1,
   f.tile_cap = reinterpret_cast<int32_t*>(z + o_cap);
   f.max_depth = ctx->filt.max_depth;
   f.flag_lut = ctx->d_flag_lut.as<uint32_t>();
-  auto al = [](const void* p, uintptr_t m) { return (reinterpret_cast<uintptr_t>(p) & (m - 1)) == 0; };
   const bool off64 = a.cig_off64 != nullptr;
-  f.vec_ok = (n > 0 && al(a.tid, 16) && al(a.pos, 16) && al(off64 ? (const void*)a.cig_off64 : (const void*)a.cig_off, 16) &&
-              al(a.flag, 8) && al(a.mapq, 4)) ? 1 : 0;
+  f.vec_ok = n > 0 ? vec_ok(a) : 0;
   if (n > 0) {
     const int64_t groups = (n + kPrepPer - 1) / kPrepPer;
     // short-read hot path: SoA chunks staged by TMA bulk copies behind mbarriers (k_prep_tma.cuh); needs 32-bit
@@ -239,8 +282,8 @@ int fused_depth_sorted(mcov_ctx* ctx, const ExpandArgs& a, int64_t tile_lo = -1,
     // take k_fused_prep.
     constexpr int64_t kPrepLongOps = 16;
     const bool long_cigars = a.n_cig >= 0 && a.n_cig > kPrepLongOps * n;
-    const bool tma = !off64 && !long_cigars && al(a.tid, 16) && al(a.pos, 16) && al(a.cig_off, 16) && al(a.flag, 16) &&
-                     al(a.mapq, 16) && al(a.cig, 16);
+    const bool tma = !off64 && !long_cigars && aligned(a.tid, 16) && aligned(a.pos, 16) && aligned(a.cig_off, 16) &&
+                     aligned(a.flag, 16) && aligned(a.mapq, 16) && aligned(a.cig, 16);
     if (tma) {
       const int64_t n_chunks = (n + kPtChunk - 1) / kPtChunk;
       const unsigned grid = (unsigned)std::min<int64_t>(n_chunks, (int64_t)ctx->n_sm * MCOV_PREP_CTAS);
@@ -275,6 +318,18 @@ int fused_depth_sorted(mcov_ctx* ctx, const ExpandArgs& a, int64_t tile_lo = -1,
   return MCOV_OK;
 }
 
+// Difference array -> depth in place: the look-back scan over the whole slot space, which also records the pass's
+// depth metrics.
+int scan_depth(mcov_ctx* ctx) {
+  const int64_t n_tiles = (ctx->n_slots + kScanTile - 1) / kScanTile;
+  CU(ctx->d_status.ensure(((size_t)n_tiles + 1) * 8));            // status words + the ticket word
+  CU(cudaMemsetAsync(ctx->d_status.p, 0, ((size_t)n_tiles + 1) * 8, ctx->stream));
+  MCOV_LAUNCH(ctx, kKScan, (k_scan_inplace<true><<<(unsigned)n_tiles, kScanThreads, 0, ctx->stream>>>(
+      ctx->depth, ctx->n_slots, ctx->d_status.as<unsigned long long>(), pc_of(ctx))));
+  CU(cudaGetLastError());
+  return MCOV_OK;
+}
+
 // count_del = 0 (only M = X positions count): the any-order formulation -- clear, one +1 / -1 pair per run of M = X ops
 // (k_expand_runs), look-back scan.  Reads [i_begin, n) of the batch; `clear` / `finalize` let a stream spread the
 // pass over its batches.
@@ -288,15 +343,7 @@ int runs_depth(mcov_ctx* ctx, const ExpandArgs& a, int64_t i_begin, bool clear, 
     MCOV_LAUNCH(ctx, kKExpand, (k_expand_runs<<<grid_for(ctx, a.n - i_begin, 256, 8), 256, 0, s>>>(f, i_begin)));
     CU(cudaGetLastError());
   }
-  if (finalize) {
-    const int64_t n_tiles = (ctx->n_slots + kScanTile - 1) / kScanTile;
-    CU(ctx->d_status.ensure(((size_t)n_tiles + 1) * 8));            // status words + the ticket word
-    CU(cudaMemsetAsync(ctx->d_status.p, 0, ((size_t)n_tiles + 1) * 8, s));
-    MCOV_LAUNCH(ctx, kKScan, (k_scan_inplace<true><<<(unsigned)n_tiles, kScanThreads, 0, s>>>(ctx->depth, ctx->n_slots,
-                                                                                            ctx->d_status.as<unsigned long long>(), pc_of(ctx))));
-    CU(cudaGetLastError());
-  }
-  return MCOV_OK;
+  return finalize ? scan_depth(ctx) : MCOV_OK;
 }
 
 // per-base depth of a whole sorted batch from device columns: the fused path, or the M-run formulation when the
@@ -306,29 +353,67 @@ int depth_from_columns(mcov_ctx* ctx, const ExpandArgs& a) {
   return runs_depth(ctx, a, 0, true, true);
 }
 
+// The verdict of a pass from a host copy of its counters; changes nothing but the error text.  `n_reads` is what the
+// pass sized its bucket list of long-span reads for; `who` names the call that reports the failure.
+int check_pass(mcov_ctx* ctx, const PassCounters& h, int64_t n_reads, const char* who) {
+  auto no = [&](int code, const char* why) { return fail(ctx, code, (std::string(who) + ": " + why).c_str()); };
+  if (h.unsorted) return no(MCOV_ERR_UNSORTED, "reads are not sorted by (tid,pos); use mcov_begin/push/finalize");
+  if ((int64_t)h.n_far > std::min<int64_t>(std::max<int64_t>(n_reads, 1), kFarCapDefault))
+    return no(MCOV_ERR_RANGE, "too many long-span reads for the bucket list; use mcov_begin/push/finalize");
+  if (h.far_overflow) return no(MCOV_ERR_RANGE, "a batch held too many long-span reads for the bucket list; use mcov_begin/push/finalize");
+  if (h.cap_unreplayed)
+    return no(MCOV_ERR_STATE, "htslib's max_depth cap fires in this file (a pile deeper than max_depth); the exact replay needs "
+                              "the contig's reads in one batch -- run the file through mcov_depth_sorted, or raise max_depth");
+  return MCOV_OK;
+}
+
 // Deliver the deferred verdict of an asynchronous fused pass (stream already synchronised,
 // `h` = the pass counters just read back).
-int fused_verdict(mcov_ctx* ctx, const PassCounters& h) {
+int fused_verdict(mcov_ctx* ctx, const PassCounters& h, const char* who) {
   if (!ctx->verdict_pending) return MCOV_OK;
   ctx->verdict_pending = false;
-  if (h.unsorted) {
-    ctx->state = kIdle;
-    return fail(ctx, MCOV_ERR_UNSORTED, "mcov_depth_sorted: reads are not sorted by (tid,pos); use mcov_begin/push/finalize");
-  }
-  if ((int64_t)h.n_far > std::min<int64_t>(std::max<int64_t>(ctx->n_reads_pushed, 1), kFarCapDefault)) {
-    ctx->state = kIdle;
-    return fail(ctx, MCOV_ERR_RANGE, "mcov_depth_sorted: too many long-span reads for the bucket list; use mcov_begin/push/finalize");
-  }
-  if (h.far_overflow) {
-    ctx->state = kIdle;
-    return fail(ctx, MCOV_ERR_RANGE, "mcov_stream_push: a batch held too many long-span reads for the bucket list; use mcov_begin/push/finalize");
-  }
-  if (h.cap_unreplayed) {
-    ctx->state = kIdle;
-    return fail(ctx, MCOV_ERR_STATE, "mcov_stream_push: htslib's max_depth cap fires in this file (a pile deeper than max_depth); the exact replay needs "
-                                     "the contig's reads in one batch -- run the file through mcov_depth_sorted, or raise max_depth");
-  }
-  ctx->cap_contigs = (int32_t)h.cap_contigs;        // replayed by k_cap_replay right after the tile kernel
+  int rc = check_pass(ctx, h, ctx->n_reads_pushed, who);
+  if (rc) ctx->state = kIdle;
+  else ctx->cap_contigs = (int32_t)h.cap_contigs;        // replayed by k_cap_replay right after the tile kernel
+  return rc;
+}
+
+// Synchronise the stream behind what the caller has enqueued and deliver a pending verdict.  The counters are read
+// back only for the verdict, or into `out` when the caller wants them.
+int sync_verdict(mcov_ctx* ctx, const char* who, PassCounters* out = nullptr) {
+  PassCounters h;
+  PassCounters* hp = out ? out : &h;
+  if (out || ctx->verdict_pending) CU(cudaMemcpyAsync(hp, ctx->d_pc.p, sizeof(PassCounters), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  return fused_verdict(ctx, *hp, who);
+}
+
+// The depth pass of a whole sorted batch once its columns are on the device, and its bookkeeping.  With `wait` the
+// verdict is delivered here, else by the next synchronising call.
+int run_sorted_pass(mcov_ctx* ctx, const ExpandArgs& a, ReadStage* st, int64_t n_reads, bool wait_copy, bool wait, const char* who) {
+  CU(cudaMemsetAsync(ctx->d_pc.p, 0, sizeof(PassCounters), ctx->stream));
+  int rc = depth_from_columns(ctx, a);
+  if (rc) return rc;
+  ctx->n_reads_pushed = n_reads;
+  rc = finish_stage(ctx, st, wait_copy);
+  if (rc) return rc;
+  ctx->state = kDepthReady;
+  ctx->verdict_pending = true;
+  // sortedness is a property of the data: one small read-back decides
+  return wait ? sync_verdict(ctx, who) : MCOV_OK;
+}
+
+// Host checks of a narrow transport (a per-contig read-count prefix instead of tid[], op counts instead of offsets):
+// the device rebuilds the offsets from the op counts and reads cig[] there, so they must add up to the op array.
+template <typename NCig>
+int check_narrow(mcov_ctx* ctx, int64_t n, const int64_t* contig_read_start, const NCig* n_cigar, int64_t n_cig_total,
+                 const uint8_t* mapq, const char* who) {
+  auto bad = [&](const char* why) { return fail(ctx, MCOV_ERR_ARG, (std::string(who) + ": " + why).c_str()); };
+  if (!mapq && ctx->filt.min_mapq > 0) return bad("mapq is required when min_mapq > 0");
+  if (contig_read_start[0] != 0 || contig_read_start[ctx->n_contigs] > n) return bad("contig_read_start must start at 0 and end <= n");
+  uint64_t sum = 0;
+  for (int64_t i = 0; i < n; ++i) sum += n_cigar[i];
+  if (sum != (uint64_t)n_cig_total) return bad("the op counts do not add up to n_cig_total");
   return MCOV_OK;
 }
 
@@ -358,22 +443,20 @@ int block_stage(mcov_ctx* ctx, const void* block, int64_t bytes, ExpandArgs& a, 
       return fail(ctx, MCOV_ERR_ARG, "transport block: a section lies outside the block");
   }
   if (!h.has_mapq && ctx->filt.min_mapq > 0) return fail(ctx, MCOV_ERR_ARG, "transport block: packed without mapq, but the filter has min_mapq > 0");
-  { int wrc = wait_pending_copy(ctx); if (wrc) return wrc; }
-  ReadStage& st = ctx->stage[ctx->stage_next];
-  ctx->stage_next ^= 1;
-  if (st.in_flight) { CU(cudaEventSynchronize(st.consumed)); st.in_flight = false; }
-  const int64_t n1 = std::max<int64_t>(n, 1);
-  const int64_t off_len = (n + 1 + 3) & ~(int64_t)3;                    // scanned in place: multiple of 4
-  CU(st.raw.ensure((size_t)h.total_bytes + 16));
-  CU(st.tid.ensure((size_t)n1 * 4)); CU(st.pos.ensure((size_t)n1 * 4)); CU(st.flag.ensure((size_t)n1 * 2)); CU(st.mapq.ensure((size_t)n1));
-  CU(st.cig_off.ensure((size_t)off_len * 4)); CU(st.cig.ensure((size_t)h.n_cigar * 4 + 16));
+  ReadStage* st = nullptr;
+  int rc = acquire_stage(ctx, &st);
+  if (rc) return rc;
+  const int64_t off_len = off_len_of(n);
+  CU(st->raw.ensure((size_t)h.total_bytes + 16));
+  rc = stage_columns(ctx, *st, n, h.n_cigar);
+  if (rc) return rc;
   const int64_t n_chunks = (off_len + kBlkChunk - 1) / kBlkChunk;
-  CU(cudaMemcpyAsync(st.raw.p, block, (size_t)h.total_bytes, cudaMemcpyHostToDevice, ctx->copy_stream));
+  CU(cudaMemcpyAsync(st->raw.p, block, (size_t)h.total_bytes, cudaMemcpyHostToDevice, ctx->copy_stream));
   CU(cudaEventRecord(ctx->copied, ctx->copy_stream));
   BlockArgs b;
-  b.blk = st.raw.as<char>(); b.h = h; b.off_len = off_len;
-  b.tid = st.tid.as<int32_t>(); b.pos = st.pos.as<int32_t>(); b.flag = st.flag.as<uint16_t>(); b.mapq = st.mapq.as<uint8_t>();
-  b.cig_off = st.cig_off.as<uint32_t>(); b.cig = st.cig.as<uint32_t>();
+  b.blk = st->raw.as<char>(); b.h = h; b.off_len = off_len;
+  b.tid = st->tid.as<int32_t>(); b.pos = st->pos.as<int32_t>(); b.flag = st->flag.as<uint16_t>(); b.mapq = st->mapq.as<uint8_t>();
+  b.cig_off = st->cig_off.as<uint32_t>(); b.cig = st->cig.as<uint32_t>();
   // The unpack kernel needs the block's copy and nothing else -- it writes the columns of THIS staging set, which no kernel
   // of the previous pass reads -- so it runs on a stream of its own and fills whatever the previous pass leaves idle (the
   // tails of its kernels, the gaps between them) instead of queueing behind it.  (Per-kernel timing keeps it on the main
@@ -388,14 +471,36 @@ int block_stage(mcov_ctx* ctx, const void* block, int64_t bytes, ExpandArgs& a, 
     CU(cudaStreamWaitEvent(ctx->stream, ctx->unpacked, 0));
   }
   CU(cudaGetLastError());
-  std::memset(&a, 0, sizeof(a));
-  a.n = n; a.n_cig = h.n_cigar;
-  a.tid = b.tid; a.pos = b.pos; a.flag = b.flag; a.mapq = b.mapq; a.cig_off = b.cig_off; a.cig = b.cig;
-  a.contig_off = ctx->d_off.as<int64_t>(); a.contig_len = ctx->d_len.as<int32_t>(); a.n_contigs = ctx->n_contigs;
-  a.filt = ctx->filt; a.delta = ctx->depth; a.pc = pc_of(ctx);
-  a.cig_aligned16 = 1;
-  *used = &st;
+  a = columns_of(ctx, *st, n, h.n_cigar);
+  *used = st;
   return MCOV_OK;
+}
+
+// tile up to which a batch ending with the read (lt, lp) makes the depth final (reads without a valid contig sort
+// after every slot)
+int64_t stream_tile_of(const mcov_ctx* ctx, int32_t lt, int32_t lp) {
+  const int64_t n_tiles = (ctx->n_slots + kTile - 1) / kTile;
+  int64_t slot = ctx->n_slots;
+  if (lt >= 0 && lt < ctx->n_contigs) slot = ctx->off[lt] + std::min<int64_t>(std::max<int64_t>(lp, 0), ctx->len[lt]);
+  return std::min<int64_t>(slot >> kTileShift, n_tiles);
+}
+
+// Regions come from the caller: each needs a valid contig and 0 <= start <= end.
+int check_regions(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int32_t* start, const int32_t* end, const char* who) {
+  for (int64_t i = 0; i < g; ++i)
+    if (tid[i] < 0 || tid[i] >= ctx->n_contigs || start[i] < 0 || end[i] < start[i])
+      return fail(ctx, MCOV_ERR_ARG, (std::string(who) + ": need 0 <= start <= end and a valid tid").c_str());
+  return MCOV_OK;
+}
+
+// A region clipped to its contig: n positions from cs lie inside it.  A region may reach past its contig: the
+// reference's vector is end-start long whatever the contig length (pileup.py:10-11) and stays 0 there, so the pad
+// positions past the contig's end count as depth 0.
+struct Clip { int64_t cs, n; int32_t pad; };
+Clip clip_region(const mcov_ctx* ctx, int32_t tid, int32_t start, int32_t end) {
+  const int64_t len = ctx->len[tid];
+  const int64_t cs = std::min<int64_t>(start, len), n = std::min<int64_t>(end, len) - cs;
+  return {cs, n, (int32_t)((int64_t)end - start - n)};
 }
 
 // Every kernel of a pass asks for the same shared-memory carve-out (the maximum): consecutive kernels with
@@ -559,28 +664,20 @@ int mcov_depth_sorted_delta(mcov_ctx* ctx, int64_t n, const int64_t* contig_read
   if (n < 0 || n_exc < 0 || n_cig_total < 0 || n_cig_total > 0xFFFFFFFFll) return fail(ctx, MCOV_ERR_ARG, "mcov_depth_sorted_delta: bad sizes");
   if (!contig_read_start || (n > 0 && (!dpos || !flag || !n_cigar)) || (n_cig_total > 0 && !cig) || (n_exc > 0 && (!exc_index || !exc_delta)))
     return fail(ctx, MCOV_ERR_ARG, "mcov_depth_sorted_delta: null array");
-  if (!mapq && ctx->filt.min_mapq > 0) return fail(ctx, MCOV_ERR_ARG, "mcov_depth_sorted_delta: mapq is required when min_mapq > 0");
   CU(cudaSetDevice(ctx->device));
   int rc = ensure_depth(ctx);
   if (rc) return rc;
-  if (contig_read_start[0] != 0 || contig_read_start[ctx->n_contigs] > n)
-    return fail(ctx, MCOV_ERR_ARG, "mcov_depth_sorted_delta: contig_read_start must start at 0 and end <= n");
-  {
-    uint64_t sum = 0;
-    for (int64_t i = 0; i < n; ++i) sum += n_cigar[i];
-    if (sum != (uint64_t)n_cig_total) return fail(ctx, MCOV_ERR_ARG, "mcov_depth_sorted_delta: the op counts do not add up to n_cig_total");
-  }
-  { int wrc = wait_pending_copy(ctx); if (wrc) return wrc; }
-  CU(cudaMemsetAsync(ctx->d_pc.p, 0, sizeof(PassCounters), ctx->stream));
-  ReadStage& st = ctx->stage[ctx->stage_next];
-  ctx->stage_next ^= 1;
-  if (st.in_flight) { CU(cudaEventSynchronize(st.consumed)); st.in_flight = false; }
+  rc = check_narrow(ctx, n, contig_read_start, n_cigar, n_cig_total, mapq, "mcov_depth_sorted_delta");
+  if (rc) return rc;
+  ReadStage* pst = nullptr;
+  rc = acquire_stage(ctx, &pst);
+  if (rc) return rc;
+  ReadStage& st = *pst;
+  rc = stage_columns(ctx, st, n, n_cig_total);
+  if (rc) return rc;
   const int64_t n1 = std::max<int64_t>(n, 1);
-  const int64_t off_len = (n + 1 + 3) & ~(int64_t)3;                    // scanned in place: multiple of 4
+  const int64_t off_len = off_len_of(n);
   const size_t crs_bytes = ((size_t)ctx->n_contigs + 1) * 8;
-  CU(st.tid.ensure((size_t)n1 * 4)); CU(st.pos.ensure((size_t)n1 * 4));
-  CU(st.flag.ensure((size_t)n1 * 2)); CU(st.mapq.ensure((size_t)n1));
-  CU(st.cig_off.ensure((size_t)off_len * 4)); CU(st.cig.ensure((size_t)n_cig_total * 4 + 16));
   // staging of the narrow columns: [contig_read_start | dpos u16 | n_cigar u8 | exc_index | exc_delta | cig u16]
   const size_t o_dpos = (crs_bytes + 15) & ~(size_t)15, o_nc = (o_dpos + (size_t)n1 * 2 + 15) & ~(size_t)15,
                o_ei = (o_nc + (size_t)n1 + 15) & ~(size_t)15, o_ed = (o_ei + (size_t)std::max<int64_t>(n_exc, 1) * 4 + 15) & ~(size_t)15,
@@ -629,26 +726,7 @@ int mcov_depth_sorted_delta(mcov_ctx* ctx, int64_t n, const int64_t* contig_read
       n, d_crs, ctx->n_contigs, st.tid.as<int32_t>(), S, st.pos.as<int32_t>(), reinterpret_cast<const uint16_t*>(x + o_c16),
       st.cig.as<uint32_t>(), n_cig_total)));
   CU(cudaGetLastError());
-  ExpandArgs a;
-  std::memset(&a, 0, sizeof(a));
-  a.n = n; a.n_cig = n_cig_total;
-  a.tid = st.tid.as<int32_t>(); a.pos = st.pos.as<int32_t>(); a.flag = st.flag.as<uint16_t>();
-  a.mapq = st.mapq.as<uint8_t>(); a.cig_off = st.cig_off.as<uint32_t>(); a.cig = st.cig.as<uint32_t>();
-  a.contig_off = ctx->d_off.as<int64_t>(); a.contig_len = ctx->d_len.as<int32_t>(); a.n_contigs = ctx->n_contigs;
-  a.filt = ctx->filt; a.delta = ctx->depth; a.pc = pc_of(ctx);
-  a.cig_aligned16 = 1;
-  rc = depth_from_columns(ctx, a);
-  if (rc) return rc;
-  ctx->n_reads_pushed = n;
-  rc = finish_stage(ctx, &st);
-  if (rc) return rc;
-  ctx->state = kDepthReady;
-  ctx->verdict_pending = true;
-  if (!wait) return MCOV_OK;
-  PassCounters h;
-  CU(cudaMemcpyAsync(&h, ctx->d_pc.p, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));
-  return fused_verdict(ctx, h);
+  return run_sorted_pass(ctx, columns_of(ctx, st, n, n_cig_total), &st, n, true, wait != 0, "mcov_depth_sorted_delta");
 }
 
 int mcov_begin(mcov_ctx* ctx) {
@@ -679,11 +757,7 @@ static int push_reads_impl(mcov_ctx* ctx, int64_t n, const int32_t* tid, const i
   FusedArgs f;
   std::memset(&f, 0, sizeof(f));
   f.e = a;
-  {
-    auto al = [](const void* p, uintptr_t m) { return (reinterpret_cast<uintptr_t>(p) & (m - 1)) == 0; };
-    f.vec_ok = (al(a.tid, 16) && al(a.pos, 16) && al(off64 ? (const void*)a.cig_off64 : (const void*)a.cig_off, 16) &&
-                al(a.flag, 8) && al(a.mapq, 4)) ? 1 : 0;
-  }
+  f.vec_ok = vec_ok(a);
   const int grid = grid_for(ctx, (n + kPrepPer - 1) / kPrepPer, kPrepThreads, 8);
   if (!ctx->filt.count_del) MCOV_LAUNCH(ctx, kKExpand, (k_expand_runs<<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(f, 0)));
   else if (off64) MCOV_LAUNCH(ctx, kKExpand, (k_expand<true><<<grid, kPrepThreads, 0, ctx->stream>>>(f)));
@@ -707,12 +781,8 @@ int mcov_finalize(mcov_ctx* ctx) {
   if (!ctx) return MCOV_ERR_ARG;
   if (ctx->state != kAccumulating) return fail(ctx, MCOV_ERR_STATE, "mcov_finalize: nothing accumulated");
   CU(cudaSetDevice(ctx->device));
-  int64_t n_tiles = (ctx->n_slots + kScanTile - 1) / kScanTile;
-  CU(ctx->d_status.ensure(((size_t)n_tiles + 1) * 8));              // status words + the ticket word
-  CU(cudaMemsetAsync(ctx->d_status.p, 0, ((size_t)n_tiles + 1) * 8, ctx->stream));
-  MCOV_LAUNCH(ctx, kKScan, (k_scan_inplace<true><<<(unsigned)n_tiles, kScanThreads, 0, ctx->stream>>>(
-      ctx->depth, ctx->n_slots, ctx->d_status.as<unsigned long long>(), pc_of(ctx))));
-  CU(cudaGetLastError());
+  int rc = scan_depth(ctx);
+  if (rc) return rc;
   ctx->state = kDepthReady;
   return MCOV_OK;
 }
@@ -725,29 +795,11 @@ static int depth_sorted_impl(mcov_ctx* ctx, int64_t n, const int32_t* tid, const
   CU(cudaSetDevice(ctx->device));
   int rc = ensure_depth(ctx);
   if (rc) return rc;
-  CU(cudaMemsetAsync(ctx->d_pc.p, 0, sizeof(PassCounters), ctx->stream));
   ExpandArgs a;
   ReadStage* st = nullptr;
-  if (n > 0) {
-    rc = stage_reads(ctx, n, tid, pos, flag, mapq, cig_off, off64, cig, mem_kind, a, &st);
-    if (rc) return rc;
-  } else {
-    std::memset(&a, 0, sizeof(a));
-    a.pc = pc_of(ctx);
-  }
-  rc = depth_from_columns(ctx, a);
+  rc = stage_reads(ctx, n, tid, pos, flag, mapq, cig_off, off64, cig, mem_kind, a, &st);
   if (rc) return rc;
-  ctx->n_reads_pushed = n;
-  rc = finish_stage(ctx, st);
-  if (rc) return rc;
-  ctx->state = kDepthReady;
-  ctx->verdict_pending = true;
-  if (!wait) return MCOV_OK;
-  // sortedness is a property of the data: one small read-back decides
-  PassCounters h;
-  CU(cudaMemcpyAsync(&h, ctx->d_pc.p, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));
-  return fused_verdict(ctx, h);
+  return run_sorted_pass(ctx, a, st, n, true, wait, "mcov_depth_sorted");
 }
 
 int mcov_depth_sorted(mcov_ctx* ctx, int64_t n, const int32_t* tid, const int32_t* pos, const uint16_t* flag,
@@ -784,11 +836,7 @@ int mcov_stream_begin(mcov_ctx* ctx) {
 
 int mcov_stream_resend_point(const mcov_ctx* ctx, int32_t last_tid, int32_t last_pos, int32_t* resend_tid, int32_t* resend_pos) {
   if (!ctx || !resend_tid || !resend_pos || ctx->n_contigs <= 0) return MCOV_ERR_ARG;
-  // tile of the last read's start slot (reads without a valid contig sort after every slot)
-  int64_t slot = ctx->n_slots;
-  if (last_tid >= 0 && last_tid < ctx->n_contigs)
-    slot = ctx->off[last_tid] + std::min<int64_t>(std::max<int64_t>(last_pos, 0), ctx->len[last_tid]);
-  const int64_t tb = std::min<int64_t>(slot >> kTileShift, (ctx->n_slots + kTile - 1) / kTile);
+  const int64_t tb = stream_tile_of(ctx, last_tid, last_pos);
   // everything that starts at or after the first slot of tile tb-1, or reaches past it, is needed again
   const int64_t rs = std::max<int64_t>(tb - 1, 0) << kTileShift;
   if (rs >= ctx->n_slots) { *resend_tid = ctx->n_contigs; *resend_pos = 0; return MCOV_OK; }
@@ -796,14 +844,6 @@ int mcov_stream_resend_point(const mcov_ctx* ctx, int32_t last_tid, int32_t last
   *resend_tid = c;
   *resend_pos = (int32_t)std::min<int64_t>(rs - ctx->off[c], ctx->len[c]);
   return MCOV_OK;
-}
-
-// tile up to which a batch ending with the read (lt, lp) makes the depth final
-static int64_t stream_tile_of(const mcov_ctx* ctx, int32_t lt, int32_t lp) {
-  const int64_t n_tiles = (ctx->n_slots + kTile - 1) / kTile;
-  int64_t slot = ctx->n_slots;
-  if (lt >= 0 && lt < ctx->n_contigs) slot = ctx->off[lt] + std::min<int64_t>(std::max<int64_t>(lp, 0), ctx->len[lt]);
-  return std::min<int64_t>(slot >> kTileShift, n_tiles);
 }
 
 // the part of a stream push that follows the staging of the batch (`a` = device columns)
@@ -827,32 +867,26 @@ static int stream_push_staged(mcov_ctx* ctx, const ExpandArgs& a, ReadStage* st,
     int rc = runs_depth(ctx, a, n_carry, ctx->stream_reads == 0 && ctx->stream_tile_lo == 0 && !ctx->stream_started, last != 0);
     if (rc) return rc;
     ctx->stream_started = true;
-    ctx->stream_reads += n - n_carry;
-    ctx->n_reads_pushed = ctx->stream_reads;
-    ctx->stream_tile_lo = tile_hi;
-    rc = finish_stage(ctx, st, wait_copy);
+  } else {
+    CU(cudaMemsetAsync(ctx->d_pc.p, 0, sizeof(PassCounters), ctx->stream));
+    int rc = fused_depth_sorted(ctx, a, ctx->stream_tile_lo, tile_hi);
     if (rc) return rc;
-    if (last) { ctx->state = kDepthReady; ctx->verdict_pending = true; }
-    return MCOV_OK;
-  }
-  CU(cudaMemsetAsync(ctx->d_pc.p, 0, sizeof(PassCounters), ctx->stream));
-  int rc = fused_depth_sorted(ctx, a, ctx->stream_tile_lo, tile_hi);
-  if (rc) return rc;
-  // pass counters of the stream: this batch minus its carried reads, added to the running totals
-  unsigned long long* carry = reinterpret_cast<unsigned long long*>(ctx->d_stream_acc.as<char>() + sizeof(StreamAcc));
-  CU(cudaMemsetAsync(carry, 0, 16, ctx->stream));
-  FusedArgs f;
-  std::memcpy(&f, ctx->fused_blob.data(), sizeof(f));
-  if (n_carry > 0) {
-    MCOV_LAUNCH(ctx, kKStreamAcc, (k_carry_counts<<<grid_for(ctx, n_carry, 256, 4), 256, 0, ctx->stream>>>(f, n_carry, carry)));
+    // pass counters of the stream: this batch minus its carried reads, added to the running totals
+    unsigned long long* carry = reinterpret_cast<unsigned long long*>(ctx->d_stream_acc.as<char>() + sizeof(StreamAcc));
+    CU(cudaMemsetAsync(carry, 0, 16, ctx->stream));
+    FusedArgs f;
+    std::memcpy(&f, ctx->fused_blob.data(), sizeof(f));
+    if (n_carry > 0) {
+      MCOV_LAUNCH(ctx, kKStreamAcc, (k_carry_counts<<<grid_for(ctx, n_carry, 256, 4), 256, 0, ctx->stream>>>(f, n_carry, carry)));
+      CU(cudaGetLastError());
+    }
+    MCOV_LAUNCH(ctx, kKStreamAcc, (k_stream_accumulate<<<1, 1, 0, ctx->stream>>>(pc_of(ctx), ctx->d_stream_acc.as<StreamAcc>(), carry, f.far_cap)));
     CU(cudaGetLastError());
   }
-  MCOV_LAUNCH(ctx, kKStreamAcc, (k_stream_accumulate<<<1, 1, 0, ctx->stream>>>(pc_of(ctx), ctx->d_stream_acc.as<StreamAcc>(), carry, f.far_cap)));
-  CU(cudaGetLastError());
   ctx->stream_reads += n - n_carry;
   ctx->n_reads_pushed = ctx->stream_reads;
   ctx->stream_tile_lo = tile_hi;
-  rc = finish_stage(ctx, st, wait_copy);
+  int rc = finish_stage(ctx, st, wait_copy);
   if (rc) return rc;
   if (last) {
     ctx->state = kDepthReady;
@@ -881,13 +915,8 @@ int mcov_stream_push(mcov_ctx* ctx, int64_t n, int64_t n_carry, const int32_t* t
   }
   ExpandArgs a;
   ReadStage* st = nullptr;
-  if (n > 0) {
-    int rc = stage_reads(ctx, n, tid, pos, flag, mapq, cig_off, false, cig, mem_kind, a, &st);
-    if (rc) return rc;
-  } else {
-    std::memset(&a, 0, sizeof(a));
-    a.pc = pc_of(ctx);
-  }
+  int rc = stage_reads(ctx, n, tid, pos, flag, mapq, cig_off, false, cig, mem_kind, a, &st);
+  if (rc) return rc;
   return stream_push_staged(ctx, a, st, n, n_carry, lt, lp, last, resend_tid, resend_pos);
 }
 
@@ -938,19 +967,7 @@ int mcov_depth_sorted_block(mcov_ctx* ctx, const void* block, int64_t bytes, int
   mcov_block_hdr h;
   rc = block_stage(ctx, block, bytes, a, &st, h);
   if (rc) return rc;
-  CU(cudaMemsetAsync(ctx->d_pc.p, 0, sizeof(PassCounters), ctx->stream));
-  rc = depth_from_columns(ctx, a);
-  if (rc) return rc;
-  ctx->n_reads_pushed = h.n;
-  rc = finish_stage(ctx, st, /*wait_copy=*/false);
-  if (rc) return rc;
-  ctx->state = kDepthReady;
-  ctx->verdict_pending = true;
-  if (!wait) return MCOV_OK;
-  PassCounters hc;
-  CU(cudaMemcpyAsync(&hc, ctx->d_pc.p, sizeof(hc), cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));
-  return fused_verdict(ctx, hc);
+  return run_sorted_pass(ctx, a, st, h.n, /*wait_copy=*/false, wait != 0, "mcov_depth_sorted_block");
 }
 
 int mcov_depth_sorted_packed(mcov_ctx* ctx, int64_t n, const int64_t* contig_read_start, const int32_t* pos,
@@ -960,28 +977,19 @@ int mcov_depth_sorted_packed(mcov_ctx* ctx, int64_t n, const int64_t* contig_rea
   if (n < 0 || n_cig_total < 0 || n_cig_total > 0xFFFFFFFFll) return fail(ctx, MCOV_ERR_ARG, "mcov_depth_sorted_packed: bad sizes");
   if (!contig_read_start || (n > 0 && (!pos || !flag || !n_cigar)) || (n_cig_total > 0 && !cig))
     return fail(ctx, MCOV_ERR_ARG, "mcov_depth_sorted_packed: null array");
-  if (!mapq && ctx->filt.min_mapq > 0) return fail(ctx, MCOV_ERR_ARG, "mcov_depth_sorted_packed: mapq is required when min_mapq > 0");
   CU(cudaSetDevice(ctx->device));
   int rc = ensure_depth(ctx);
   if (rc) return rc;
-  if (contig_read_start[0] != 0 || contig_read_start[ctx->n_contigs] > n)
-    return fail(ctx, MCOV_ERR_ARG, "mcov_depth_sorted_packed: contig_read_start must start at 0 and end <= n");
-  {
-    // the op counts must add up to the op array: the device rebuilds the offsets from them and reads cig[] there
-    uint64_t sum = 0;
-    for (int64_t i = 0; i < n; ++i) sum += n_cigar[i];
-    if (sum != (uint64_t)n_cig_total) return fail(ctx, MCOV_ERR_ARG, "mcov_depth_sorted_packed: the op counts do not add up to n_cig_total");
-  }
-  { int wrc = wait_pending_copy(ctx); if (wrc) return wrc; }
-  CU(cudaMemsetAsync(ctx->d_pc.p, 0, sizeof(PassCounters), ctx->stream));
-  ReadStage& st = ctx->stage[ctx->stage_next];
-  ctx->stage_next ^= 1;
-  if (st.in_flight) { CU(cudaEventSynchronize(st.consumed)); st.in_flight = false; }
-  const int64_t off_len = (n + 1 + 3) & ~(int64_t)3;                    // scanned in place: multiple of 4
+  rc = check_narrow(ctx, n, contig_read_start, n_cigar, n_cig_total, mapq, "mcov_depth_sorted_packed");
+  if (rc) return rc;
+  ReadStage* pst = nullptr;
+  rc = acquire_stage(ctx, &pst);
+  if (rc) return rc;
+  ReadStage& st = *pst;
+  rc = stage_columns(ctx, st, n, n_cig_total);
+  if (rc) return rc;
+  const int64_t off_len = off_len_of(n);
   const size_t crs_bytes = ((size_t)ctx->n_contigs + 1) * 8;
-  CU(st.tid.ensure((size_t)std::max<int64_t>(n, 1) * 4)); CU(st.pos.ensure((size_t)std::max<int64_t>(n, 1) * 4));
-  CU(st.flag.ensure((size_t)std::max<int64_t>(n, 1) * 2)); CU(st.mapq.ensure((size_t)std::max<int64_t>(n, 1)));
-  CU(st.cig_off.ensure((size_t)off_len * 4)); CU(st.cig.ensure((size_t)n_cig_total * 4 + 16));
   CU(st.raw.ensure((size_t)std::max<int64_t>(n, 1) * 2 + crs_bytes + 16));     // [contig_read_start | n_cigar]
   cudaStream_t cs = ctx->copy_stream;
   char* extra = st.raw.as<char>();
@@ -1010,26 +1018,7 @@ int mcov_depth_sorted_packed(mcov_ctx* ctx, int64_t n, const int64_t* contig_rea
         st.cig_off.as<int32_t>(), off_len, ctx->d_tile_cnt.as<unsigned long long>(), pc_of(ctx))));
     CU(cudaGetLastError());
   }
-  ExpandArgs a;
-  std::memset(&a, 0, sizeof(a));
-  a.n = n; a.n_cig = n_cig_total;
-  a.tid = st.tid.as<int32_t>(); a.pos = st.pos.as<int32_t>(); a.flag = st.flag.as<uint16_t>();
-  a.mapq = st.mapq.as<uint8_t>(); a.cig_off = st.cig_off.as<uint32_t>(); a.cig = st.cig.as<uint32_t>();
-  a.contig_off = ctx->d_off.as<int64_t>(); a.contig_len = ctx->d_len.as<int32_t>(); a.n_contigs = ctx->n_contigs;
-  a.filt = ctx->filt; a.delta = ctx->depth; a.pc = pc_of(ctx);
-  a.cig_aligned16 = 1;
-  rc = depth_from_columns(ctx, a);
-  if (rc) return rc;
-  ctx->n_reads_pushed = n;
-  rc = finish_stage(ctx, &st);
-  if (rc) return rc;
-  ctx->state = kDepthReady;
-  ctx->verdict_pending = true;
-  if (!wait) return MCOV_OK;
-  PassCounters h;
-  CU(cudaMemcpyAsync(&h, ctx->d_pc.p, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));
-  return fused_verdict(ctx, h);
+  return run_sorted_pass(ctx, columns_of(ctx, st, n, n_cig_total), &st, n, true, wait != 0, "mcov_depth_sorted_packed");
 }
 
 int mcov_pass_info_get(mcov_ctx* ctx, mcov_pass_info* out) {
@@ -1037,9 +1026,7 @@ int mcov_pass_info_get(mcov_ctx* ctx, mcov_pass_info* out) {
   if (ctx->state == kIdle) return fail(ctx, MCOV_ERR_STATE, "mcov_pass_info_get: no pass has run");
   CU(cudaSetDevice(ctx->device));
   PassCounters h;
-  CU(cudaMemcpyAsync(&h, ctx->d_pc.p, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));
-  { int vr = fused_verdict(ctx, h); if (vr) return vr; }
+  { int vr = sync_verdict(ctx, "mcov_pass_info_get", &h); if (vr) return vr; }
   out->n_reads = ctx->n_reads_pushed;
   out->n_pass = (int64_t)h.n_pass;
   out->aligned_bases = (int64_t)h.aligned_bases;
@@ -1115,17 +1102,13 @@ int mcov_copy_depth(mcov_ctx* ctx, int32_t tid, int32_t start, int32_t end, int3
   CU(cudaSetDevice(ctx->device));
   CU(cudaMemcpyAsync(host_out, ctx->depth + ctx->off[tid] + start, (size_t)(end - start) * 4, cudaMemcpyDeviceToHost,
                      ctx->stream));
-  PassCounters h;
-  if (ctx->verdict_pending) CU(cudaMemcpyAsync(&h, ctx->d_pc.p, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));
-  if (ctx->verdict_pending) return fused_verdict(ctx, h);
-  return MCOV_OK;
+  return sync_verdict(ctx, "mcov_copy_depth");
 }
 
 // Build (or reuse) the plan of a region set and enqueue the statistics kernels writing g
 // records to d_out (device memory).
 static int stats_launch(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int32_t* start, const int32_t* end,
-                        int32_t breadth_n, mcov_region_stats* d_out) {
+                        int32_t breadth_n, mcov_region_stats* d_out, const char* who) {
   cudaStream_t s = ctx->stream;
   RegionPlan& rp = ctx->plan;
   // The plan of a region set is cached on the device: a caller that asks for the same
@@ -1136,26 +1119,19 @@ static int stats_launch(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int3
                     std::memcmp(rp.end.data(), end, (size_t)g * 4) == 0;
   if (!same && g > 0) {
     rp.valid = false;
-    for (int64_t i = 0; i < g; ++i) {
-      if (tid[i] < 0 || tid[i] >= ctx->n_contigs || start[i] < 0 || end[i] < start[i])
-        return fail(ctx, MCOV_ERR_ARG, "mcov_region_stats_run: need 0 <= start <= end and a valid tid");
-    }
-    // A region may reach past its contig: the reference's vector is end-start long whatever the
-    // contig length (pileup.py:10-11) and stays 0 there, so those positions count as depth 0.
+    int rc = check_regions(ctx, g, tid, start, end, who);
+    if (rc) return rc;
     // A region is LARGE (k_stats_stream) when more than kSmallRegion of its slots lie inside the
     // contig, SMALL (k_region_stats_warp) when it has fewer but at least one slot or one padding
     // position; a region with neither is in no list.
     std::vector<StatTask> small;
     rp.rlen.assign((size_t)g, 0); rp.rpad.assign((size_t)g, 0);
     for (int64_t i = 0; i < g; ++i) {
-      int64_t len = ctx->len[tid[i]];
-      int64_t cs = std::min<int64_t>(start[i], len), ce = std::min<int64_t>(end[i], len);
-      int64_t n = ce - cs;
-      int32_t pad = (int32_t)((int64_t)end[i] - start[i] - n);
-      rp.rlen[i] = (int32_t)n; rp.rpad[i] = pad;
-      if (n <= kSmallRegion && n + pad > 0) {
+      const Clip c = clip_region(ctx, tid[i], start[i], end[i]);
+      rp.rlen[i] = (int32_t)c.n; rp.rpad[i] = c.pad;
+      if (c.n <= kSmallRegion && c.n + c.pad > 0) {
         StatTask t;
-        t.slot = ctx->off[tid[i]] + cs; t.n = (int32_t)n; t.region = (int32_t)i;
+        t.slot = ctx->off[tid[i]] + c.cs; t.n = (int32_t)c.n; t.region = (int32_t)i;
         small.push_back(t);
       }
     }
@@ -1172,7 +1148,7 @@ static int stats_launch(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int3
     for (int64_t i = 0; i < g && total_big > 0; ++i) {
       if (rp.rlen[i] <= kSmallRegion) continue;
       int64_t rem = rp.rlen[i];
-      int64_t slot = ctx->off[tid[i]] + std::min<int64_t>(start[i], ctx->len[tid[i]]);
+      int64_t slot = ctx->off[tid[i]] + clip_region(ctx, tid[i], start[i], end[i]).cs;
       const size_t first_piece = pieces.size();
       while (rem > 0) {
         const int64_t take = std::min(rem, room);
@@ -1262,7 +1238,6 @@ int mcov_region_stats_run(mcov_ctx* ctx, int64_t g, const int32_t* tid, const in
   if (g > INT32_MAX) return fail(ctx, MCOV_ERR_RANGE, "mcov_region_stats_run: more than 2^31-1 regions");
   CU(cudaSetDevice(ctx->device));
   cudaStream_t s = ctx->stream;
-  RegionPlan& rp = ctx->plan;
   // Results and the pending verdict come back through pinned memory (a pageable destination would
   // make the copy synchronous and slow): straight into host_out when the caller's buffer is itself
   // pinned, else through the context's staging buffer.
@@ -1277,14 +1252,14 @@ int mcov_region_stats_run(mcov_ctx* ctx, int64_t g, const int32_t* tid, const in
   char* stage = ctx->h_pin.as<char>();
   if (g > 0) {
     CU(ctx->d_out.ensure(out_bytes));
-    int rc = stats_launch(ctx, g, tid, start, end, breadth_n, ctx->d_out.as<mcov_region_stats>());
+    int rc = stats_launch(ctx, g, tid, start, end, breadth_n, ctx->d_out.as<mcov_region_stats>(), "mcov_region_stats_run");
     if (rc) return rc;
     CU(cudaMemcpyAsync(direct ? (void*)host_out : (void*)stage, ctx->d_out.p, out_bytes, cudaMemcpyDeviceToHost, s));
   }
   PassCounters* hp = reinterpret_cast<PassCounters*>(stage + (direct ? 0 : out_bytes));
   if (ctx->verdict_pending) CU(cudaMemcpyAsync(hp, ctx->d_pc.p, sizeof(PassCounters), cudaMemcpyDeviceToHost, s));
   CU(cudaStreamSynchronize(s));
-  if (ctx->verdict_pending) { PassCounters h = *hp; int vr = fused_verdict(ctx, h); if (vr) return vr; }
+  { int vr = fused_verdict(ctx, *hp, "mcov_region_stats_run"); if (vr) return vr; }
   if (g > 0 && !direct) std::memcpy(host_out, stage, out_bytes);
   // htslib's cap fired in this pass (rare: a pile deeper than max_depth).  The depth store holds the replay of the
   // WHOLE-CONTIG iterator; the reference builds one iterator per region (metacov/cli.py:85-95 -> pileup.py:13), which is
@@ -1322,9 +1297,8 @@ int mcov_region_stats_run(mcov_ctx* ctx, int64_t g, const int32_t* tid, const in
       CU(cudaGetLastError());
       for (size_t q = 0; q < k; ++q) {
         const int64_t i = idx[q];
-        const int64_t len = ctx->len[tid[i]];
-        const int64_t cs = std::min<int64_t>(start[i], len), ce = std::min<int64_t>(end[i], len);
-        int rc = mcov_order_stats_by_sort(ctx, d_scr + soff[q] + cs, ce - cs, (int64_t)end[i] - start[i] - (ce - cs), breadth_n,
+        const Clip c = clip_region(ctx, tid[i], start[i], end[i]);
+        int rc = mcov_order_stats_by_sort(ctx, d_scr + soff[q] + c.cs, c.n, c.pad, breadth_n,
                                           ctx->d_out.as<mcov_region_stats>() + i, ctx->d_win_slot, ctx->d_win_out);
         if (rc) return fail(ctx, rc, "mcov_region_stats_run: per-region cap replay failed");
         CU(cudaMemcpyAsync(&host_out[i], ctx->d_out.as<mcov_region_stats>() + i, sizeof(mcov_region_stats), cudaMemcpyDeviceToHost, s));
@@ -1339,9 +1313,9 @@ int mcov_region_stats_run(mcov_ctx* ctx, int64_t g, const int32_t* tid, const in
   for (int64_t i = 0; i < g; ++i) {
     if (end[i] == start[i]) { std::memset(&host_out[i], 0, sizeof(mcov_region_stats)); continue; }
     if (host_out[i].flags & kStatOverflow) {
-      int rc = mcov_order_stats_by_sort(ctx, ctx->depth + ctx->off[tid[i]] + std::min<int64_t>(start[i], ctx->len[tid[i]]),
-                                        rp.rlen[i], rp.rpad[i], breadth_n, ctx->d_out.as<mcov_region_stats>() + i,
-                                        ctx->d_win_slot, ctx->d_win_out);
+      const Clip c = clip_region(ctx, tid[i], start[i], end[i]);
+      int rc = mcov_order_stats_by_sort(ctx, ctx->depth + ctx->off[tid[i]] + c.cs, c.n, c.pad, breadth_n,
+                                        ctx->d_out.as<mcov_region_stats>() + i, ctx->d_win_slot, ctx->d_win_out);
       if (rc) return fail(ctx, rc, "mcov_region_stats_run: radix statistics failed");
       redo = true;
     }
@@ -1372,7 +1346,7 @@ int mcov_region_stats_submit(mcov_ctx* ctx, int64_t g, const int32_t* tid, const
   if (!sl.ready) CU(cudaEventCreateWithFlags(&sl.ready, cudaEventDisableTiming));
   if (g > 0) {
     CU(sl.d_rec.ensure(out_bytes));
-    int rc = stats_launch(ctx, g, tid, start, end, breadth_n, sl.d_rec.as<mcov_region_stats>());
+    int rc = stats_launch(ctx, g, tid, start, end, breadth_n, sl.d_rec.as<mcov_region_stats>(), "mcov_region_stats_submit");
     if (rc) return rc;
   }
   sl.has_verdict = ctx->verdict_pending;
@@ -1411,11 +1385,11 @@ static int stats_collect_common(mcov_ctx* ctx, int slot, mcov_region_stats** vie
   sl.g = -1;
   const size_t out_bytes = (size_t)g * sizeof(mcov_region_stats);
   if (sl.has_verdict) {
+    // (the context may hold the next pass by now: its state and pending verdict are not this slot's)
     PassCounters h;
     std::memcpy(&h, sl.buf.as<char>() + out_bytes, sizeof(h));
-    if (h.unsorted) return fail(ctx, MCOV_ERR_UNSORTED, "mcov_region_stats_collect: the reads of that pass were not sorted by (tid,pos)");
-    if ((int64_t)h.n_far > std::min<int64_t>(std::max<int64_t>(sl.n_reads, 1), kFarCapDefault))
-      return fail(ctx, MCOV_ERR_RANGE, "mcov_region_stats_collect: too many long-span reads in that pass");
+    int rc = check_pass(ctx, h, sl.n_reads, "mcov_region_stats_collect");
+    if (rc) return rc;
     ctx->cap_contigs = (int32_t)h.cap_contigs;      // (the replay ran on the device before the statistics kernels)
     sl.cap_contigs = (int32_t)h.cap_contigs;
   }
@@ -1464,7 +1438,7 @@ int mcov_region_stats_enqueue(mcov_ctx* ctx, int64_t g, const int32_t* tid, cons
   if (g > INT32_MAX) return fail(ctx, MCOV_ERR_RANGE, "mcov_region_stats_enqueue: more than 2^31-1 regions");
   if (g == 0) return MCOV_OK;
   CU(cudaSetDevice(ctx->device));
-  return stats_launch(ctx, g, tid, start, end, breadth_n, dev_out);
+  return stats_launch(ctx, g, tid, start, end, breadth_n, dev_out, "mcov_region_stats_enqueue");
 }
 
 int mcov_region_hist_enqueue(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int32_t* start, const int32_t* end,
@@ -1475,21 +1449,18 @@ int mcov_region_hist_enqueue(mcov_ctx* ctx, int64_t g, const int32_t* tid, const
   if (g > INT32_MAX) return fail(ctx, MCOV_ERR_RANGE, "mcov_region_hist_enqueue: more than 2^31-1 regions");
   if (g == 0) return MCOV_OK;
   CU(cudaSetDevice(ctx->device));
+  int rc = check_regions(ctx, g, tid, start, end, "mcov_region_hist_enqueue");
+  if (rc) return rc;
   constexpr int64_t kChunk = 65536;
   std::vector<HistTask> tasks;
   for (int64_t i = 0; i < g; ++i) {
-    if (tid[i] < 0 || tid[i] >= ctx->n_contigs || start[i] < 0 || end[i] < start[i])
-      return fail(ctx, MCOV_ERR_ARG, "mcov_region_hist_enqueue: need 0 <= start <= end and a valid tid");
-    const int64_t len = ctx->len[tid[i]];
-    const int64_t cs = std::min<int64_t>(start[i], len), ce = std::min<int64_t>(end[i], len);
-    const int64_t n = ce - cs;
-    int32_t pad = (int32_t)((int64_t)end[i] - start[i] - n);       // beyond the contig end: depth 0 (pileup.py:10-11)
-    const int64_t nch = std::max<int64_t>((n + kChunk - 1) / kChunk, pad > 0 ? 1 : 0);
+    const Clip c = clip_region(ctx, tid[i], start[i], end[i]);
+    const int64_t nch = std::max<int64_t>((c.n + kChunk - 1) / kChunk, c.pad > 0 ? 1 : 0);
     for (int64_t k = 0; k < nch; ++k) {
       HistTask t;
-      t.slot = ctx->off[tid[i]] + cs + k * kChunk;
-      t.n = (int32_t)std::max<int64_t>(0, std::min<int64_t>(kChunk, n - k * kChunk));
-      t.region = (int32_t)i; t.pad = k == 0 ? pad : 0; t.reserved = 0;
+      t.slot = ctx->off[tid[i]] + c.cs + k * kChunk;
+      t.n = (int32_t)std::max<int64_t>(0, std::min<int64_t>(kChunk, c.n - k * kChunk));
+      t.region = (int32_t)i; t.pad = k == 0 ? c.pad : 0; t.reserved = 0;
       tasks.push_back(t);
     }
   }
@@ -1542,11 +1513,8 @@ int mcov_depth_runs(mcov_ctx* ctx, int32_t tid0, int32_t tid1, int64_t* n_runs_o
   MCOV_LAUNCH(ctx, kKRunOffsets, (k_run_offsets<<<1, 1024, 0, s>>>(counts, nt)));
   CU(cudaGetLastError());
   long long total = 0;
-  PassCounters h;
   CU(cudaMemcpyAsync(&total, counts + nt, 8, cudaMemcpyDeviceToHost, s));
-  if (ctx->verdict_pending) CU(cudaMemcpyAsync(&h, ctx->d_pc.p, sizeof(h), cudaMemcpyDeviceToHost, s));
-  CU(cudaStreamSynchronize(s));                    // (also: `tasks` has been consumed)
-  if (ctx->verdict_pending) { int vr = fused_verdict(ctx, h); if (vr) return vr; }
+  { int vr = sync_verdict(ctx, "mcov_depth_runs"); if (vr) return vr; }     // (the synchronise also: `tasks` has been consumed)
   if (total > 0) {
     CU(ctx->d_run_out.ensure((size_t)total * 16));
     int32_t* o = ctx->d_run_out.as<int32_t>();

@@ -79,3 +79,35 @@ def test_stream_rejects_misuse():
         eng.stream_push(sub_batch(b, np.arange(n // 2, n)), last=False)
         with pytest.raises(McovError):                                    # a batch that ends before the previous one
             eng.stream_push(sub_batch(b, np.arange(0, n // 4)), last=False)
+
+
+def test_stream_cap_verdict_reaches_every_consumer():
+    """Where htslib's max_depth cap fires in a streamed pass, the pass cannot be replayed exactly (the pile's contig
+    may be spread over batches) and its depth is not the capped one.  Every call that delivers the verdict of such a
+    pass must refuse it with MCOV_ERR_STATE, the pipelined statistics included."""
+    from metacov_b200 import CoverageEngine, McovError, ReadBatch, _capi
+    rng = np.random.default_rng(23)
+    lengths = np.array([20000], np.int32)
+    pos = np.sort(np.r_[np.full(400, 9000), rng.integers(0, 19900, 3000)]).astype(np.int32)     # a pile 400 deep
+    n = len(pos)
+    reflen = np.full(n, 100, np.int64)
+    b = ReadBatch(np.zeros(n, np.int32), pos, np.zeros(n, np.uint16), np.full(n, 30, np.uint8),
+                  np.arange(n + 1, dtype=np.uint32), reflen.astype(np.uint32) << 4)
+    cuts = np.r_[0, n // 3, 2 * n // 3, n]
+    tid, start, end = np.zeros(1, np.int32), np.zeros(1, np.int32), lengths
+
+    def refused(call):
+        with pytest.raises(McovError) as ei:
+            call()
+        assert ei.value.code == _capi.MCOV_ERR_STATE
+
+    with CoverageEngine(lengths) as eng:
+        eng.set_filter(max_depth=100)
+        push_in_batches(eng, b, reflen, cuts)
+        refused(lambda: eng.region_stats(tid, start, end))
+        push_in_batches(eng, b, reflen, cuts)
+        refused(eng.pass_info)
+        for copy in (True, False):
+            push_in_batches(eng, b, reflen, cuts)
+            ticket = eng.region_stats_submit(tid, start, end, slot=0)
+            refused(lambda: eng.region_stats_collect(ticket, copy=copy))
