@@ -100,7 +100,9 @@ int64_t mcov_n_slots(const mcov_ctx* ctx);
 int64_t mcov_contig_offset(const mcov_ctx* ctx, int32_t tid);
 
 /* Optional: caller-owned device buffer (e.g. a torch.int32 tensor) of at
- * least mcov_n_slots() elements to hold the depth. */
+ * least mcov_n_slots() elements to hold the depth.  The caller must not write
+ * it between a depth pass and the statistics of that pass: the statistics of
+ * large regions may be taken from per-tile histograms counted by the pass. */
 int  mcov_bind_depth(mcov_ctx* ctx, int32_t* dev, int64_t n_slots);
 
 int  mcov_set_filter(mcov_ctx* ctx, const mcov_filter* f);
@@ -377,7 +379,8 @@ int  mcov_window_means(mcov_ctx* ctx, int32_t window, double* host_out, int64_t 
 
 /* Replaces reading `column.n` back one column at a time (pileup.py:13-16). */
 int  mcov_copy_depth(mcov_ctx* ctx, int32_t tid, int32_t start, int32_t end, int32_t* host_out);
-/* Device pointer to the depth array (valid after finalize / depth_sorted). */
+/* Device pointer to the depth array (valid after finalize / depth_sorted).
+ * The caller may write through it: later statistics read the depth again. */
 int32_t* mcov_depth_ptr(mcov_ctx* ctx);
 
 /* Counters of the last pass. */

@@ -65,6 +65,8 @@ struct RegionPlan {
   int64_t g = 0, n_small = 0;
   int32_t ss_grid = 0, n_split = 0;      // balanced stream over the large regions (k_stats_stream.cuh): CTAs, split regions
   int64_t n_contigs_epoch = -1;
+  int64_t id = 0;                        // distinct for every plan the context builds
+  int64_t hist_tiles = 0;                // tiles that lie wholly inside a large region (their histograms spare the statistics the depth)
   std::vector<int32_t> tid, start, end, rlen, rpad;
 };
 
@@ -138,6 +140,12 @@ struct mcov_ctx {
 
   // fused (sorted) path scratch
   mcov::DevBuf d_start_slot, d_far_list, d_tile_cnt, d_tile_off, d_far_sorted;
+  // per-tile depth histograms of the last one-shot fused pass (FusedArgs::tile_hist), written because of plan
+  // tile_hist_plan; tile_hist_valid: they describe the depth store as it is now (cleared by every call that writes the
+  // depth otherwise, and by mcov_depth_ptr, which hands the store to the caller)
+  mcov::DevBuf d_tile_hist;
+  bool tile_hist_valid = false;
+  int64_t tile_hist_plan = 0, plan_serial = 0;
 
   // stats scratch
   mcov::DevBuf d_ss_pieces, d_ss_cta, d_ss_split, d_ss_pool;

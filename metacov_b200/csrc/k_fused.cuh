@@ -56,6 +56,13 @@ constexpr int kFusedThreads = kTile / 16; // 16 slots per thread
 constexpr int kTileVec = 4;               // = four int4 per thread (independent of the push path's scan shape)
 static_assert(kFusedThreads * kTileVec * 4 == kTile, "tile kernel: threads x vectors x 4 slots must cover the tile");
 static_assert(kTileShift >= 9 && kTileShift <= 12, "record format: 12-bit offset, 13-bit span code");
+// Depth histogram of one tile, written by the tile kernel so that the statistics of large regions need not read the
+// depth of the tiles that lie wholly inside them (k_stats_stream.cuh): kTileHistWords u16, [0] = anchor A, [1 + b] =
+// slots of the tile with depth A + b (b < kTileHistBins).  A = kTileHistNone: some depth of the tile lies outside the
+// window (or the tile's depth was rewritten afterwards), the tile is counted from the depth.
+constexpr int kTileHistWords = 128;
+constexpr int kTileHistBins = kTileHistWords - 1;
+constexpr uint16_t kTileHistNone = 0xFFFF;
 constexpr int kPrepThreads = 256;
 constexpr int kPrepPer = 4;               // reads per thread
 constexpr uint32_t kFarCapDefault = 1u << 26;
@@ -76,6 +83,7 @@ struct FusedArgs {
   uint32_t* tile_first;       // [n_tiles+1] (a fused batch holds < 2^32 reads)
   int32_t* depth;
   int32_t* tile_cap;          // [n_tiles] max of depth[p-1]+starts[p] in the tile, written only when > max_depth
+  uint16_t* tile_hist;        // [n_tiles][kTileHistWords] depth histograms of the tiles (k_tile_tma.cuh), nullptr: not written
   uint32_t* tile_heavy;       // [n_tiles] ids of the tiles with >= heavy_min reads (k_far_scatter; pc->n_heavy of them)
   uint32_t heavy_min;
   int32_t max_depth;          // htslib maxcnt (<= 0: cap disabled)
@@ -706,6 +714,11 @@ __global__ void k_cap_replay(FusedArgs f, uint8_t* __restrict__ contig_capped) {
   }
   atomicAdd(&f.e.pc->cap_contigs, 1u);
   contig_capped[c] = 1;
+  if (f.tile_hist) {                                // the histograms of the contig's tiles describe the uncapped depth
+    const int64_t b0 = f.e.contig_off[c];
+    const int64_t T1 = min((b0 + f.e.contig_len[c]) >> kTileShift, f.n_tiles - 1);
+    for (int64_t T = b0 >> kTileShift; T <= T1; ++T) f.tile_hist[T * kTileHistWords] = kTileHistNone;
+  }
   cap_replay_contig(f, c, f.depth + f.e.contig_off[c], 0, (int64_t)f.e.contig_len[c] + 1);
 }
 

@@ -15,7 +15,13 @@
 //     histogram in global memory (fire-and-forget reductions, nobody waits), and the CTA whose
 //     piece of it arrives last pulls the merged bin range back and walks the region.
 // The walk is hist_walk (k_stats.cuh), the same as for the small regions.
+//
+// When the tile kernel has left a depth histogram of every tile (FusedArgs::tile_hist, k_fused.cuh) that still
+// describes the depth, the tiles that lie wholly inside a piece are counted from their histograms (256 bytes each
+// instead of 8 KB of depth); only the piece's ends, and the tiles whose depth left the histogram's window, are read
+// from the depth.
 #pragma once
+#include "k_fused.cuh"
 #include "k_stats.cuh"
 
 namespace mcov {
@@ -43,7 +49,10 @@ struct SsPiece {          // a region, or the part of a region inside one slice
   int32_t split;          // -1: the whole region is this piece; else index of the region's global histogram
 };
 
-struct SsDesc { int32_t region, split, pad, skip, cnt, last; };     // cnt < 0: end of the slice
+// cnt < 0: end of the slice.  tile < 0: the stage holds depth, valid elements [skip, skip + cnt); else the histograms
+// of the cnt tiles from `tile` on
+struct SsDesc { int32_t region, split, pad, skip, cnt, last, tile; };
+constexpr int kSsHistTiles = kSsBlk * 4 / (kTileHistWords * 2);     // tile histograms per stage
 
 struct SsArgs {
   const int32_t* depth;
@@ -54,6 +63,7 @@ struct SsArgs {
   uint32_t* split_hist;             // [n_split][kHistBins], zero between runs
   RegionScratch* split_scratch;     // [n_split] arrival counter + bin range of the merged histogram, zero between runs
   const int32_t* split_pieces;      // [n_split] pieces of the split region: the CTA that merges the last one walks the region
+  const uint16_t* tile_hist;        // [n_tiles][kTileHistWords] histograms of the depth's tiles (k_fused.cuh), nullptr: none
   mcov_region_stats* out;
   int32_t breadth_n;
 };
@@ -100,21 +110,36 @@ k_stats_stream(const __grid_constant__ SsArgs a) {
       }
       ++it;
     };
-    for (int p = p0; p < p1; ++p) {
-      const SsPiece pc = a.pieces[p];
-      const int64_t a0 = pc.slot & ~(int64_t)3, end = pc.slot + pc.n;
-      const int64_t nblk = pc.n > 0 ? (end - a0 + kSsBlk - 1) / kSsBlk : 1;      // a piece without slots still finishes its region
+    // the depth of the slots [s0, s1) of a piece; `last`: the piece ends there (a piece without slots still finishes its region)
+    auto depth_stages = [&](const SsPiece& pc, int64_t s0, int64_t s1, bool last) {
+      const int64_t a0 = s0 & ~(int64_t)3;
+      const int64_t nblk = s1 > s0 ? (s1 - a0 + kSsBlk - 1) / kSsBlk : (last ? 1 : 0);
       for (int64_t k = 0; k < nblk; ++k) {
         const int64_t b0 = a0 + k * kSsBlk;
-        const int64_t lo = max(b0, pc.slot), hi = min(b0 + kSsBlk, end);
+        const int64_t lo = max(b0, s0), hi = min(b0 + kSsBlk, s1);
         SsDesc d;
-        d.region = pc.region; d.split = pc.split; d.pad = pc.pad;
-        d.skip = (int32_t)(lo - b0); d.cnt = (int32_t)max((int64_t)0, hi - lo); d.last = (k == nblk - 1) ? 1 : 0;
+        d.region = pc.region; d.split = pc.split; d.pad = pc.pad; d.tile = -1;
+        d.skip = (int32_t)(lo - b0); d.cnt = (int32_t)max((int64_t)0, hi - lo); d.last = (last && k == nblk - 1) ? 1 : 0;
         const uint32_t bytes = d.cnt > 0 ? (uint32_t)((d.skip + d.cnt + 3) & ~3) * 4u : 0u;   // whole 16-byte vectors inside the padded depth array
         publish(d, a.depth + b0, bytes);
       }
+    };
+    for (int p = p0; p < p1; ++p) {
+      const SsPiece pc = a.pieces[p];
+      const int64_t end = pc.slot + pc.n;
+      // tiles [t0, t1) lie wholly inside the piece
+      const int64_t t0 = a.tile_hist ? (pc.slot + kTile - 1) >> kTileShift : 0, t1 = a.tile_hist ? end >> kTileShift : 0;
+      if (t1 <= t0) { depth_stages(pc, pc.slot, end, true); continue; }
+      depth_stages(pc, pc.slot, t0 << kTileShift, false);
+      for (int64_t t = t0; t < t1; t += kSsHistTiles) {
+        SsDesc d;
+        d.region = pc.region; d.split = pc.split; d.pad = pc.pad;
+        d.skip = 0; d.cnt = (int32_t)min((int64_t)kSsHistTiles, t1 - t); d.last = 0; d.tile = (int32_t)t;
+        publish(d, reinterpret_cast<const int32_t*>(a.tile_hist + t * kTileHistWords), (uint32_t)d.cnt * kTileHistWords * 2u);
+      }
+      depth_stages(pc, t1 << kTileShift, end, true);
     }
-    SsDesc e; e.region = -1; e.split = -1; e.pad = 0; e.skip = 0; e.cnt = -1; e.last = 0;
+    SsDesc e; e.region = -1; e.split = -1; e.pad = 0; e.skip = 0; e.cnt = -1; e.last = 0; e.tile = -1;
     publish(e, nullptr, 0u);
     return;
   }
@@ -127,7 +152,29 @@ k_stats_stream(const __grid_constant__ SsArgs a) {
     mbar_wait(&s_full[s], k & 1);
     const SsDesc d = s_desc[s];
     if (d.cnt < 0) break;
-    if (d.cnt > 0) {
+    if (d.tile >= 0) {
+      // 64 threads per tile histogram, a u32 (two u16 words) each: word 2w holds bin 2w - 1, word 2w + 1 bin 2w
+      const uint32_t* h = reinterpret_cast<const uint32_t*>(s_ring + (size_t)s * kSsBlk);
+      constexpr int kPer = kTileHistWords / 2;
+      for (int q = t; q < d.cnt * kPer; q += kSsConsumers) {
+        const int r = q / kPer, w = q % kPer;
+        const int anchor = (int)(h[r * kPer] & 0xffffu);
+        if (anchor != kTileHistNone) {
+          const uint32_t x = h[q];
+          const int b = anchor + 2 * w;
+          if (w > 0 && (x & 0xffffu)) { atomicAdd(&s_hist[b - 1], x & 0xffffu); lo = min(lo, b - 1); hi = max(hi, b - 1); }
+          if (x >> 16) { atomicAdd(&s_hist[b], x >> 16); lo = min(lo, b); hi = max(hi, b); }
+        } else {
+          // no histogram: the tile's depth, read by the 64 threads of its histogram (eight loads in flight each)
+          const int4* v = reinterpret_cast<const int4*>(a.depth + ((int64_t)(d.tile + r) << kTileShift)) + w;
+          int4 x[kTile / 4 / kPer];
+#pragma unroll
+          for (int u = 0; u < kTile / 4 / kPer; ++u) x[u] = __ldcs(v + u * kPer);
+#pragma unroll
+          for (int u = 0; u < kTile / 4 / kPer; ++u) hist_vec(s_hist, x[u], lo, hi);
+        }
+      }
+    } else if (d.cnt > 0) {
       const int4* v = reinterpret_cast<const int4*>(s_ring + (size_t)s * kSsBlk);
       const int stop = d.skip + d.cnt;                                  // valid elements [skip, stop)
       const int nvec = (stop + 3) >> 2;

@@ -21,6 +21,7 @@
 // the tile range [tile_lo, tile_hi) (streaming: successive batches of a sorted file).
 #pragma once
 #include "k_fused.cuh"
+#include "k_stats.cuh"
 
 namespace mcov {
 
@@ -138,6 +139,25 @@ __device__ __forceinline__ int tt_scatter(const FusedArgs& f, const TtMeta& m, c
   return open;
 }
 
+// The depth histogram of the previous tile (f.tile_hist): one u16 per consumer thread, and its bins cleared for the
+// next tile.  Called after the current tile's first barrier, which every consumer passes only when it has counted the
+// previous tile; the current tile counts after its second barrier.
+static_assert(kFusedThreads == kTileHistWords, "one histogram word per consumer thread");
+static_assert(kHistBins - 1 - kTileHistBins < (int)kTileHistNone, "anchors stay below kTileHistNone");
+__device__ __forceinline__ void tt_hist_flush(const FusedArgs& f, uint32_t* s_th, const int* s_th_tile) {
+  const int tile = s_th_tile[0];
+  if (tile < 0) return;
+  const int t = threadIdx.x, b = (t + kTileHistWords - 1) & (kTileHistWords - 1);      // thread 0: the outside-window bin
+  const uint32_t c = s_th[b];
+  s_th[b] = 0u;
+  const int anchor = s_th_tile[1];
+  // anchor + kTileHistBins <= kHistBins - 1: the histogram holds no value of the statistics' overflow bin
+  const bool ok = c == 0u && anchor + kTileHistBins <= kHistBins - 1;
+  f.tile_hist[(int64_t)tile * kTileHistWords + t] = t == 0 ? (ok ? (uint16_t)anchor : kTileHistNone) : (uint16_t)c;
+}
+
+// HIST: also write the depth histogram of every tile to f.tile_hist (a pass without histograms runs code without them)
+template <bool HIST>
 __global__ void __launch_bounds__(kTtThreads, MCOV_TT_CTAS)
 k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
   __shared__ __align__(16) int s_cnt[kTile + 36];       // [kTile ..]: spare counters (tt_scatter)
@@ -146,11 +166,17 @@ k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
   __shared__ TtMeta s_meta[kTtStages];
   __shared__ int s_warp[kFusedThreads / 32], s_warp2[kFusedThreads / 32];
   __shared__ int s_open[2];
+  // depth histogram of the tile (f.tile_hist): bins [anchor, anchor + kTileHistBins), then one bin for everything
+  // outside; the tile and the anchor it was counted with, kept for tt_hist_flush
+  __shared__ uint32_t s_th[kTileHistWords];
+  __shared__ int s_th_tile[2];
   PassCounters* pc = f.e.pc;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   {                                                     // (before the dependency wait: touches nothing global)
     int4* z0 = reinterpret_cast<int4*>(s_cnt);
     for (int k = threadIdx.x; k < kTile / 4; k += kTtThreads) z0[k] = make_int4(0, 0, 0, 0);
+    if (HIST && threadIdx.x < kTileHistWords) s_th[threadIdx.x] = 0u;
+    if (HIST && threadIdx.x == 0) s_th_tile[0] = -1;
     if (threadIdx.x < 2) s_open[threadIdx.x] = 0;
     if (threadIdx.x == 0) {
       for (int s = 0; s < kTtStages; ++s) { mbar_init(&s_full[s], 1); mbar_init(&s_empty[s], kFusedThreads / 32); }
@@ -250,6 +276,7 @@ k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
       open = __reduce_add_sync(0xffffffffu, open);
       if (lane == 0) { if (open) atomicAdd(&s_open[par], open); mbar_arrive(&s_empty[s]); }   // stage free: the records have been read
       named_bar_sync<1, kFusedThreads>();
+      if (HIST) tt_hist_flush(f, s_th, s_th_tile);
       const int4* vs = reinterpret_cast<const int4*>(s_cnt);
 #pragma unroll
       for (int j = 0; j < kTileVec; ++j) {
@@ -269,6 +296,7 @@ k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
       // dense tile: starts and ends counted in two 32-bit passes over the same counters
       tt_scatter<1, false>(f, m, rec, s_cnt, reach, has_far);
       named_bar_sync<1, kFusedThreads>();
+      if (HIST) tt_hist_flush(f, s_th, s_th_tile);
 #pragma unroll
       for (int j = 0; j < kTileVec; ++j) {
         const int idx = (warp * kTileVec + j) * 32 + lane;
@@ -332,6 +360,9 @@ k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
     if (threadIdx.x == 0) s_open[par ^ 1] = 0;
     named_bar_sync<1, kFusedThreads>();
     int off = m.carry + s_open[par];                     // far reads + near reads open at the border
+    // the histogram window is centred on the depth entering the tile
+    const int anchor = max(0, off - kTileHistBins / 2);
+    if (HIST && threadIdx.x == 0) { s_th_tile[0] = (int)m.tile; s_th_tile[1] = anchor; }
 #pragma unroll
     for (int w = 0; w < kFusedThreads / 32; ++w) off += (w < warp) ? s_warp[w] : 0;
     const int64_t base = m.tile << kTileShift;
@@ -345,7 +376,16 @@ k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
       cap_t = max(cap_t, o + capv[j]);
       v[j].x += o; v[j].y += o; v[j].z += o; v[j].w += o;
       mx = max(mx, max(max(v[j].x, v[j].y), max(v[j].z, v[j].w)));
-      if (idx < n_vec) st_stream_int4(out + idx, v[j]);
+      if (idx < n_vec) {
+        st_stream_int4(out + idx, v[j]);
+        if (HIST) {
+          // plain +1 updates (ATOMS.POPC.INC, see hist_vec); a value outside the window lands in the last bin
+          atomicAdd(&s_th[min((unsigned)(v[j].x - anchor), (unsigned)kTileHistBins)], 1u);
+          atomicAdd(&s_th[min((unsigned)(v[j].y - anchor), (unsigned)kTileHistBins)], 1u);
+          atomicAdd(&s_th[min((unsigned)(v[j].z - anchor), (unsigned)kTileHistBins)], 1u);
+          atomicAdd(&s_th[min((unsigned)(v[j].w - anchor), (unsigned)kTileHistBins)], 1u);
+        }
+      }
     }
     cap = max(cap, cap_t);
     // htslib's cap could fire somewhere in this tile (rare): remember the tile for the exact replay
@@ -355,6 +395,7 @@ k_fused_tile_tma(const __grid_constant__ FusedArgs f) {
   cap = warp_max(cap);
   if (lane == 0) { s_warp2[warp] = cap; }
   named_bar_sync<1, kFusedThreads>();                    // (s_warp of the last tile has been read by everyone)
+  if (HIST) tt_hist_flush(f, s_th, s_th_tile);
   if (lane == 0) s_warp[warp] = mx;
   named_bar_sync<1, kFusedThreads>();
   if (threadIdx.x == 0) {
