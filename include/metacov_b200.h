@@ -620,8 +620,45 @@ typedef struct mcov_bam_dev {
 int  mcov_bam_decode_gpu(mcov_ctx* ctx, const void* file_bytes, int64_t n_bytes, int verify_crc, mcov_bam_dev* out);
 /* The same straight from the file (the image is mapped, not read into a buffer of the caller's). */
 int  mcov_bam_decode_gpu_file(mcov_ctx* ctx, const char* path, int verify_crc, mcov_bam_dev* out);
-/* Read names and SEQ of the file last decoded on this context, computed on the
- * device from the inflated stream (no host reader is opened).  Each output is
+/* SAM text decoded on the device into the same columns.  The header (the '@'
+ * lines before the first record; references from @SQ SN:/LN:) is read on the
+ * host; the whole image goes to the device in chunks of chunk_bytes (0: 64 MiB)
+ * while the newlines of each copied chunk are counted, and the lines are parsed
+ * there (SAM spec 1.4 with the BAM encoding of htslib's sam_parse1: POS-1,
+ * RNAME '*' -> -1, an RNAME that is not an @SQ name is an error, CIGAR ops
+ * len<<4|op, l_seq = length of SEQ or 0 for '*'; optional fields are skipped).
+ * `inflated` points at the text and header_bytes is the header's length;
+ * n_segments is 0.  A malformed line is MCOV_ERR_IO and mcov_last_error names
+ * its 1-based line number and the field; more than 2^32-1 CIGAR ops in the file
+ * is MCOV_ERR_RANGE.  The columns are valid until the next decode on the
+ * context, like those of mcov_bam_decode_gpu.  Synchronises. */
+int  mcov_sam_decode_gpu(mcov_ctx* ctx, const void* bytes, int64_t n_bytes, int64_t chunk_bytes, mcov_bam_dev* out);
+int  mcov_sam_decode_gpu_file(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, mcov_bam_dev* out);
+/* pysam's `mapped` / `unmapped` of the file last decoded on this context (BAM or
+ * SAM), counted on the device from its columns with the BAI metadata
+ * definitions: mapped = records with tid >= 0 and without flag 0x4, unmapped =
+ * every other record.  Synchronises. */
+int  mcov_bam_gpu_mapped(mcov_ctx* ctx, int64_t* mapped, int64_t* unmapped);
+/* Test hook: the SAM rules of mcov_sam_decode_gpu (the same field helpers,
+ * csrc/k_sam.cuh) run line by line on the host, so that the CPU suite can
+ * check them.  Not a product path: the decoders have no CPU fallback.  With
+ * tid == NULL only the counts are filled (n_records, n_cigar, n_ref,
+ * header_bytes); otherwise every non-NULL array must hold n_records entries
+ * (cig_off n_records + 1, cig n_cigar, seq_win n_records x (win_bases+1)/2).
+ * name_hash / kmer_code / seq_win are the outputs of mcov_bam_gpu_names_seq.
+ * MCOV_ERR_IO on a malformed line: fail_line (1-based) and fail_field (0-10 =
+ * QNAME..QUAL, 11 = fewer than 11 fields or an empty line, 12 = a header line
+ * after a record) are set and err holds the message. */
+typedef struct mcov_sam_host_cols {
+  int64_t n_records, n_cigar, header_bytes, fail_line;
+  int32_t n_ref, fail_field, k_len, win_bases;
+  int32_t* tid; int32_t* pos; uint16_t* flag; uint8_t* mapq; int32_t* l_seq; int32_t* isize;
+  uint32_t* cig_off; uint32_t* cig;
+  uint64_t* name_hash; int32_t* kmer_code; uint8_t* seq_win;
+} mcov_sam_host_cols;
+int  mcov_sam_parse_host(const void* bytes, int64_t n_bytes, mcov_sam_host_cols* cols, char* err, int err_len);
+/* Read names and SEQ of the file last decoded on this context (BAM or SAM), computed on the
+ * device from the inflated stream or the SAM text (no host reader is opened).  Each output is
  * optional (NULL = not wanted) and lies in host or device memory per mem_kind:
  *   name_hash_out  u64[n]  FNV-1a 64 of `read.query_name`, the key of the
  *                  reference's mate dict (metacov/pileup.py:101-118)

@@ -69,6 +69,15 @@ class BamDev(C.Structure):
                 ("isize", C.c_void_p), ("cig_off", C.c_void_p), ("cig", C.c_void_p), ("inflated", C.c_void_p)]
 
 
+class SamHostCols(C.Structure):
+    """mcov_sam_host_cols: columns of the host-compiled SAM rules (test hook mcov_sam_parse_host)."""
+    _fields_ = [("n_records", C.c_int64), ("n_cigar", C.c_int64), ("header_bytes", C.c_int64), ("fail_line", C.c_int64),
+                ("n_ref", C.c_int32), ("fail_field", C.c_int32), ("k_len", C.c_int32), ("win_bases", C.c_int32),
+                ("tid", C.c_void_p), ("pos", C.c_void_p), ("flag", C.c_void_p), ("mapq", C.c_void_p), ("l_seq", C.c_void_p),
+                ("isize", C.c_void_p), ("cig_off", C.c_void_p), ("cig", C.c_void_p), ("name_hash", C.c_void_p),
+                ("kmer_code", C.c_void_p), ("seq_win", C.c_void_p)]
+
+
 class BamBatch(C.Structure):
     """mcov_bam_batch: one batch of the streaming host reader (pinned SoA views)."""
     _fields_ = [("n", C.c_int64), ("n_carry", C.c_int64), ("n_cigar", C.c_int64), ("last", C.c_int32), ("reserved", C.c_int32),
@@ -141,6 +150,10 @@ SIGNATURES = {
     "mcov_bam_decode_gpu_file": (C.c_int, [_vp, C.c_char_p, C.c_int, _vp]),
     "mcov_bam_gpu_names_seq": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _vp, C.c_int]),
     "mcov_bam_gpu_stream_depth": (C.c_int, [_vp, C.c_char_p, _i64, C.c_int, _vp]),
+    "mcov_sam_decode_gpu": (C.c_int, [_vp, _vp, C.c_int64, C.c_int64, _vp]),
+    "mcov_sam_decode_gpu_file": (C.c_int, [_vp, C.c_char_p, C.c_int64, _vp]),
+    "mcov_bam_gpu_mapped": (C.c_int, [_vp, C.POINTER(_i64), C.POINTER(_i64)]),
+    "mcov_sam_parse_host": (C.c_int, [_vp, C.c_int64, C.POINTER(SamHostCols), C.c_char_p, C.c_int]),
     "mcov_inflate_host": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint32]),
     "mcov_inflate_host_win": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint32, C.c_uint32]),
     "mcov_crc32_host": (C.c_uint32, [_vp, C.c_uint32]),

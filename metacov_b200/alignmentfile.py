@@ -133,6 +133,29 @@ def stream_depth(engine, stream):
     return k
 
 
+def is_sam_text(filename):
+    """The format decision of ``AlignmentFile``: SAM text when the file does not start with the gzip magic and its first
+    line is a header line ('@' + two letters + TAB) or has at least 11 TAB-separated fields.  Everything else (BAM, an
+    empty file, an index, garbage) is left to the BAM readers, which reject what is not BAM."""
+    try:
+        fh = open(filename, "rb")
+    except OSError:
+        return False
+    with fh:
+        line = fh.read(1 << 16)
+        if not line or line[:2] == b"\x1f\x8b":
+            return False
+        while b"\n" not in line and line.count(b"\t") < 10:        # (a long first record: read on to its tenth TAB)
+            more = fh.read(1 << 20)
+            if not more:
+                break
+            line += more
+    line = line.split(b"\n", 1)[0]
+    if len(line) >= 4 and line[:1] == b"@" and line[1:3].isalpha() and line[3:4] == b"\t":
+        return True
+    return line.count(b"\t") >= 10
+
+
 class AlignmentFile:
     def __init__(self, filename, mode="rb", device=0, decode="host", **kw):
         """decode="host": BGZF inflate and record parsing by the native host reader (csrc/bamio.cpp), streamed batch by
@@ -143,11 +166,21 @@ class AlignmentFile:
         inflated, parsed and pushed into the streamed depth pass on the device (mcov_bam_gpu_stream_depth) -- any file size,
         the host only reads; accessors that need every record on the host (soa(), read names) open the host reader on
         demand; decode="auto": "gpu" when the whole file fits the device (file size x GPU_DECODE_FOOTPRINT below the free
-        device memory), else "gpu-stream"."""
+        device memory), else "gpu-stream".
+
+        The format comes from the content (``is_sam_text``).  SAM text is always parsed whole on the device
+        (csrc/sam_gpu.cu): "host", "gpu" and "auto" all do that and ``decode`` reads "gpu"; "gpu-stream" is refused, and a
+        file whose decode does not fit the free device memory raises OSError."""
         if "w" in mode:
             raise ValueError("metacov_b200.AlignmentFile is read-only")
         if decode not in ("host", "gpu", "gpu-stream", "auto"):
             raise ValueError("decode must be 'host', 'gpu', 'gpu-stream' or 'auto'")
+        self.format = "sam" if is_sam_text(filename) else "bam"
+        if self.format == "sam":
+            if decode == "gpu-stream":
+                raise ValueError("%s: SAM text is not streamed; use decode='gpu' (or BAM input)" % filename)
+            self._check_sam_fits(filename, device)
+            decode = "gpu"
         if decode == "auto":
             decode = "gpu" if self._fits_device(filename, device) else "gpu-stream"
         self._gpu_chunk_bytes = int(kw.get("gpu_chunk_bytes", 64 << 20))
@@ -188,12 +221,35 @@ class AlignmentFile:
             return False
         return size * cls.GPU_DECODE_FOOTPRINT < free
 
+    # device bytes per byte of SAM text that the decode holds: the text (1), and per line -- 23 bytes at the least -- its
+    # end (8), the columns (23), the record offset (8), the field offsets (16) and the op count (8): 63 / 23 < 2.8; each
+    # CIGAR op (4 bytes, at least 2 of text) stays below that ratio.  With DevBuf's 1/8 growth margin: 1.125 x 3.8 < 4.3,
+    # rounded up to leave room for the depth pass that follows.
+    SAM_DECODE_FOOTPRINT = 5
+
+    @classmethod
+    def _check_sam_fits(cls, filename, device):
+        import torch
+        try:
+            size = os.path.getsize(filename)
+            free, _total = torch.cuda.mem_get_info(device)
+        except (OSError, RuntimeError):
+            return                                          # (no size or no device: the decode itself reports it)
+        if size * cls.SAM_DECODE_FOOTPRINT >= free:
+            raise OSError("%s: a SAM file of %d bytes needs about %d bytes of device memory to decode, %d are free; "
+                          "SAM is decoded whole on the device, while BAM input streams (decode='gpu-stream')"
+                          % (filename, size, size * cls.SAM_DECODE_FOOTPRINT, free))
+
     def _open_gpu(self, filename, device):
         from . import bamgpu
         self._h = None
         eng = CoverageEngine([1], device=device)            # the contig table follows once the header is decoded
         try:
-            dsoa = bamgpu.decode(eng, os.fspath(filename))      # (the library maps the file: no host copy of the image)
+            # (the library maps the file: no host copy of the image)
+            if self.format == "sam":
+                dsoa = bamgpu.decode_sam(eng, os.fspath(filename))
+            else:
+                dsoa = bamgpu.decode(eng, os.fspath(filename))
             self.text, refs = dsoa.header()
         except McovError as e:
             eng.close()
@@ -265,6 +321,8 @@ class AlignmentFile:
         return self.references[tid]
 
     def _idx(self):
+        if self._index_stats is None and self.format == "sam":
+            self._index_stats = self._gpu[1].mapped_counts()      # (SAM has no index: counted from the decoded columns)
         if self._index_stats is None:
             m, u = C.c_int64(0), C.c_int64(0)
             rc = lib.mcov_bai_stats(str(self.filename).encode(), C.byref(m), C.byref(u))
@@ -282,6 +340,8 @@ class AlignmentFile:
         return self._idx()[1]
 
     def has_index(self):
+        if self.format == "sam":
+            return False
         try:
             self._idx()
             return True

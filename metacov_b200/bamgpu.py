@@ -1,10 +1,11 @@
-"""BAM decode on the GPU (SURVEY.md 8(f) row 3): the compressed file goes to the device, BGZF blocks are
+"""BAM and SAM decode on the GPU (SURVEY.md 8(f) row 3): the compressed file goes to the device, BGZF blocks are
 inflated and the records parsed there (csrc/bam_gpu.cu), and the SoA columns stay in HBM for the coverage
 kernels.  Replaces, for this path, ``pysam.AlignmentFile`` + ``IteratorRowAll`` (reference
 metacov/scan.pyx:204, 216; cli.py:56) without the host decode of ``alignmentfile.AlignmentFile``.
 
     eng = CoverageEngine(lengths)
     soa = bamgpu.decode(eng, "reads.bam")        # device-resident columns, owned by the engine's context
+    soa = bamgpu.decode_sam(eng, "reads.sam")    # (the same columns from SAM text)
     bamgpu.depth_sorted(eng, soa)                # per-base depth straight from them
 """
 import ctypes as C
@@ -32,14 +33,16 @@ class DevView:
 
 
 class DeviceSoA:
-    """Device pointers of a decoded BAM (``mcov_bam_dev``); valid until the next decode on the same engine."""
+    """Device pointers of a decoded BAM or SAM (``mcov_bam_dev``; ``format`` "bam" or "sam"); valid until the next decode
+    on the same engine."""
 
     COLS = (("tid", np.int32), ("pos", np.int32), ("flag", np.uint16), ("mapq", np.uint8), ("l_seq", np.int32),
             ("isize", np.int32), ("cig_off", np.uint32), ("cig", np.uint32))
 
-    def __init__(self, engine, raw):
+    def __init__(self, engine, raw, format="bam"):
         self._engine = engine
         self.raw = raw
+        self.format = format
         self.n_records, self.n_cigar, self.n_ref = raw.n_records, raw.n_cigar, raw.n_ref
         self.inflated_bytes, self.header_bytes, self.n_segments = raw.inflated_bytes, raw.header_bytes, raw.n_segments
 
@@ -85,11 +88,27 @@ class DeviceSoA:
                                                        p("kmer_code"), p("seq_win"), _capi.MEM_HOST))
         return out
 
+    def mapped_counts(self):
+        """(mapped, unmapped) counted on the device from the columns, with the BAI metadata definitions
+        (``mcov_bam_gpu_mapped``)."""
+        m, u = C.c_int64(0), C.c_int64(0)
+        self._engine._check(lib.mcov_bam_gpu_mapped(self._engine._ctx, C.byref(m), C.byref(u)))
+        return m.value, u.value
+
     def header(self):
-        """(text, [(name, length)]) parsed from the inflated stream's header (SAM spec 4.2)."""
+        """(text, [(name, length)]) parsed from the inflated stream's header (SAM spec 4.2), or from the '@' lines of a
+        SAM file (text: those lines as in the file; references: @SQ SN / LN in order)."""
         buf = np.empty(self.header_bytes, dtype=np.uint8)
-        self._engine._check(lib.mcov_copy_to_host(self._engine._ctx, self.raw.inflated, _capi.ptr(buf), buf.nbytes))
+        if buf.nbytes:
+            self._engine._check(lib.mcov_copy_to_host(self._engine._ctx, self.raw.inflated, _capi.ptr(buf), buf.nbytes))
         b = buf.tobytes()
+        if self.format == "sam":
+            refs = []
+            for line in b.decode().splitlines():
+                if line.startswith("@SQ\t"):
+                    tags = dict(t.split(":", 1) for t in line.split("\t")[1:] if ":" in t)
+                    refs.append((tags["SN"], int(tags["LN"])))
+            return b.decode(), refs
         l_text = int.from_bytes(b[4:8], "little")
         text = b[8:8 + l_text].split(b"\0")[0].decode()
         p = 8 + l_text
@@ -125,6 +144,28 @@ def decode(engine, source, verify_crc=True):
     engine._check(lib.mcov_bam_decode_gpu(engine._ctx, ptr, n, 1 if verify_crc else 0, C.byref(raw)))
     del keep
     return DeviceSoA(engine, raw)
+
+
+def decode_sam(engine, source, chunk_bytes=0):
+    """Parse a SAM text file on the GPU into the same device-resident columns as ``decode`` (csrc/sam_gpu.cu).
+    ``source``: a path, ``bytes`` or a uint8 numpy array / pinned torch tensor holding the file image; ``chunk_bytes``: the
+    size of the copies the newline count overlaps (0 = 64 MiB).  Returns a ``DeviceSoA`` of format "sam"."""
+    raw = _capi.BamDev()
+    if isinstance(source, (str, os.PathLike)):
+        engine._check(lib.mcov_sam_decode_gpu_file(engine._ctx, os.fsencode(source), int(chunk_bytes), C.byref(raw)))
+        return DeviceSoA(engine, raw, "sam")
+    if isinstance(source, bytes):
+        keep = np.frombuffer(source, dtype=np.uint8)
+        ptr, n = keep.ctypes.data, keep.nbytes
+    elif hasattr(source, "data_ptr"):
+        keep = source
+        ptr, n = source.data_ptr(), source.numel() * source.element_size()
+    else:
+        keep = np.ascontiguousarray(source, dtype=np.uint8)
+        ptr, n = keep.ctypes.data, keep.nbytes
+    engine._check(lib.mcov_sam_decode_gpu(engine._ctx, ptr, n, int(chunk_bytes), C.byref(raw)))
+    del keep
+    return DeviceSoA(engine, raw, "sam")
 
 
 def depth_sorted(engine, soa, wait=True):

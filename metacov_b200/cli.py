@@ -35,7 +35,7 @@ def main():
 
 @main.command()
 @click.option("--bamfile", "-b", type=click.File("rb"), required=True,
-              help="Input BAM file. Must be sorted and indexed.")
+              help="Input BAM (sorted, indexed) or SAM file.")
 @click.option("--reference-fasta", "-f", type=click.File("rb"))
 @click.option("--regionfile-blast7", "-rb", type=click.File("r"), help="Input Region file in BLAST7 format")
 @click.option("--regionfile-csv", "-rc", type=click.File("r"), help="Input Region file in CSV format")
@@ -50,7 +50,8 @@ def main():
 @click.option("--window-out", "-wo", type=click.File("w"), metavar="FILE", help="Output CSV of --window (sacc,start,end,avg)")
 @click.option("--bam-decode", type=click.Choice(["host", "gpu", "gpu-stream", "auto"]), default="auto", show_default=True,
               help="Where the BAM file is inflated and parsed: host threads (zlib), the GPU (whole file / streamed in chunks), or "
-                   "auto = the GPU, streamed when the file does not fit it. Not in the reference: additive.")
+                   "auto = the GPU, streamed when the file does not fit it. Applies to BAM only: SAM text is always parsed whole "
+                   "on the GPU (gpu-stream is refused for it). Not in the reference: additive.")
 def pileup(bamfile, reference_fasta, regionfile_blast7, regionfile_csv, kmer_histogram, kmer_length, outfile,
            bedgraph=None, window=None, window_out=None, bam_decode="auto"):
     """
@@ -155,7 +156,8 @@ def write_windows(bam, window, out):
               help="Compute histogram of insert sizes.")
 @click.option("--bam-decode", type=click.Choice(["host", "gpu", "gpu-stream", "auto"]), default="auto", show_default=True,
               help="Where the BAM file is inflated and parsed (see `pileup`); with the GPU the accumulators run on the "
-                   "device-resident columns. Not in the reference: additive.")
+                   "device-resident columns. Applies to BAM only: SAM text is always parsed on the GPU. Not in the "
+                   "reference: additive.")
 @click.argument("readfile", nargs=-1, required=True)
 def scan(readfile, readfile_type, out_basehist, boffset, out_kmerhist, k, number, step, offset, max_reads,
          reference_fasta, out_mirrorhist, mirror_offset, mirror_length, out_isizehist, group_by, bam_decode="auto"):

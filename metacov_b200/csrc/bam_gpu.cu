@@ -466,6 +466,7 @@ extern "C" int mcov_bam_decode_gpu(mcov_ctx* ctx, const void* file_bytes, int64_
   if (!file_bytes || n_bytes <= 0 || !out) return bfail(ctx, MCOV_ERR_ARG, "mcov_bam_decode_gpu: bad arguments");
   std::memset(out, 0, sizeof(*out));
   CUB(cudaSetDevice(ctx->device));
+  ctx->bam.sam = false;
   cudaStream_t s = ctx->stream;
   const uint8_t* raw = static_cast<const uint8_t*>(file_bytes);
   std::vector<BgzfBlock> blocks;
@@ -520,6 +521,8 @@ extern "C" int mcov_bam_decode_gpu(mcov_ctx* ctx, const void* file_bytes, int64_
   return MCOV_OK;
 }
 
+int mcov_sam_gpu_names_seq(mcov_ctx* ctx, int32_t k_len, int32_t win_bases, uint64_t* d_hash, int32_t* d_kmer, uint8_t* d_win);   // sam_gpu.cu
+
 extern "C" int mcov_bam_gpu_names_seq(mcov_ctx* ctx, int32_t k_len, int32_t win_bases, uint64_t* name_hash_out,
                                       int32_t* kmer_code_out, uint8_t* seq_win_out, int mem_kind) {
   if (!ctx) return MCOV_ERR_ARG;
@@ -541,8 +544,13 @@ extern "C" int mcov_bam_gpu_names_seq(mcov_ctx* ctx, int32_t k_len, int32_t win_
     if (seq_win_out) { CUB(B.win.ensure((size_t)n * W)); d_win = B.win.as<uint8_t>(); }
   }
   CUB(cudaMemsetAsync(B.status.as<int>() + 2, 0, 4, s));
-  MCOV_LAUNCH(ctx, kKBamNamesSeq, (k_bam_names_seq<<<(unsigned)((n + 127) / 128), 128, 0, s>>>(
-      B.data.as<uint8_t>(), B.rec_off.as<uint64_t>(), n, k_len, win_bases, d_hash, d_kmer, d_win, B.status.as<int>())));
+  if (B.sam) {                                                 // a SAM decode: the same outputs from the text
+    const int src = mcov_sam_gpu_names_seq(ctx, k_len, win_bases, d_hash, d_kmer, d_win);
+    if (src) return src;
+  } else {
+    MCOV_LAUNCH(ctx, kKBamNamesSeq, (k_bam_names_seq<<<(unsigned)((n + 127) / 128), 128, 0, s>>>(
+        B.data.as<uint8_t>(), B.rec_off.as<uint64_t>(), n, k_len, win_bases, d_hash, d_kmer, d_win, B.status.as<int>())));
+  }
   CUB(cudaGetLastError());
   int bad = 0;
   CUB(cudaMemcpyAsync(&bad, B.status.as<int>() + 2, 4, cudaMemcpyDeviceToHost, s));
@@ -601,6 +609,7 @@ extern "C" int mcov_bam_gpu_stream_depth(mcov_ctx* ctx, const char* path, int64_
   cudaStream_t s = ctx->stream;
   mcov_ctx::BamDev& B = ctx->bam;
   B.n_rec = -1;                                                   // (the whole-file decode's columns are gone after this)
+  B.sam = false;
   FILE* fh = std::fopen(path, "rb");
   if (!fh) return bfail(ctx, MCOV_ERR_IO, "mcov_bam_gpu_stream_depth: cannot open the file");
   struct Closer { FILE* f; ~Closer() { if (f) std::fclose(f); } } closer{fh};

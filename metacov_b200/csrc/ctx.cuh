@@ -54,6 +54,7 @@ enum KernelId {
   kKExpand = 0, kKScan, kKFusedPrep, kKScanCounts, kKFarScatter,
   kKWindowSums, kKIsizeHist, kKGroupCount, kKSortedStats, kKClear, kKRegionStatsSmall, kKCapReplay, kKUnpack, kKKmerHist, kKRegionStatsWarp,
   kKExpPrep, kKExpEntries, kKExpRegion, kKExpRevsum, kKRegionHist, kKHistFinish, kKRunCount, kKRunOffsets, kKRunWrite, kKRunEnds, kKBgzfInflate, kKBamGuess, kKBamWalkCount, kKBamWalkWrite, kKDeltaUnpack, kKStreamAcc, kKFusedPrepTma, kKFusedTileTma, kKStatsStream, kKBlockUnpack, kKBamNamesSeq,
+  kKSamNlCount, kKSamNlWrite, kKSamFields, kKSamCigar, kKSamNamesSeq, kKMapCounts,
   kKernelCount
 };
 
@@ -128,11 +129,17 @@ struct mcov_ctx {
     // carried into the next batch
     mcov::PinBuf pin[2];
     mcov::DevBuf tail, tail2, c_tid, c_pos, c_flag, c_mapq, c_off, c_cig;
+    // SAM decode (sam_gpu.cu): `data` holds the text; tile newline counts, line ends, per-record field offsets, op counts,
+    // the @SQ name table, CUB scratch
+    mcov::DevBuf sam_tiles, sam_lines, sam_aux, sam_ops, sam_ref, sam_tmp;
     int64_t n_rec = -1;                              // records of the last decode (-1: none)
+    bool sam = false;                                // the last decode read SAM text (names / SEQ come from the text)
     void release() {
       n_rec = -1;
+      sam = false;
       mcov::DevBuf* b[] = {&raw, &blocks, &data, &status, &starts, &segs, &wout, &tid, &pos, &flag, &mapq, &lseq, &isize, &cig_off, &cig,
-                           &rec_off, &name_hash, &kmer, &win, &tail, &tail2, &c_tid, &c_pos, &c_flag, &c_mapq, &c_off, &c_cig};
+                           &rec_off, &name_hash, &kmer, &win, &tail, &tail2, &c_tid, &c_pos, &c_flag, &c_mapq, &c_off, &c_cig,
+                           &sam_tiles, &sam_lines, &sam_aux, &sam_ops, &sam_ref, &sam_tmp};
       for (mcov::DevBuf* x : b) x->release();
       pin[0].release(); pin[1].release();
     }

@@ -1065,7 +1065,8 @@ static const char* kKernelNames[kKernelCount] = {
     "memset_depth", "k_region_stats_small", "k_cap_replay", "k_unpack_reads", "k_kmer_hist", "k_region_stats_warp",
     "k_exp_prep", "k_exp_entries", "k_exp_region", "k_exp_revsum", "k_region_hist", "k_hist_finish", "k_run_count", "k_run_offsets", "k_run_write", "k_run_ends",
     "k_bgzf_inflate", "k_bam_guess", "k_bam_walk_count", "k_bam_walk_write", "k_delta_unpack", "k_stream_accumulate",
-    "k_fused_prep_tma", "k_fused_tile_tma", "k_stats_stream", "k_block_unpack", "k_bam_names_seq"};
+    "k_fused_prep_tma", "k_fused_tile_tma", "k_stats_stream", "k_block_unpack", "k_bam_names_seq",
+    "k_sam_nl_count", "k_sam_nl_write", "k_sam_fields", "k_sam_cigar", "k_sam_names_seq", "k_dev_map_counts"};
 
 int mcov_copy_to_host(mcov_ctx* ctx, const void* dev, void* host, int64_t n_bytes) {
   if (!ctx) return MCOV_ERR_ARG;
