@@ -111,6 +111,18 @@ void mcov_default_filter(mcov_filter* f);
 /* Start a new pass: clears the difference array and all counters. */
 int  mcov_begin(mcov_ctx* ctx);
 
+/* mcov_begin with flags.  MCOV_BEGIN_EXACT_CAP: the pass also counts, per
+ * slot, the passing reads that start there (an int32 array the size of the
+ * depth store, allocated on first use), and mcov_finalize reports the exact
+ * cap_metric max_p depth[p-1]+starts[p] within each contig (depth[-1] = 0) --
+ * the value the fused path reports for the same reads, whatever their order:
+ * when it does not exceed max_depth, htslib's cap cannot fire.  Without a cap
+ * (max_depth <= 0) nothing is counted, and with count_del = 0 cap_metric stays
+ * the upper bound of mcov_begin -- also when mcov_set_filter switches to either
+ * inside the pass (the starts would miss the reads pushed after it). */
+#define MCOV_BEGIN_EXACT_CAP 1
+int  mcov_begin_ex(mcov_ctx* ctx, int flags);
+
 /* Replaces the per-record work of htslib's pileup engine behind
  * `bam.pileup()` (reference metacov/pileup.py:13): filter each record, reduce
  * its CIGAR to a reference length, and add +1 @ pos / -1 @ pos+reflen to the
@@ -389,8 +401,9 @@ typedef struct mcov_pass_info {
   int64_t n_pass;         /* records that passed the filter with reflen > 0   */
   int64_t aligned_bases;  /* sum of reflen over passing reads (unclipped)     */
   int32_t max_depth_seen; /* max depth over all contigs (before the cap)      */
-  int32_t cap_metric;     /* max_p depth[p-1]+starts[p] (fused path) or an
-                             upper bound of it (push path)                    */
+  int32_t cap_metric;     /* max_p depth[p-1]+starts[p] (fused path, and
+                             push passes begun with MCOV_BEGIN_EXACT_CAP) or
+                             an upper bound of it (other push passes)         */
   int32_t sorted;         /* 1 if the input was coordinate-sorted             */
   int32_t cap_contigs;    /* contigs whose depth was replayed under the max_depth
                              cap (fused path; 0 = the cap never fired)        */
@@ -634,6 +647,29 @@ int  mcov_bam_decode_gpu_file(mcov_ctx* ctx, const char* path, int verify_crc, m
  * context, like those of mcov_bam_decode_gpu.  Synchronises. */
 int  mcov_sam_decode_gpu(mcov_ctx* ctx, const void* bytes, int64_t n_bytes, int64_t chunk_bytes, mcov_bam_dev* out);
 int  mcov_sam_decode_gpu_file(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, mcov_bam_dev* out);
+/* SAM text that arrives in pieces (a pipe, stdin), decoded a chunk of whole
+ * lines at a time into the same columns.  mcov_sam_chunk_begin takes the
+ * header -- every '@' line in front of the first record and nothing else --,
+ * validates it like mcov_sam_decode_gpu, uploads the @SQ table and starts the
+ * line count; n_ref (optional) receives the number of @SQ lines.
+ * mcov_sam_chunk_decode parses every complete line of bytes[0, n) (through
+ * its last LF; everything when `last` is set, the final line may then lack its
+ * LF) and sets *consumed to the bytes it parsed: the caller keeps the rest in
+ * front of its next piece.  *consumed == 0 without `last` means the piece held
+ * no complete line.  The columns of `out` describe this chunk only (indices
+ * local to it, header_bytes 0) and stay valid until the next decode on the
+ * context, as do mcov_bam_gpu_names_seq and mcov_bam_gpu_mapped, which serve
+ * this chunk.  A malformed line is MCOV_ERR_IO naming its 1-based line number
+ * in the whole stream (header lines and the lines of earlier chunks
+ * included); a '@' line after the header is such an error.  Synchronises: the
+ * caller may reuse `bytes` when the call returns. */
+int  mcov_sam_chunk_begin(mcov_ctx* ctx, const void* header_bytes, int64_t n, int32_t* n_ref);
+int  mcov_sam_chunk_decode(mcov_ctx* ctx, const void* bytes, int64_t n, int last, int64_t* consumed, mcov_bam_dev* out);
+/* The longest line of the stream begun by mcov_sam_chunk_begin, over the chunks
+ * decoded so far: its bytes with the LF (a last line without an LF: to the end
+ * of the stream); counted on the device from each chunk's line index.  -1
+ * without a chunked decode. */
+int64_t mcov_sam_chunk_longest_line(const mcov_ctx* ctx);
 /* pysam's `mapped` / `unmapped` of the file last decoded on this context (BAM or
  * SAM), counted on the device from its columns with the BAI metadata
  * definitions: mapped = records with tid >= 0 and without flag 0x4, unmapped =

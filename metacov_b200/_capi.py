@@ -20,6 +20,7 @@ MCOV_ERR_NOMEM = -4
 MCOV_ERR_IO = -5
 MCOV_ERR_RANGE = -6
 MCOV_ERR_UNSORTED = -7
+MCOV_BEGIN_EXACT_CAP = 1     # mcov_begin_ex: the any-order pass reports the exact cap metric
 MEM_HOST = 0
 MEM_DEVICE = 1
 
@@ -124,6 +125,7 @@ SIGNATURES = {
     "mcov_set_filter": (C.c_int, [_vp, C.POINTER(Filter)]),
     "mcov_default_filter": (None, [C.POINTER(Filter)]),
     "mcov_begin": (C.c_int, [_vp]),
+    "mcov_begin_ex": (C.c_int, [_vp, C.c_int]),
     "mcov_push_reads": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int]),
     "mcov_finalize": (C.c_int, [_vp]),
     "mcov_depth_sorted": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int]),
@@ -152,6 +154,9 @@ SIGNATURES = {
     "mcov_bam_gpu_stream_depth": (C.c_int, [_vp, C.c_char_p, _i64, C.c_int, _vp]),
     "mcov_sam_decode_gpu": (C.c_int, [_vp, _vp, C.c_int64, C.c_int64, _vp]),
     "mcov_sam_decode_gpu_file": (C.c_int, [_vp, C.c_char_p, C.c_int64, _vp]),
+    "mcov_sam_chunk_begin": (C.c_int, [_vp, _vp, C.c_int64, C.POINTER(_i32)]),
+    "mcov_sam_chunk_decode": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, C.POINTER(_i64), _vp]),
+    "mcov_sam_chunk_longest_line": (_i64, [_vp]),
     "mcov_bam_gpu_mapped": (C.c_int, [_vp, C.POINTER(_i64), C.POINTER(_i64)]),
     "mcov_sam_parse_host": (C.c_int, [_vp, C.c_int64, C.POINTER(SamHostCols), C.c_char_p, C.c_int]),
     "mcov_inflate_host": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint32]),

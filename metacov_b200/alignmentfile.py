@@ -13,7 +13,7 @@ import os
 
 import numpy as np
 
-from . import _capi
+from . import _capi, samstream
 from ._capi import McovError, lib
 from .engine import CoverageEngine, ReadBatch
 
@@ -170,11 +170,26 @@ class AlignmentFile:
 
         The format comes from the content (``is_sam_text``).  SAM text is always parsed whole on the device
         (csrc/sam_gpu.cu): "host", "gpu" and "auto" all do that and ``decode`` reads "gpu"; "gpu-stream" is refused, and a
-        file whose decode does not fit the free device memory raises OSError."""
+        file whose decode does not fit the free device memory raises OSError.
+
+        A stream -- "-" (standard input), a binary file object, or a path that is not a regular file (a FIFO, the
+        /dev/fd/N of a pipe) -- is read once, as SAM text, in chunks of whole lines (``gpu_chunk_bytes``, default 64 MiB):
+        ``piped`` is True and ``decode`` reads "gpu-stream".  Its header is read by the constructor.  The first consumer
+        reads the records: the depth (``coverage_engine`` and everything built on it, ``mapped`` / ``unmapped``
+        included) or ``scan_reads``; the other kind, and the accessors that need every record (``soa``, ``len``, read
+        names, SEQ), raise ValueError.  Gzip data on a stream (BAM) raises OSError: BAM is read from a file path.
+        ``mapped`` / ``unmapped`` of a stream count the records read: all of them after the depth pass, and after a
+        ``scan_reads`` that ``maxreads`` stopped, every record of the chunks read up to that point.  The host buffers are
+        pageable; ``pinned_buffers=True`` makes them page-locked (tools/bench_pipe.py compares the two)."""
         if "w" in mode:
             raise ValueError("metacov_b200.AlignmentFile is read-only")
         if decode not in ("host", "gpu", "gpu-stream", "auto"):
             raise ValueError("decode must be 'host', 'gpu', 'gpu-stream' or 'auto'")
+        self.piped = False
+        self._pipe = None
+        if samstream.is_stream(filename):
+            self._open_pipe(filename, device, kw)
+            return
         self.format = "sam" if is_sam_text(filename) else "bam"
         if self.format == "sam":
             if decode == "gpu-stream":
@@ -206,6 +221,130 @@ class AlignmentFile:
         self.references, self.lengths, self.text = self._stream.references, self._stream.lengths, self._stream.text
         self.nreferences = len(self.references)
         self._tid = {name: i for i, name in enumerate(self.references)}
+
+    def _open_pipe(self, source, device, kw):
+        """A stream: the header now, the records by the first consumer (``_pipe_pass``)."""
+        src, head, rest, owned = samstream.open_stream(source)
+        self.format = "sam"
+        self.piped = True
+        self.decode = "gpu-stream"
+        self.filename = source if isinstance(source, str) else getattr(source, "name", "<stream>")
+        self._device = device
+        self._gpu_chunk_bytes = int(kw.get("gpu_chunk_bytes", 64 << 20))
+        self.gpu_stream_info = None
+        self.pipe_info = None
+        self.stream_batches = 0
+        self._gpu = self._soa = self._engine = self._filter_kw = self._index_stats = None
+        self._h = self._stream = None
+        self._pipe_consumer = None
+        self._pipe_read = False
+        self._pipe_reader = None
+        self._pipe_pinned = bool(kw.get("pinned_buffers", False))
+        self.text = head.decode()
+        refs = samstream.header_refs(self.text)
+        eng = CoverageEngine([1], device=device)
+        try:
+            n_ref = C.c_int32(0)
+            keep = np.frombuffer(head, dtype=np.uint8) if head else None
+            rc = lib.mcov_sam_chunk_begin(eng._ctx, keep.ctypes.data if keep is not None else None, len(head), C.byref(n_ref))
+            if rc != 0:
+                raise OSError("%s: %s" % (self.filename, lib.mcov_last_error(eng._ctx).decode()))
+        except BaseException:
+            eng.close()
+            if owned is not None:
+                owned.close()
+            raise
+        self.references = tuple(r for r, _ in refs)
+        self.lengths = tuple(l for _, l in refs)
+        self.nreferences = len(refs)
+        self._tid = {name: i for i, name in enumerate(self.references)}
+        if self.lengths:
+            eng.set_contigs(self.lengths)
+        self._pipe_eng = eng
+        self._pipe = (src, rest, owned)
+
+    def _pipe_claim(self, consumer):
+        """The stream goes to its first consumer; a second kind of consumer cannot have it."""
+        if self._pipe_consumer is None:
+            self._pipe_consumer = consumer
+        elif self._pipe_consumer != consumer:
+            raise ValueError("%s: a piped SAM stream is read once, and it has been read by %s; %s needs the records again "
+                             "(write the stream to a file to use both)" % (self.filename, self._pipe_consumer, consumer))
+
+    def _no_records(self, what):
+        if self.piped:
+            raise ValueError("%s: %s needs every record, and a piped SAM stream is read once by the depth pass or "
+                             "scan_reads without keeping its records (write it to a file instead)" % (self.filename, what))
+
+    def _pipe_pass(self, per_chunk, stop_after=0):
+        """Read the stream: every chunk is decoded on the device (``mcov_sam_chunk_decode``) and ``per_chunk(dsoa, n)``
+        sees its columns (n: the records of the chunk to use; ``stop_after`` > 0 ends the read after that many records).
+        Counts records and mapped / unmapped (BAI definitions) of the chunks read."""
+        from . import bamgpu
+        if self._pipe_read:
+            raise ValueError("%s: the piped SAM stream has been read already (by a pass that did not complete)" % self.filename)
+        self._pipe_read = True
+        src, rest, _owned = self._pipe
+        eng = self._pipe_eng
+        reader = samstream.ChunkReader(src, rest, self._gpu_chunk_bytes, pinned=self._pipe_pinned)
+        self._pipe_reader = reader
+        tot = {"records": 0, "mapped": 0, "unmapped": 0}
+
+        def decode(view, last):
+            raw, used = _capi.BamDev(), C.c_int64(0)
+            a = np.frombuffer(view, dtype=np.uint8)
+            try:
+                rc = lib.mcov_sam_chunk_decode(eng._ctx, a.ctypes.data if len(a) else None, len(a), 1 if last else 0,
+                                               C.byref(used), C.byref(raw))
+            finally:
+                del a
+            if rc != 0:
+                raise OSError("%s: %s" % (self.filename, lib.mcov_last_error(eng._ctx).decode()))
+            assert used.value == len(view), (used.value, len(view))
+            if raw.n_records == 0:
+                return True
+            dsoa = bamgpu.DeviceSoA(eng, raw, "sam")
+            n = raw.n_records
+            if stop_after:
+                n = min(n, stop_after - tot["records"])
+            per_chunk(dsoa, n)
+            m, u = dsoa.mapped_counts()
+            tot["records"] += raw.n_records
+            tot["mapped"] += m
+            tot["unmapped"] += u
+            return not (stop_after and tot["records"] >= stop_after)
+
+        reader.run(decode)
+        self._index_stats = (tot["mapped"], tot["unmapped"])
+        self.pipe_info = dict(records=tot["records"], longest_line=int(lib.mcov_sam_chunk_longest_line(eng._ctx)),
+                              **reader.info())
+        self.stream_batches = reader.chunks
+        return tot["records"]
+
+    def _pipe_depth(self):
+        """The depth of a stream: one any-order pass with the exact cap verdict (``mcov_begin_ex``)."""
+        self._pipe_claim("the depth pass")
+        eng = self._pipe_eng
+        if self._filter_kw:
+            eng.set_filter(**self._filter_kw)
+        eng.begin(exact_cap=True)
+
+        def push(dsoa, n):
+            r = dsoa.raw
+            eng._check(lib.mcov_push_reads(eng._ctx, n, r.tid, r.pos, r.flag, r.mapq, r.cig_off, r.cig, _capi.MEM_DEVICE))
+
+        self._pipe_pass(push)
+        eng.finalize()
+        info = eng.pass_info()
+        md = eng.filter.max_depth
+        if md > 0 and info["cap_metric"] > md:
+            from .pileup import DepthCapError
+            raise DepthCapError(
+                "%s: depth[p-1]+starts[p] reaches %d > max_depth=%d: htslib's pileup would drop reads here, and a piped "
+                "stream cannot be read again to replay its cap; write the input to a coordinate-sorted file instead, or "
+                "raise max_depth via set_pileup_filter(max_depth=...) before the first use" % (self.filename, info["cap_metric"], md))
+        self._engine = eng
+        return eng
 
     # device bytes per byte of BAM that a GPU decode needs: the image itself, the inflated stream (BAM records deflate
     # ~4-5x), the SoA columns, and as much again for the depth arrays and scratch of the pass that follows
@@ -290,6 +429,17 @@ class AlignmentFile:
 
     # -- lifetime ---------------------------------------------------------
     def close(self):
+        if getattr(self, "_pipe", None) is not None:
+            if self._engine is self._pipe_eng:
+                self._engine = None
+            self._pipe_eng.close()
+            owned = self._pipe[2]
+            if owned is not None:
+                if self._pipe_reader is not None:
+                    self._pipe_reader.release(owned.close)   # (after an early stop: once the reader thread is out)
+                else:
+                    owned.close()
+            self._pipe = None
         if getattr(self, "_engine", None) is not None:
             self._engine.close()
             self._engine = None
@@ -321,6 +471,8 @@ class AlignmentFile:
         return self.references[tid]
 
     def _idx(self):
+        if self._index_stats is None and self.piped:
+            self.coverage_engine()                          # (counted while the stream is read)
         if self._index_stats is None and self.format == "sam":
             self._index_stats = self._gpu[1].mapped_counts()      # (SAM has no index: counted from the decoded columns)
         if self._index_stats is None:
@@ -352,6 +504,7 @@ class AlignmentFile:
     def soa(self):
         """Every record of the file as SoA numpy views (file order; the arrays
         the reference reads field by field at scan.pyx:243-294)."""
+        self._no_records("soa()")
         if self._soa is None and self._gpu is not None:
             self._soa = {c: self._gpu[1].to_host(c) for c, _ in self._gpu[1].COLS}
         if self._soa is None:
@@ -376,6 +529,7 @@ class AlignmentFile:
     def seq_windows(self, win_bases):
         """uint8[n, (win_bases+1)//2]: per read the first (forward) / last (reverse) win_bases bases,
         nt16 two per byte -- the part of SEQ the k-mer histogram looks at."""
+        self._no_records("seq_windows()")
         if self._gpu is not None:                       # decoded on the GPU: SEQ is read there too
             return self._gpu[1].names_seq(win_bases=win_bases)["seq_win"]
         n = len(self.soa()["tid"])
@@ -389,11 +543,13 @@ class AlignmentFile:
         return out
 
     def __len__(self):
+        self._no_records("len()")
         return len(self.soa()["tid"])
 
     # -- pileup.experimental ------------------------------------------------
     def name_hashes(self):
         """uint64[n]: FNV-1a of every read name (the key of the reference's mate dict, pileup.py:101)."""
+        self._no_records("name_hashes()")
         if self._gpu is not None:
             return self._gpu[1].names_seq(name_hash=True)["name_hash"]
         n = len(self.soa()["tid"])
@@ -404,6 +560,7 @@ class AlignmentFile:
 
     def qas_kmer_codes(self, k_len):
         """int32[n]: code of ``read.query_alignment_sequence[0:k_len]`` (pileup.py:109, 123), -1 = no key."""
+        self._no_records("qas_kmer_codes()")
         if self._gpu is not None:
             return self._gpu[1].names_seq(k_len=k_len)["kmer_code"]
         n = len(self.soa()["tid"])
@@ -436,6 +593,7 @@ class AlignmentFile:
 
     def experimental_stats(self, refs, starts, ends, k_len, kc_val, kc_has):
         """``mcov_exp_stats`` records of the regions (the read loop of pileup.py:90-146 on the GPU)."""
+        self._no_records("experimental_stats()")
         s = self.soa()
         cstart, max_span = self._fetch_index()
         pos = s["pos"]
@@ -474,7 +632,11 @@ class AlignmentFile:
     # -- coverage ---------------------------------------------------------
     def set_pileup_filter(self, **kw):
         """Override pysam's implicit pileup arguments (flag_filter, flag_require,
-        min_mapq, ignore_orphans, max_depth); invalidates the cached depth."""
+        min_mapq, ignore_orphans, max_depth); invalidates the cached depth.  A piped stream takes it before its
+        records are read only."""
+        if self.piped and self._pipe_consumer is not None:
+            raise ValueError("%s: set_pileup_filter after the piped stream has been read: its depth cannot be computed "
+                             "again; set the filter before the first use" % self.filename)
         self._filter_kw = kw
         if self._engine is not None:
             if self._gpu is None:
@@ -483,6 +645,8 @@ class AlignmentFile:
 
     def coverage_engine(self):
         """The per-base depth of the whole file, computed once on the GPU."""
+        if self.piped:
+            return self._engine if self._engine is not None else self._pipe_depth()
         if self._engine is None and self._gpu is not None:
             eng, path = self._gpu_depth()
         elif self._engine is None and self._soa is None:

@@ -18,6 +18,7 @@ from . import pileup as _pileup
 from . import scan as _scan
 from . import util
 from .alignmentfile import AlignmentFile
+from .samstream import is_stream
 from .fasta import FastaFile
 
 logging.basicConfig(level=logging.INFO, format="[%(relativeCreated)6.1f %(funcName)s]  %(message)s",
@@ -35,7 +36,8 @@ def main():
 
 @main.command()
 @click.option("--bamfile", "-b", type=click.File("rb"), required=True,
-              help="Input BAM (sorted, indexed) or SAM file.")
+              help="Input BAM (sorted, indexed) or SAM file; '-' or a pipe (e.g. <(minimap2 -a ...)) reads SAM text as it "
+                   "is written, in any read order.")
 @click.option("--reference-fasta", "-f", type=click.File("rb"))
 @click.option("--regionfile-blast7", "-rb", type=click.File("r"), help="Input Region file in BLAST7 format")
 @click.option("--regionfile-csv", "-rc", type=click.File("r"), help="Input Region file in CSV format")
@@ -59,7 +61,11 @@ def pileup(bamfile, reference_fasta, regionfile_blast7, regionfile_csv, kmer_his
     """
     if (window is None) != (window_out is None):
         raise click.UsageError("--window and --window-out go together")
-    bam = AlignmentFile(bamfile.name, decode=bam_decode)
+    source = "-" if _is_stdin(bamfile) else bamfile.name
+    if kmer_histogram and is_stream(source):
+        raise click.UsageError("-k/--kmer-histogram (the experimental model) fetches reads per region, which a piped "
+                               "stream cannot give; write the alignments to a sorted file for it")
+    bam = AlignmentFile(source, decode=bam_decode)
     fasta = FastaFile(reference_fasta.name) if reference_fasta else None          # cli.py:59
     regions = util.make_region_iterator(regionfile_blast7, regionfile_csv, bam)
     try:
@@ -101,6 +107,12 @@ def pileup(bamfile, reference_fasta, regionfile_blast7, regionfile_csv, kmer_his
     if window is not None:
         write_windows(bam, window, window_out)
     bam.close()
+
+
+def _is_stdin(f):
+    """click.File gives standard input for '-' (named "<stdin>", or unnamed under a test runner)."""
+    name = getattr(f, "name", None)
+    return not isinstance(name, str) or name in ("<stdin>", "-")
 
 
 def write_bedgraph(bam, out):
@@ -158,12 +170,14 @@ def write_windows(bam, window, out):
               help="Where the BAM file is inflated and parsed (see `pileup`); with the GPU the accumulators run on the "
                    "device-resident columns. Applies to BAM only: SAM text is always parsed on the GPU. Not in the "
                    "reference: additive.")
-@click.argument("readfile", nargs=-1, required=True)
+@click.argument("readfile", nargs=-1, required=True, metavar="READFILE...  ('-' or a pipe: SAM text as it is written)")
 def scan(readfile, readfile_type, out_basehist, boffset, out_kmerhist, k, number, step, offset, max_reads,
          reference_fasta, out_mirrorhist, mirror_offset, mirror_length, out_isizehist, group_by, bam_decode="auto"):
     """
     Gather read statistics
     """
+    if not readfile_type and is_stream(readfile[0]):
+        readfile_type = "bam"                           # (a stream is read as SAM text)
     if not readfile_type:
         for ext, ft in ((".bam", "bam"), (".sam", "bam"), (".fq", "fq"), (".fq.gz", "fq"), (".fastq", "fq"),
                         (".fastq.gz", "fq")):
@@ -190,9 +204,12 @@ def scan(readfile, readfile_type, out_basehist, boffset, out_kmerhist, k, number
         update_every = int(max_reads + 50 / 100)        # sic (reference cli.py:205-206)
 
     infile = AlignmentFile(readfile[0], decode=bam_decode)
-    log.info("mapped = {}, unmapped = {}, total = {}".format(infile.mapped, infile.unmapped,
-                                                             infile.mapped + infile.unmapped))
-    length = infile.mapped + infile.unmapped
+    if infile.piped:
+        length = max_reads or 0                         # (the counts of a stream are known once it has been read)
+    else:
+        log.info("mapped = {}, unmapped = {}, total = {}".format(infile.mapped, infile.unmapped,
+                                                                 infile.mapped + infile.unmapped))
+        length = infile.mapped + infile.unmapped
     if max_reads and 0 < max_reads < length:
         length = max_reads
 
@@ -207,6 +224,9 @@ def scan(readfile, readfile_type, out_basehist, boffset, out_kmerhist, k, number
         with infile:
             nreads = _scan.scan_reads(infile, None, counters, update_every, lambda: bar.update(update_every),
                                       max_reads)
+            if infile.piped:
+                log.info("mapped = {}, unmapped = {}, total = {}".format(infile.mapped, infile.unmapped,
+                                                                         infile.mapped + infile.unmapped))
         bar.update(update_every)
     log.info("Processed {} reads".format(nreads))
 

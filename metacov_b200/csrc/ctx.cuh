@@ -55,6 +55,7 @@ enum KernelId {
   kKWindowSums, kKIsizeHist, kKGroupCount, kKSortedStats, kKClear, kKRegionStatsSmall, kKCapReplay, kKUnpack, kKKmerHist, kKRegionStatsWarp,
   kKExpPrep, kKExpEntries, kKExpRegion, kKExpRevsum, kKRegionHist, kKHistFinish, kKRunCount, kKRunOffsets, kKRunWrite, kKRunEnds, kKBgzfInflate, kKBamGuess, kKBamWalkCount, kKBamWalkWrite, kKDeltaUnpack, kKStreamAcc, kKFusedPrepTma, kKFusedTileTma, kKStatsStream, kKBlockUnpack, kKBamNamesSeq,
   kKSamNlCount, kKSamNlWrite, kKSamFields, kKSamCigar, kKSamNamesSeq, kKMapCounts,
+  kKCapExact, kKSamLineMax,
   kKernelCount
 };
 
@@ -115,6 +116,8 @@ struct mcov_ctx {
   int stage_next = 0;
   int64_t n_reads_pushed = 0;
   bool verdict_pending = false;   // an asynchronous fused pass has not been checked for sortedness yet
+  bool exact_cap = false;         // the any-order pass counts starts for the exact cap metric (mcov_begin_ex)
+  mcov::DevBuf d_starts;          // [n_slots] passing reads that start at each slot (exact_cap passes)
   int64_t contig_epoch = 0;
   mcov::RegionPlan plan;
   int32_t cap_contigs = 0;        // contigs replayed under htslib's max_depth cap in the last fused pass
@@ -134,6 +137,12 @@ struct mcov_ctx {
     mcov::DevBuf sam_tiles, sam_lines, sam_aux, sam_ops, sam_ref, sam_tmp;
     int64_t n_rec = -1;                              // records of the last decode (-1: none)
     bool sam = false;                                // the last decode read SAM text (names / SEQ come from the text)
+    uint32_t sam_ref_mask = 0;                       // the @SQ table in sam_ref: slot mask, bytes of slots / name offsets, names
+    size_t sam_tab_bytes = 0, sam_off_bytes = 0;
+    int32_t sam_n_ref = 0;
+    bool sam_chunked = false;                        // a chunked SAM decode has begun (mcov_sam_chunk_begin)
+    int64_t sam_line0 = 0;                           // lines of that stream in front of the next chunk
+    int64_t sam_longest = 0;                         // its longest line so far (LF included)
     void release() {
       n_rec = -1;
       sam = false;

@@ -82,7 +82,10 @@ struct FusedArgs {
   uint32_t* far_sorted;       // [far_cap] in-tile offsets bucketed by tile
   uint32_t* tile_first;       // [n_tiles+1] (a fused batch holds < 2^32 reads)
   int32_t* depth;
-  int32_t* tile_cap;          // [n_tiles] max of depth[p-1]+starts[p] in the tile, written only when > max_depth
+  union {                     // (one slot: the fused path and the push path never need both, and the layout stays)
+    int32_t* tile_cap;        // fused: [n_tiles] max of depth[p-1]+starts[p] in the tile, written only when > max_depth
+    int32_t* starts;          // push (k_expand<., true>): [n_slots] passing reads that start at each slot
+  };
   uint16_t* tile_hist;        // [n_tiles][kTileHistWords] depth histograms of the tiles (k_tile_tma.cuh), nullptr: not written
   uint32_t* tile_heavy;       // [n_tiles] ids of the tiles with >= heavy_min reads (k_far_scatter; pc->n_heavy of them)
   uint32_t heavy_min;
@@ -421,7 +424,9 @@ __device__ __forceinline__ void prep_flush_counters(PassCounters* pc, uint32_t n
 
 // K1 of the push path (any read order): filter + CIGAR reduce + difference-array deltas, see
 // k_expand.cuh.  Shares prep_load_reduce with the fused path (only f.e and f.vec_ok are read).
-template <bool OFF64>
+// STARTS: also count the passing reads that start at each slot (starts[slot] += 1), for the exact cap metric of
+// mcov_begin_ex(MCOV_BEGIN_EXACT_CAP) into f.starts -- the same reads the fused path's tile kernel counts as starts.
+template <bool OFF64, bool STARTS>
 __global__ void __launch_bounds__(kPrepThreads, 4)
 k_expand(const __grid_constant__ FusedArgs f) {
   const ExpandArgs& a = f.e;
@@ -469,6 +474,7 @@ k_expand(const __grid_constant__ FusedArgs f) {
         if (e > s) {                                          // reflen == 0 or entirely outside the contig: nothing
           atomicAdd(delta + c_base + s, 1);
           atomicAdd(delta + c_base + e, -1);
+          if (STARTS) atomicAdd(f.starts + c_base + s, 1);
           n_pass += 1;
           aligned += R.reflen[r];
         }
@@ -476,6 +482,30 @@ k_expand(const __grid_constant__ FusedArgs f) {
     }
   }
   prep_flush_counters(a.pc, n_pass, aligned, unsorted, 0u);
+}
+
+// The exact cap metric of an any-order pass, after the scan: max_p depth[p-1] + starts[p] over the slot space.  Every
+// contig ends in a sentinel slot of depth 0 that no read starts at, so the maximum over the concatenation is the maximum
+// within each contig with depth[-1] = 0.  Four slots per thread and step, 128-bit loads of both arrays.
+__global__ void __launch_bounds__(256)
+k_cap_exact(const int32_t* __restrict__ depth, const int32_t* __restrict__ starts, int64_t n_slots, PassCounters* pc) {
+  const int64_t n_vec = n_slots >> 2;                            // (n_slots is a multiple of 4)
+  int m = 0;
+  for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n_vec; k += (int64_t)gridDim.x * blockDim.x) {
+    const int4 d = __ldg(reinterpret_cast<const int4*>(depth) + k);
+    const int4 s = __ldg(reinterpret_cast<const int4*>(starts) + k);
+    const int prev = k ? __ldg(depth + 4 * k - 1) : 0;
+    m = max(m, max(max(prev + s.x, d.x + s.y), max(d.y + s.z, d.z + s.w)));
+  }
+  m = warp_max(m);
+  __shared__ int s_m[8];
+  if ((threadIdx.x & 31) == 0) s_m[threadIdx.x >> 5] = m;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int b = 0;
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) b = max(b, s_m[w]);
+    if (b > 0) atomicMax(&pc->cap_metric, b);
+  }
 }
 
 // Per-warp state of a prep kernel: pass counters and the constants of the warp's current contig

@@ -604,7 +604,8 @@ void mcov_destroy(mcov_ctx* ctx) {
                     &ctx->d_start_slot, &ctx->d_far_list, &ctx->d_tile_cnt, &ctx->d_tile_off, &ctx->d_far_sorted, &ctx->d_tile_hist,
                     &ctx->d_tasks, &ctx->d_rlen, &ctx->d_done,
                     &ctx->d_cap_scratch, &ctx->d_flag_lut, &ctx->d_stream_acc, &ctx->d_ss_pieces, &ctx->d_ss_cta, &ctx->d_ss_split, &ctx->d_ss_pool,
-                    &ctx->d_out, &ctx->d_win_slot, &ctx->d_win_n, &ctx->d_win_out, &ctx->d_htasks, &ctx->d_tile_heavy, &ctx->d_run_tasks, &ctx->d_run_counts, &ctx->d_run_out};
+                    &ctx->d_out, &ctx->d_win_slot, &ctx->d_win_n, &ctx->d_win_out, &ctx->d_htasks, &ctx->d_tile_heavy, &ctx->d_run_tasks, &ctx->d_run_counts, &ctx->d_run_out,
+                    &ctx->d_starts};
   for (DevBuf* b : bufs) b->release();
   ctx->bam.release();
   ctx->h_pin.release();
@@ -746,19 +747,28 @@ int mcov_depth_sorted_delta(mcov_ctx* ctx, int64_t n, const int64_t* contig_read
   return run_sorted_pass(ctx, columns_of(ctx, st, n, n_cig_total), &st, n, true, wait != 0, "mcov_depth_sorted_delta");
 }
 
-int mcov_begin(mcov_ctx* ctx) {
+int mcov_begin_ex(mcov_ctx* ctx, int flags) {
   if (!ctx) return MCOV_ERR_ARG;
+  if (flags & ~MCOV_BEGIN_EXACT_CAP) return fail(ctx, MCOV_ERR_ARG, "mcov_begin_ex: unknown flags");
   CU(cudaSetDevice(ctx->device));
   int rc = ensure_depth(ctx);
   if (rc) return rc;
   MCOV_LAUNCH(ctx, kKClear, CU(cudaMemsetAsync(ctx->depth, 0, (size_t)ctx->n_slots * 4, ctx->stream)));
   CU(cudaMemsetAsync(ctx->d_pc.p, 0, sizeof(PassCounters), ctx->stream));
+  // the starts array of the exact cap metric: only where a cap exists and k_expand counts (count_del = 0 keeps the bound)
+  ctx->exact_cap = (flags & MCOV_BEGIN_EXACT_CAP) && ctx->filt.max_depth > 0 && ctx->filt.count_del;
+  if (ctx->exact_cap) {
+    CU(ctx->d_starts.ensure((size_t)ctx->n_slots * 4));
+    MCOV_LAUNCH(ctx, kKClear, CU(cudaMemsetAsync(ctx->d_starts.p, 0, (size_t)ctx->n_slots * 4, ctx->stream)));
+  }
   ctx->n_reads_pushed = 0;
   ctx->verdict_pending = false;
   ctx->tile_hist_valid = false;
   ctx->state = kAccumulating;
   return MCOV_OK;
 }
+
+int mcov_begin(mcov_ctx* ctx) { return mcov_begin_ex(ctx, 0); }
 
 static int push_reads_impl(mcov_ctx* ctx, int64_t n, const int32_t* tid, const int32_t* pos, const uint16_t* flag,
                            const uint8_t* mapq, const void* cig_off, bool off64, const uint32_t* cig, int mem_kind) {
@@ -778,9 +788,16 @@ static int push_reads_impl(mcov_ctx* ctx, int64_t n, const int32_t* tid, const i
   f.e = a;
   f.vec_ok = vec_ok(a);
   const int grid = grid_for(ctx, (n + kPrepPer - 1) / kPrepPer, kPrepThreads, 8);
+  // a filter changed inside the pass so that starts are no longer counted (count_del = 0, or no cap): the pass keeps the
+  // scan's bound rather than report a metric over starts that miss these reads
+  if (ctx->exact_cap && (!ctx->filt.count_del || ctx->filt.max_depth <= 0)) ctx->exact_cap = false;
   if (!ctx->filt.count_del) MCOV_LAUNCH(ctx, kKExpand, (k_expand_runs<<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(f, 0)));
-  else if (off64) MCOV_LAUNCH(ctx, kKExpand, (k_expand<true><<<grid, kPrepThreads, 0, ctx->stream>>>(f)));
-  else MCOV_LAUNCH(ctx, kKExpand, (k_expand<false><<<grid, kPrepThreads, 0, ctx->stream>>>(f)));
+  else if (ctx->exact_cap) {
+    f.starts = ctx->d_starts.as<int32_t>();
+    if (off64) MCOV_LAUNCH(ctx, kKExpand, (k_expand<true, true><<<grid, kPrepThreads, 0, ctx->stream>>>(f)));
+    else MCOV_LAUNCH(ctx, kKExpand, (k_expand<false, true><<<grid, kPrepThreads, 0, ctx->stream>>>(f)));
+  } else if (off64) MCOV_LAUNCH(ctx, kKExpand, (k_expand<true, false><<<grid, kPrepThreads, 0, ctx->stream>>>(f)));
+  else MCOV_LAUNCH(ctx, kKExpand, (k_expand<false, false><<<grid, kPrepThreads, 0, ctx->stream>>>(f)));
   CU(cudaGetLastError());
   ctx->n_reads_pushed += n;
   return finish_stage(ctx, st);
@@ -803,6 +820,12 @@ int mcov_finalize(mcov_ctx* ctx) {
   ctx->tile_hist_valid = false;
   int rc = scan_depth(ctx);
   if (rc) return rc;
+  if (ctx->exact_cap) {                  // the scan's bound is replaced by the exact value
+    CU(cudaMemsetAsync(&pc_of(ctx)->cap_metric, 0, sizeof(int), ctx->stream));
+    MCOV_LAUNCH(ctx, kKCapExact, (k_cap_exact<<<grid_for(ctx, ctx->n_slots / 4, 256, 8), 256, 0, ctx->stream>>>(
+        ctx->depth, ctx->d_starts.as<int32_t>(), ctx->n_slots, pc_of(ctx))));
+    CU(cudaGetLastError());
+  }
   ctx->state = kDepthReady;
   return MCOV_OK;
 }
@@ -1066,7 +1089,8 @@ static const char* kKernelNames[kKernelCount] = {
     "k_exp_prep", "k_exp_entries", "k_exp_region", "k_exp_revsum", "k_region_hist", "k_hist_finish", "k_run_count", "k_run_offsets", "k_run_write", "k_run_ends",
     "k_bgzf_inflate", "k_bam_guess", "k_bam_walk_count", "k_bam_walk_write", "k_delta_unpack", "k_stream_accumulate",
     "k_fused_prep_tma", "k_fused_tile_tma", "k_stats_stream", "k_block_unpack", "k_bam_names_seq",
-    "k_sam_nl_count", "k_sam_nl_write", "k_sam_fields", "k_sam_cigar", "k_sam_names_seq", "k_dev_map_counts"};
+    "k_sam_nl_count", "k_sam_nl_write", "k_sam_fields", "k_sam_cigar", "k_sam_names_seq", "k_dev_map_counts",
+    "k_cap_exact", "k_sam_line_max"};
 
 int mcov_copy_to_host(mcov_ctx* ctx, const void* dev, void* host, int64_t n_bytes) {
   if (!ctx) return MCOV_ERR_ARG;

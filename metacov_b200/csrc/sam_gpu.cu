@@ -12,6 +12,11 @@
 //   k_sam_cigar       one warp per line again, behind a scan of the op counts: every op letter found by ballot takes the
 //                     digits in front of it, and the op goes to its slot (a 100 KB CIGAR is 32 lanes' work, not one's)
 //   k_sam_names_seq   read-name hashes, k-mer keys and SEQ windows (the outputs of k_bam_names_seq) from the text
+//   k_sam_line_max    the longest line of a chunk of a stream, from its line index (mcov_sam_chunk_longest_line)
+//
+// A decode is a header part (sam_upload_header: the @SQ table) and a lines part (sam_decode_lines: everything above).  A
+// file is one of each; a stream (mcov_sam_chunk_begin / mcov_sam_chunk_decode) is one header part and a lines part per
+// chunk of whole lines, with indices local to the chunk.
 //
 // Validation failures do not stop the kernels: each one takes the smallest (record, field) with atomicMin, and the host
 // reports that line.  The per-field rules live in k_sam.cuh, shared with the host-compiled test hook mcov_sam_parse_host.
@@ -256,6 +261,20 @@ k_dev_map_counts(const int32_t* __restrict__ tid, const uint16_t* __restrict__ f
   if (threadIdx.x == 0 && tot) atomicAdd(out, (unsigned long long)tot);
 }
 
+// The longest line of a chunk, its LF included (a last line without one: up to the end of the text); from the line index.
+__global__ void __launch_bounds__(256)
+k_sam_line_max(const uint64_t* __restrict__ line_end, int64_t n_rec, uint64_t body, uint64_t n, unsigned long long* __restrict__ out) {
+  using BR = cub::BlockReduce<unsigned long long, 256>;
+  __shared__ typename BR::TempStorage tmp;
+  unsigned long long m = 0;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_rec; i += (int64_t)gridDim.x * blockDim.x) {
+    const uint64_t start = i ? line_end[i - 1] + 1 : body;
+    m = max(m, (unsigned long long)(min(line_end[i] + 1, n) - start));
+  }
+  const unsigned long long b = BR(tmp).Reduce(m, cub::Max());
+  if (threadIdx.x == 0 && b) atomicMax(out, b);
+}
+
 // ---- host side ------------------------------------------------------------------------------------
 
 // The header: the '@' lines in front of the first record.  References from @SQ SN:/LN:, in order.
@@ -356,36 +375,45 @@ using namespace mcov;
 
 static int sfail(mcov_ctx* ctx, int code, const std::string& msg) { ctx->err = msg; return code; }
 
-extern "C" int mcov_sam_decode_gpu(mcov_ctx* ctx, const void* bytes, int64_t n_bytes, int64_t chunk_bytes, mcov_bam_dev* out) {
-  if (!ctx) return MCOV_ERR_ARG;
-  if (!bytes || n_bytes <= 0 || !out || chunk_bytes < 0) return sfail(ctx, MCOV_ERR_ARG, "mcov_sam_decode_gpu: bad arguments");
-  std::memset(out, 0, sizeof(*out));
-  SCU(cudaSetDevice(ctx->device));
-  cudaStream_t s = ctx->stream;
+// The header part of a decode: the @SQ name table to the device (B.sam_ref), kept for the lines that follow.
+static int sam_upload_header(mcov_ctx* ctx, const SamHeader& h) {
   mcov_ctx::BamDev& B = ctx->bam;
-  B.n_rec = -1;                                                        // (the last decode's columns are overwritten below)
-  B.sam = false;
-  const uint8_t* raw = static_cast<const uint8_t*>(bytes);
-  const uint64_t n = (uint64_t)n_bytes;
-  SamHeader h;
-  if (!sam_parse_header(raw, n, h)) return sfail(ctx, MCOV_ERR_IO, "mcov_sam_decode_gpu: " + h.err);
-  const int32_t n_ref = (int32_t)h.names.size();
   RefTableHost rt;
   rt.build(h.names);
-  // the whole image to the device, chunk by chunk on the copy stream; the newline count of each chunk's tiles follows
-  // its copy on the main stream
-  const uint64_t n_tiles = (n + kSamTile - 1) / kSamTile;
-  uint64_t chunk = chunk_bytes > 0 ? (uint64_t)chunk_bytes : (64ull << 20);
-  chunk = (chunk + kSamTile - 1) / kSamTile * kSamTile;
   const size_t tab_bytes = rt.slot.size() * 4, name_bytes = rt.names.size(), off_bytes = rt.off.size() * 8;
-  SCU(B.data.ensure((size_t)n + 64));
-  SCU(B.status.ensure(64));
-  SCU(B.sam_tiles.ensure((size_t)(n_tiles + 1) * 8));
   SCU(B.sam_ref.ensure(tab_bytes + off_bytes + name_bytes + 16));
   uint8_t* refd = B.sam_ref.as<uint8_t>();
+  cudaStream_t s = ctx->stream;
   SCU(cudaMemcpyAsync(refd, rt.slot.data(), tab_bytes, cudaMemcpyHostToDevice, s));
   SCU(cudaMemcpyAsync(refd + tab_bytes, rt.off.data(), off_bytes, cudaMemcpyHostToDevice, s));
   SCU(cudaMemcpyAsync(refd + tab_bytes + off_bytes, rt.names.data(), name_bytes, cudaMemcpyHostToDevice, s));
+  B.sam_ref_mask = (uint32_t)(rt.slot.size() - 1);
+  B.sam_tab_bytes = tab_bytes; B.sam_off_bytes = off_bytes;
+  B.sam_n_ref = (int32_t)h.names.size();
+  return MCOV_OK;
+}
+
+static SamRefTable sam_ref_view(const mcov_ctx::BamDev& B) {
+  const uint8_t* refd = B.sam_ref.as<uint8_t>();
+  return SamRefTable{reinterpret_cast<const int32_t*>(refd), B.sam_ref_mask, refd + B.sam_tab_bytes + B.sam_off_bytes,
+                     reinterpret_cast<const uint64_t*>(refd + B.sam_tab_bytes)};
+}
+
+// The lines part of a decode: raw[body, n) holds whole record lines (the last one may lack its LF) and nothing after
+// them; it goes to the device with raw[0, body), in copies of `chunk` bytes, and is parsed into the columns.  A malformed
+// line is reported as line `line0` + its index + 1 (line0: the lines of the stream in front of raw[body]).
+static int sam_decode_lines(mcov_ctx* ctx, const uint8_t* raw, uint64_t n, uint64_t body, uint64_t chunk, int64_t line0,
+                            const char* who, mcov_bam_dev* out) {
+  cudaStream_t s = ctx->stream;
+  mcov_ctx::BamDev& B = ctx->bam;
+  // the whole image to the device, chunk by chunk on the copy stream; the newline count of each chunk's tiles follows
+  // its copy on the main stream
+  const uint64_t n_tiles = (n + kSamTile - 1) / kSamTile;
+  chunk = chunk > 0 ? chunk : (64ull << 20);
+  chunk = (chunk + kSamTile - 1) / kSamTile * kSamTile;
+  SCU(B.data.ensure((size_t)n + 64));
+  SCU(B.status.ensure(64));
+  SCU(B.sam_tiles.ensure((size_t)(n_tiles + 1) * 8));
   SCU(cudaMemsetAsync(B.data.as<uint8_t>() + n, 0, 64, s));
   SCU(cudaMemsetAsync(B.sam_tiles.p, 0, (size_t)(n_tiles + 1) * 8, s));
   unsigned long long* d_err = reinterpret_cast<unsigned long long*>(B.status.as<int>() + 8);
@@ -402,8 +430,8 @@ extern "C" int mcov_sam_decode_gpu(mcov_ctx* ctx, const void* bytes, int64_t n_b
     SCU(cudaEventRecord(ev, ctx->copy_stream));
     SCU(cudaStreamWaitEvent(s, ev, 0));
     const uint64_t t0 = c0 / kSamTile, t1 = (c1 + kSamTile - 1) / kSamTile;
-    if (c1 > h.body)
-      MCOV_LAUNCH(ctx, kKSamNlCount, (k_sam_nl_count<<<(unsigned)(t1 - t0), kSamThreads, 0, s>>>(B.data.as<uint8_t>(), h.body, n, t0, tiles)));
+    if (c1 > body)
+      MCOV_LAUNCH(ctx, kKSamNlCount, (k_sam_nl_count<<<(unsigned)(t1 - t0), kSamThreads, 0, s>>>(B.data.as<uint8_t>(), body, n, t0, tiles)));
   }
   SCU(cudaGetLastError());
   size_t tb = 0;
@@ -413,11 +441,11 @@ extern "C" int mcov_sam_decode_gpu(mcov_ctx* ctx, const void* bytes, int64_t n_b
   unsigned long long n_nl = 0;
   SCU(cudaMemcpyAsync(&n_nl, tiles + n_tiles, 8, cudaMemcpyDeviceToHost, s));
   SCU(cudaStreamSynchronize(s));
-  const bool tail = h.body < n && raw[n - 1] != '\n';                 // a last line without its newline
+  const bool tail = body < n && raw[n - 1] != '\n';                   // a last line without its newline
   const uint64_t n_rec = n_nl + (tail ? 1 : 0);
   SCU(B.sam_lines.ensure((size_t)(n_rec + 1) * 8));
   if (n_nl)
-    MCOV_LAUNCH(ctx, kKSamNlWrite, (k_sam_nl_write<<<(unsigned)n_tiles, kSamThreads, 0, s>>>(B.data.as<uint8_t>(), h.body, n, tiles,
+    MCOV_LAUNCH(ctx, kKSamNlWrite, (k_sam_nl_write<<<(unsigned)n_tiles, kSamThreads, 0, s>>>(B.data.as<uint8_t>(), body, n, tiles,
                                                                                          B.sam_lines.as<uint64_t>())));
   if (tail) SCU(cudaMemcpyAsync(B.sam_lines.as<uint64_t>() + n_nl, &n, 8, cudaMemcpyHostToDevice, s));
   // columns
@@ -428,12 +456,10 @@ extern "C" int mcov_sam_decode_gpu(mcov_ctx* ctx, const void* bytes, int64_t n_b
   o.tid = B.tid.as<int32_t>(); o.pos = B.pos.as<int32_t>(); o.flag = B.flag.as<uint16_t>(); o.mapq = B.mapq.as<uint8_t>();
   o.l_seq = B.lseq.as<int32_t>(); o.isize = B.isize.as<int32_t>(); o.rec_off = B.rec_off.as<uint64_t>(); o.aux = B.sam_aux.as<SamAux>();
   o.ops = B.sam_ops.as<unsigned long long>();
-  SamRefTable refs{reinterpret_cast<const int32_t*>(refd), (uint32_t)(rt.slot.size() - 1), refd + tab_bytes + off_bytes,
-                   reinterpret_cast<const uint64_t*>(refd + tab_bytes)};
   SCU(cudaMemsetAsync(o.ops + n_rec, 0, 8, s));
   if (n_rec)
     MCOV_LAUNCH(ctx, kKSamFields, (k_sam_fields<<<(unsigned)((n_rec + kSamWarps - 1) / kSamWarps), kSamThreads, 0, s>>>(
-        B.data.as<uint8_t>(), h.body, B.sam_lines.as<uint64_t>(), (int64_t)n_rec, refs, o, d_err)));
+        B.data.as<uint8_t>(), body, B.sam_lines.as<uint64_t>(), (int64_t)n_rec, sam_ref_view(B), o, d_err)));
   SCU(cudaGetLastError());
   SCU(cub::DeviceScan::ExclusiveSum(nullptr, tb, o.ops, o.ops, (int64_t)(n_rec + 1), s));
   SCU(B.sam_tmp.ensure(tb + 16));
@@ -442,9 +468,9 @@ extern "C" int mcov_sam_decode_gpu(mcov_ctx* ctx, const void* bytes, int64_t n_b
   SCU(cudaMemcpyAsync(&hv[0], d_err, 8, cudaMemcpyDeviceToHost, s));
   SCU(cudaMemcpyAsync(&hv[1], o.ops + n_rec, 8, cudaMemcpyDeviceToHost, s));
   SCU(cudaStreamSynchronize(s));
-  if (hv[0] != kSamNoErr) return sfail(ctx, MCOV_ERR_IO, sam_err_text("mcov_sam_decode_gpu", h.lines + (int64_t)(hv[0] >> 8) + 1, (int)(hv[0] & 255)));
+  if (hv[0] != kSamNoErr) return sfail(ctx, MCOV_ERR_IO, sam_err_text(who, line0 + (int64_t)(hv[0] >> 8) + 1, (int)(hv[0] & 255)));
   const uint64_t n_cig = hv[1];
-  if (n_cig > 0xFFFFFFFFull) return sfail(ctx, MCOV_ERR_RANGE, "mcov_sam_decode_gpu: more than 2^32-1 CIGAR ops");
+  if (n_cig > 0xFFFFFFFFull) return sfail(ctx, MCOV_ERR_RANGE, std::string(who) + ": more than 2^32-1 CIGAR ops");
   SCU(B.cig.ensure((n_cig + 4) * 4));
   if (n_rec)
     MCOV_LAUNCH(ctx, kKSamCigar, (k_sam_cigar<<<(unsigned)((n_rec + kSamWarps - 1) / kSamWarps), kSamThreads, 0, s>>>(
@@ -454,13 +480,89 @@ extern "C" int mcov_sam_decode_gpu(mcov_ctx* ctx, const void* bytes, int64_t n_b
   SCU(cudaMemcpyAsync(B.cig_off.as<uint32_t>() + n_rec, &last, 4, cudaMemcpyHostToDevice, s));
   SCU(cudaMemcpyAsync(&hv[0], d_err, 8, cudaMemcpyDeviceToHost, s));
   SCU(cudaStreamSynchronize(s));
-  if (hv[0] != kSamNoErr) return sfail(ctx, MCOV_ERR_IO, sam_err_text("mcov_sam_decode_gpu", h.lines + (int64_t)(hv[0] >> 8) + 1, (int)(hv[0] & 255)));
-  out->n_records = (int64_t)n_rec; out->n_cigar = (int64_t)n_cig; out->n_ref = n_ref;
-  out->inflated_bytes = (int64_t)n; out->header_bytes = (int64_t)h.body; out->n_segments = 0;
+  if (hv[0] != kSamNoErr) return sfail(ctx, MCOV_ERR_IO, sam_err_text(who, line0 + (int64_t)(hv[0] >> 8) + 1, (int)(hv[0] & 255)));
+  out->n_records = (int64_t)n_rec; out->n_cigar = (int64_t)n_cig; out->n_ref = B.sam_n_ref;
+  out->inflated_bytes = (int64_t)n; out->header_bytes = (int64_t)body; out->n_segments = 0;
   out->tid = o.tid; out->pos = o.pos; out->flag = o.flag; out->mapq = o.mapq; out->l_seq = o.l_seq; out->isize = o.isize;
   out->cig_off = B.cig_off.as<uint32_t>(); out->cig = B.cig.as<uint32_t>(); out->inflated = B.data.as<uint8_t>();
   B.n_rec = (int64_t)n_rec;
   B.sam = true;
+  return MCOV_OK;
+}
+
+extern "C" int mcov_sam_decode_gpu(mcov_ctx* ctx, const void* bytes, int64_t n_bytes, int64_t chunk_bytes, mcov_bam_dev* out) {
+  if (!ctx) return MCOV_ERR_ARG;
+  if (!bytes || n_bytes <= 0 || !out || chunk_bytes < 0) return sfail(ctx, MCOV_ERR_ARG, "mcov_sam_decode_gpu: bad arguments");
+  std::memset(out, 0, sizeof(*out));
+  SCU(cudaSetDevice(ctx->device));
+  mcov_ctx::BamDev& B = ctx->bam;
+  B.n_rec = -1;                                                        // (the last decode's columns are overwritten below)
+  B.sam = false;
+  B.sam_chunked = false;
+  const uint8_t* raw = static_cast<const uint8_t*>(bytes);
+  SamHeader h;
+  if (!sam_parse_header(raw, (uint64_t)n_bytes, h)) return sfail(ctx, MCOV_ERR_IO, "mcov_sam_decode_gpu: " + h.err);
+  int rc = sam_upload_header(ctx, h);
+  if (rc) return rc;
+  return sam_decode_lines(ctx, raw, (uint64_t)n_bytes, h.body, (uint64_t)chunk_bytes, h.lines, "mcov_sam_decode_gpu", out);
+}
+
+extern "C" int mcov_sam_chunk_begin(mcov_ctx* ctx, const void* header_bytes, int64_t n, int32_t* n_ref) {
+  if (!ctx) return MCOV_ERR_ARG;
+  if ((!header_bytes && n) || n < 0) return sfail(ctx, MCOV_ERR_ARG, "mcov_sam_chunk_begin: bad arguments");
+  SCU(cudaSetDevice(ctx->device));
+  mcov_ctx::BamDev& B = ctx->bam;
+  B.n_rec = -1;
+  B.sam = false;
+  B.sam_chunked = false;
+  const uint8_t* raw = static_cast<const uint8_t*>(header_bytes);
+  SamHeader h;
+  if (!sam_parse_header(raw, (uint64_t)n, h)) return sfail(ctx, MCOV_ERR_IO, "mcov_sam_chunk_begin: " + h.err);
+  if (h.body != (uint64_t)n) return sfail(ctx, MCOV_ERR_ARG, "mcov_sam_chunk_begin: the header holds a line that is not a header line");
+  int rc = sam_upload_header(ctx, h);
+  if (rc) return rc;
+  B.sam_line0 = h.lines;
+  B.sam_longest = 0;
+  B.sam_chunked = true;
+  if (n_ref) *n_ref = B.sam_n_ref;
+  return MCOV_OK;
+}
+
+extern "C" int mcov_sam_chunk_decode(mcov_ctx* ctx, const void* bytes, int64_t n, int last, int64_t* consumed, mcov_bam_dev* out) {
+  if (!ctx) return MCOV_ERR_ARG;
+  if ((!bytes && n) || n < 0 || !consumed || !out) return sfail(ctx, MCOV_ERR_ARG, "mcov_sam_chunk_decode: bad arguments");
+  mcov_ctx::BamDev& B = ctx->bam;
+  if (!B.sam_chunked) return sfail(ctx, MCOV_ERR_STATE, "mcov_sam_chunk_decode: call mcov_sam_chunk_begin first");
+  std::memset(out, 0, sizeof(*out));
+  *consumed = 0;
+  SCU(cudaSetDevice(ctx->device));
+  const uint8_t* raw = static_cast<const uint8_t*>(bytes);
+  uint64_t cut = (uint64_t)n;
+  if (!last && n) {
+    const void* nl = memrchr(raw, '\n', (size_t)n);
+    cut = nl ? (uint64_t)(static_cast<const uint8_t*>(nl) - raw) + 1 : 0;
+  }
+  B.n_rec = -1;
+  B.sam = false;
+  ctx->ncig_key_ptr = nullptr;                                         // (the offset column is rewritten in place)
+  if (cut == 0) { out->n_ref = B.sam_n_ref; return MCOV_OK; }
+  const int rc = sam_decode_lines(ctx, raw, cut, 0, 0, B.sam_line0, "mcov_sam_chunk_decode", out);
+  if (rc) return rc;
+  B.sam_line0 += out->n_records;
+  *consumed = (int64_t)cut;
+  if (out->n_records) {                                                // (the line index of this chunk is still in sam_lines)
+    cudaStream_t s = ctx->stream;
+    unsigned long long* d_max = reinterpret_cast<unsigned long long*>(B.status.as<int>() + 12);
+    SCU(cudaMemsetAsync(d_max, 0, 8, s));
+    const int64_t grid = std::min<int64_t>((out->n_records + 255) / 256, (int64_t)std::max(ctx->n_sm, 1) * 4);
+    MCOV_LAUNCH(ctx, kKSamLineMax, (k_sam_line_max<<<(unsigned)grid, 256, 0, s>>>(B.sam_lines.as<uint64_t>(), out->n_records, 0,
+                                                                                  cut, d_max)));
+    SCU(cudaGetLastError());
+    unsigned long long m = 0;
+    SCU(cudaMemcpyAsync(&m, d_max, 8, cudaMemcpyDeviceToHost, s));
+    SCU(cudaStreamSynchronize(s));
+    B.sam_longest = std::max<int64_t>(B.sam_longest, (int64_t)m);
+  }
   return MCOV_OK;
 }
 
@@ -594,4 +696,8 @@ extern "C" int mcov_sam_parse_host(const void* bytes, int64_t n_bytes, mcov_sam_
   c->n_records = i;
   c->n_cigar = (int64_t)k_op;
   return MCOV_OK;
+}
+
+extern "C" int64_t mcov_sam_chunk_longest_line(const mcov_ctx* ctx) {
+  return ctx && ctx->bam.sam_chunked ? ctx->bam.sam_longest : -1;
 }

@@ -143,8 +143,13 @@ class CoverageEngine:
         self._check(lib.mcov_bind_depth(self._ctx, tensor.data_ptr(), tensor.numel()))
 
     # -- depth ------------------------------------------------------------
-    def begin(self):
-        self._check(lib.mcov_begin(self._ctx))
+    def begin(self, exact_cap=False):
+        """Start an any-order pass.  exact_cap: the pass reports the exact cap metric max depth[p-1]+starts[p]
+        (mcov_begin_ex, MCOV_BEGIN_EXACT_CAP) instead of an upper bound of it."""
+        if exact_cap:
+            self._check(lib.mcov_begin_ex(self._ctx, _capi.MCOV_BEGIN_EXACT_CAP))
+        else:
+            self._check(lib.mcov_begin(self._ctx))
 
     def push(self, batch):
         b = _canon(batch)

@@ -85,6 +85,10 @@ class ReadProcessorList(ReadProcessor):
     def get_rows(self, i):
         return self.processors[i].get_rows()
 
+    def _merge(self, other):
+        for p, q in zip(self.processors, other.processors):
+            p._merge(q)
+
     def _accumulate(self, ctx, group_flags, targets):
         # targets: the copies of this list, one per ByFlag group (or just [self])
         for i, p in enumerate(self.processors):
@@ -153,6 +157,14 @@ class IsizeHist(ReadProcessor):
         data[:m] = row[:m]
         self._counts_data = data
 
+    def _merge(self, other):
+        """Add the counts of another IsizeHist (tables of any widths): the rows one call over both sets of reads gives."""
+        a, b = self._counts_data, other._counts_data
+        row = np.zeros(max(len(a), len(b)), dtype=np.uint32)
+        row[:len(a)] += a
+        row[:len(b)] += b
+        self._ingest(row)
+
     def _accumulate(self, ctx, group_flags, targets):
         hist, _, _ = ctx["engine"].isize_hist(ctx["flag"], ctx["isize"], group_flags)
         for g, t in enumerate(targets):
@@ -180,6 +192,9 @@ class KmerHist(ReadProcessor):
         yield ["N" * self.K] + list(self.counts[4 ** self.K])
         for i in range(4 ** self.K):
             yield [kmer_base2_to_ascii(i, self.K)] + list(self._counts_data[i])
+
+    def _merge(self, other):
+        self._counts_data = self._counts_data + other._counts_data
 
     def _accumulate(self, ctx, group_flags, targets):
         if self.OFFSET < 0:
@@ -236,6 +251,12 @@ def scan_reads(infile, fasta, counters, progress_interval=10000000, progress_cb=
     else:
         raise Exception("mah")               # scan.pyx:649
     processor.set_max_readlen(50)
+    if infile.piped:
+        n = _scan_pipe(infile, processor, maxreads)
+        if progress_cb:
+            for _ in range(n // max(int(progress_interval), 1)):
+                progress_cb()
+        return n
     gpu = getattr(infile, "_gpu", None)
     if gpu is not None:
         # a file decoded on the GPU: flag / isize / l_seq (and, for KmerHist, the SEQ windows) stay where the decoder left
@@ -268,3 +289,26 @@ def scan_reads(infile, fasta, counters, progress_interval=10000000, progress_cb=
         for _ in range(n // max(int(progress_interval), 1)):
             progress_cb()
     return n
+
+
+def _scan_pipe(infile, processor, maxreads):
+    """``scan_reads`` over a piped SAM stream: the accumulators run on the device columns of every chunk as it is decoded,
+    and the chunks' histograms are added up.  ``maxreads`` ends the read after that many records."""
+    infile._pipe_claim("scan_reads")
+    state = {"n": 0, "rlen": 0}
+
+    def per_chunk(dsoa, n):
+        target = processor if state["n"] == 0 else copy(processor)
+        ctx = {"engine": dsoa._engine, "infile": infile, "flag": dsoa.device_view("flag", n), "isize": dsoa.device_view("isize", n),
+               "l_seq": dsoa.device_view("l_seq", n), "device_soa": dsoa}
+        target._accumulate(ctx, [], [target])
+        if target is not processor:
+            processor._merge(target)
+        if n:
+            state["rlen"] = max(state["rlen"], int(dsoa.to_host("l_seq")[:n].max()))
+        state["n"] += n
+
+    infile._pipe_pass(per_chunk, stop_after=int(maxreads or 0))
+    if state["n"]:
+        processor.set_max_readlen(max(50, state["rlen"]))
+    return state["n"]
