@@ -726,6 +726,44 @@ typedef struct mcov_bam_gpu_stream_info {
 } mcov_bam_gpu_stream_info;
 int  mcov_bam_gpu_stream_depth(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, int verify_crc,
                                mcov_bam_gpu_stream_info* info);
+/* A / C / G / T counts at every reference position: pysam's
+ * AlignmentFile.count_coverage over the whole file, on the device.
+ * mcov_base_counts counts the records of the file last decoded on this
+ * context (mcov_bam_decode_gpu*, mcov_sam_decode_gpu*: path NULL), or of the BAM
+ * file at `path` read through the streamed decoder chunk_bytes at a time (<= 0:
+ * 64 MiB; like mcov_bam_gpu_stream_depth, the context's contig table must be
+ * the file's, and the columns of an earlier decode are gone afterwards).  The
+ * context's contig table (mcov_set_contigs) places the counts.
+ *   Records: those placed on a contig (0 <= tid < n_contigs, pos >= 0), minus
+ *   those with a flag of 0x4 | 0x100 | 0x200 | 0x400 (MCOV_BC_ALL, pysam's
+ *   read_callback="all"; MCOV_BC_NOFILTER skips none).  A record without SEQ
+ *   counts nothing.  Every (query, reference) pair of an M, = or X op counts
+ *   at its reference position when the base is A, C, G or T and, with
+ *   quality_threshold != 0, the read has qualities (BAM: first QUAL byte not
+ *   0xFF; SAM: QUAL not '*') and the base's quality is >= quality_threshold
+ *   (a negative threshold only asks for qualities).  Pairs at or past the
+ *   contig's end are dropped.  No MAPQ or orphan filter, no max_depth cap;
+ *   the pileup filter of mcov_set_filter does not apply.
+ *   Any read order: one warp per read (k_bc_any), global atomics.
+ * The counts live apart from the depth store, which, with its statistics
+ * caches, is left as it was.  MCOV_ERR_NOMEM, before anything is allocated,
+ * when the 16 bytes a slot do not fit the free device memory (the message
+ * holds both byte counts); MCOV_ERR_IO naming the first record (0-based, file
+ * order) whose CIGAR consumes more query bases than its SEQ holds -- nothing
+ * is read past SEQ or QUAL --, or whose SEQ / QUAL leave the BAM record;
+ * MCOV_ERR_STATE without contigs or a decoded file.  After an error the
+ * context is usable and holds no counts.  Synchronises. */
+enum {
+  MCOV_BC_ALL = 0,        /* skip unmapped, secondary, QC-fail and duplicate records */
+  MCOV_BC_NOFILTER = 1    /* count every placed record                               */
+};
+int  mcov_base_counts(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, int32_t quality_threshold, int mode);
+/* The counts of the last mcov_base_counts at [start, end) of contig tid into
+ * host_out[4 * (end - start)]: the A counts, then C, G and T, each end - start
+ * long.  MCOV_ERR_STATE without counts for the current contig table,
+ * MCOV_ERR_ARG for a region outside the contig.  Synchronises. */
+int  mcov_copy_base_counts(mcov_ctx* ctx, int32_t tid, int32_t start, int32_t end, uint32_t* host_out);
+
 /* Test hooks: the device inflate / CRC-32 code (csrc/inflate.cuh) compiled for the host, so that the CPU
  * suite can check it against zlib.  mcov_inflate_host returns 0 or a positive decoder status. */
 int  mcov_inflate_host(const uint8_t* src, uint32_t clen, uint8_t* dst, uint32_t ulen);

@@ -23,6 +23,8 @@ MCOV_ERR_UNSORTED = -7
 MCOV_BEGIN_EXACT_CAP = 1     # mcov_begin_ex: the any-order pass reports the exact cap metric
 MEM_HOST = 0
 MEM_DEVICE = 1
+MCOV_BC_ALL = 0              # mcov_base_counts: pysam's read_callback="all" (skip flags 0x4 | 0x100 | 0x200 | 0x400)
+MCOV_BC_NOFILTER = 1         # read_callback="nofilter"
 
 _STATUS_NAMES = {
     MCOV_ERR_ARG: "MCOV_ERR_ARG", MCOV_ERR_STATE: "MCOV_ERR_STATE", MCOV_ERR_CUDA: "MCOV_ERR_CUDA",
@@ -158,6 +160,8 @@ SIGNATURES = {
     "mcov_sam_chunk_decode": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, C.POINTER(_i64), _vp]),
     "mcov_sam_chunk_longest_line": (_i64, [_vp]),
     "mcov_bam_gpu_mapped": (C.c_int, [_vp, C.POINTER(_i64), C.POINTER(_i64)]),
+    "mcov_base_counts": (C.c_int, [_vp, C.c_char_p, _i64, _i32, C.c_int]),
+    "mcov_copy_base_counts": (C.c_int, [_vp, _i32, _i32, _i32, _vp]),
     "mcov_sam_parse_host": (C.c_int, [_vp, C.c_int64, C.POINTER(SamHostCols), C.c_char_p, C.c_int]),
     "mcov_inflate_host": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint32]),
     "mcov_inflate_host_win": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint32, C.c_uint32]),

@@ -6,7 +6,9 @@ Protocol provided (reference call sites): constructor from a path
 (metacov/cli.py:56, 211); context manager (cli.py:258); ``references`` /
 ``lengths`` (util.py:67-68, cli.py:80); ``mapped`` / ``unmapped``
 (cli.py:73-75, 214-216); ``pileup(ref, start, end)`` yielding objects with
-``.pos`` / ``.n`` (pileup.py:13-16).
+``.pos`` / ``.n`` (pileup.py:13-16); ``count_coverage(contig, start, stop,
+quality_threshold, read_callback)``, the A / C / G / T counts per position
+(pysam's signature; computed on the GPU, csrc/basecount.cu).
 """
 import ctypes as C
 import os
@@ -212,6 +214,8 @@ class AlignmentFile:
         self.stream_batches = 0
         self._h = None
         self._stream = None
+        self._bc_eng = None                                 # count_coverage of a file that is not resident on the device
+        self._bc_key = None                                 # (threshold, mode) of the counts held
         if decode == "gpu":
             self._open_gpu(filename, device)
             return
@@ -236,6 +240,7 @@ class AlignmentFile:
         self.stream_batches = 0
         self._gpu = self._soa = self._engine = self._filter_kw = self._index_stats = None
         self._h = self._stream = None
+        self._bc_eng = self._bc_key = None
         self._pipe_consumer = None
         self._pipe_read = False
         self._pipe_reader = None
@@ -446,6 +451,9 @@ class AlignmentFile:
         if getattr(self, "_gpu", None) is not None:
             self._gpu[0].close()                            # (the same engine, if the depth was computed)
             self._gpu = None
+        if getattr(self, "_bc_eng", None) is not None:
+            self._bc_eng.close()
+            self._bc_eng = None
         if getattr(self, "_h", None):
             lib.mcov_bam_close(self._h)
             self._h = None
@@ -736,3 +744,65 @@ class AlignmentFile:
         """Per-base depth as an int32 array (additive helper)."""
         tid = self._tid[contig]
         return self.coverage_engine().copy_depth(tid, 0 if start is None else start, stop)
+
+    def count_coverage(self, contig, start=None, stop=None, quality_threshold=15, read_callback="all"):
+        """pysam's ``count_coverage``: four ``numpy.uint32`` arrays (A, C, G, T), each ``stop - start`` long, index k =
+        position start + k, counted on the GPU over the whole file once per (threshold, read_callback) and sliced.
+
+        ``start`` None -> 0, ``stop`` None -> the contig length (a larger ``stop`` is clipped to it); an empty or
+        negative interval or a negative ``start`` raises ValueError, an unknown contig KeyError.  ``read_callback``
+        "all" skips records flagged 0x4, 0x100, 0x200 or 0x400, "nofilter" none; anything else, a callable included,
+        raises ValueError.  Every (qpos, refpos) pair of an M / = / X op counts where the base is A, C, G or T and,
+        with ``quality_threshold`` (None = 0) non-zero, the read has qualities and the base's quality is at least the
+        threshold.  No MAPQ, orphan or max_depth filter; ``set_pileup_filter`` does not apply.  A record whose CIGAR
+        consumes more query bases than its SEQ holds raises IndexError naming it, as pysam does; counters that do not fit
+        the free device memory raise MemoryError.
+
+        Deliberate differences from pysam: the file need not be coordinate-sorted or indexed (pysam's ``fetch`` needs
+        both); under "nofilter", a record flagged unmapped that carries a CIGAR counts by its CIGAR everywhere, where
+        pysam's ``fetch`` returns it only for intervals that contain its POS.  Files decoded on the device count from
+        the resident records; others (``decode="host"`` / ``"gpu-stream"``) go through the GPU decoder chunk by chunk.
+        The depth and its statistics are left as they were.  A piped stream raises ValueError."""
+        self._no_records("count_coverage()")
+        if callable(read_callback) or read_callback not in ("all", "nofilter"):
+            raise ValueError("read_callback must be 'all' or 'nofilter' (a callable is not supported: the counts are "
+                             "computed on the GPU), got %r" % (read_callback,))
+        tid = self._tid[contig]                             # KeyError for unknown contigs, like pysam
+        length = int(self.lengths[tid])
+        start = 0 if start is None else int(start)
+        stop = length if stop is None else min(int(stop), length)
+        if start < 0:
+            raise ValueError("start out of range (%d)" % start)
+        if stop == start:
+            raise ValueError("interval of size 0")
+        if stop < start:
+            raise ValueError("interval of size less than 0")
+        t = max(min(int(quality_threshold or 0), 2 ** 31 - 1), -2 ** 31)
+        mode = _capi.MCOV_BC_NOFILTER if read_callback == "nofilter" else _capi.MCOV_BC_ALL
+        eng = self._count_engine()
+        if self._bc_key != (t, mode):
+            self._bc_key = None
+            try:
+                if self._gpu is not None:
+                    eng.base_counts(t, mode)
+                else:
+                    eng.base_counts(t, mode, path=self.filename, chunk_bytes=self._gpu_chunk_bytes)
+            except McovError as e:
+                if e.code == _capi.MCOV_ERR_IO and "consumes more query bases" in str(e):
+                    raise IndexError("%s: %s" % (self.filename, e))         # (pysam's error there)
+                if e.code == _capi.MCOV_ERR_NOMEM:
+                    raise MemoryError("%s: %s" % (self.filename, e))
+                if e.code == _capi.MCOV_ERR_IO:
+                    raise OSError("%s: %s" % (self.filename, e))
+                raise
+            self._bc_key = (t, mode)
+        c = eng.copy_base_counts(tid, start, stop)
+        return c[0], c[1], c[2], c[3]
+
+    def _count_engine(self):
+        """The engine that counts: a device-decoded file's own (it holds the records); else one of the counts' own."""
+        if self._gpu is not None:
+            return self._gpu[0]
+        if self._bc_eng is None:
+            self._bc_eng = CoverageEngine(self.lengths, device=self._device)
+        return self._bc_eng

@@ -598,11 +598,12 @@ extern "C" int mcov_bam_decode_gpu_file(mcov_ctx* ctx, const char* path, int ver
   return rc;
 }
 
-extern "C" int mcov_bam_gpu_stream_depth(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, int verify_crc,
-                                         mcov_bam_gpu_stream_info* info) {
-  if (!ctx) return MCOV_ERR_ARG;
-  if (!path || !info) return bfail(ctx, MCOV_ERR_ARG, "mcov_bam_gpu_stream_depth: bad arguments");
-  std::memset(info, 0, sizeof(*info));
+// The chunk loop of the streamed decode: every chunk inflated, chained and written into columns behind the reads the
+// sink carried, then handed to the sink.  The depth pass (mcov_bam_gpu_stream_depth) and the base counts
+// (mcov_base_counts) are its two consumers.
+int mcov::bam_gpu_chunks(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, int verify_crc, mcov_bam_gpu_stream_info* info,
+                         const char* who, BamChunkSink& sink) {
+  auto F = [&](int code, const char* why) { ctx->err = std::string(who) + ": " + why; return code; };
   if (chunk_bytes <= 0) chunk_bytes = 64ll << 20;
   chunk_bytes = std::max<int64_t>(chunk_bytes, 1 << 17);          // at least one BGZF block (<= 64 KiB) beside a leftover
   CUB(cudaSetDevice(ctx->device));
@@ -611,7 +612,7 @@ extern "C" int mcov_bam_gpu_stream_depth(mcov_ctx* ctx, const char* path, int64_
   B.n_rec = -1;                                                   // (the whole-file decode's columns are gone after this)
   B.sam = false;
   FILE* fh = std::fopen(path, "rb");
-  if (!fh) return bfail(ctx, MCOV_ERR_IO, "mcov_bam_gpu_stream_depth: cannot open the file");
+  if (!fh) return F(MCOV_ERR_IO, "cannot open the file");
   struct Closer { FILE* f; ~Closer() { if (f) std::fclose(f); } } closer{fh};
   // a file smaller than the chunk: buffers no larger than the file needs.  The two host buffers are PINNED only for a long
   // stream (>= 1 GiB of file): pinning costs 0.6 - 2.4 ms per MB on these boxes (and as much again to free), which a short
@@ -629,7 +630,7 @@ extern "C" int mcov_bam_gpu_stream_depth(mcov_ctx* ctx, const char* path, int64_
   CUB(B.pin[0].ensure(cap, pin)); CUB(B.pin[1].ensure(cap, pin));
   CUB(B.status.ensure(64));
   auto read_into = [fh](uint8_t* dst, size_t want) -> size_t { return std::fread(dst, 1, want, fh); };
-  int rc = mcov_stream_begin(ctx);
+  int rc = sink.begin(ctx);
   if (rc) return rc;
   int cur = 0;
   size_t left = 0;                                                // bytes of an incomplete block at the front of pin[cur]
@@ -639,7 +640,6 @@ extern "C" int mcov_bam_gpu_stream_depth(mcov_ctx* ctx, const char* path, int64_
   int64_t n_carry = 0, carry_ops = 0;
   int32_t n_ref = -1;
   bool first = true, pushed_last = false;
-  int32_t rt = -1, rp = 0;
   std::vector<BgzfBlock> blocks;
   std::vector<WalkSeg> segs;
   std::vector<WalkOut> wo;
@@ -650,9 +650,9 @@ extern "C" int mcov_bam_gpu_stream_depth(mcov_ctx* ctx, const char* path, int64_
     blocks.clear();
     uint64_t total = 0;
     size_t consumed = 0;
-    if (!index_bgzf(raw, have, blocks, total, &consumed, tail_len)) return bfail(ctx, MCOV_ERR_IO, "mcov_bam_gpu_stream_depth: not a valid BGZF file");
-    if (eof && consumed != have) return bfail(ctx, MCOV_ERR_IO, "mcov_bam_gpu_stream_depth: the file ends inside a BGZF block");
-    if (!eof && consumed == 0) return bfail(ctx, MCOV_ERR_IO, "mcov_bam_gpu_stream_depth: a BGZF block larger than the chunk");
+    if (!index_bgzf(raw, have, blocks, total, &consumed, tail_len)) return F(MCOV_ERR_IO, "not a valid BGZF file");
+    if (eof && consumed != have) return F(MCOV_ERR_IO, "the file ends inside a BGZF block");
+    if (!eof && consumed == 0) return F(MCOV_ERR_IO, "a BGZF block larger than the chunk");
     const size_t next_left = have - consumed;
     std::future<size_t> next_read;
     const bool was_eof = eof;
@@ -666,7 +666,7 @@ extern "C" int mcov_bam_gpu_stream_depth(mcov_ctx* ctx, const char* path, int64_
     do {                                                          // (one pass; `break` = leave with err_rc set, after joining the reader)
       // inflate behind the carried record bytes
       if (B.raw.ensure(consumed + 16) != cudaSuccess || B.blocks.ensure((size_t)std::max<int64_t>(nb, 1) * sizeof(BgzfBlock)) != cudaSuccess ||
-          B.data.ensure((size_t)total + 64) != cudaSuccess) { err_rc = bfail(ctx, MCOV_ERR_NOMEM, "mcov_bam_gpu_stream_depth: out of device memory"); break; }
+          B.data.ensure((size_t)total + 64) != cudaSuccess) { err_rc = F(MCOV_ERR_NOMEM, "out of device memory"); break; }
       if (tail_len) cudaMemcpyAsync(B.data.p, B.tail.p, (size_t)tail_len, cudaMemcpyDeviceToDevice, s);
       if (consumed) cudaMemcpyAsync(B.raw.p, raw, consumed, cudaMemcpyHostToDevice, s);
       cudaMemsetAsync(B.status.p, 0, 64, s);
@@ -675,19 +675,19 @@ extern "C" int mcov_bam_gpu_stream_depth(mcov_ctx* ctx, const char* path, int64_
         MCOV_LAUNCH(ctx, kKBgzfInflate, (k_bgzf_inflate<<<(unsigned)((nb + kInflateGroupsPerCta - 1) / kInflateGroupsPerCta), kInflateThreads, 0, s>>>(
             B.raw.as<uint8_t>(), B.blocks.as<BgzfBlock>(), nb, B.data.as<uint8_t>(), verify_crc, B.status.as<int>())));
       }
-      if (cudaGetLastError() != cudaSuccess) { err_rc = bfail(ctx, MCOV_ERR_CUDA, "mcov_bam_gpu_stream_depth: inflate launch failed"); break; }
+      if (cudaGetLastError() != cudaSuccess) { err_rc = F(MCOV_ERR_CUDA, "inflate launch failed"); break; }
       uint64_t rec_begin = 0;
       if (first) {
-        if (total < 12) { err_rc = bfail(ctx, MCOV_ERR_IO, "mcov_bam_gpu_stream_depth: not a valid BAM file"); break; }
+        if (total < 12) { err_rc = F(MCOV_ERR_IO, "not a valid BAM file"); break; }
         err_rc = bam_dev_header(ctx, total, &rec_begin, &n_ref);             // (a header that does not fit the first chunk reads as truncated)
         if (err_rc) break;
-        if (n_ref != ctx->n_contigs) { err_rc = bfail(ctx, MCOV_ERR_ARG, "mcov_bam_gpu_stream_depth: the context's contig table is not this file's"); break; }
+        if (n_ref != ctx->n_contigs) { err_rc = F(MCOV_ERR_ARG, "the context's contig table is not this file's"); break; }
         first = false;
       } else {
         int st2[2] = {0, 0};
         cudaMemcpyAsync(st2, B.status.p, sizeof(st2), cudaMemcpyDeviceToHost, s);
-        if (cudaStreamSynchronize(s) != cudaSuccess) { err_rc = bfail(ctx, MCOV_ERR_CUDA, "mcov_bam_gpu_stream_depth: inflate failed"); break; }
-        if (st2[0]) { err_rc = bfail(ctx, MCOV_ERR_IO, st2[0] == 100 ? "mcov_bam_gpu_stream_depth: CRC mismatch in a BGZF block" : "mcov_bam_gpu_stream_depth: corrupt deflate stream in a BGZF block"); break; }
+        if (cudaStreamSynchronize(s) != cudaSuccess) { err_rc = F(MCOV_ERR_CUDA, "inflate failed"); break; }
+        if (st2[0]) { err_rc = F(MCOV_ERR_IO, st2[0] == 100 ? "CRC mismatch in a BGZF block" : "corrupt deflate stream in a BGZF block"); break; }
       }
       // the record chain of this chunk
       uint64_t chain_end = rec_begin;
@@ -700,18 +700,18 @@ extern "C" int mcov_bam_gpu_stream_depth(mcov_ctx* ctx, const char* path, int64_
       uint64_t n_rec = 0, n_cig = 0;
       for (size_t i = 0; i < segs.size(); ++i) { segs[i].rec_base = (uint64_t)n_carry + n_rec; segs[i].cig_base = (uint64_t)carry_ops + n_cig; n_rec += wo[i].n_rec; n_cig += wo[i].n_cig; }
       const uint64_t n_tot = (uint64_t)n_carry + n_rec, ops_tot = (uint64_t)carry_ops + n_cig;
-      if (ops_tot > 0xFFFFFFF0ull || n_tot > 0x7FFFFFF0ull) { err_rc = bfail(ctx, MCOV_ERR_RANGE, "mcov_bam_gpu_stream_depth: a chunk holds too many records; use a smaller chunk"); break; }
+      if (ops_tot > 0xFFFFFFF0ull || n_tot > 0x7FFFFFF0ull) { err_rc = F(MCOV_ERR_RANGE, "a chunk holds too many records; use a smaller chunk"); break; }
       // the bytes of the record this chunk ends in: kept for the front of the next chunk's stream
       const uint64_t new_tail = total - chain_end;
       if (new_tail) {
-        if (B.tail2.ensure((size_t)new_tail) != cudaSuccess) { err_rc = bfail(ctx, MCOV_ERR_NOMEM, "mcov_bam_gpu_stream_depth: out of device memory"); break; }
+        if (B.tail2.ensure((size_t)new_tail) != cudaSuccess) { err_rc = F(MCOV_ERR_NOMEM, "out of device memory"); break; }
         cudaMemcpyAsync(B.tail2.p, B.data.as<uint8_t>() + chain_end, (size_t)new_tail, cudaMemcpyDeviceToDevice, s);
       }
       // columns: [carried reads | this chunk's]
       bool okm = B.tid.ensure((n_tot + 4) * 4) == cudaSuccess && B.pos.ensure((n_tot + 4) * 4) == cudaSuccess && B.flag.ensure((n_tot + 4) * 2) == cudaSuccess &&
                  B.mapq.ensure(n_tot + 4) == cudaSuccess && B.lseq.ensure((n_tot + 4) * 4) == cudaSuccess && B.isize.ensure((n_tot + 4) * 4) == cudaSuccess &&
                  B.cig_off.ensure((n_tot + 5) * 4) == cudaSuccess && B.cig.ensure((ops_tot + 4) * 4) == cudaSuccess && B.rec_off.ensure((n_tot + 4) * 8) == cudaSuccess;
-      if (!okm) { err_rc = bfail(ctx, MCOV_ERR_NOMEM, "mcov_bam_gpu_stream_depth: out of device memory"); break; }
+      if (!okm) { err_rc = F(MCOV_ERR_NOMEM, "out of device memory"); break; }
       if (n_carry) {
         cudaMemcpyAsync(B.tid.p, B.c_tid.p, (size_t)n_carry * 4, cudaMemcpyDeviceToDevice, s);
         cudaMemcpyAsync(B.pos.p, B.c_pos.p, (size_t)n_carry * 4, cudaMemcpyDeviceToDevice, s);
@@ -731,47 +731,22 @@ extern "C" int mcov_bam_gpu_stream_depth(mcov_ctx* ctx, const char* path, int64_
       }
       const uint32_t last_off = (uint32_t)ops_tot;
       cudaMemcpyAsync(o.cig_off + n_tot, &last_off, 4, cudaMemcpyHostToDevice, s);
-      if (cudaStreamSynchronize(s) != cudaSuccess) { err_rc = bfail(ctx, MCOV_ERR_CUDA, "mcov_bam_gpu_stream_depth: record walk failed"); break; }
+      if (cudaStreamSynchronize(s) != cudaSuccess) { err_rc = F(MCOV_ERR_CUDA, "record walk failed"); break; }
       std::swap(B.tail, B.tail2);
       info->inflated_bytes += (int64_t)(total - tail_len);
       tail_len = new_tail;
-      if (was_eof && tail_len) { err_rc = bfail(ctx, MCOV_ERR_IO, "mcov_bam_gpu_stream_depth: the last BAM record is truncated"); break; }
-      // the batch -> streamed depth pass
-      const int last = was_eof ? 1 : 0;
-      err_rc = mcov_stream_push(ctx, (int64_t)n_tot, n_carry, o.tid, o.pos, o.flag, o.mapq, o.cig_off, o.cig, MCOV_MEM_DEVICE, last, &rt, &rp);
+      if (was_eof && tail_len) { err_rc = F(MCOV_ERR_IO, "the last BAM record is truncated"); break; }
+      // the batch -> the consumer
+      BamChunk bc;
+      bc.n = (int64_t)n_tot; bc.n_carry = n_carry; bc.n_ops = (int64_t)ops_tot;
+      bc.tid = o.tid; bc.pos = o.pos; bc.flag = o.flag; bc.mapq = o.mapq; bc.l_seq = o.l_seq; bc.cig_off = o.cig_off; bc.cig = o.cig;
+      bc.data = B.data.as<uint8_t>(); bc.rec_off = o.rec_off; bc.last = was_eof;
+      err_rc = sink.batch(ctx, bc, &n_carry, &carry_ops);
       if (err_rc) break;
       info->n_records += (int64_t)n_rec; info->n_chunks += 1; info->n_segments += (int64_t)segs.size();
       info->file_bytes += (int64_t)consumed;
-      if (last) { pushed_last = true; break; }
-      // what the next batch must begin with: the suffix from the first read that starts at / reaches past the resend point
-      n_carry = 0; carry_ops = 0;
-      if (n_tot) {
-        unsigned long long* d_first = reinterpret_cast<unsigned long long*>(B.status.as<int>() + 4);
-        const unsigned long long init = n_tot;
-        cudaMemcpyAsync(d_first, &init, 8, cudaMemcpyHostToDevice, s);
-        k_bam_carry_first<<<(unsigned)((n_tot + 255) / 256), 256, 0, s>>>((int64_t)n_tot, o.tid, o.pos, o.cig_off, o.cig, rt, rp, ctx->n_contigs, d_first);
-        unsigned long long j0 = n_tot;
-        cudaMemcpyAsync(&j0, d_first, 8, cudaMemcpyDeviceToHost, s);
-        if (cudaStreamSynchronize(s) != cudaSuccess) { err_rc = bfail(ctx, MCOV_ERR_CUDA, "mcov_bam_gpu_stream_depth: carry selection failed"); break; }
-        if (j0 < n_tot) {
-          uint32_t o0 = 0;
-          cudaMemcpyAsync(&o0, o.cig_off + j0, 4, cudaMemcpyDeviceToHost, s);
-          cudaStreamSynchronize(s);
-          n_carry = (int64_t)(n_tot - j0); carry_ops = (int64_t)ops_tot - (int64_t)o0;
-          okm = B.c_tid.ensure((size_t)n_carry * 4) == cudaSuccess && B.c_pos.ensure((size_t)n_carry * 4) == cudaSuccess &&
-                B.c_flag.ensure((size_t)n_carry * 2) == cudaSuccess && B.c_mapq.ensure((size_t)n_carry) == cudaSuccess &&
-                B.c_off.ensure((size_t)n_carry * 4) == cudaSuccess && B.c_cig.ensure((size_t)std::max<int64_t>(carry_ops, 1) * 4) == cudaSuccess;
-          if (!okm) { err_rc = bfail(ctx, MCOV_ERR_NOMEM, "mcov_bam_gpu_stream_depth: out of device memory"); break; }
-          cudaMemcpyAsync(B.c_tid.p, o.tid + j0, (size_t)n_carry * 4, cudaMemcpyDeviceToDevice, s);
-          cudaMemcpyAsync(B.c_pos.p, o.pos + j0, (size_t)n_carry * 4, cudaMemcpyDeviceToDevice, s);
-          cudaMemcpyAsync(B.c_flag.p, o.flag + j0, (size_t)n_carry * 2, cudaMemcpyDeviceToDevice, s);
-          cudaMemcpyAsync(B.c_mapq.p, o.mapq + j0, (size_t)n_carry, cudaMemcpyDeviceToDevice, s);
-          k_bam_rebase_offsets<<<(unsigned)((n_carry + 255) / 256), 256, 0, s>>>(n_carry, o.cig_off + j0, o0, B.c_off.as<uint32_t>());
-          if (carry_ops) cudaMemcpyAsync(B.c_cig.p, o.cig + o0, (size_t)carry_ops * 4, cudaMemcpyDeviceToDevice, s);
-          info->max_carry = std::max<int64_t>(info->max_carry, n_carry);
-        }
-      }
-      if (cudaGetLastError() != cudaSuccess) { err_rc = bfail(ctx, MCOV_ERR_CUDA, "mcov_bam_gpu_stream_depth: carry copy failed"); break; }
+      info->max_carry = std::max<int64_t>(info->max_carry, n_carry);
+      if (was_eof) { pushed_last = true; break; }
     } while (false);
     if (next_read.valid()) {                                      // always join the reader before leaving or going on
       got = next_read.get();
@@ -782,6 +757,64 @@ extern "C" int mcov_bam_gpu_stream_depth(mcov_ctx* ctx, const char* path, int64_
     if (err_rc) return err_rc;
   }
   return MCOV_OK;
+}
+
+namespace {
+
+// The streamed depth pass as a consumer of the chunk loop: every batch goes to mcov_stream_push, and what the next batch
+// must begin with is the suffix from the first read that starts at / reaches past the pass's resend point.
+struct DepthSink : mcov::BamChunkSink {
+  int32_t rt = -1, rp = 0;
+  int begin(mcov_ctx* ctx) override { return mcov_stream_begin(ctx); }
+  int batch(mcov_ctx* ctx, const BamChunk& b, int64_t* n_carry_out, int64_t* carry_ops_out) override {
+    cudaStream_t s = ctx->stream;
+    mcov_ctx::BamDev& B = ctx->bam;
+    const int last = b.last ? 1 : 0;
+    int rc = mcov_stream_push(ctx, b.n, b.n_carry, b.tid, b.pos, b.flag, b.mapq, b.cig_off, b.cig, MCOV_MEM_DEVICE, last, &rt, &rp);
+    if (rc) return rc;
+    *n_carry_out = 0; *carry_ops_out = 0;
+    if (last) return MCOV_OK;
+    const uint64_t n_tot = (uint64_t)b.n, ops_tot = (uint64_t)b.n_ops;
+    if (n_tot) {
+      unsigned long long* d_first = reinterpret_cast<unsigned long long*>(B.status.as<int>() + 4);
+      const unsigned long long init = n_tot;
+      cudaMemcpyAsync(d_first, &init, 8, cudaMemcpyHostToDevice, s);
+      k_bam_carry_first<<<(unsigned)((n_tot + 255) / 256), 256, 0, s>>>((int64_t)n_tot, b.tid, b.pos, b.cig_off, b.cig, rt, rp, ctx->n_contigs, d_first);
+      unsigned long long j0 = n_tot;
+      cudaMemcpyAsync(&j0, d_first, 8, cudaMemcpyDeviceToHost, s);
+      if (cudaStreamSynchronize(s) != cudaSuccess) return bfail(ctx, MCOV_ERR_CUDA, "mcov_bam_gpu_stream_depth: carry selection failed");
+      if (j0 < n_tot) {
+        uint32_t o0 = 0;
+        cudaMemcpyAsync(&o0, b.cig_off + j0, 4, cudaMemcpyDeviceToHost, s);
+        cudaStreamSynchronize(s);
+        const int64_t n_carry = (int64_t)(n_tot - j0), carry_ops = (int64_t)ops_tot - (int64_t)o0;
+        const bool okm = B.c_tid.ensure((size_t)n_carry * 4) == cudaSuccess && B.c_pos.ensure((size_t)n_carry * 4) == cudaSuccess &&
+                         B.c_flag.ensure((size_t)n_carry * 2) == cudaSuccess && B.c_mapq.ensure((size_t)n_carry) == cudaSuccess &&
+                         B.c_off.ensure((size_t)n_carry * 4) == cudaSuccess && B.c_cig.ensure((size_t)std::max<int64_t>(carry_ops, 1) * 4) == cudaSuccess;
+        if (!okm) return bfail(ctx, MCOV_ERR_NOMEM, "mcov_bam_gpu_stream_depth: out of device memory");
+        cudaMemcpyAsync(B.c_tid.p, b.tid + j0, (size_t)n_carry * 4, cudaMemcpyDeviceToDevice, s);
+        cudaMemcpyAsync(B.c_pos.p, b.pos + j0, (size_t)n_carry * 4, cudaMemcpyDeviceToDevice, s);
+        cudaMemcpyAsync(B.c_flag.p, b.flag + j0, (size_t)n_carry * 2, cudaMemcpyDeviceToDevice, s);
+        cudaMemcpyAsync(B.c_mapq.p, b.mapq + j0, (size_t)n_carry, cudaMemcpyDeviceToDevice, s);
+        k_bam_rebase_offsets<<<(unsigned)((n_carry + 255) / 256), 256, 0, s>>>(n_carry, b.cig_off + j0, o0, B.c_off.as<uint32_t>());
+        if (carry_ops) cudaMemcpyAsync(B.c_cig.p, b.cig + o0, (size_t)carry_ops * 4, cudaMemcpyDeviceToDevice, s);
+        *n_carry_out = n_carry; *carry_ops_out = carry_ops;
+      }
+    }
+    if (cudaGetLastError() != cudaSuccess) return bfail(ctx, MCOV_ERR_CUDA, "mcov_bam_gpu_stream_depth: carry copy failed");
+    return MCOV_OK;
+  }
+};
+
+}  // namespace
+
+extern "C" int mcov_bam_gpu_stream_depth(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, int verify_crc,
+                                         mcov_bam_gpu_stream_info* info) {
+  if (!ctx) return MCOV_ERR_ARG;
+  if (!path || !info) return bfail(ctx, MCOV_ERR_ARG, "mcov_bam_gpu_stream_depth: bad arguments");
+  std::memset(info, 0, sizeof(*info));
+  DepthSink sink;
+  return bam_gpu_chunks(ctx, path, chunk_bytes, verify_crc, info, "mcov_bam_gpu_stream_depth", sink);
 }
 
 // The device decoder compiled for the host: lets the CPU test suite check inflate.cuh against zlib

@@ -56,6 +56,7 @@ enum KernelId {
   kKExpPrep, kKExpEntries, kKExpRegion, kKExpRevsum, kKRegionHist, kKHistFinish, kKRunCount, kKRunOffsets, kKRunWrite, kKRunEnds, kKBgzfInflate, kKBamGuess, kKBamWalkCount, kKBamWalkWrite, kKDeltaUnpack, kKStreamAcc, kKFusedPrepTma, kKFusedTileTma, kKStatsStream, kKBlockUnpack, kKBamNamesSeq,
   kKSamNlCount, kKSamNlWrite, kKSamFields, kKSamCigar, kKSamNamesSeq, kKMapCounts,
   kKCapExact, kKSamLineMax,
+  kKBcAny,
   kKernelCount
 };
 
@@ -78,6 +79,33 @@ struct ReadStage {            // one staging set for host-resident batches
   cudaEvent_t consumed = nullptr;   // recorded after the kernel that read this set
   bool in_flight = false;
 };
+
+}  // namespace mcov
+
+struct mcov_bam_gpu_stream_info;
+
+namespace mcov {
+
+// One batch of the streamed BAM decode (bam_gpu_chunks): device columns of n records, the first n_carry of them carried
+// over from the previous batch (their rec_off points into bytes that are gone); data / rec_off locate the records
+// [n_carry, n) in this chunk's inflated stream.
+struct BamChunk {
+  int64_t n, n_carry, n_ops;
+  const int32_t* tid; const int32_t* pos; const uint16_t* flag; const uint8_t* mapq; const int32_t* l_seq;
+  const uint32_t* cig_off; const uint32_t* cig;
+  const uint8_t* data; const uint64_t* rec_off;
+  bool last;
+};
+// A consumer of the streamed decode: begin() once the file is open, batch() for every chunk.  batch() sets how many of
+// the batch's last reads (and their ops) lead the next one.
+struct BamChunkSink {
+  virtual int begin(mcov_ctx*) { return 0; }
+  virtual int batch(mcov_ctx* ctx, const BamChunk& b, int64_t* n_carry, int64_t* carry_ops) = 0;
+  virtual ~BamChunkSink() {}
+};
+// bam_gpu.cu: the chunk loop of mcov_bam_gpu_stream_depth; `who` prefixes the error texts
+int bam_gpu_chunks(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, int verify_crc, mcov_bam_gpu_stream_info* info,
+                   const char* who, BamChunkSink& sink);
 
 }  // namespace mcov
 
@@ -153,6 +181,13 @@ struct mcov_ctx {
       pin[0].release(); pin[1].release();
     }
   } bam;
+
+  // A / C / G / T counts of the last mcov_base_counts (basecount.cu): [n_slots][4] uint32, for (bc_qthr, bc_mode) of
+  // the contig table of epoch bc_epoch; the error word.  Apart from the depth store and its caches.
+  mcov::DevBuf d_bc, d_bc_word;
+  bool bc_ready = false;
+  int32_t bc_qthr = 0, bc_mode = 0;
+  int64_t bc_epoch = -1;
 
   // fused (sorted) path scratch
   mcov::DevBuf d_start_slot, d_far_list, d_tile_cnt, d_tile_off, d_far_sorted;

@@ -19,6 +19,8 @@ constexpr unsigned long long kSamNoErr = ~0ull;
 
 constexpr uint64_t kSamMaxOpLen = (1u << 28) - 1u;
 
+struct SamAux { uint32_t l_qname, cig_b, cig_e, seq_b; };              // field offsets from the line start (device decode)
+
 // unsigned decimal of [p, p + n) in [0, max]; false for an empty field, a non-digit or a value past max
 MCOV_HD bool sam_dec_u(const uint8_t* p, uint32_t n, uint64_t max, uint64_t* v) {
   if (n == 0) return false;

@@ -44,8 +44,6 @@ constexpr int kSamRounds = 8;                                          // 16-byt
 constexpr uint64_t kSamTile = (uint64_t)kSamThreads * 16 * kSamRounds; // 32 KiB
 constexpr int kSamWarps = kSamThreads / 32;
 
-struct SamAux { uint32_t l_qname, cig_b, cig_e, seq_b; };              // field offsets from the line start
-
 // 16-bit mask of the bytes of v equal to c (exact SWAR zero-byte test per 32-bit word)
 __device__ __forceinline__ uint32_t byte_eq_mask16(uint4 v, uint32_t c) {
   const uint32_t rep = c * 0x01010101u;

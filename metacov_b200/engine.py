@@ -5,6 +5,7 @@ depth of every contig of one BAM (the quantity reference metacov/pileup.py:
 10-16 rebuilds per region) and answers region queries from it.
 """
 import ctypes as C
+import os
 from collections import namedtuple
 
 import numpy as np
@@ -269,6 +270,21 @@ class CoverageEngine:
     def sync(self):
         """Wait for everything enqueued on the engine's stream."""
         self._check(lib.mcov_sync(self._ctx))
+
+    # -- A / C / G / T counts -------------------------------------------------
+    def base_counts(self, quality_threshold=15, mode=_capi.MCOV_BC_ALL, path=None, chunk_bytes=0):
+        """A / C / G / T counts at every position of every contig (``mcov_base_counts``): of the file last decoded on this
+        engine (``bamgpu.decode`` / ``decode_sam``), or of the BAM at ``path`` through the streamed decoder.  ``mode``:
+        MCOV_BC_ALL or MCOV_BC_NOFILTER.  The depth is left as it was."""
+        p = os.fsencode(path) if path is not None else None
+        self._check(lib.mcov_base_counts(self._ctx, p, int(chunk_bytes), int(quality_threshold), int(mode)))
+
+    def copy_base_counts(self, tid, start=0, end=None):
+        """uint32 [4, end - start]: the A, C, G and T counts of [start, end) of contig ``tid`` (``base_counts`` first)."""
+        end = int(self.lengths[tid]) if end is None else int(end)
+        out = np.empty((4, max(end - int(start), 0)), dtype=np.uint32)
+        self._check(lib.mcov_copy_base_counts(self._ctx, int(tid), int(start), end, _capi.ptr(out)))
+        return out
 
     # -- accounting ---------------------------------------------------------
     def launch_count(self):
