@@ -764,6 +764,64 @@ int  mcov_base_counts(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, int3
  * MCOV_ERR_ARG for a region outside the contig.  Synchronises. */
 int  mcov_copy_base_counts(mcov_ctx* ctx, int32_t tid, int32_t start, int32_t end, uint32_t* host_out);
 
+/* Alleles from the counts of the last mcov_base_counts (csrc/alleles.cu; the
+ * rules are restated in oracle/alleles.py).  At a position with counts n_A,
+ * n_C, n_G, n_T and N their 64-bit sum:
+ *   covered    N >= min_coverage;
+ *   present    allele b: n_b >= min_count and (double)n_b >= min_freq * (double)N;
+ *   consensus  the largest count, ties to the first of A C G T;
+ *   pi_p       1 - ((fA*fA + fC*fC) + (fG*fG + fT*fT)), f_b = (double)n_b / N,
+ *              in this order and without FMA contraction (bit-identical to numpy);
+ *   kind       at a covered position: 1 SNV (two or more alleles present),
+ *              2 SUB (reference base known, consensus differs), 4 POPSUB
+ *              (reference base known, some allele present, the reference's not).
+ * The reference base of a position is A, C, G or T from mcov_set_reference
+ * (case-insensitive); anything else, or use_reference = 0, is unknown.
+ * min_coverage >= 1, min_count >= 1, 0 <= min_freq <= 1, use_reference 0 / 1,
+ * else MCOV_ERR_ARG.  MCOV_ERR_STATE without counts for the current contig
+ * table, or with use_reference while some contig has had no mcov_set_reference
+ * since the last mcov_set_contigs.  The depth store, its statistics caches and
+ * the counts are never written; after an error the context is usable. */
+typedef struct mcov_allele_params {
+  uint32_t min_coverage, min_count;
+  double   min_freq;
+  int32_t  use_reference;
+  int32_t  pad;
+} mcov_allele_params;
+/* One region: length = end - start (positions past the contig end have zero
+ * counts), depth_sum = sum of N, pi_sum = sum of pi_p over covered positions
+ * (summed in a fixed order: the same counts give the same bits), the others
+ * count positions.  64 bytes. */
+typedef struct mcov_allele_stats {
+  int64_t length, covered, depth_sum;
+  double  pi_sum;
+  int64_t snv, ref_covered, sub, popsub;
+} mcov_allele_stats;
+/* One site (kind != 0): 0-based position, the counts, ref 'A' 'C' 'G' 'T' or
+ * 'N' (unknown), consensus 'A' 'C' 'G' or 'T', kind bits.  32 bytes. */
+typedef struct mcov_allele_site {
+  int32_t  tid, pos;
+  uint32_t cnt[4];
+  uint8_t  ref, consensus, kind, pad[5];
+} mcov_allele_site;
+/* The reference of contig tid: n ASCII bytes, n the contig's length, kept on
+ * the device (one byte a slot) until the next mcov_set_contigs.  MCOV_ERR_NOMEM,
+ * before anything is allocated, when the store does not fit the free device
+ * memory (the message holds both byte counts).  Synchronises. */
+int  mcov_set_reference(mcov_ctx* ctx, int32_t tid, const char* ascii, int32_t n);
+/* The records of g regions [start, end) of contig tid (0 <= start <= end; a
+ * region may overlap others and reach past its contig) into host_out[g].
+ * Synchronises. */
+int  mcov_allele_stats_run(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int32_t* start, const int32_t* end,
+                           const mcov_allele_params* params, mcov_allele_stats* host_out);
+/* Every site of every contig, in slot order (= by tid, then pos), into a list
+ * kept on the device; their number in *n_sites_out.  Synchronises. */
+int  mcov_allele_sites(mcov_ctx* ctx, const mcov_allele_params* params, int64_t* n_sites_out);
+/* The sites [first, first + n) of the last mcov_allele_sites into host_out[n].
+ * MCOV_ERR_STATE without a list for the current contig table, MCOV_ERR_ARG for
+ * a range outside it.  Synchronises. */
+int  mcov_allele_sites_read(mcov_ctx* ctx, int64_t first, int64_t n, mcov_allele_site* host_out);
+
 /* Test hooks: the device inflate / CRC-32 code (csrc/inflate.cuh) compiled for the host, so that the CPU
  * suite can check it against zlib.  mcov_inflate_host returns 0 or a positive decoder status. */
 int  mcov_inflate_host(const uint8_t* src, uint32_t clen, uint8_t* dst, uint32_t ulen);

@@ -59,6 +59,25 @@ REGION_STATS_DTYPE = np.dtype([
 assert REGION_STATS_DTYPE.itemsize == C.sizeof(RegionStats) == 64
 
 
+class AlleleParams(C.Structure):
+    """mcov_allele_params."""
+    _fields_ = [("min_coverage", C.c_uint32), ("min_count", C.c_uint32), ("min_freq", C.c_double),
+                ("use_reference", C.c_int32), ("pad", C.c_int32)]
+
+
+ALLELE_STATS_DTYPE = np.dtype([
+    ("length", "<i8"), ("covered", "<i8"), ("depth_sum", "<i8"), ("pi_sum", "<f8"), ("snv", "<i8"),
+    ("ref_covered", "<i8"), ("sub", "<i8"), ("popsub", "<i8")])
+assert ALLELE_STATS_DTYPE.itemsize == 64      # mcov_allele_stats
+
+# mcov_allele_site: the counts as A C G T, ref / consensus as one ASCII letter, kind bits (1 SNV, 2 SUB, 4 POPSUB)
+ALLELE_SITE_DTYPE = np.dtype({
+    "names": ["tid", "pos", "A", "C", "G", "T", "ref", "consensus", "kind"],
+    "formats": ["<i4", "<i4", "<u4", "<u4", "<u4", "<u4", "S1", "S1", "u1"],
+    "offsets": [0, 4, 8, 12, 16, 20, 24, 25, 26], "itemsize": 32})
+ALLELE_SNV, ALLELE_SUB, ALLELE_POPSUB = 1, 2, 4
+
+
 class BamGpuStreamInfo(C.Structure):
     _fields_ = [("n_records", C.c_int64), ("n_chunks", C.c_int64), ("n_segments", C.c_int64), ("inflated_bytes", C.c_int64),
                 ("file_bytes", C.c_int64), ("max_carry", C.c_int64)]
@@ -162,6 +181,10 @@ SIGNATURES = {
     "mcov_bam_gpu_mapped": (C.c_int, [_vp, C.POINTER(_i64), C.POINTER(_i64)]),
     "mcov_base_counts": (C.c_int, [_vp, C.c_char_p, _i64, _i32, C.c_int]),
     "mcov_copy_base_counts": (C.c_int, [_vp, _i32, _i32, _i32, _vp]),
+    "mcov_set_reference": (C.c_int, [_vp, _i32, C.c_char_p, _i32]),
+    "mcov_allele_stats_run": (C.c_int, [_vp, _i64, _vp, _vp, _vp, C.POINTER(AlleleParams), _vp]),
+    "mcov_allele_sites": (C.c_int, [_vp, C.POINTER(AlleleParams), C.POINTER(_i64)]),
+    "mcov_allele_sites_read": (C.c_int, [_vp, _i64, _i64, _vp]),
     "mcov_sam_parse_host": (C.c_int, [_vp, C.c_int64, C.POINTER(SamHostCols), C.c_char_p, C.c_int]),
     "mcov_inflate_host": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint32]),
     "mcov_inflate_host_win": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint32, C.c_uint32]),

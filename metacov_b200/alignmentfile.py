@@ -158,6 +158,12 @@ def is_sam_text(filename):
     return line.count(b"\t") >= 10
 
 
+def _check_read_callback(read_callback):
+    if callable(read_callback) or read_callback not in ("all", "nofilter"):
+        raise ValueError("read_callback must be 'all' or 'nofilter' (a callable is not supported: the counts are "
+                         "computed on the GPU), got %r" % (read_callback,))
+
+
 class AlignmentFile:
     def __init__(self, filename, mode="rb", device=0, decode="host", **kw):
         """decode="host": BGZF inflate and record parsing by the native host reader (csrc/bamio.cpp), streamed batch by
@@ -216,6 +222,7 @@ class AlignmentFile:
         self._stream = None
         self._bc_eng = None                                 # count_coverage of a file that is not resident on the device
         self._bc_key = None                                 # (threshold, mode) of the counts held
+        self._ref_fasta = None                              # the FASTA whose sequences the count engine holds
         if decode == "gpu":
             self._open_gpu(filename, device)
             return
@@ -240,7 +247,7 @@ class AlignmentFile:
         self.stream_batches = 0
         self._gpu = self._soa = self._engine = self._filter_kw = self._index_stats = None
         self._h = self._stream = None
-        self._bc_eng = self._bc_key = None
+        self._bc_eng = self._bc_key = self._ref_fasta = None
         self._pipe_consumer = None
         self._pipe_read = False
         self._pipe_reader = None
@@ -764,9 +771,7 @@ class AlignmentFile:
         the resident records; others (``decode="host"`` / ``"gpu-stream"``) go through the GPU decoder chunk by chunk.
         The depth and its statistics are left as they were.  A piped stream raises ValueError."""
         self._no_records("count_coverage()")
-        if callable(read_callback) or read_callback not in ("all", "nofilter"):
-            raise ValueError("read_callback must be 'all' or 'nofilter' (a callable is not supported: the counts are "
-                             "computed on the GPU), got %r" % (read_callback,))
+        _check_read_callback(read_callback)
         tid = self._tid[contig]                             # KeyError for unknown contigs, like pysam
         length = int(self.lengths[tid])
         start = 0 if start is None else int(start)
@@ -777,6 +782,12 @@ class AlignmentFile:
             raise ValueError("interval of size 0")
         if stop < start:
             raise ValueError("interval of size less than 0")
+        eng = self._counted(quality_threshold, read_callback)
+        c = eng.copy_base_counts(tid, start, stop)
+        return c[0], c[1], c[2], c[3]
+
+    def _counted(self, quality_threshold, read_callback):
+        """The count engine holding the counts of (threshold, read_callback): counted now unless they are held."""
         t = max(min(int(quality_threshold or 0), 2 ** 31 - 1), -2 ** 31)
         mode = _capi.MCOV_BC_NOFILTER if read_callback == "nofilter" else _capi.MCOV_BC_ALL
         eng = self._count_engine()
@@ -796,8 +807,72 @@ class AlignmentFile:
                     raise OSError("%s: %s" % (self.filename, e))
                 raise
             self._bc_key = (t, mode)
-        c = eng.copy_base_counts(tid, start, stop)
-        return c[0], c[1], c[2], c[3]
+        return eng
+
+    def allele_stats(self, contigs=None, starts=None, stops=None, fasta=None, quality_threshold=15, read_callback="all",
+                     min_coverage=5, min_freq=0.05, min_count=2):
+        """Allele statistics of regions from the A / C / G / T counts of ``count_coverage`` (same counts, same cache):
+        a structured array (``_capi.ALLELE_STATS_DTYPE``) with one record per region -- length, covered, depth_sum,
+        pi_sum, snv, ref_covered, sub, popsub; ``alleles.derive`` turns it into breadth, depth, pi, SNVs per kbp and the
+        consensus / population ANI.  The rules are those of ``mcov_allele_stats_run`` (include/metacov_b200.h).
+
+        Regions: ``contigs`` (names; default every contig), ``starts`` (default 0) and ``stops`` (default the contig
+        length), 0-based half-open; they may overlap and reach past the contig end.  ``fasta`` (a ``FastaFile``, or
+        anything with ``references`` and ``fetch``) gives the reference bases for SUB / POPSUB: each contig is looked up
+        by the first word of its name and must have the contig's length, else ValueError naming it; a FASTA is sent to
+        the GPU once per file.  Without it the reference is unknown everywhere.  Bad parameters or regions raise
+        ValueError, an unknown contig KeyError, a piped stream ValueError."""
+        eng, use_ref = self._allele_engine("allele_stats()", fasta, quality_threshold, read_callback,
+                                           min_coverage, min_freq, min_count)
+        if contigs is None:
+            contigs = self.references
+        elif isinstance(contigs, str):
+            contigs = [contigs]
+        tid = np.array([self._tid[c] for c in contigs], dtype=np.int64)
+        lengths = np.asarray(self.lengths, dtype=np.int64)
+        start = np.zeros(len(tid), np.int64) if starts is None else np.asarray(starts, dtype=np.int64).reshape(-1)
+        stop = lengths[tid] if stops is None else np.asarray(stops, dtype=np.int64).reshape(-1)
+        if not len(start) == len(stop) == len(tid):
+            raise ValueError("contigs, starts and stops differ in length")
+        if len(tid) and (start.min() < 0 or (stop < start).any() or stop.max() >= 2 ** 31):
+            raise ValueError("regions need 0 <= start <= stop < 2^31")
+        return eng.allele_stats(tid, start, stop, min_coverage, min_freq, min_count, use_reference=use_ref)
+
+    def allele_sites(self, fasta=None, quality_threshold=15, read_callback="all", min_coverage=5, min_freq=0.05,
+                     min_count=2):
+        """Every site -- a covered position where two or more alleles are present (SNV, kind bit 1) or, with ``fasta``,
+        where the consensus differs from the reference (SUB, 2) or the reference base is not present (POPSUB, 4) -- in
+        (tid, pos) order: a structured array (``_capi.ALLELE_SITE_DTYPE``: tid pos A C G T ref consensus kind).
+        Arguments as in ``allele_stats``."""
+        eng, use_ref = self._allele_engine("allele_sites()", fasta, quality_threshold, read_callback,
+                                           min_coverage, min_freq, min_count)
+        return eng.allele_sites(min_coverage, min_freq, min_count, use_reference=use_ref)
+
+    def _allele_engine(self, what, fasta, quality_threshold, read_callback, min_coverage, min_freq, min_count):
+        """The count engine with the counts of (threshold, read_callback) and, given a FASTA, its reference."""
+        self._no_records(what)
+        _check_read_callback(read_callback)
+        CoverageEngine._allele_params(min_coverage, min_freq, min_count, False)      # (ValueError before any work)
+        eng = self._counted(quality_threshold, read_callback)
+        if fasta is not None and self._ref_fasta is not fasta:
+            self._ref_fasta = None
+            names = set(fasta.references)
+            for tid, name in enumerate(self.references):
+                key = (name.split() or [name])[0]
+                if key not in names:
+                    raise ValueError("%s: contig %r is not in the reference FASTA" % (self.filename, name))
+                seq = fasta.fetch(key)
+                if len(seq) != int(self.lengths[tid]):
+                    raise ValueError("%s: contig %r is %d long in the reference FASTA and %d in the alignments"
+                                     % (self.filename, name, len(seq), int(self.lengths[tid])))
+                try:
+                    eng.set_reference(tid, seq)
+                except McovError as e:
+                    if e.code == _capi.MCOV_ERR_NOMEM:
+                        raise MemoryError("%s: %s" % (self.filename, e))
+                    raise
+            self._ref_fasta = fasta
+        return eng, fasta is not None
 
     def _count_engine(self):
         """The engine that counts: a device-decoded file's own (it holds the records); else one of the counts' own."""

@@ -18,6 +18,7 @@ from . import pileup as _pileup
 from . import scan as _scan
 from . import util
 from .alignmentfile import AlignmentFile
+from .alleles import derive
 from .samstream import is_stream
 from .fasta import FastaFile
 
@@ -237,6 +238,76 @@ def scan(readfile, readfile_type, out_basehist, boffset, out_kmerhist, k, number
     if out_isizehist:
         csv.writer(out_isizehist).writerows(counters.get_rows(n))
         n += 1
+
+
+@main.command()
+@click.option("--bamfile", "-b", type=click.Path(dir_okay=False, allow_dash=True), required=True,
+              help="Input BAM or SAM file (any read order, no index needed). Not a pipe: the counts need every record.")
+@click.option("--reference-fasta", "-f", type=click.Path(exists=True, dir_okay=False),
+              help="Reference the reads were mapped to: enables SUB / POPSUB, con_ani and pop_ani.")
+@click.option("--regionfile-blast7", "-rb", type=click.File("r"), help="Input Region file in BLAST7 format")
+@click.option("--regionfile-csv", "-rc", type=click.File("r"), help="Input Region file in CSV format")
+@click.option("--outfile", "-o", type=click.File("w"), default="-", help="Output CSV (default STDOUT)")
+@click.option("--sites-out", type=click.File("w"), metavar="FILE",
+              help="Also write every site as TSV: contig pos ref A C G T consensus snv sub popsub (pos 0-based).")
+@click.option("--quality-threshold", "-q", type=int, default=15, show_default=True,
+              help="Count a base only with a quality of at least this (0: every base).")
+@click.option("--read-callback", type=click.Choice(["all", "nofilter"]), default="all", show_default=True,
+              help="all: skip unmapped, secondary, QC-fail and duplicate reads; nofilter: count every placed read.")
+@click.option("--min-coverage", type=click.IntRange(1), default=5, show_default=True)
+@click.option("--min-freq", type=click.FloatRange(0, 1), default=0.05, show_default=True)
+@click.option("--min-count", type=click.IntRange(1), default=2, show_default=True)
+@click.option("--bam-decode", type=click.Choice(["host", "gpu", "gpu-stream", "auto"]), default="auto", show_default=True,
+              help="Where the BAM file is inflated and parsed (see `pileup`).")
+def alleles(bamfile, reference_fasta, regionfile_blast7, regionfile_csv, outfile, sites_out, quality_threshold,
+            read_callback, min_coverage, min_freq, min_count, bam_decode):
+    """
+    Allele statistics per region from the A/C/G/T counts on the GPU: breadth, depth, nucleotide diversity (pi), SNVs
+    per kbp and, with a reference, consensus and population ANI.  Not in the reference: additive.
+    """
+    if is_stream(bamfile):
+        raise click.UsageError("-b/--bamfile: the allele counts need every record of a file; a piped stream cannot give "
+                               "them (write the alignments to a file)")
+    regions = None
+    if regionfile_blast7 or regionfile_csv:
+        regions = util.make_region_iterator(regionfile_blast7, regionfile_csv, None)
+    bam = AlignmentFile(bamfile, decode=bam_decode)
+    fasta = FastaFile(reference_fasta) if reference_fasta else None
+    if regions is None:
+        regions = util.get_regions_from_bam(bam)
+    name2ref = {word.split()[0]: word for word in bam.references}
+    hits = list(regions)
+    refs, starts, ends = [], [], []
+    for hit in hits:
+        refs.append(name2ref[hit.sacc])
+        start, end = sorted((int(hit.sstart), int(hit.send)))      # (as `pileup`: blast's reverse strand has end < start)
+        starts.append(start)
+        ends.append(end)
+    kw = dict(fasta=fasta, quality_threshold=quality_threshold, read_callback=read_callback,
+              min_coverage=min_coverage, min_freq=min_freq, min_count=min_count)
+    if hits:
+        derived = derive(bam.allele_stats(refs, starts, ends, **kw))
+        writer = csv.DictWriter(outfile, fieldnames=["sacc", "start", "end"] + sorted(derived))
+        writer.writeheader()
+        for k, hit in enumerate(hits):
+            row = {name: float(v[k]) for name, v in derived.items()}
+            row.update({"sacc": hit.sacc, "start": hit.sstart, "end": hit.send})
+            writer.writerow(row)
+    if sites_out is not None:
+        write_sites(bam, bam.allele_sites(**kw), sites_out)
+    bam.close()
+
+
+def write_sites(bam, sites, out):
+    """Sites as TSV lines: contig (first word of its name), 0-based position, reference base (N: unknown), the A C G T
+    counts, the consensus and the SNV / SUB / POPSUB flags as 0 / 1."""
+    names = [ref.split()[0] for ref in bam.references]
+    out.write("contig\tpos\tref\tA\tC\tG\tT\tconsensus\tsnv\tsub\tpopsub\n")
+    kind = sites["kind"]
+    cols = [sites[k].tolist() for k in ("tid", "pos", "A", "C", "G", "T")]
+    for (t, p, a, c, g, tt), r, cons, k in zip(zip(*cols), sites["ref"].tolist(), sites["consensus"].tolist(), kind.tolist()):
+        out.write("%s\t%d\t%s\t%d\t%d\t%d\t%d\t%s\t%d\t%d\t%d\n" % (names[t], p, r.decode(), a, c, g, tt, cons.decode(),
+                                                                    k & 1, (k >> 1) & 1, (k >> 2) & 1))
 
 
 if __name__ == "__main__":

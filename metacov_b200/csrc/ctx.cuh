@@ -57,6 +57,7 @@ enum KernelId {
   kKSamNlCount, kKSamNlWrite, kKSamFields, kKSamCigar, kKSamNamesSeq, kKMapCounts,
   kKCapExact, kKSamLineMax,
   kKBcAny,
+  kKRefEncode, kKAlleleChunks, kKAlleleCombine, kKAlleleSiteCount, kKAlleleSiteWrite,
   kKernelCount
 };
 
@@ -188,6 +189,14 @@ struct mcov_ctx {
   bool bc_ready = false;
   int32_t bc_qthr = 0, bc_mode = 0;
   int64_t bc_epoch = -1;
+
+  // Alleles (alleles.cu): the reference store ([n_slots] codes 0-3 A C G T, 4 unknown) of the contig table of epoch
+  // ref_epoch and which contigs have been given one; the region and site scratch; the site list of the last
+  // mcov_allele_sites (n_sites of them, -1 = none) for the contig table of epoch sites_epoch.
+  mcov::DevBuf d_ref, d_ref_stage, d_al_chunks, d_al_part, d_al_meta, d_al_out, d_al_tiles, d_al_scan, d_sites;
+  std::vector<uint8_t> ref_set;
+  int64_t ref_epoch = -1;
+  int64_t n_sites = -1, sites_epoch = -1;
 
   // fused (sorted) path scratch
   mcov::DevBuf d_start_slot, d_far_list, d_tile_cnt, d_tile_off, d_far_sorted;

@@ -605,7 +605,9 @@ void mcov_destroy(mcov_ctx* ctx) {
                     &ctx->d_tasks, &ctx->d_rlen, &ctx->d_done,
                     &ctx->d_cap_scratch, &ctx->d_flag_lut, &ctx->d_stream_acc, &ctx->d_ss_pieces, &ctx->d_ss_cta, &ctx->d_ss_split, &ctx->d_ss_pool,
                     &ctx->d_out, &ctx->d_win_slot, &ctx->d_win_n, &ctx->d_win_out, &ctx->d_htasks, &ctx->d_tile_heavy, &ctx->d_run_tasks, &ctx->d_run_counts, &ctx->d_run_out,
-                    &ctx->d_starts, &ctx->d_bc, &ctx->d_bc_word};
+                    &ctx->d_starts, &ctx->d_bc, &ctx->d_bc_word,
+                    &ctx->d_ref, &ctx->d_ref_stage, &ctx->d_al_chunks, &ctx->d_al_part, &ctx->d_al_meta, &ctx->d_al_out,
+                    &ctx->d_al_tiles, &ctx->d_al_scan, &ctx->d_sites};
   for (DevBuf* b : bufs) b->release();
   ctx->bam.release();
   ctx->h_pin.release();
@@ -1091,7 +1093,8 @@ static const char* kKernelNames[kKernelCount] = {
     "k_fused_prep_tma", "k_fused_tile_tma", "k_stats_stream", "k_block_unpack", "k_bam_names_seq",
     "k_sam_nl_count", "k_sam_nl_write", "k_sam_fields", "k_sam_cigar", "k_sam_names_seq", "k_dev_map_counts",
     "k_cap_exact", "k_sam_line_max",
-    "k_bc_any"};
+    "k_bc_any",
+    "k_ref_encode", "k_allele_chunks", "k_allele_combine", "k_allele_site_count", "k_allele_site_write"};
 
 int mcov_copy_to_host(mcov_ctx* ctx, const void* dev, void* host, int64_t n_bytes) {
   if (!ctx) return MCOV_ERR_ARG;

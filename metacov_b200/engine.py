@@ -286,6 +286,50 @@ class CoverageEngine:
         self._check(lib.mcov_copy_base_counts(self._ctx, int(tid), int(start), end, _capi.ptr(out)))
         return out
 
+    # -- alleles (from the counts of base_counts) ---------------------------------------------------------------------
+    def set_reference(self, tid, seq):
+        """The reference of contig ``tid`` (str or bytes, exactly the contig's length) for ``use_reference=True``."""
+        b = seq.encode("ascii") if isinstance(seq, str) else bytes(seq)
+        self._check(lib.mcov_set_reference(self._ctx, int(tid), b, len(b)))
+
+    @staticmethod
+    def _allele_params(min_coverage, min_freq, min_count, use_reference):
+        p = _capi.AlleleParams()
+        for name, v, lo in (("min_coverage", min_coverage, 1), ("min_count", min_count, 1)):
+            if int(v) != v or not lo <= int(v) < 2 ** 32:
+                raise ValueError("%s must be an integer >= %d, got %r" % (name, lo, v))
+        if not 0.0 <= float(min_freq) <= 1.0:
+            raise ValueError("min_freq must be in [0, 1], got %r" % (min_freq,))
+        p.min_coverage, p.min_count, p.min_freq = int(min_coverage), int(min_count), float(min_freq)
+        p.use_reference = 1 if use_reference else 0
+        return p
+
+    def allele_stats(self, tid, start, end, min_coverage=5, min_freq=0.05, min_count=2, use_reference=False):
+        """Allele statistics of g regions (``mcov_allele_stats_run``) -> structured array ``_capi.ALLELE_STATS_DTYPE``
+        (length, covered, depth_sum, pi_sum, snv, ref_covered, sub, popsub).  Needs ``base_counts`` first, and with
+        ``use_reference`` a ``set_reference`` of every contig."""
+        tid = np.ascontiguousarray(tid, dtype=np.int32)
+        start = np.ascontiguousarray(start, dtype=np.int32)
+        end = np.ascontiguousarray(end, dtype=np.int32)
+        g = len(tid)
+        if not (len(start) == len(end) == g):
+            raise ValueError("tid/start/end lengths differ")
+        p = self._allele_params(min_coverage, min_freq, min_count, use_reference)
+        out = np.zeros(g, dtype=_capi.ALLELE_STATS_DTYPE)
+        self._check(lib.mcov_allele_stats_run(self._ctx, g, _capi.ptr(tid), _capi.ptr(start), _capi.ptr(end), C.byref(p),
+                                              _capi.ptr(out)))
+        return out
+
+    def allele_sites(self, min_coverage=5, min_freq=0.05, min_count=2, use_reference=False):
+        """Every site (a covered position of kind SNV, SUB or POPSUB) in (tid, pos) order -> structured array
+        ``_capi.ALLELE_SITE_DTYPE`` (tid pos A C G T ref consensus kind)."""
+        p = self._allele_params(min_coverage, min_freq, min_count, use_reference)
+        n = C.c_int64(0)
+        self._check(lib.mcov_allele_sites(self._ctx, C.byref(p), C.byref(n)))
+        out = np.zeros(n.value, dtype=_capi.ALLELE_SITE_DTYPE)
+        self._check(lib.mcov_allele_sites_read(self._ctx, 0, n.value, _capi.ptr(out)))
+        return out
+
     # -- accounting ---------------------------------------------------------
     def launch_count(self):
         return lib.mcov_launch_count(self._ctx)
