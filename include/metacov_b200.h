@@ -822,6 +822,56 @@ int  mcov_allele_sites(mcov_ctx* ctx, const mcov_allele_params* params, int64_t*
  * a range outside it.  Synchronises. */
 int  mcov_allele_sites_read(mcov_ctx* ctx, int64_t first, int64_t n, mcov_allele_site* host_out);
 
+/* Samples compared position by position (csrc/compare.cu; the rules are
+ * restated in oracle/compare.py).  A sample keeps one signature byte a slot,
+ * made from its counts with the allele rules above (no reference):
+ *   0x80       covered;
+ *   bits 4-5   the consensus (0-3 = A C G T);
+ *   bits 0-3   the present mask (bit b: allele b present);
+ * 0x00 where not covered, and in every padding and end slot.  For a pair
+ * (a, b) at a position: compared = covered in both; the allele set of a sample
+ * is its present mask OR its consensus' bit (never empty where covered);
+ * con_snp = compared and the consensuses differ; pop_snp = compared and the
+ * two allele sets are disjoint (a pop_snp is always a con_snp).  The pair calls
+ * take sig[n_sig], device arrays of mcov_n_slots(ctx) signature bytes on ctx's
+ * GPU (4-byte aligned) made under a contig table equal to ctx's, and
+ * pairs[2 * n_pairs], indices into sig with a != b.  MCOV_ERR_ARG for fewer
+ * than two signatures, no pair, a pair index out of range or a == b, a pointer
+ * that is null or not device memory on ctx's GPU, or a bad region;
+ * MCOV_ERR_STATE without a contig table.  The depth store, its caches, the
+ * counts and the reference store are never written; after an error the
+ * context is usable. */
+/* One (pair, region): length = end - start, positions covered in a, in b, in
+ * both (compared), con_snp and pop_snp positions.  48 bytes. */
+typedef struct mcov_compare_stats {
+  int64_t length, covered_a, covered_b, compared, con_snp, pop_snp;
+} mcov_compare_stats;
+/* One site of a pair (a con_snp position): the pair's index, the position, both
+ * signature bytes, kind bits 1 con_snp (always set), 2 pop_snp.  16 bytes. */
+typedef struct mcov_compare_site {
+  int32_t pair, tid, pos;
+  uint8_t sig_a, sig_b, kind, pad;
+} mcov_compare_site;
+/* The signature of every slot from the counts of the last mcov_base_counts into
+ * dev_out[mcov_n_slots(ctx)] (device memory on ctx's GPU).
+ * params->use_reference must be 0 (else MCOV_ERR_ARG).  MCOV_ERR_STATE without
+ * counts for the current contig table.  Synchronises. */
+int  mcov_allele_signature(mcov_ctx* ctx, const mcov_allele_params* params, uint8_t* dev_out);
+/* The records of every pair over g regions [start, end) of contig tid
+ * (0 <= start <= end; regions may overlap and reach past their contig, where
+ * nothing is covered) into host_out[n_pairs * g], pair-major.  Synchronises. */
+int  mcov_compare_run(mcov_ctx* ctx, int32_t n_sig, const uint8_t* const* sig, int32_t n_pairs, const int32_t* pairs,
+                      int64_t g, const int32_t* tid, const int32_t* start, const int32_t* end, mcov_compare_stats* host_out);
+/* Every site of every pair, in (pair, tid, pos) order, into a list kept on the
+ * device; their number in *n_sites_out.  MCOV_ERR_NOMEM, with the byte count,
+ * when the list does not fit.  Synchronises. */
+int  mcov_compare_sites(mcov_ctx* ctx, int32_t n_sig, const uint8_t* const* sig, int32_t n_pairs, const int32_t* pairs,
+                        int64_t* n_sites_out);
+/* The sites [first, first + n) of the last mcov_compare_sites into
+ * host_out[n].  MCOV_ERR_STATE without a list for the current contig table,
+ * MCOV_ERR_ARG for a range outside it.  Synchronises. */
+int  mcov_compare_sites_read(mcov_ctx* ctx, int64_t first, int64_t n, mcov_compare_site* host_out);
+
 /* Test hooks: the device inflate / CRC-32 code (csrc/inflate.cuh) compiled for the host, so that the CPU
  * suite can check it against zlib.  mcov_inflate_host returns 0 or a positive decoder status. */
 int  mcov_inflate_host(const uint8_t* src, uint32_t clen, uint8_t* dst, uint32_t ulen);

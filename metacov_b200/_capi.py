@@ -77,6 +77,20 @@ ALLELE_SITE_DTYPE = np.dtype({
     "offsets": [0, 4, 8, 12, 16, 20, 24, 25, 26], "itemsize": 32})
 ALLELE_SNV, ALLELE_SUB, ALLELE_POPSUB = 1, 2, 4
 
+COMPARE_STATS_DTYPE = np.dtype([
+    ("length", "<i8"), ("covered_a", "<i8"), ("covered_b", "<i8"), ("compared", "<i8"), ("con_snp", "<i8"),
+    ("pop_snp", "<i8")])
+assert COMPARE_STATS_DTYPE.itemsize == 48     # mcov_compare_stats
+
+# mcov_compare_site: the pair's index, the position, both signature bytes (0x80 covered, bits 4-5 consensus, bits 0-3
+# present mask), kind bits (1 con_snp, 2 pop_snp), pad (always 0).  The pad is a field so that every byte of a record
+# is defined: numpy leaves the gaps of a structured dtype uninitialised when it copies records (e.g. by a mask), and a
+# site list's bytes are then not comparable.
+COMPARE_SITE_DTYPE = np.dtype([("pair", "<i4"), ("tid", "<i4"), ("pos", "<i4"), ("sig_a", "u1"), ("sig_b", "u1"),
+                               ("kind", "u1"), ("pad", "u1")])
+assert COMPARE_SITE_DTYPE.itemsize == 16      # mcov_compare_site
+COMPARE_CON_SNP, COMPARE_POP_SNP = 1, 2
+
 
 class BamGpuStreamInfo(C.Structure):
     _fields_ = [("n_records", C.c_int64), ("n_chunks", C.c_int64), ("n_segments", C.c_int64), ("inflated_bytes", C.c_int64),
@@ -185,6 +199,10 @@ SIGNATURES = {
     "mcov_allele_stats_run": (C.c_int, [_vp, _i64, _vp, _vp, _vp, C.POINTER(AlleleParams), _vp]),
     "mcov_allele_sites": (C.c_int, [_vp, C.POINTER(AlleleParams), C.POINTER(_i64)]),
     "mcov_allele_sites_read": (C.c_int, [_vp, _i64, _i64, _vp]),
+    "mcov_allele_signature": (C.c_int, [_vp, C.POINTER(AlleleParams), _vp]),
+    "mcov_compare_run": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i64, _vp, _vp, _vp, _vp]),
+    "mcov_compare_sites": (C.c_int, [_vp, _i32, _vp, _i32, _vp, C.POINTER(_i64)]),
+    "mcov_compare_sites_read": (C.c_int, [_vp, _i64, _i64, _vp]),
     "mcov_sam_parse_host": (C.c_int, [_vp, C.c_int64, C.POINTER(SamHostCols), C.c_char_p, C.c_int]),
     "mcov_inflate_host": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint32]),
     "mcov_inflate_host_win": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint32, C.c_uint32]),

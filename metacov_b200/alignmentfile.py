@@ -824,6 +824,12 @@ class AlignmentFile:
         ValueError, an unknown contig KeyError, a piped stream ValueError."""
         eng, use_ref = self._allele_engine("allele_stats()", fasta, quality_threshold, read_callback,
                                            min_coverage, min_freq, min_count)
+        tid, start, stop = self._regions(contigs, starts, stops)
+        return eng.allele_stats(tid, start, stop, min_coverage, min_freq, min_count, use_reference=use_ref)
+
+    def _regions(self, contigs, starts, stops):
+        """(tid, start, stop) int64 arrays of regions given as in ``allele_stats``: ValueError for bad regions,
+        KeyError for an unknown contig."""
         if contigs is None:
             contigs = self.references
         elif isinstance(contigs, str):
@@ -836,7 +842,7 @@ class AlignmentFile:
             raise ValueError("contigs, starts and stops differ in length")
         if len(tid) and (start.min() < 0 or (stop < start).any() or stop.max() >= 2 ** 31):
             raise ValueError("regions need 0 <= start <= stop < 2^31")
-        return eng.allele_stats(tid, start, stop, min_coverage, min_freq, min_count, use_reference=use_ref)
+        return tid, start, stop
 
     def allele_sites(self, fasta=None, quality_threshold=15, read_callback="all", min_coverage=5, min_freq=0.05,
                      min_count=2):
@@ -847,6 +853,15 @@ class AlignmentFile:
         eng, use_ref = self._allele_engine("allele_sites()", fasta, quality_threshold, read_callback,
                                            min_coverage, min_freq, min_count)
         return eng.allele_sites(min_coverage, min_freq, min_count, use_reference=use_ref)
+
+    def allele_signature(self, quality_threshold=15, read_callback="all", min_coverage=5, min_freq=0.05, min_count=2):
+        """The signature of every slot of the count engine's table from the counts of ``count_coverage`` (same counts,
+        same cache): a CUDA ``torch.uint8`` tensor of ``n_slots`` bytes, 0x80 covered, bits 4-5 the consensus (0-3 =
+        A C G T), bits 0-3 the present mask, 0 where not covered.  It is what ``compare`` keeps of a file.  Arguments as
+        in ``allele_stats``; a piped stream raises ValueError."""
+        eng, _ = self._allele_engine("allele_signature()", None, quality_threshold, read_callback,
+                                     min_coverage, min_freq, min_count)
+        return eng.allele_signature(min_coverage, min_freq, min_count)
 
     def _allele_engine(self, what, fasta, quality_threshold, read_callback, min_coverage, min_freq, min_count):
         """The count engine with the counts of (threshold, read_callback) and, given a FASTA, its reference."""

@@ -26,3 +26,18 @@ def derive(stats):
         "con_ani": 1.0 - _ratio(s["sub"], s["ref_covered"]),
         "pop_ani": 1.0 - _ratio(s["popsub"], s["ref_covered"]),
     }
+
+
+COMPARE_DERIVED = ("con_ani", "percent_compared", "pop_ani")
+
+
+def derive_compare(stats):
+    """{name: float64 array} of the pair records of ``compare`` / ``CoverageEngine.compare_stats``:
+    con_ani = 1 - con_snp / compared, pop_ani = 1 - pop_snp / compared, percent_compared = compared / length.  A
+    division by zero gives NaN."""
+    s = stats
+    return {
+        "con_ani": 1.0 - _ratio(s["con_snp"], s["compared"]),
+        "percent_compared": _ratio(s["compared"], s["length"]),
+        "pop_ani": 1.0 - _ratio(s["pop_snp"], s["compared"]),
+    }

@@ -18,7 +18,8 @@ from . import pileup as _pileup
 from . import scan as _scan
 from . import util
 from .alignmentfile import AlignmentFile
-from .alleles import derive
+from .alleles import derive, derive_compare
+from .compare import compare as _compare, read_references
 from .samstream import is_stream
 from .fasta import FastaFile
 
@@ -308,6 +309,88 @@ def write_sites(bam, sites, out):
     for (t, p, a, c, g, tt), r, cons, k in zip(zip(*cols), sites["ref"].tolist(), sites["consensus"].tolist(), kind.tolist()):
         out.write("%s\t%d\t%s\t%d\t%d\t%d\t%d\t%s\t%d\t%d\t%d\n" % (names[t], p, r.decode(), a, c, g, tt, cons.decode(),
                                                                     k & 1, (k >> 1) & 1, (k >> 2) & 1))
+
+
+@main.command()
+@click.option("--bamfile", "-b", "bamfiles", type=click.Path(dir_okay=False, allow_dash=True), multiple=True, required=True,
+              help="Input BAM or SAM file, two or more times (any read order, no index; every file with the same "
+                   "reference names and lengths). Not a pipe: the counts need every record.")
+@click.option("--regionfile-blast7", "-rb", type=click.File("r"), help="Input Region file in BLAST7 format")
+@click.option("--regionfile-csv", "-rc", type=click.File("r"), help="Input Region file in CSV format")
+@click.option("--outfile", "-o", type=click.File("w"), default="-", help="Output CSV (default STDOUT)")
+@click.option("--sites-out", type=click.File("w"), metavar="FILE",
+              help="Also write every con_snp site of every pair as TSV: sample_a sample_b contig pos cons_a cons_b "
+                   "alleles_a alleles_b con_snp pop_snp (pos 0-based; alleles: the present alleles plus the consensus).")
+@click.option("--quality-threshold", "-q", type=int, default=15, show_default=True,
+              help="Count a base only with a quality of at least this (0: every base).")
+@click.option("--read-callback", type=click.Choice(["all", "nofilter"]), default="all", show_default=True,
+              help="all: skip unmapped, secondary, QC-fail and duplicate reads; nofilter: count every placed read.")
+@click.option("--min-coverage", type=click.IntRange(1), default=5, show_default=True)
+@click.option("--min-freq", type=click.FloatRange(0, 1), default=0.05, show_default=True)
+@click.option("--min-count", type=click.IntRange(1), default=2, show_default=True)
+@click.option("--bam-decode", type=click.Choice(["host", "gpu", "gpu-stream", "auto"]), default="auto", show_default=True,
+              help="Where the BAM file is inflated and parsed (see `pileup`).")
+def compare(bamfiles, regionfile_blast7, regionfile_csv, outfile, sites_out, quality_threshold, read_callback,
+            min_coverage, min_freq, min_count, bam_decode):
+    """
+    Compare samples per region and pair on the GPU: positions covered in both, consensus and population ANI (conANI /
+    popANI) from the A/C/G/T counts of each file.  Not in the reference: additive.
+    """
+    if len(bamfiles) < 2:
+        raise click.UsageError("-b/--bamfile: a comparison needs at least two files")
+    for f in bamfiles:
+        if is_stream(f):
+            raise click.UsageError("-b/--bamfile %s: the allele counts need every record of a file; a piped stream "
+                                   "cannot give them (write the alignments to a file)" % f)
+    names, lengths = read_references(bamfiles[0])
+    if regionfile_blast7 or regionfile_csv:
+        hits = list(util.make_region_iterator(regionfile_blast7, regionfile_csv, None))
+    else:
+        hits = [util.Region(n, name, 0, length) for n, (name, length) in enumerate(zip(names, lengths))]
+    name2ref = {word.split()[0]: word for word in names}
+    refs, starts, ends = [], [], []
+    for hit in hits:
+        refs.append(name2ref[hit.sacc])
+        start, end = sorted((int(hit.sstart), int(hit.send)))      # (as `pileup`: blast's reverse strand has end < start)
+        starts.append(start)
+        ends.append(end)
+    res = _compare(bamfiles, refs, starts, ends, sites=sites_out is not None, decode=bam_decode,
+                   quality_threshold=quality_threshold, read_callback=read_callback, min_coverage=min_coverage,
+                   min_freq=min_freq, min_count=min_count)
+    derived = derive_compare(res.stats)
+    cols = {"compared": res.stats["compared"], "con_snps": res.stats["con_snp"], "covered_a": res.stats["covered_a"],
+            "covered_b": res.stats["covered_b"], "pop_snps": res.stats["pop_snp"]}
+    cols.update(derived)
+    writer = csv.DictWriter(outfile, fieldnames=["sacc", "start", "end", "sample_a", "sample_b"] + sorted(cols))
+    writer.writeheader()
+    for k, hit in enumerate(hits):
+        for p, (a, b) in enumerate(res.pairs.tolist()):
+            row = {name: (int(v[p, k]) if v.dtype.kind == "i" else float(v[p, k])) for name, v in cols.items()}
+            row.update({"sacc": hit.sacc, "start": hit.sstart, "end": hit.send, "sample_a": bamfiles[a],
+                        "sample_b": bamfiles[b]})
+            writer.writerow(row)
+    if sites_out is not None:
+        write_compare_sites(names, bamfiles, res.pairs, res.sites, sites_out)
+
+
+def _alleles_of(sig):
+    """Letters of a signature byte's allele set: the present alleles plus the consensus, in A C G T order."""
+    bits = (sig & 0x0F) | (1 << ((sig >> 4) & 3))
+    return "".join(ch for b, ch in enumerate("ACGT") if bits >> b & 1)
+
+
+def write_compare_sites(references, samples, pairs, sites, out):
+    """Compare sites as TSV lines: the two samples as given, contig (first word of its name), 0-based position, both
+    consensus bases, both allele sets as letters (e.g. AG) and the con_snp / pop_snp flags as 0 / 1."""
+    names = [ref.split()[0] for ref in references]
+    out.write("sample_a\tsample_b\tcontig\tpos\tcons_a\tcons_b\talleles_a\talleles_b\tcon_snp\tpop_snp\n")
+    pairs = pairs.tolist()
+    cols = [sites[k].tolist() for k in ("pair", "tid", "pos", "sig_a", "sig_b", "kind")]
+    for p, t, pos, sa, sb, k in zip(*cols):
+        a, b = pairs[p]
+        out.write("%s\t%s\t%s\t%d\t%s\t%s\t%s\t%s\t%d\t%d\n" % (
+            samples[a], samples[b], names[t], pos, "ACGT"[(sa >> 4) & 3], "ACGT"[(sb >> 4) & 3], _alleles_of(sa),
+            _alleles_of(sb), k & 1, (k >> 1) & 1))
 
 
 if __name__ == "__main__":

@@ -23,9 +23,9 @@ static_assert(sizeof(mcov_allele_stats) == 64, "mcov_allele_stats is 64 bytes");
 static_assert(sizeof(mcov_allele_site) == 32, "mcov_allele_site is 32 bytes");
 static_assert(sizeof(AlPart) == 64, "AlPart is 64 bytes");
 
-namespace {
+namespace mcov {
 
-int al_fail(mcov_ctx* ctx, int code, const std::string& what, cudaError_t e = cudaSuccess) {
+int al_fail(mcov_ctx* ctx, int code, const std::string& what, cudaError_t e) {
   ctx->err = what;
   if (e != cudaSuccess) { ctx->err += ": "; ctx->err += cudaGetErrorString(e); }
   return code;
@@ -36,8 +36,6 @@ int al_fail(mcov_ctx* ctx, int code, const std::string& what, cudaError_t e = cu
     cudaError_t e__ = (call);                                                                             \
     if (e__ != cudaSuccess) return al_fail(ctx, MCOV_ERR_CUDA, std::string(who) + ": " + #call, e__);     \
   } while (0)
-
-constexpr int64_t kRefStageBytes = 64 << 20;      // the reference goes up in pieces of this size
 
 // Parameters and state shared by the region and site calls: the kernel's parameters, or an error.
 int al_check(mcov_ctx* ctx, const mcov_allele_params* p, AlleleParams* out, const char* who) {
@@ -65,6 +63,12 @@ int al_check(mcov_ctx* ctx, const mcov_allele_params* p, AlleleParams* out, cons
 unsigned al_grid(const mcov_ctx* ctx, int64_t items, int per) {
   return (unsigned)std::max<int64_t>(1, std::min<int64_t>((items + per - 1) / per, (int64_t)std::max(ctx->n_sm, 1) * 64));
 }
+
+}  // namespace mcov
+
+namespace {
+
+constexpr int64_t kRefStageBytes = 64 << 20;      // the reference goes up in pieces of this size
 
 }  // namespace
 

@@ -58,6 +58,7 @@ enum KernelId {
   kKCapExact, kKSamLineMax,
   kKBcAny,
   kKRefEncode, kKAlleleChunks, kKAlleleCombine, kKAlleleSiteCount, kKAlleleSiteWrite,
+  kKAlleleSignature, kKCompareChunks, kKCompareCombine, kKCompareSiteCount, kKCompareSiteWrite,
   kKernelCount
 };
 
@@ -197,6 +198,11 @@ struct mcov_ctx {
   std::vector<uint8_t> ref_set;
   int64_t ref_epoch = -1;
   int64_t n_sites = -1, sites_epoch = -1;
+
+  // Comparisons (compare.cu): the (sample a, sample b) signature pointers of each pair, the region and site scratch; the
+  // site list of the last mcov_compare_sites (n_cmp_sites of them, -1 = none) for the contig table of cmp_sites_epoch.
+  mcov::DevBuf d_cmp_pairs, d_cmp_chunks, d_cmp_part, d_cmp_meta, d_cmp_out, d_cmp_tiles, d_cmp_scan, d_cmp_sites;
+  int64_t n_cmp_sites = -1, cmp_sites_epoch = -1;
 
   // fused (sorted) path scratch
   mcov::DevBuf d_start_slot, d_far_list, d_tile_cnt, d_tile_off, d_far_sorted;

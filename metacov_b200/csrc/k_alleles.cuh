@@ -14,7 +14,7 @@
 // pi_p is computed with _rn intrinsics so that nothing is contracted into an FMA: it is bit-identical to numpy's.
 #pragma once
 #include <stdint.h>
-#include "common.cuh"
+#include "k_allele_rules.cuh"
 
 namespace mcov {
 
@@ -24,14 +24,6 @@ constexpr int kAlChunk = 2048;           // positions a chunk (64 a lane)
 constexpr int kAlTile = 4096;            // slots a site tile
 constexpr int kAlTileThreads = 256;
 constexpr uint8_t kRefUnknown = 4;
-
-struct AlleleParams {
-  uint32_t min_cov, min_count;
-  double min_freq;
-  int32_t use_ref;
-};
-
-struct AlChunk { int64_t slot; int64_t n; };   // n positions from slot, all inside one contig
 
 struct AlPart {                                // a chunk's partial record (a region's record minus its length)
   int64_t covered, depth_sum;
@@ -54,14 +46,8 @@ __device__ __forceinline__ AlPos allele_eval(const uint4 c, const uint32_t r, co
   o.pi = 0.0; o.kind = 0; o.cons = 0;
   if (!o.covered) return o;
   const double dn = (double)o.n;
-  const double thr = __dmul_rn(P.min_freq, dn);
-  const uint32_t v[4] = {c.x, c.y, c.z, c.w};
-  uint32_t mask = 0, best = 0;
-#pragma unroll
-  for (int b = 0; b < 4; ++b) {
-    if (v[b] >= P.min_count && (double)v[b] >= thr) mask |= 1u << b;
-    if (b > 0 && v[b] > v[best]) best = b;
-  }
+  const AlRules ru = allele_rules(c, dn, P);
+  const uint32_t mask = ru.mask, best = ru.best;
   const double fa = __ddiv_rn((double)c.x, dn), fc = __ddiv_rn((double)c.y, dn);
   const double fg = __ddiv_rn((double)c.z, dn), ft = __ddiv_rn((double)c.w, dn);
   o.pi = __dsub_rn(1.0, __dadd_rn(__dadd_rn(__dmul_rn(fa, fa), __dmul_rn(fc, fc)), __dadd_rn(__dmul_rn(fg, fg), __dmul_rn(ft, ft))));
@@ -93,11 +79,6 @@ struct AlRegionArgs {
 __device__ __forceinline__ double warp_sum_f64(double v) {
 #pragma unroll
   for (int s = 16; s > 0; s >>= 1) v = __dadd_rn(v, __shfl_xor_sync(0xffffffffu, v, s));
-  return v;
-}
-__device__ __forceinline__ long long warp_sum_i64(long long v) {
-#pragma unroll
-  for (int s = 16; s > 0; s >>= 1) v += __shfl_xor_sync(0xffffffffu, v, s);
   return v;
 }
 

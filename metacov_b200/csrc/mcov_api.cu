@@ -607,7 +607,9 @@ void mcov_destroy(mcov_ctx* ctx) {
                     &ctx->d_out, &ctx->d_win_slot, &ctx->d_win_n, &ctx->d_win_out, &ctx->d_htasks, &ctx->d_tile_heavy, &ctx->d_run_tasks, &ctx->d_run_counts, &ctx->d_run_out,
                     &ctx->d_starts, &ctx->d_bc, &ctx->d_bc_word,
                     &ctx->d_ref, &ctx->d_ref_stage, &ctx->d_al_chunks, &ctx->d_al_part, &ctx->d_al_meta, &ctx->d_al_out,
-                    &ctx->d_al_tiles, &ctx->d_al_scan, &ctx->d_sites};
+                    &ctx->d_al_tiles, &ctx->d_al_scan, &ctx->d_sites,
+                    &ctx->d_cmp_pairs, &ctx->d_cmp_chunks, &ctx->d_cmp_part, &ctx->d_cmp_meta, &ctx->d_cmp_out,
+                    &ctx->d_cmp_tiles, &ctx->d_cmp_scan, &ctx->d_cmp_sites};
   for (DevBuf* b : bufs) b->release();
   ctx->bam.release();
   ctx->h_pin.release();
@@ -1094,7 +1096,8 @@ static const char* kKernelNames[kKernelCount] = {
     "k_sam_nl_count", "k_sam_nl_write", "k_sam_fields", "k_sam_cigar", "k_sam_names_seq", "k_dev_map_counts",
     "k_cap_exact", "k_sam_line_max",
     "k_bc_any",
-    "k_ref_encode", "k_allele_chunks", "k_allele_combine", "k_allele_site_count", "k_allele_site_write"};
+    "k_ref_encode", "k_allele_chunks", "k_allele_combine", "k_allele_site_count", "k_allele_site_write",
+    "k_allele_signature", "k_compare_chunks", "k_compare_combine", "k_compare_site_count", "k_compare_site_write"};
 
 int mcov_copy_to_host(mcov_ctx* ctx, const void* dev, void* host, int64_t n_bytes) {
   if (!ctx) return MCOV_ERR_ARG;

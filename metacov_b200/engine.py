@@ -330,6 +330,66 @@ class CoverageEngine:
         self._check(lib.mcov_allele_sites_read(self._ctx, 0, n.value, _capi.ptr(out)))
         return out
 
+    # -- comparisons (signatures of base_counts, then pairs of signatures) --------------------------------------------
+    def allele_signature(self, min_coverage=5, min_freq=0.05, min_count=2):
+        """The signature of every slot (``mcov_allele_signature``) -> CUDA ``torch.uint8`` tensor of ``n_slots``: 0x80
+        covered, bits 4-5 the consensus, bits 0-3 the present mask, 0 where not covered.  Needs ``base_counts`` first."""
+        import torch
+        p = self._allele_params(min_coverage, min_freq, min_count, False)
+        dev = torch.device("cuda", self.device)
+        out = torch.empty(int(self.n_slots), dtype=torch.uint8, device=dev)
+        torch.cuda.current_stream(dev).synchronize()         # (the tensor's memory may still be read by earlier work)
+        self._check(lib.mcov_allele_signature(self._ctx, C.byref(p), _capi.ptr(out)))
+        return out
+
+    def _compare_args(self, signatures, pairs):
+        """(ctypes pointer table, pairs as int32 [n, 2]) after checking every tensor and pair, else ValueError."""
+        import torch
+        sigs = list(signatures)
+        if len(sigs) < 2:
+            raise ValueError("a comparison needs at least two signatures, got %d" % len(sigs))
+        for i, s in enumerate(sigs):
+            if not isinstance(s, torch.Tensor) or s.device.type != "cuda" or s.device.index != self.device:
+                raise ValueError("signature %d must be a CUDA tensor on device %d" % (i, self.device))
+            if s.dtype != torch.uint8 or s.dim() != 1 or not s.is_contiguous() or s.numel() != int(self.n_slots):
+                raise ValueError("signature %d must be a contiguous torch.uint8 vector of n_slots = %d, got %s %s"
+                                 % (i, int(self.n_slots), s.dtype, tuple(s.shape)))
+        pairs = np.asarray(pairs, dtype=np.int64).reshape(-1, 2)
+        if len(pairs) == 0:
+            raise ValueError("pairs must hold at least one pair of signatures")
+        if pairs.min() < 0 or pairs.max() >= len(sigs) or (pairs[:, 0] == pairs[:, 1]).any():
+            raise ValueError("pairs must index two different signatures of 0 .. %d" % (len(sigs) - 1))
+        tab = (C.c_void_p * len(sigs))(*[s.data_ptr() for s in sigs])
+        torch.cuda.current_stream(torch.device("cuda", self.device)).synchronize()   # (the signatures are written)
+        return tab, np.ascontiguousarray(pairs, dtype=np.int32), sigs
+
+    def compare_stats(self, signatures, pairs, tid, start, end):
+        """Every pair's records over g regions (``mcov_compare_run``) -> structured array
+        ``_capi.COMPARE_STATS_DTYPE`` of shape [n_pairs, g] (length, covered_a, covered_b, compared, con_snp,
+        pop_snp).  ``signatures``: tensors of ``allele_signature`` made under this contig table; ``pairs``: [n, 2]
+        indices into them."""
+        tab, pairs, _keep = self._compare_args(signatures, pairs)
+        tid = np.ascontiguousarray(tid, dtype=np.int32)
+        start = np.ascontiguousarray(start, dtype=np.int32)
+        end = np.ascontiguousarray(end, dtype=np.int32)
+        g = len(tid)
+        if not (len(start) == len(end) == g):
+            raise ValueError("tid/start/end lengths differ")
+        out = np.zeros((len(pairs), g), dtype=_capi.COMPARE_STATS_DTYPE)
+        self._check(lib.mcov_compare_run(self._ctx, len(tab), tab, len(pairs), _capi.ptr(pairs), g, _capi.ptr(tid),
+                                         _capi.ptr(start), _capi.ptr(end), _capi.ptr(out)))
+        return out
+
+    def compare_sites(self, signatures, pairs):
+        """Every con_snp position of every pair in (pair, tid, pos) order (``mcov_compare_sites``) -> structured array
+        ``_capi.COMPARE_SITE_DTYPE`` (pair tid pos sig_a sig_b kind; kind 1 con_snp, 2 pop_snp)."""
+        tab, pairs, _keep = self._compare_args(signatures, pairs)
+        n = C.c_int64(0)
+        self._check(lib.mcov_compare_sites(self._ctx, len(tab), tab, len(pairs), _capi.ptr(pairs), C.byref(n)))
+        out = np.zeros(n.value, dtype=_capi.COMPARE_SITE_DTYPE)
+        self._check(lib.mcov_compare_sites_read(self._ctx, 0, n.value, _capi.ptr(out)))
+        return out
+
     # -- accounting ---------------------------------------------------------
     def launch_count(self):
         return lib.mcov_launch_count(self._ctx)
