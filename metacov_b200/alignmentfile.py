@@ -801,8 +801,7 @@ class AlignmentFile:
             except McovError as e:
                 if e.code == _capi.MCOV_ERR_IO and "consumes more query bases" in str(e):
                     raise IndexError("%s: %s" % (self.filename, e))         # (pysam's error there)
-                if e.code == _capi.MCOV_ERR_NOMEM:
-                    raise MemoryError("%s: %s" % (self.filename, e))
+                self._raise_nomem(e)
                 if e.code == _capi.MCOV_ERR_IO:
                     raise OSError("%s: %s" % (self.filename, e))
                 raise
@@ -883,11 +882,15 @@ class AlignmentFile:
                 try:
                     eng.set_reference(tid, seq)
                 except McovError as e:
-                    if e.code == _capi.MCOV_ERR_NOMEM:
-                        raise MemoryError("%s: %s" % (self.filename, e))
+                    self._raise_nomem(e)
                     raise
             self._ref_fasta = fasta
         return eng, fasta is not None
+
+    def _raise_nomem(self, e):
+        """MemoryError naming the file for an McovError of device memory that does not fit (MCOV_ERR_NOMEM)."""
+        if e.code == _capi.MCOV_ERR_NOMEM:
+            raise MemoryError("%s: %s" % (self.filename, e))
 
     def _count_engine(self):
         """The engine that counts: a device-decoded file's own (it holds the records); else one of the counts' own."""

@@ -241,34 +241,60 @@ def scan(readfile, readfile_type, out_basehist, boffset, out_kmerhist, k, number
         n += 1
 
 
+def _allele_options(sites_help):
+    """The options `alleles` and `compare` share, in this order behind their own; ``sites_help``: --sites-out's help."""
+    def apply(f):
+        for option in reversed([
+                click.option("--regionfile-blast7", "-rb", type=click.File("r"), help="Input Region file in BLAST7 format"),
+                click.option("--regionfile-csv", "-rc", type=click.File("r"), help="Input Region file in CSV format"),
+                click.option("--outfile", "-o", type=click.File("w"), default="-", help="Output CSV (default STDOUT)"),
+                click.option("--sites-out", type=click.File("w"), metavar="FILE", help=sites_help),
+                click.option("--quality-threshold", "-q", type=int, default=15, show_default=True,
+                             help="Count a base only with a quality of at least this (0: every base)."),
+                click.option("--read-callback", type=click.Choice(["all", "nofilter"]), default="all", show_default=True,
+                             help="all: skip unmapped, secondary, QC-fail and duplicate reads; nofilter: count every "
+                                  "placed read."),
+                click.option("--min-coverage", type=click.IntRange(1), default=5, show_default=True),
+                click.option("--min-freq", type=click.FloatRange(0, 1), default=0.05, show_default=True),
+                click.option("--min-count", type=click.IntRange(1), default=2, show_default=True),
+                click.option("--bam-decode", type=click.Choice(["host", "gpu", "gpu-stream", "auto"]), default="auto",
+                             show_default=True, help="Where the BAM file is inflated and parsed (see `pileup`).")]):
+            f = option(f)
+        return f
+    return apply
+
+
+def _refuse_stream(path, option="-b/--bamfile"):
+    if is_stream(path):
+        raise click.UsageError(option + ": the allele counts need every record of a file; a piped stream cannot give "
+                               "them (write the alignments to a file)")
+
+
+def _hit_columns(hits, references):
+    """(refs, starts, ends) of region hits: the full reference name of each hit's contig and its 0-based interval."""
+    name2ref = {word.split()[0]: word for word in references}
+    refs, starts, ends = [], [], []
+    for hit in hits:
+        refs.append(name2ref[hit.sacc])
+        start, end = sorted((int(hit.sstart), int(hit.send)))      # (as `pileup`: blast's reverse strand has end < start)
+        starts.append(start)
+        ends.append(end)
+    return refs, starts, ends
+
+
 @main.command()
 @click.option("--bamfile", "-b", type=click.Path(dir_okay=False, allow_dash=True), required=True,
               help="Input BAM or SAM file (any read order, no index needed). Not a pipe: the counts need every record.")
 @click.option("--reference-fasta", "-f", type=click.Path(exists=True, dir_okay=False),
               help="Reference the reads were mapped to: enables SUB / POPSUB, con_ani and pop_ani.")
-@click.option("--regionfile-blast7", "-rb", type=click.File("r"), help="Input Region file in BLAST7 format")
-@click.option("--regionfile-csv", "-rc", type=click.File("r"), help="Input Region file in CSV format")
-@click.option("--outfile", "-o", type=click.File("w"), default="-", help="Output CSV (default STDOUT)")
-@click.option("--sites-out", type=click.File("w"), metavar="FILE",
-              help="Also write every site as TSV: contig pos ref A C G T consensus snv sub popsub (pos 0-based).")
-@click.option("--quality-threshold", "-q", type=int, default=15, show_default=True,
-              help="Count a base only with a quality of at least this (0: every base).")
-@click.option("--read-callback", type=click.Choice(["all", "nofilter"]), default="all", show_default=True,
-              help="all: skip unmapped, secondary, QC-fail and duplicate reads; nofilter: count every placed read.")
-@click.option("--min-coverage", type=click.IntRange(1), default=5, show_default=True)
-@click.option("--min-freq", type=click.FloatRange(0, 1), default=0.05, show_default=True)
-@click.option("--min-count", type=click.IntRange(1), default=2, show_default=True)
-@click.option("--bam-decode", type=click.Choice(["host", "gpu", "gpu-stream", "auto"]), default="auto", show_default=True,
-              help="Where the BAM file is inflated and parsed (see `pileup`).")
+@_allele_options("Also write every site as TSV: contig pos ref A C G T consensus snv sub popsub (pos 0-based).")
 def alleles(bamfile, reference_fasta, regionfile_blast7, regionfile_csv, outfile, sites_out, quality_threshold,
             read_callback, min_coverage, min_freq, min_count, bam_decode):
     """
     Allele statistics per region from the A/C/G/T counts on the GPU: breadth, depth, nucleotide diversity (pi), SNVs
     per kbp and, with a reference, consensus and population ANI.  Not in the reference: additive.
     """
-    if is_stream(bamfile):
-        raise click.UsageError("-b/--bamfile: the allele counts need every record of a file; a piped stream cannot give "
-                               "them (write the alignments to a file)")
+    _refuse_stream(bamfile)
     regions = None
     if regionfile_blast7 or regionfile_csv:
         regions = util.make_region_iterator(regionfile_blast7, regionfile_csv, None)
@@ -276,14 +302,8 @@ def alleles(bamfile, reference_fasta, regionfile_blast7, regionfile_csv, outfile
     fasta = FastaFile(reference_fasta) if reference_fasta else None
     if regions is None:
         regions = util.get_regions_from_bam(bam)
-    name2ref = {word.split()[0]: word for word in bam.references}
     hits = list(regions)
-    refs, starts, ends = [], [], []
-    for hit in hits:
-        refs.append(name2ref[hit.sacc])
-        start, end = sorted((int(hit.sstart), int(hit.send)))      # (as `pileup`: blast's reverse strand has end < start)
-        starts.append(start)
-        ends.append(end)
+    refs, starts, ends = _hit_columns(hits, bam.references)
     kw = dict(fasta=fasta, quality_threshold=quality_threshold, read_callback=read_callback,
               min_coverage=min_coverage, min_freq=min_freq, min_count=min_count)
     if hits:
@@ -315,21 +335,8 @@ def write_sites(bam, sites, out):
 @click.option("--bamfile", "-b", "bamfiles", type=click.Path(dir_okay=False, allow_dash=True), multiple=True, required=True,
               help="Input BAM or SAM file, two or more times (any read order, no index; every file with the same "
                    "reference names and lengths). Not a pipe: the counts need every record.")
-@click.option("--regionfile-blast7", "-rb", type=click.File("r"), help="Input Region file in BLAST7 format")
-@click.option("--regionfile-csv", "-rc", type=click.File("r"), help="Input Region file in CSV format")
-@click.option("--outfile", "-o", type=click.File("w"), default="-", help="Output CSV (default STDOUT)")
-@click.option("--sites-out", type=click.File("w"), metavar="FILE",
-              help="Also write every con_snp site of every pair as TSV: sample_a sample_b contig pos cons_a cons_b "
-                   "alleles_a alleles_b con_snp pop_snp (pos 0-based; alleles: the present alleles plus the consensus).")
-@click.option("--quality-threshold", "-q", type=int, default=15, show_default=True,
-              help="Count a base only with a quality of at least this (0: every base).")
-@click.option("--read-callback", type=click.Choice(["all", "nofilter"]), default="all", show_default=True,
-              help="all: skip unmapped, secondary, QC-fail and duplicate reads; nofilter: count every placed read.")
-@click.option("--min-coverage", type=click.IntRange(1), default=5, show_default=True)
-@click.option("--min-freq", type=click.FloatRange(0, 1), default=0.05, show_default=True)
-@click.option("--min-count", type=click.IntRange(1), default=2, show_default=True)
-@click.option("--bam-decode", type=click.Choice(["host", "gpu", "gpu-stream", "auto"]), default="auto", show_default=True,
-              help="Where the BAM file is inflated and parsed (see `pileup`).")
+@_allele_options("Also write every con_snp site of every pair as TSV: sample_a sample_b contig pos cons_a cons_b "
+                 "alleles_a alleles_b con_snp pop_snp (pos 0-based; alleles: the present alleles plus the consensus).")
 def compare(bamfiles, regionfile_blast7, regionfile_csv, outfile, sites_out, quality_threshold, read_callback,
             min_coverage, min_freq, min_count, bam_decode):
     """
@@ -339,21 +346,13 @@ def compare(bamfiles, regionfile_blast7, regionfile_csv, outfile, sites_out, qua
     if len(bamfiles) < 2:
         raise click.UsageError("-b/--bamfile: a comparison needs at least two files")
     for f in bamfiles:
-        if is_stream(f):
-            raise click.UsageError("-b/--bamfile %s: the allele counts need every record of a file; a piped stream "
-                                   "cannot give them (write the alignments to a file)" % f)
+        _refuse_stream(f, "-b/--bamfile " + f)
     names, lengths = read_references(bamfiles[0])
     if regionfile_blast7 or regionfile_csv:
         hits = list(util.make_region_iterator(regionfile_blast7, regionfile_csv, None))
     else:
         hits = [util.Region(n, name, 0, length) for n, (name, length) in enumerate(zip(names, lengths))]
-    name2ref = {word.split()[0]: word for word in names}
-    refs, starts, ends = [], [], []
-    for hit in hits:
-        refs.append(name2ref[hit.sacc])
-        start, end = sorted((int(hit.sstart), int(hit.send)))      # (as `pileup`: blast's reverse strand has end < start)
-        starts.append(start)
-        ends.append(end)
+    refs, starts, ends = _hit_columns(hits, names)
     res = _compare(bamfiles, refs, starts, ends, sites=sites_out is not None, decode=bam_decode,
                    quality_threshold=quality_threshold, read_callback=read_callback, min_coverage=min_coverage,
                    min_freq=min_freq, min_count=min_count)

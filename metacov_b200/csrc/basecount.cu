@@ -6,7 +6,6 @@
 // streamed decoder chunk by chunk (bam_gpu_chunks), each chunk's records counted while they are resident.
 #include <algorithm>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -18,25 +17,13 @@ using namespace mcov;
 
 namespace {
 
-int bc_fail(mcov_ctx* ctx, int code, const std::string& what, cudaError_t e = cudaSuccess) {
-  ctx->err = what;
-  if (e != cudaSuccess) { ctx->err += ": "; ctx->err += cudaGetErrorString(e); }
-  return code;
-}
-
-#define BCU(call)                                                                                   \
-  do {                                                                                              \
-    cudaError_t e__ = (call);                                                                       \
-    if (e__ != cudaSuccess) return bc_fail(ctx, MCOV_ERR_CUDA, std::string("mcov_base_counts: ") + #call, e__); \
-  } while (0)
-
 // Count the records [i0, n) of one set of device columns.
 int count_records(mcov_ctx* ctx, const BcArgs& a, bool sam) {
   if (a.n <= a.i0) return MCOV_OK;
   const int64_t grid = std::min<int64_t>((a.n - a.i0 + kBcWarps - 1) / kBcWarps, (int64_t)std::max(ctx->n_sm, 1) * 8);
   if (sam) MCOV_LAUNCH(ctx, kKBcAny, (k_bc_any<BcSamRec><<<(unsigned)grid, kBcThreads, 0, ctx->stream>>>(a)));
   else MCOV_LAUNCH(ctx, kKBcAny, (k_bc_any<BcBamRec><<<(unsigned)grid, kBcThreads, 0, ctx->stream>>>(a)));
-  BCU(cudaGetLastError());
+  CTX_CU("mcov_base_counts", cudaGetLastError());
   return MCOV_OK;
 }
 
@@ -71,37 +58,28 @@ struct CountSink : BamChunkSink {
 }  // namespace
 
 extern "C" int mcov_base_counts(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, int32_t quality_threshold, int mode) {
+  const char* who = "mcov_base_counts";
   if (!ctx) return MCOV_ERR_ARG;
-  if (mode != MCOV_BC_ALL && mode != MCOV_BC_NOFILTER) return bc_fail(ctx, MCOV_ERR_ARG, "mcov_base_counts: mode must be MCOV_BC_ALL or MCOV_BC_NOFILTER");
-  if (ctx->n_contigs <= 0) return bc_fail(ctx, MCOV_ERR_STATE, "mcov_base_counts: mcov_set_contigs has not been called");
+  if (mode != MCOV_BC_ALL && mode != MCOV_BC_NOFILTER) return ctx_fail(ctx, MCOV_ERR_ARG, "mcov_base_counts: mode must be MCOV_BC_ALL or MCOV_BC_NOFILTER");
+  if (ctx->n_contigs <= 0) return ctx_fail(ctx, MCOV_ERR_STATE, "mcov_base_counts: mcov_set_contigs has not been called");
   mcov_ctx::BamDev& B = ctx->bam;
-  if (!path && (B.n_rec < 0 || !B.data.p)) return bc_fail(ctx, MCOV_ERR_STATE, "mcov_base_counts: no file decoded on this context");
-  BCU(cudaSetDevice(ctx->device));
+  if (!path && (B.n_rec < 0 || !B.data.p)) return ctx_fail(ctx, MCOV_ERR_STATE, "mcov_base_counts: no file decoded on this context");
+  CTX_CU(who, cudaSetDevice(ctx->device));
   ctx->bc_ready = false;
   // the counters: 16 bytes a slot, checked against the free device memory before anything is allocated
   const size_t need = (size_t)ctx->n_slots * 16;
-  if (ctx->d_bc.cap < need) {
-    size_t free_b = 0, total_b = 0;
-    BCU(cudaMemGetInfo(&free_b, &total_b));
-    if (const char* h = std::getenv("MCOV_BC_FREE_BYTES")) free_b = (size_t)std::strtoull(h, nullptr, 10);   // test hook
-    const size_t want = need + need / 8 + 256;                   // (DevBuf's growth margin)
-    if (want > free_b + ctx->d_bc.cap) {
-      char msg[256];
-      std::snprintf(msg, sizeof(msg), "mcov_base_counts: the A/C/G/T counters of %lld reference slots need %zu bytes of device memory, %zu are free",
-                    (long long)ctx->n_slots, want, free_b + ctx->d_bc.cap);
-      return bc_fail(ctx, MCOV_ERR_NOMEM, msg);
-    }
-  }
-  BCU(ctx->d_bc.ensure(need));
-  BCU(ctx->d_bc_word.ensure(8));
+  if (int rc = ensure_fits(ctx, ctx->d_bc, need, "MCOV_BC_FREE_BYTES", who,
+                           "the A/C/G/T counters of %lld reference slots need %zu bytes of device memory, %zu are free"))
+    return rc;
+  CTX_CU(who, ctx->d_bc_word.ensure(8));
   cudaStream_t s = ctx->stream;
-  BCU(cudaMemsetAsync(ctx->d_bc.p, 0, need, s));
-  BCU(cudaMemsetAsync(ctx->d_bc_word.p, 0xFF, 8, s));
+  CTX_CU(who, cudaMemsetAsync(ctx->d_bc.p, 0, need, s));
+  CTX_CU(who, cudaMemsetAsync(ctx->d_bc_word.p, 0xFF, 8, s));
   if (path) {
     mcov_bam_gpu_stream_info info;
     std::memset(&info, 0, sizeof(info));
     CountSink sink(quality_threshold, mode);
-    const int rc = bam_gpu_chunks(ctx, path, chunk_bytes, 1, &info, "mcov_base_counts", sink);
+    const int rc = bam_gpu_chunks(ctx, path, chunk_bytes, 1, &info, who, sink);
     if (rc) return rc;
   } else {
     BcArgs a = context_bc_args(ctx, quality_threshold, mode);
@@ -113,15 +91,15 @@ extern "C" int mcov_base_counts(mcov_ctx* ctx, const char* path, int64_t chunk_b
     if (rc) return rc;
   }
   unsigned long long e = 0;
-  BCU(cudaMemcpyAsync(&e, ctx->d_bc_word.p, 8, cudaMemcpyDeviceToHost, s));
-  BCU(cudaStreamSynchronize(s));
+  CTX_CU(who, cudaMemcpyAsync(&e, ctx->d_bc_word.p, 8, cudaMemcpyDeviceToHost, s));
+  CTX_CU(who, cudaStreamSynchronize(s));
   if (e != ~0ull) {
     char msg[256];
     std::snprintf(msg, sizeof(msg), (e & 3) == kBcErrQueryLong
                       ? "mcov_base_counts: record %lld (0-based, file order): its CIGAR consumes more query bases than SEQ holds"
                       : "mcov_base_counts: record %lld (0-based, file order): its SEQ / QUAL leave the record",
                   (long long)(e >> 2));
-    return bc_fail(ctx, MCOV_ERR_IO, msg);
+    return ctx_fail(ctx, MCOV_ERR_IO, msg);
   }
   ctx->bc_ready = true;
   ctx->bc_qthr = quality_threshold; ctx->bc_mode = mode;
@@ -130,17 +108,18 @@ extern "C" int mcov_base_counts(mcov_ctx* ctx, const char* path, int64_t chunk_b
 }
 
 extern "C" int mcov_copy_base_counts(mcov_ctx* ctx, int32_t tid, int32_t start, int32_t end, uint32_t* host_out) {
+  const char* who = "mcov_copy_base_counts";
   if (!ctx) return MCOV_ERR_ARG;
   if (!ctx->bc_ready || ctx->bc_epoch != ctx->contig_epoch)
-    return bc_fail(ctx, MCOV_ERR_STATE, "mcov_copy_base_counts: no counts for this contig table (call mcov_base_counts first)");
+    return ctx_fail(ctx, MCOV_ERR_STATE, "mcov_copy_base_counts: no counts for this contig table (call mcov_base_counts first)");
   if (tid < 0 || tid >= ctx->n_contigs || start < 0 || end < start || end > ctx->len[tid] || (end > start && !host_out))
-    return bc_fail(ctx, MCOV_ERR_ARG, "mcov_copy_base_counts: region out of range");
+    return ctx_fail(ctx, MCOV_ERR_ARG, "mcov_copy_base_counts: region out of range");
   const int64_t n = (int64_t)end - start;
   if (n == 0) return MCOV_OK;
-  BCU(cudaSetDevice(ctx->device));
+  CTX_CU(who, cudaSetDevice(ctx->device));
   std::vector<uint32_t> tmp((size_t)n * 4);
-  BCU(cudaMemcpyAsync(tmp.data(), ctx->d_bc.as<uint32_t>() + (ctx->off[tid] + start) * 4, (size_t)n * 16, cudaMemcpyDeviceToHost, ctx->stream));
-  BCU(cudaStreamSynchronize(ctx->stream));
+  CTX_CU(who, cudaMemcpyAsync(tmp.data(), ctx->d_bc.as<uint32_t>() + (ctx->off[tid] + start) * 4, (size_t)n * 16, cudaMemcpyDeviceToHost, ctx->stream));
+  CTX_CU(who, cudaStreamSynchronize(ctx->stream));
   for (int64_t k = 0; k < n; ++k)
     for (int b = 0; b < 4; ++b) host_out[b * n + k] = tmp[(size_t)k * 4 + b];
   return MCOV_OK;

@@ -10,8 +10,6 @@
 #include <string>
 #include <vector>
 
-#include <cub/device/device_scan.cuh>
-
 #include "ctx.cuh"
 #include "k_compare.cuh"
 
@@ -23,28 +21,22 @@ static_assert(sizeof(CmpPart) == 24, "CmpPart is 24 bytes");
 
 namespace {
 
-#define CMU(who, call)                                                                                    \
-  do {                                                                                                    \
-    cudaError_t e__ = (call);                                                                             \
-    if (e__ != cudaSuccess) return al_fail(ctx, MCOV_ERR_CUDA, std::string(who) + ": " + #call, e__);     \
-  } while (0)
-
 // p is 4-byte aligned device memory on ctx's GPU, or an error naming `what`.
 int cmp_device_ptr(mcov_ctx* ctx, const void* p, const char* who, const std::string& what) {
   cudaPointerAttributes at;
   const cudaError_t e = p ? cudaPointerGetAttributes(&at, p) : cudaErrorInvalidValue;
   if (e != cudaSuccess) (void)cudaGetLastError();
   if (e != cudaSuccess || at.type != cudaMemoryTypeDevice || at.device != ctx->device || (reinterpret_cast<uintptr_t>(p) & 3))
-    return al_fail(ctx, MCOV_ERR_ARG, std::string(who) + ": " + what + " is not 4-byte aligned device memory on the context's GPU");
+    return ctx_fail(ctx, MCOV_ERR_ARG, std::string(who) + ": " + what + " is not 4-byte aligned device memory on the context's GPU");
   return MCOV_OK;
 }
 
 // The checks the pair calls share; on success the device table [2 * n_pairs] of (sample a, sample b) signature pointers
-// is in ctx->d_cmp_pairs (copied on ctx->stream).
+// is in ctx->d_pair_sigs (copied on ctx->stream).
 int cmp_pairs(mcov_ctx* ctx, int32_t n_sig, const uint8_t* const* sig, int32_t n_pairs, const int32_t* pairs, const char* who) {
-  if (ctx->n_contigs <= 0) return al_fail(ctx, MCOV_ERR_STATE, std::string(who) + ": no contig table (mcov_set_contigs)");
+  if (ctx->n_contigs <= 0) return ctx_fail(ctx, MCOV_ERR_STATE, std::string(who) + ": no contig table (mcov_set_contigs)");
   if (n_sig < 2 || !sig || n_pairs < 1 || !pairs)
-    return al_fail(ctx, MCOV_ERR_ARG, std::string(who) + ": need at least two signatures and one pair");
+    return ctx_fail(ctx, MCOV_ERR_ARG, std::string(who) + ": need at least two signatures and one pair");
   for (int32_t i = 0; i < n_sig; ++i)
     if (int rc = cmp_device_ptr(ctx, sig[i], who, "signature " + std::to_string(i))) return rc;
   std::vector<const uint8_t*> tab((size_t)2 * n_pairs);
@@ -53,12 +45,12 @@ int cmp_pairs(mcov_ctx* ctx, int32_t n_sig, const uint8_t* const* sig, int32_t n
     if (a < 0 || a >= n_sig || b < 0 || b >= n_sig || a == b) {
       char msg[200];
       std::snprintf(msg, sizeof(msg), "%s: pair %d is (%d, %d); need two different signatures of 0 .. %d", who, p, a, b, n_sig - 1);
-      return al_fail(ctx, MCOV_ERR_ARG, msg);
+      return ctx_fail(ctx, MCOV_ERR_ARG, msg);
     }
     tab[2 * (size_t)p] = sig[a]; tab[2 * (size_t)p + 1] = sig[b];
   }
-  CMU(who, ctx->d_cmp_pairs.ensure(tab.size() * sizeof(void*)));
-  CMU(who, cudaMemcpyAsync(ctx->d_cmp_pairs.p, tab.data(), tab.size() * sizeof(void*), cudaMemcpyHostToDevice, ctx->stream));
+  CTX_CU(who, ctx->d_pair_sigs.ensure(tab.size() * sizeof(void*)));
+  CTX_CU(who, cudaMemcpyAsync(ctx->d_pair_sigs.p, tab.data(), tab.size() * sizeof(void*), cudaMemcpyHostToDevice, ctx->stream));
   return MCOV_OK;
 }
 
@@ -67,16 +59,16 @@ int cmp_pairs(mcov_ctx* ctx, int32_t n_sig, const uint8_t* const* sig, int32_t n
 extern "C" int mcov_allele_signature(mcov_ctx* ctx, const mcov_allele_params* params, uint8_t* dev_out) {
   const char* who = "mcov_allele_signature";
   if (!ctx) return MCOV_ERR_ARG;
-  if (params && params->use_reference != 0) return al_fail(ctx, MCOV_ERR_ARG, "mcov_allele_signature: use_reference must be 0");
+  if (params && params->use_reference != 0) return ctx_fail(ctx, MCOV_ERR_ARG, "mcov_allele_signature: use_reference must be 0");
   AlleleParams P;
   if (int rc = al_check(ctx, params, &P, who)) return rc;
-  CMU(who, cudaSetDevice(ctx->device));
+  CTX_CU(who, cudaSetDevice(ctx->device));
   if (int rc = cmp_device_ptr(ctx, dev_out, who, "dev_out")) return rc;
   cudaStream_t s = ctx->stream;
   MCOV_LAUNCH(ctx, kKAlleleSignature, (k_allele_signature<<<al_grid(ctx, ctx->n_slots, kSigThreads * kSigUnroll), kSigThreads, 0, s>>>(
                                           ctx->d_bc.as<uint4>(), ctx->n_slots, P, dev_out)));
-  CMU(who, cudaGetLastError());
-  CMU(who, cudaStreamSynchronize(s));
+  CTX_CU(who, cudaGetLastError());
+  CTX_CU(who, cudaStreamSynchronize(s));
   return MCOV_OK;
 }
 
@@ -85,51 +77,30 @@ extern "C" int mcov_compare_run(mcov_ctx* ctx, int32_t n_sig, const uint8_t* con
                                 mcov_compare_stats* host_out) {
   const char* who = "mcov_compare_run";
   if (!ctx) return MCOV_ERR_ARG;
-  if (g < 0 || (g > 0 && (!tid || !start || !end || !host_out))) return al_fail(ctx, MCOV_ERR_ARG, "mcov_compare_run: bad arguments");
-  for (int64_t i = 0; i < g; ++i)
-    if (tid[i] < 0 || tid[i] >= ctx->n_contigs || start[i] < 0 || end[i] < start[i])
-      return al_fail(ctx, MCOV_ERR_ARG, "mcov_compare_run: need 0 <= start <= end and a valid tid");
-  CMU(who, cudaSetDevice(ctx->device));
+  if (int rc = check_regions(ctx, g, tid, start, end, host_out, who)) return rc;
+  CTX_CU(who, cudaSetDevice(ctx->device));
   if (int rc = cmp_pairs(ctx, n_sig, sig, n_pairs, pairs, who)) return rc;
   if (g == 0) return MCOV_OK;
   cudaStream_t s = ctx->stream;
-  // Every region cut into chunks of kCmpChunk positions inside its contig (as mcov_allele_stats_run); first[g + 1]
-  // locates each region's chunks, length[g] follows it.
-  std::vector<AlChunk> chunks;
-  std::vector<int64_t> meta((size_t)(2 * g + 1));
-  int64_t* first = meta.data();
-  int64_t* length = meta.data() + g + 1;
-  for (int64_t i = 0; i < g; ++i) {
-    first[i] = (int64_t)chunks.size();
-    length[i] = (int64_t)end[i] - start[i];
-    const int64_t len = ctx->len[tid[i]];
-    const int64_t a = std::min<int64_t>(start[i], len), b = std::min<int64_t>(end[i], len);
-    for (int64_t p = a; p < b; p += kCmpChunk) chunks.push_back({ctx->off[tid[i]] + p, std::min<int64_t>(kCmpChunk, b - p)});
-  }
-  first[g] = (int64_t)chunks.size();
-  const int64_t nc = (int64_t)chunks.size();
-  const auto* tab = ctx->d_cmp_pairs.as<const uint8_t* const>();
-  CMU(who, ctx->d_cmp_meta.ensure(meta.size() * 8));
-  CMU(who, ctx->d_cmp_out.ensure((size_t)g * n_pairs * sizeof(mcov_compare_stats)));
-  CMU(who, cudaMemcpyAsync(ctx->d_cmp_meta.p, meta.data(), meta.size() * 8, cudaMemcpyHostToDevice, s));
+  int64_t nc = 0;
+  if (int rc = upload_region_chunks(ctx, g, tid, start, end, kCmpChunk, (size_t)n_pairs * sizeof(CmpPart),
+                                    (size_t)g * n_pairs * sizeof(mcov_compare_stats), who, &nc))
+    return rc;
   if (nc > 0) {
-    CMU(who, ctx->d_cmp_chunks.ensure((size_t)nc * sizeof(AlChunk)));
-    CMU(who, ctx->d_cmp_part.ensure((size_t)nc * n_pairs * sizeof(CmpPart)));
-    CMU(who, cudaMemcpyAsync(ctx->d_cmp_chunks.p, chunks.data(), (size_t)nc * sizeof(AlChunk), cudaMemcpyHostToDevice, s));
     CmpRegionArgs a;
-    a.sig = tab; a.n_pairs = n_pairs;
-    a.chunks = ctx->d_cmp_chunks.as<AlChunk>(); a.n_chunks = nc;
-    a.part = ctx->d_cmp_part.as<CmpPart>();
+    a.sig = ctx->d_pair_sigs.as<const uint8_t* const>(); a.n_pairs = n_pairs;
+    a.chunks = ctx->d_chunks.as<AlChunk>(); a.n_chunks = nc;
+    a.part = ctx->d_chunk_part.as<CmpPart>();
     MCOV_LAUNCH(ctx, kKCompareChunks, (k_compare_chunks<<<al_grid(ctx, nc * n_pairs, kCmpWarps), kCmpThreads, 0, s>>>(a)));
-    CMU(who, cudaGetLastError());
+    CTX_CU(who, cudaGetLastError());
   }
-  const int64_t* d_meta = ctx->d_cmp_meta.as<int64_t>();
+  const int64_t* d_meta = ctx->d_chunk_meta.as<int64_t>();
   MCOV_LAUNCH(ctx, kKCompareCombine, (k_compare_combine<<<al_grid(ctx, g * n_pairs, kCmpWarps), kCmpThreads, 0, s>>>(
-                                          ctx->d_cmp_part.as<CmpPart>(), n_pairs, d_meta, d_meta + g + 1, g,
-                                          ctx->d_cmp_out.as<mcov_compare_stats>())));
-  CMU(who, cudaGetLastError());
-  CMU(who, cudaMemcpyAsync(host_out, ctx->d_cmp_out.p, (size_t)g * n_pairs * sizeof(mcov_compare_stats), cudaMemcpyDeviceToHost, s));
-  CMU(who, cudaStreamSynchronize(s));
+                                          ctx->d_chunk_part.as<CmpPart>(), n_pairs, d_meta, d_meta + g + 1, g,
+                                          ctx->d_region_out.as<mcov_compare_stats>())));
+  CTX_CU(who, cudaGetLastError());
+  CTX_CU(who, cudaMemcpyAsync(host_out, ctx->d_region_out.p, (size_t)g * n_pairs * sizeof(mcov_compare_stats), cudaMemcpyDeviceToHost, s));
+  CTX_CU(who, cudaStreamSynchronize(s));
   return MCOV_OK;
 }
 
@@ -137,60 +108,39 @@ extern "C" int mcov_compare_sites(mcov_ctx* ctx, int32_t n_sig, const uint8_t* c
                                   int64_t* n_sites_out) {
   const char* who = "mcov_compare_sites";
   if (!ctx) return MCOV_ERR_ARG;
-  ctx->n_cmp_sites = -1;
-  if (!n_sites_out) return al_fail(ctx, MCOV_ERR_ARG, "mcov_compare_sites: null n_sites_out");
-  CMU(who, cudaSetDevice(ctx->device));
+  ctx->compare_sites.n = -1;
+  if (!n_sites_out) return ctx_fail(ctx, MCOV_ERR_ARG, "mcov_compare_sites: null n_sites_out");
+  CTX_CU(who, cudaSetDevice(ctx->device));
   if (int rc = cmp_pairs(ctx, n_sig, sig, n_pairs, pairs, who)) return rc;
   cudaStream_t s = ctx->stream;
   const int64_t n_tiles = (ctx->n_slots + kCmpTile - 1) / kCmpTile;
   const int64_t items = n_tiles * n_pairs;
   // [items] site counts (pair-major), then [items] their inclusive scan
-  CMU(who, ctx->d_cmp_tiles.ensure((size_t)items * 16));
+  CTX_CU(who, ctx->d_site_tiles.ensure((size_t)items * 16));
   CmpSiteArgs a;
-  a.sig = ctx->d_cmp_pairs.as<const uint8_t* const>(); a.n_pairs = n_pairs;
+  a.sig = ctx->d_pair_sigs.as<const uint8_t* const>(); a.n_pairs = n_pairs;
   a.n_slots = ctx->n_slots; a.n_tiles = n_tiles;
   a.contig_off = ctx->d_off.as<int64_t>(); a.n_contigs = ctx->n_contigs;
-  a.tile_n = ctx->d_cmp_tiles.as<int64_t>(); a.tile_incl = a.tile_n + items;
+  a.tile_n = ctx->d_site_tiles.as<int64_t>(); a.tile_incl = a.tile_n + items;
   a.sites = nullptr;
   MCOV_LAUNCH(ctx, kKCompareSiteCount, (k_compare_site_count<<<al_grid(ctx, items, 1), kCmpTileThreads, 0, s>>>(a)));
-  CMU(who, cudaGetLastError());
-  size_t tb = 0;
-  CMU(who, cub::DeviceScan::InclusiveSum(nullptr, tb, a.tile_n, a.tile_n + items, items, s));
-  CMU(who, ctx->d_cmp_scan.ensure(tb));
-  CMU(who, cub::DeviceScan::InclusiveSum(ctx->d_cmp_scan.p, tb, a.tile_n, a.tile_n + items, items, s));
+  CTX_CU(who, cudaGetLastError());
   int64_t total = 0;
-  CMU(who, cudaMemcpyAsync(&total, a.tile_n + 2 * items - 1, 8, cudaMemcpyDeviceToHost, s));
-  CMU(who, cudaStreamSynchronize(s));
+  if (int rc = size_site_list(ctx, ctx->compare_sites, items, sizeof(mcov_compare_site), who, &total)) return rc;
   if (total > 0) {
-    const size_t bytes = (size_t)total * sizeof(mcov_compare_site);
-    if (ctx->d_cmp_sites.ensure(bytes) != cudaSuccess) {
-      (void)cudaGetLastError();
-      char msg[200];
-      std::snprintf(msg, sizeof(msg), "mcov_compare_sites: %lld sites need %zu bytes of device memory", (long long)total, bytes);
-      return al_fail(ctx, MCOV_ERR_NOMEM, msg);
-    }
-    a.sites = ctx->d_cmp_sites.as<mcov_compare_site>();
+    a.sites = ctx->compare_sites.list.as<mcov_compare_site>();
     MCOV_LAUNCH(ctx, kKCompareSiteWrite, (k_compare_site_write<<<al_grid(ctx, items, 1), kCmpTileThreads, 0, s>>>(a)));
-    CMU(who, cudaGetLastError());
-    CMU(who, cudaStreamSynchronize(s));
+    CTX_CU(who, cudaGetLastError());
+    CTX_CU(who, cudaStreamSynchronize(s));
   }
-  ctx->n_cmp_sites = total;
-  ctx->cmp_sites_epoch = ctx->contig_epoch;
+  ctx->compare_sites.n = total;
+  ctx->compare_sites.epoch = ctx->contig_epoch;
   *n_sites_out = total;
   return MCOV_OK;
 }
 
 extern "C" int mcov_compare_sites_read(mcov_ctx* ctx, int64_t first, int64_t n, mcov_compare_site* host_out) {
-  const char* who = "mcov_compare_sites_read";
   if (!ctx) return MCOV_ERR_ARG;
-  if (ctx->n_cmp_sites < 0 || ctx->cmp_sites_epoch != ctx->contig_epoch)
-    return al_fail(ctx, MCOV_ERR_STATE, "mcov_compare_sites_read: no site list for this contig table (call mcov_compare_sites first)");
-  if (first < 0 || n < 0 || first > ctx->n_cmp_sites - n || (n > 0 && !host_out))
-    return al_fail(ctx, MCOV_ERR_ARG, "mcov_compare_sites_read: range outside the site list");
-  if (n == 0) return MCOV_OK;
-  CMU(who, cudaSetDevice(ctx->device));
-  CMU(who, cudaMemcpyAsync(host_out, ctx->d_cmp_sites.as<mcov_compare_site>() + first, (size_t)n * sizeof(mcov_compare_site),
-                           cudaMemcpyDeviceToHost, ctx->stream));
-  CMU(who, cudaStreamSynchronize(ctx->stream));
-  return MCOV_OK;
+  return read_site_list(ctx, ctx->compare_sites, first, n, host_out, sizeof(mcov_compare_site), "mcov_compare_sites_read",
+                        "mcov_compare_sites");
 }

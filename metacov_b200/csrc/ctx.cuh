@@ -1,5 +1,6 @@
 // ctx.cuh -- the context behind the C-ABI (device buffers, streams, state).
 #pragma once
+#include <cstdio>
 #include <cstdlib>
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -13,16 +14,24 @@ namespace mcov {
 struct DevBuf {
   void* p = nullptr;
   size_t cap = 0;
+  // what ensure(bytes) allocates when it has to grow (ensure_fits checks this much against the free memory)
+  static size_t grown(size_t bytes) { return bytes + bytes / 8 + 256; }
   cudaError_t ensure(size_t bytes) {
     if (bytes <= cap) return cudaSuccess;
     if (p) { cudaFree(p); p = nullptr; cap = 0; }
-    size_t want = bytes + bytes / 8 + 256;
+    size_t want = grown(bytes);
     cudaError_t e = cudaMalloc(&p, want);
     if (e == cudaSuccess) cap = want;
     return e;
   }
   void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
   template <typename T> T* as() const { return reinterpret_cast<T*>(p); }
+};
+
+// a site list on the device: n records for the contig table of epoch `epoch` (n = -1: none)
+struct SiteList {
+  DevBuf list;
+  int64_t n = -1, epoch = -1;
 };
 
 struct PinBuf {
@@ -192,17 +201,17 @@ struct mcov_ctx {
   int64_t bc_epoch = -1;
 
   // Alleles (alleles.cu): the reference store ([n_slots] codes 0-3 A C G T, 4 unknown) of the contig table of epoch
-  // ref_epoch and which contigs have been given one; the region and site scratch; the site list of the last
-  // mcov_allele_sites (n_sites of them, -1 = none) for the contig table of epoch sites_epoch.
-  mcov::DevBuf d_ref, d_ref_stage, d_al_chunks, d_al_part, d_al_meta, d_al_out, d_al_tiles, d_al_scan, d_sites;
+  // ref_epoch and which contigs have been given one.  Comparisons (compare.cu): the (sample a, sample b) signature
+  // pointers of each pair.
+  mcov::DevBuf d_ref, d_ref_stage, d_pair_sigs;
   std::vector<uint8_t> ref_set;
   int64_t ref_epoch = -1;
-  int64_t n_sites = -1, sites_epoch = -1;
-
-  // Comparisons (compare.cu): the (sample a, sample b) signature pointers of each pair, the region and site scratch; the
-  // site list of the last mcov_compare_sites (n_cmp_sites of them, -1 = none) for the contig table of cmp_sites_epoch.
-  mcov::DevBuf d_cmp_pairs, d_cmp_chunks, d_cmp_part, d_cmp_meta, d_cmp_out, d_cmp_tiles, d_cmp_scan, d_cmp_sites;
-  int64_t n_cmp_sites = -1, cmp_sites_epoch = -1;
+  // Scratch of the allele and compare region / site calls, one set for both: every such call synchronises before it
+  // returns.  Regions: the chunks (AlChunk), the meta [first[g + 1] | length[g]] (int64), a partial record per chunk,
+  // the region records.  Sites: the tile counts followed by their inclusive scan (int64), the scan's temporary storage.
+  mcov::DevBuf d_chunks, d_chunk_meta, d_chunk_part, d_region_out, d_site_tiles, d_site_scan;
+  // the site lists of the last mcov_allele_sites and mcov_compare_sites (both stay readable)
+  mcov::SiteList allele_sites, compare_sites;
 
   // fused (sorted) path scratch
   mcov::DevBuf d_start_slot, d_far_list, d_tile_cnt, d_tile_off, d_far_sorted;
@@ -278,3 +287,85 @@ struct mcov_ctx {
 
 // wrap one kernel launch (or memset) for accounting / timing
 #define MCOV_LAUNCH(ctx, id, ...) do { (ctx)->prof_begin(id); __VA_ARGS__; (ctx)->prof_end(); } while (0)
+
+// Host helpers of the count, allele and compare calls (basecount.cu, alleles.cu, compare.cu).  `who`, the entry point,
+// starts every error text.
+
+// return from the enclosing call with MCOV_ERR_CUDA ("who: call: CUDA error text") when a CUDA call fails
+#define CTX_CU(who, call)                                                                                  \
+  do {                                                                                                     \
+    cudaError_t e__ = (call);                                                                              \
+    if (e__ != cudaSuccess) return mcov::ctx_fail(ctx, MCOV_ERR_CUDA, std::string(who) + ": " + #call, e__); \
+  } while (0)
+
+namespace mcov {
+
+struct AlleleParams;
+
+// ctx->err = what (+ ": " and the CUDA error's text); returns code.
+inline int ctx_fail(mcov_ctx* ctx, int code, const std::string& what, cudaError_t e = cudaSuccess) {
+  ctx->err = what;
+  if (e != cudaSuccess) { ctx->err += ": "; ctx->err += cudaGetErrorString(e); }
+  return code;
+}
+
+// buf.ensure(need), unless the allocation that takes (DevBuf::grown) exceeds the free device memory plus buf's own:
+// then MCOV_ERR_NOMEM, "who: " + msg, a format of (n_slots, bytes wanted, bytes free).  The environment variable
+// free_hook, when set, stands in for the free bytes (a test hook).
+inline int ensure_fits(mcov_ctx* ctx, DevBuf& buf, size_t need, const char* free_hook, const char* who, const char* msg) {
+  if (buf.cap < need) {
+    size_t free_b = 0, total_b = 0;
+    CTX_CU(who, cudaMemGetInfo(&free_b, &total_b));
+    if (const char* h = std::getenv(free_hook)) free_b = (size_t)std::strtoull(h, nullptr, 10);
+    const size_t want = DevBuf::grown(need);
+    if (want > free_b + buf.cap) {
+      char text[256];
+      std::snprintf(text, sizeof(text), msg, (long long)ctx->n_slots, want, free_b + buf.cap);
+      return ctx_fail(ctx, MCOV_ERR_NOMEM, std::string(who) + ": " + text);
+    }
+  }
+  CTX_CU(who, buf.ensure(need));
+  return MCOV_OK;
+}
+
+// g regions of the contig table, and where their records go
+inline int check_regions(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int32_t* start, const int32_t* end,
+                         const void* out, const char* who) {
+  if (g < 0 || (g > 0 && (!tid || !start || !end || !out))) return ctx_fail(ctx, MCOV_ERR_ARG, std::string(who) + ": bad arguments");
+  for (int64_t i = 0; i < g; ++i)
+    if (tid[i] < 0 || tid[i] >= ctx->n_contigs || start[i] < 0 || end[i] < start[i])
+      return ctx_fail(ctx, MCOV_ERR_ARG, std::string(who) + ": need 0 <= start <= end and a valid tid");
+  return MCOV_OK;
+}
+
+// Records [first, first + n) of a site list to the host; `builder` is the call that builds the list.
+inline int read_site_list(mcov_ctx* ctx, const SiteList& sl, int64_t first, int64_t n, void* host_out, size_t site_bytes,
+                          const char* who, const char* builder) {
+  if (sl.n < 0 || sl.epoch != ctx->contig_epoch)
+    return ctx_fail(ctx, MCOV_ERR_STATE, std::string(who) + ": no site list for this contig table (call " + builder + " first)");
+  if (first < 0 || n < 0 || first > sl.n - n || (n > 0 && !host_out))
+    return ctx_fail(ctx, MCOV_ERR_ARG, std::string(who) + ": range outside the site list");
+  if (n == 0) return MCOV_OK;
+  CTX_CU(who, cudaSetDevice(ctx->device));
+  CTX_CU(who, cudaMemcpyAsync(host_out, sl.list.as<uint8_t>() + first * site_bytes, (size_t)n * site_bytes,
+                              cudaMemcpyDeviceToHost, ctx->stream));
+  CTX_CU(who, cudaStreamSynchronize(ctx->stream));
+  return MCOV_OK;
+}
+
+// alleles.cu: the checked parameters or an error (MCOV_ERR_STATE without counts for the contig table); the grid of a
+// grid-stride kernel over `items` work items, `per` of them a CTA.
+int al_check(mcov_ctx* ctx, const mcov_allele_params* p, AlleleParams* out, const char* who);
+unsigned al_grid(const mcov_ctx* ctx, int64_t items, int per);
+
+// alleles.cu: every region cut into chunks of at most `chunk` positions inside its contig (positions past its end add
+// to the length only); chunks to ctx->d_chunks, meta to d_chunk_meta, d_region_out sized to out_bytes, d_chunk_part to
+// part_bytes a chunk.
+int upload_region_chunks(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int32_t* start, const int32_t* end,
+                         int64_t chunk, size_t part_bytes, size_t out_bytes, const char* who, int64_t* n_chunks);
+
+// alleles.cu: between a site list's count launch, which wrote `items` tile counts to ctx->d_site_tiles, and its write
+// launch: the counts' inclusive scan into the `items` words behind them, the total read back, sl.list sized for it.
+int size_site_list(mcov_ctx* ctx, SiteList& sl, int64_t items, size_t site_bytes, const char* who, int64_t* total);
+
+}  // namespace mcov

@@ -172,16 +172,7 @@ k_allele_site_count(AlSiteArgs a) {
       const int64_t s = s0 + k * kAlTileThreads + threadIdx.x;
       if (s < a.n_slots) n += allele_eval(__ldg(a.cnt + s), al_ref_at(a, s), a.P).kind != 0;
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
-    if ((threadIdx.x & 31) == 0) s_w[threadIdx.x >> 5] = n;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      int64_t tot = 0;
-      for (int w = 0; w < kAlTileThreads / 32; ++w) tot += s_w[w];
-      a.tile_n[t] = tot;
-    }
-    __syncthreads();
+    store_tile_count<kAlTileThreads>(n, s_w, a.tile_n, t, threadIdx.x);
   }
 }
 
@@ -207,9 +198,7 @@ k_allele_site_write(AlSiteArgs a) {
 #pragma unroll
       for (int w = 0; w < kAlTileThreads / 32; ++w) { before += w < warp ? s_w[w] : 0; tot += s_w[w]; }
       if (o.kind != 0) {
-        // contig of slot s: the last contig_off <= s
-        int32_t lo = 0, hi = a.n_contigs - 1;
-        while (lo < hi) { const int32_t m = (lo + hi + 1) >> 1; if (__ldg(a.contig_off + m) <= s) lo = m; else hi = m - 1; }
+        const int32_t lo = contig_of(a.contig_off, a.n_contigs, s);
         mcov_allele_site st;
         st.tid = lo; st.pos = (int32_t)(s - a.contig_off[lo]);
         st.cnt[0] = c.x; st.cnt[1] = c.y; st.cnt[2] = c.z; st.cnt[3] = c.w;

@@ -180,16 +180,7 @@ k_compare_site_count(CmpSiteArgs a) {
       const int64_t q = q0 + k * kCmpTileThreads + threadIdx.x;
       if (q < n_words) n += __popc(cmp_flags(__ldg(pa + q), __ldg(pb + q)).con);
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
-    if ((threadIdx.x & 31) == 0) s_w[threadIdx.x >> 5] = n;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      int64_t tot = 0;
-      for (int w = 0; w < kCmpTileThreads / 32; ++w) tot += s_w[w];
-      a.tile_n[pair * a.n_tiles + t] = tot;
-    }
-    __syncthreads();
+    store_tile_count<kCmpTileThreads>(n, s_w, a.tile_n, pair * a.n_tiles + t, threadIdx.x);
   }
 }
 
@@ -213,11 +204,8 @@ k_compare_site_write(CmpSiteArgs a) {
     const uint32_t* pb = reinterpret_cast<const uint32_t*>(a.sig[2 * pair + 1]);
     const int64_t s0 = t * kCmpTile, s1 = s0 + kCmpTile < a.n_slots ? s0 + kCmpTile : a.n_slots;
     if (threadIdx.x < 2) {
-      // contig of the tile's first (thread 0) and last (thread 1) slot: the last contig_off <= s
-      const int64_t s = threadIdx.x == 0 ? s0 : s1 - 1;
-      int32_t lo = 0, hi = a.n_contigs - 1;
-      while (lo < hi) { const int32_t m = (lo + hi + 1) >> 1; if (__ldg(a.contig_off + m) <= s) lo = m; else hi = m - 1; }
-      s_c[threadIdx.x] = lo;
+      // contig of the tile's first (thread 0) and last (thread 1) slot
+      s_c[threadIdx.x] = contig_of(a.contig_off, a.n_contigs, threadIdx.x == 0 ? s0 : s1 - 1);
     }
     __syncthreads();
     const int32_t c0 = s_c[0], nc = s_c[1] - s_c[0] + 1;

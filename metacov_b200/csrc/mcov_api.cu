@@ -606,10 +606,8 @@ void mcov_destroy(mcov_ctx* ctx) {
                     &ctx->d_cap_scratch, &ctx->d_flag_lut, &ctx->d_stream_acc, &ctx->d_ss_pieces, &ctx->d_ss_cta, &ctx->d_ss_split, &ctx->d_ss_pool,
                     &ctx->d_out, &ctx->d_win_slot, &ctx->d_win_n, &ctx->d_win_out, &ctx->d_htasks, &ctx->d_tile_heavy, &ctx->d_run_tasks, &ctx->d_run_counts, &ctx->d_run_out,
                     &ctx->d_starts, &ctx->d_bc, &ctx->d_bc_word,
-                    &ctx->d_ref, &ctx->d_ref_stage, &ctx->d_al_chunks, &ctx->d_al_part, &ctx->d_al_meta, &ctx->d_al_out,
-                    &ctx->d_al_tiles, &ctx->d_al_scan, &ctx->d_sites,
-                    &ctx->d_cmp_pairs, &ctx->d_cmp_chunks, &ctx->d_cmp_part, &ctx->d_cmp_meta, &ctx->d_cmp_out,
-                    &ctx->d_cmp_tiles, &ctx->d_cmp_scan, &ctx->d_cmp_sites};
+                    &ctx->d_ref, &ctx->d_ref_stage, &ctx->d_pair_sigs, &ctx->d_chunks, &ctx->d_chunk_meta, &ctx->d_chunk_part,
+                    &ctx->d_region_out, &ctx->d_site_tiles, &ctx->d_site_scan, &ctx->allele_sites.list, &ctx->compare_sites.list};
   for (DevBuf* b : bufs) b->release();
   ctx->bam.release();
   ctx->h_pin.release();

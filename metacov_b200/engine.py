@@ -304,16 +304,21 @@ class CoverageEngine:
         p.use_reference = 1 if use_reference else 0
         return p
 
+    @staticmethod
+    def _region_columns(tid, start, end):
+        """(tid, start, end) as contiguous int32 arrays of one length g, and g; else ValueError."""
+        tid = np.ascontiguousarray(tid, dtype=np.int32)
+        start = np.ascontiguousarray(start, dtype=np.int32)
+        end = np.ascontiguousarray(end, dtype=np.int32)
+        if not (len(start) == len(end) == len(tid)):
+            raise ValueError("tid/start/end lengths differ")
+        return tid, start, end, len(tid)
+
     def allele_stats(self, tid, start, end, min_coverage=5, min_freq=0.05, min_count=2, use_reference=False):
         """Allele statistics of g regions (``mcov_allele_stats_run``) -> structured array ``_capi.ALLELE_STATS_DTYPE``
         (length, covered, depth_sum, pi_sum, snv, ref_covered, sub, popsub).  Needs ``base_counts`` first, and with
         ``use_reference`` a ``set_reference`` of every contig."""
-        tid = np.ascontiguousarray(tid, dtype=np.int32)
-        start = np.ascontiguousarray(start, dtype=np.int32)
-        end = np.ascontiguousarray(end, dtype=np.int32)
-        g = len(tid)
-        if not (len(start) == len(end) == g):
-            raise ValueError("tid/start/end lengths differ")
+        tid, start, end, g = self._region_columns(tid, start, end)
         p = self._allele_params(min_coverage, min_freq, min_count, use_reference)
         out = np.zeros(g, dtype=_capi.ALLELE_STATS_DTYPE)
         self._check(lib.mcov_allele_stats_run(self._ctx, g, _capi.ptr(tid), _capi.ptr(start), _capi.ptr(end), C.byref(p),
@@ -369,12 +374,7 @@ class CoverageEngine:
         pop_snp).  ``signatures``: tensors of ``allele_signature`` made under this contig table; ``pairs``: [n, 2]
         indices into them."""
         tab, pairs, _keep = self._compare_args(signatures, pairs)
-        tid = np.ascontiguousarray(tid, dtype=np.int32)
-        start = np.ascontiguousarray(start, dtype=np.int32)
-        end = np.ascontiguousarray(end, dtype=np.int32)
-        g = len(tid)
-        if not (len(start) == len(end) == g):
-            raise ValueError("tid/start/end lengths differ")
+        tid, start, end, g = self._region_columns(tid, start, end)
         out = np.zeros((len(pairs), g), dtype=_capi.COMPARE_STATS_DTYPE)
         self._check(lib.mcov_compare_run(self._ctx, len(tab), tab, len(pairs), _capi.ptr(pairs), g, _capi.ptr(tid),
                                          _capi.ptr(start), _capi.ptr(end), _capi.ptr(out)))

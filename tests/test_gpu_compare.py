@@ -214,6 +214,34 @@ def test_invariance(samples):
     assert np.array_equal(sw.sites["sig_a"], allp.sites["sig_b"]) and np.array_equal(sw.sites["pos"], allp.sites["pos"])
 
 
+def test_allele_and_compare_calls_share_an_engine(samples):
+    """The allele and compare calls of one engine share their region and site scratch but keep separate site lists:
+    building the compare list leaves the allele list readable, and a compare pass in between leaves allele_stats
+    bit-identical."""
+    from metacov_b200 import AlignmentFile, _capi
+    from metacov_b200._capi import lib
+    kw = dict(min_coverage=1, min_freq=0.0, min_count=1)
+    with AlignmentFile(samples[1]["bam"], decode="gpu") as af:
+        other = af.allele_signature(**kw)
+    reg = _regions(np.random.default_rng(37))
+    tid, lo, hi = (np.array([r[k] for r in reg]) for k in range(3))
+    with AlignmentFile(samples[0]["bam"], decode="gpu") as af:
+        sigs, pairs = [af.allele_signature(**kw), other], [(0, 1)]
+        eng = af._count_engine()
+        sites = eng.allele_sites(**kw)
+        csites = eng.compare_sites(sigs, pairs)
+        first = eng.allele_stats(tid, lo, hi, **kw)
+        cstats = eng.compare_stats(sigs, pairs, tid, lo, hi)
+        again = eng.allele_stats(tid, lo, hi, **kw)
+        assert len(sites) > 50 and len(csites) > 50 and int(cstats["con_snp"].sum()) > 0
+        assert again.tobytes() == first.tobytes()
+        for read, want, dtype in ((lib.mcov_allele_sites_read, sites, _capi.ALLELE_SITE_DTYPE),
+                                  (lib.mcov_compare_sites_read, csites, _capi.COMPARE_SITE_DTYPE)):
+            got = np.zeros(len(want), dtype=dtype)
+            eng._check(read(eng._ctx, 0, len(want), _capi.ptr(got)))
+            assert got.tobytes() == want.tobytes()
+
+
 def test_one_counter_store_at_a_time(samples, monkeypatch):
     """compare counts a file only after the engine of every file counted before it is closed."""
     from metacov_b200 import CoverageEngine
