@@ -13,7 +13,7 @@ import os
 
 import numpy as np
 
-from . import _capi
+from . import _capi, samstream
 from ._capi import lib
 
 
@@ -103,12 +103,8 @@ class DeviceSoA:
             self._engine._check(lib.mcov_copy_to_host(self._engine._ctx, self.raw.inflated, _capi.ptr(buf), buf.nbytes))
         b = buf.tobytes()
         if self.format == "sam":
-            refs = []
-            for line in b.decode().splitlines():
-                if line.startswith("@SQ\t"):
-                    tags = dict(t.split(":", 1) for t in line.split("\t")[1:] if ":" in t)
-                    refs.append((tags["SN"], int(tags["LN"])))
-            return b.decode(), refs
+            text = b.decode()
+            return text, samstream.header_refs(text)
         l_text = int.from_bytes(b[4:8], "little")
         text = b[8:8 + l_text].split(b"\0")[0].decode()
         p = 8 + l_text

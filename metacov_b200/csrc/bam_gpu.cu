@@ -34,12 +34,11 @@
 #include <string>
 #include <vector>
 
+#include "bamfmt.h"
 #include "ctx.cuh"
 #include "inflate.cuh"
 
 namespace mcov {
-
-struct BgzfBlock { uint64_t coff; uint64_t uoff; uint32_t clen; uint32_t ulen; uint32_t crc; uint32_t pad; };
 
 #ifndef MCOV_INFLATE_WINDOW
 #define MCOV_INFLATE_WINDOW 2048              /* bytes of recent output mirrored in shared memory, per warp */
@@ -290,63 +289,6 @@ __global__ void k_bam_rebase_offsets(int64_t m, const uint32_t* __restrict__ src
   if (i < m) dst[i] = src[i] - base;
 }
 
-// ---- host side ------------------------------------------------------------------------------------
-
-static inline uint16_t h16(const uint8_t* p) { return (uint16_t)(p[0] | (p[1] << 8)); }
-static inline uint32_t h32(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24); }
-
-// BGZF block table of a file image (SAM spec 4.1: gzip members with a 'BC' extra field holding BSIZE)
-// consumed (optional): a trailing INCOMPLETE block is not an error -- indexing stops in front of it and *consumed tells
-// how many bytes the complete blocks take (chunks of a larger file)
-static bool index_bgzf(const uint8_t* raw, size_t n, std::vector<BgzfBlock>& blocks, uint64_t& total, size_t* consumed = nullptr,
-                       uint64_t uoff0 = 0) {
-  size_t off = 0;
-  uint64_t uoff = uoff0;
-  if (consumed) *consumed = 0;
-  while (off < n) {
-    if (consumed) {
-      // is the whole block here?  (BSIZE sits at a fixed place in every BGZF writer's header, but walk the extra field anyway)
-      if (off + 18 > n) break;
-      const uint16_t xl = h16(raw + off + 10);
-      if (off + 12 + xl > n) break;
-      int bs = -1;
-      for (size_t q = off + 12; q + 4 <= off + 12 + xl; q += 4 + h16(raw + q + 2))
-        if (raw[q] == 'B' && raw[q + 1] == 'C' && h16(raw + q + 2) == 2 && q + 6 <= off + 12 + xl) bs = h16(raw + q + 4);
-      if (bs >= 0 && off + (size_t)bs + 1 > n) break;
-    }
-    if (off + 18 > n) return false;
-    const uint8_t* h = raw + off;
-    if (h[0] != 0x1f || h[1] != 0x8b || h[2] != 8 || !(h[3] & 4)) return false;
-    const uint16_t xlen = h16(h + 10);
-    if (off + 12 + xlen > n) return false;
-    int bsize = -1;
-    size_t p = off + 12;
-    const size_t xend = off + 12 + xlen;
-    while (p + 4 <= xend) {
-      const uint16_t slen = h16(raw + p + 2);
-      if (raw[p] == 'B' && raw[p + 1] == 'C' && slen == 2 && p + 6 <= xend) bsize = h16(raw + p + 4);
-      p += 4 + slen;
-    }
-    if (bsize < 0) return false;
-    const size_t bend = off + (size_t)bsize + 1;
-    if (bend > n || (size_t)bsize + 1 < (size_t)(12 + xlen + 8)) return false;
-    BgzfBlock b;
-    b.coff = off + 12 + xlen;
-    b.clen = (uint32_t)(bend - 8 - b.coff);
-    b.crc = h32(raw + bend - 8);
-    b.ulen = h32(raw + bend - 4);
-    if (b.ulen > 65536u) return false;
-    b.uoff = uoff;
-    b.pad = 0;
-    uoff += b.ulen;
-    blocks.push_back(b);
-    off = bend;
-    if (consumed) *consumed = off;
-  }
-  total = uoff;
-  return true;
-}
-
 }  // namespace mcov
 
 using namespace mcov;
@@ -359,16 +301,15 @@ using namespace mcov;
 
 static int bfail(mcov_ctx* ctx, int code, const char* msg) { ctx->err = msg; return code; }
 
-// Header of the inflated stream at B.data (host side: magic, text, reference table) -> n_ref and the offset of the
-// first alignment record.  Also the place where the inflate status is looked at.
+// Header of the inflated stream at B.data (read on the host) -> n_ref and the offset of the first alignment record.  Also
+// the place where the inflate status is looked at.
 static int bam_dev_header(mcov_ctx* ctx, uint64_t total, uint64_t* rec_begin_out, int32_t* n_ref_out) {
   mcov_ctx::BamDev& B = ctx->bam;
   cudaStream_t s = ctx->stream;
   int st[2] = {0, 0};
   std::vector<uint8_t> head;
   size_t want = (size_t)std::min<uint64_t>(total, 1u << 20);
-  uint64_t rec_begin = 0;
-  int32_t n_ref = 0;
+  BamHeader h;
   for (;;) {
     head.resize(want);
     CUB(cudaMemcpyAsync(head.data(), B.data.p, want, cudaMemcpyDeviceToHost, s));
@@ -378,31 +319,14 @@ static int bam_dev_header(mcov_ctx* ctx, uint64_t total, uint64_t* rec_begin_out
       ctx->err = st[0] == 100 ? "mcov_bam_decode_gpu: CRC mismatch in a BGZF block" : "mcov_bam_decode_gpu: corrupt deflate stream in a BGZF block";
       return MCOV_ERR_IO;
     }
-    if (std::memcmp(head.data(), "BAM\1", 4) != 0) return bfail(ctx, MCOV_ERR_IO, "mcov_bam_decode_gpu: not a valid BAM file");
-    bool need_more = false;
-    size_t p = 8;
-    const uint64_t l_text = h32(head.data() + 4);
-    if (p + l_text + 4 > total) return bfail(ctx, MCOV_ERR_IO, "mcov_bam_decode_gpu: truncated BAM header");
-    if (p + l_text + 4 > want) need_more = true;
-    if (!need_more) {
-      p += (size_t)l_text;
-      n_ref = (int32_t)h32(head.data() + p);
-      p += 4;
-      if (n_ref < 0) return bfail(ctx, MCOV_ERR_IO, "mcov_bam_decode_gpu: bad reference count");
-      for (int32_t i = 0; i < n_ref; ++i) {
-        if (p + 4 > want) { need_more = true; break; }
-        const uint64_t l_name = h32(head.data() + p);
-        if (p + 8 + l_name > total) return bfail(ctx, MCOV_ERR_IO, "mcov_bam_decode_gpu: truncated reference table");
-        if (p + 8 + l_name > want) { need_more = true; break; }
-        p += 8 + (size_t)l_name;
-      }
-      rec_begin = p;
-    }
-    if (!need_more) break;
-    if (want >= total) return bfail(ctx, MCOV_ERR_IO, "mcov_bam_decode_gpu: truncated BAM header");
+    const HeaderParse r = parse_bam_header(head.data(), want, false, h);
+    if (r == HeaderParse::kOk) break;
+    if (r == HeaderParse::kBad) { ctx->err = std::string("mcov_bam_decode_gpu: ") + h.bad; return MCOV_ERR_IO; }
+    if (want >= total)
+      return bfail(ctx, MCOV_ERR_IO, r == HeaderParse::kMoreText ? "mcov_bam_decode_gpu: truncated BAM header" : "mcov_bam_decode_gpu: truncated reference table");
     want = (size_t)std::min<uint64_t>(total, (uint64_t)want * 4);
   }
-  *rec_begin_out = rec_begin; *n_ref_out = n_ref;
+  *rec_begin_out = h.rec_begin; *n_ref_out = h.n_ref;
   return MCOV_OK;
 }
 
@@ -461,6 +385,30 @@ static int bam_dev_chain(mcov_ctx* ctx, uint64_t total, uint64_t rec_begin, int3
   return MCOV_OK;
 }
 
+// The columns of n records and `ops` CIGAR ops: sized, written from the records of `segs` (k_bam_walk_write) and closed
+// with cig_off[n] = ops.  The rows in front of the segments' rec_base (reads carried into a chunk) are the caller's.
+static cudaError_t bam_dev_columns(mcov_ctx* ctx, const std::vector<WalkSeg>& segs, uint64_t n, uint64_t ops, SoaOut& o) {
+  mcov_ctx::BamDev& B = ctx->bam;
+  cudaStream_t s = ctx->stream;
+  const struct { DevBuf* buf; uint64_t bytes; } cols[] = {
+      {&B.tid, (n + 4) * 4}, {&B.pos, (n + 4) * 4}, {&B.flag, (n + 4) * 2}, {&B.mapq, n + 4}, {&B.lseq, (n + 4) * 4},
+      {&B.isize, (n + 4) * 4}, {&B.cig_off, (n + 5) * 4}, {&B.cig, (ops + 4) * 4}, {&B.rec_off, (n + 4) * 8}};
+  cudaError_t e;
+  for (const auto& c : cols)
+    if ((e = c.buf->ensure((size_t)c.bytes)) != cudaSuccess) return e;
+  o.tid = B.tid.as<int32_t>(); o.pos = B.pos.as<int32_t>(); o.flag = B.flag.as<uint16_t>(); o.mapq = B.mapq.as<uint8_t>();
+  o.l_seq = B.lseq.as<int32_t>(); o.isize = B.isize.as<int32_t>(); o.cig_off = B.cig_off.as<uint32_t>(); o.cig = B.cig.as<uint32_t>();
+  o.rec_off = B.rec_off.as<uint64_t>();
+  if (!segs.empty()) {
+    if ((e = cudaMemcpyAsync(B.segs.p, segs.data(), segs.size() * sizeof(WalkSeg), cudaMemcpyHostToDevice, s)) != cudaSuccess) return e;
+    MCOV_LAUNCH(ctx, kKBamWalkWrite, (k_bam_walk_write<<<(unsigned)((segs.size() + 127) / 128), 128, 0, s>>>(
+        B.data.as<uint8_t>(), B.segs.as<WalkSeg>(), (int64_t)segs.size(), o)));
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  }
+  const uint32_t last = (uint32_t)ops;                   // (a pageable source is copied before the call returns)
+  return cudaMemcpyAsync(o.cig_off + n, &last, 4, cudaMemcpyHostToDevice, s);
+}
+
 extern "C" int mcov_bam_decode_gpu(mcov_ctx* ctx, const void* file_bytes, int64_t n_bytes, int verify_crc, mcov_bam_dev* out) {
   if (!ctx) return MCOV_ERR_ARG;
   if (!file_bytes || n_bytes <= 0 || !out) return bfail(ctx, MCOV_ERR_ARG, "mcov_bam_decode_gpu: bad arguments");
@@ -471,7 +419,8 @@ extern "C" int mcov_bam_decode_gpu(mcov_ctx* ctx, const void* file_bytes, int64_
   const uint8_t* raw = static_cast<const uint8_t*>(file_bytes);
   std::vector<BgzfBlock> blocks;
   uint64_t total = 0;
-  if (!index_bgzf(raw, (size_t)n_bytes, blocks, total)) return bfail(ctx, MCOV_ERR_IO, "mcov_bam_decode_gpu: not a valid BGZF file");
+  size_t used = 0;
+  if (!bgzf_index(raw, (size_t)n_bytes, 0, false, blocks, total, used)) return bfail(ctx, MCOV_ERR_IO, "mcov_bam_decode_gpu: not a valid BGZF file");
   if (total < 12) return bfail(ctx, MCOV_ERR_IO, "mcov_bam_decode_gpu: not a valid BAM file");
   const int64_t nb = (int64_t)blocks.size();
   mcov_ctx::BamDev& B = ctx->bam;
@@ -496,22 +445,9 @@ extern "C" int mcov_bam_decode_gpu(mcov_ctx* ctx, const void* file_bytes, int64_
   uint64_t n_rec = 0, n_cig = 0;
   for (size_t i = 0; i < segs.size(); ++i) { segs[i].rec_base = n_rec; segs[i].cig_base = n_cig; n_rec += wo[i].n_rec; n_cig += wo[i].n_cig; }
   if (n_cig > 0xFFFFFFFFull) return bfail(ctx, MCOV_ERR_RANGE, "mcov_bam_decode_gpu: more than 2^32-1 CIGAR ops");
-  CUB(B.tid.ensure((n_rec + 4) * 4)); CUB(B.pos.ensure((n_rec + 4) * 4)); CUB(B.flag.ensure((n_rec + 4) * 2)); CUB(B.mapq.ensure(n_rec + 4));
-  CUB(B.lseq.ensure((n_rec + 4) * 4)); CUB(B.isize.ensure((n_rec + 4) * 4)); CUB(B.cig_off.ensure((n_rec + 5) * 4)); CUB(B.cig.ensure((n_cig + 4) * 4));
-  SoaOut o;
-  o.tid = B.tid.as<int32_t>(); o.pos = B.pos.as<int32_t>(); o.flag = B.flag.as<uint16_t>(); o.mapq = B.mapq.as<uint8_t>();
-  o.l_seq = B.lseq.as<int32_t>(); o.isize = B.isize.as<int32_t>(); o.cig_off = B.cig_off.as<uint32_t>(); o.cig = B.cig.as<uint32_t>();
-  CUB(B.rec_off.ensure((n_rec + 4) * 8));
-  o.rec_off = B.rec_off.as<uint64_t>();
   B.n_rec = 0;
-  if (!segs.empty()) {
-    CUB(cudaMemcpyAsync(B.segs.p, segs.data(), segs.size() * sizeof(WalkSeg), cudaMemcpyHostToDevice, s));
-    MCOV_LAUNCH(ctx, kKBamWalkWrite, (k_bam_walk_write<<<(unsigned)((segs.size() + 127) / 128), 128, 0, s>>>(
-        B.data.as<uint8_t>(), B.segs.as<WalkSeg>(), (int64_t)segs.size(), o)));
-    CUB(cudaGetLastError());
-  }
-  const uint32_t last = (uint32_t)n_cig;
-  CUB(cudaMemcpyAsync(o.cig_off + n_rec, &last, 4, cudaMemcpyHostToDevice, s));
+  SoaOut o;
+  CUB(bam_dev_columns(ctx, segs, n_rec, n_cig, o));
   CUB(cudaStreamSynchronize(s));
   out->n_records = (int64_t)n_rec; out->n_cigar = (int64_t)n_cig; out->n_ref = n_ref;
   out->inflated_bytes = (int64_t)total; out->header_bytes = (int64_t)rec_begin; out->n_segments = (int64_t)segs.size();
@@ -647,10 +583,9 @@ int mcov::bam_gpu_chunks(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, i
     uint8_t* raw = B.pin[cur].as<uint8_t>();
     const size_t have = left + got;
     // the next chunk of the file, behind the bytes this one will leave over (their number is known once the blocks are indexed)
-    blocks.clear();
     uint64_t total = 0;
     size_t consumed = 0;
-    if (!index_bgzf(raw, have, blocks, total, &consumed, tail_len)) return F(MCOV_ERR_IO, "not a valid BGZF file");
+    if (!bgzf_index(raw, have, tail_len, true, blocks, total, consumed)) return F(MCOV_ERR_IO, "not a valid BGZF file");
     if (eof && consumed != have) return F(MCOV_ERR_IO, "the file ends inside a BGZF block");
     if (!eof && consumed == 0) return F(MCOV_ERR_IO, "a BGZF block larger than the chunk");
     const size_t next_left = have - consumed;
@@ -708,10 +643,9 @@ int mcov::bam_gpu_chunks(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, i
         cudaMemcpyAsync(B.tail2.p, B.data.as<uint8_t>() + chain_end, (size_t)new_tail, cudaMemcpyDeviceToDevice, s);
       }
       // columns: [carried reads | this chunk's]
-      bool okm = B.tid.ensure((n_tot + 4) * 4) == cudaSuccess && B.pos.ensure((n_tot + 4) * 4) == cudaSuccess && B.flag.ensure((n_tot + 4) * 2) == cudaSuccess &&
-                 B.mapq.ensure(n_tot + 4) == cudaSuccess && B.lseq.ensure((n_tot + 4) * 4) == cudaSuccess && B.isize.ensure((n_tot + 4) * 4) == cudaSuccess &&
-                 B.cig_off.ensure((n_tot + 5) * 4) == cudaSuccess && B.cig.ensure((ops_tot + 4) * 4) == cudaSuccess && B.rec_off.ensure((n_tot + 4) * 8) == cudaSuccess;
-      if (!okm) { err_rc = F(MCOV_ERR_NOMEM, "out of device memory"); break; }
+      SoaOut o;
+      const cudaError_t ce = bam_dev_columns(ctx, segs, n_tot, ops_tot, o);
+      if (ce != cudaSuccess) { err_rc = ce == cudaErrorMemoryAllocation ? F(MCOV_ERR_NOMEM, "out of device memory") : F(MCOV_ERR_CUDA, "record walk failed"); break; }
       if (n_carry) {
         cudaMemcpyAsync(B.tid.p, B.c_tid.p, (size_t)n_carry * 4, cudaMemcpyDeviceToDevice, s);
         cudaMemcpyAsync(B.pos.p, B.c_pos.p, (size_t)n_carry * 4, cudaMemcpyDeviceToDevice, s);
@@ -720,17 +654,6 @@ int mcov::bam_gpu_chunks(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, i
         cudaMemcpyAsync(B.cig_off.p, B.c_off.p, (size_t)n_carry * 4, cudaMemcpyDeviceToDevice, s);
         if (carry_ops) cudaMemcpyAsync(B.cig.p, B.c_cig.p, (size_t)carry_ops * 4, cudaMemcpyDeviceToDevice, s);
       }
-      SoaOut o;
-      o.tid = B.tid.as<int32_t>(); o.pos = B.pos.as<int32_t>(); o.flag = B.flag.as<uint16_t>(); o.mapq = B.mapq.as<uint8_t>();
-      o.l_seq = B.lseq.as<int32_t>(); o.isize = B.isize.as<int32_t>(); o.cig_off = B.cig_off.as<uint32_t>(); o.cig = B.cig.as<uint32_t>();
-      o.rec_off = B.rec_off.as<uint64_t>();
-      if (!segs.empty()) {
-        cudaMemcpyAsync(B.segs.p, segs.data(), segs.size() * sizeof(WalkSeg), cudaMemcpyHostToDevice, s);
-        MCOV_LAUNCH(ctx, kKBamWalkWrite, (k_bam_walk_write<<<(unsigned)((segs.size() + 127) / 128), 128, 0, s>>>(
-            B.data.as<uint8_t>(), B.segs.as<WalkSeg>(), (int64_t)segs.size(), o)));
-      }
-      const uint32_t last_off = (uint32_t)ops_tot;
-      cudaMemcpyAsync(o.cig_off + n_tot, &last_off, 4, cudaMemcpyHostToDevice, s);
       if (cudaStreamSynchronize(s) != cudaSuccess) { err_rc = F(MCOV_ERR_CUDA, "record walk failed"); break; }
       std::swap(B.tail, B.tail2);
       info->inflated_bytes += (int64_t)(total - tail_len);

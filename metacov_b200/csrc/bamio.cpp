@@ -20,6 +20,7 @@
 #include <thread>
 #include <vector>
 
+#include "bamfmt.h"
 #include "metacov_b200.h"
 
 struct mcov_bam {
@@ -41,51 +42,13 @@ struct mcov_bam {
   std::vector<uint64_t> name_hash;   // FNV-1a 64 of the read name (filled with the SEQ pass)
 };
 
-namespace {
+using namespace mcov;
 
-struct Block { size_t coff, clen, uoff, ulen; uint32_t crc; };
+namespace {
 
 int set_err(char* err, int errlen, const char* msg) {
   if (err && errlen > 0) std::snprintf(err, (size_t)errlen, "%s", msg);
   return MCOV_ERR_IO;
-}
-
-inline uint16_t rd16(const uint8_t* p) { return (uint16_t)(p[0] | (p[1] << 8)); }
-inline uint32_t rd32(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24); }
-inline uint64_t rd64(const uint8_t* p) { return (uint64_t)rd32(p) | ((uint64_t)rd32(p + 4) << 32); }
-
-bool index_blocks(const std::vector<uint8_t>& raw, std::vector<Block>& blocks, size_t& total) {
-  size_t off = 0, uoff = 0;
-  const size_t n = raw.size();
-  while (off < n) {
-    if (off + 18 > n) return false;
-    const uint8_t* h = raw.data() + off;
-    if (h[0] != 0x1f || h[1] != 0x8b || h[2] != 8 || !(h[3] & 4)) return false;
-    uint16_t xlen = rd16(h + 10);
-    if (off + 12 + xlen > n) return false;
-    int bsize = -1;
-    size_t p = off + 12, xend = off + 12 + xlen;
-    while (p + 4 <= xend) {
-      uint16_t slen = rd16(raw.data() + p + 2);
-      if (raw[p] == 'B' && raw[p + 1] == 'C' && slen == 2 && p + 6 <= xend) bsize = rd16(raw.data() + p + 4);
-      p += 4 + slen;
-    }
-    if (bsize < 0) return false;
-    size_t bend = off + (size_t)bsize + 1;
-    if (bend > n || (size_t)bsize + 1 < (size_t)(12 + xlen + 8)) return false;
-    Block b;
-    b.coff = off + 12 + xlen;
-    b.clen = bend - 8 - b.coff;
-    b.crc = rd32(raw.data() + bend - 8);
-    b.ulen = rd32(raw.data() + bend - 4);
-    if (b.ulen > 65536) return false;          // BGZF: a block inflates to at most 64 KiB (SAM spec 4.1)
-    b.uoff = uoff;
-    uoff += b.ulen;
-    blocks.push_back(b);
-    off = bend;
-  }
-  total = uoff;
-  return true;
 }
 
 bool inflate_block(const uint8_t* src, size_t clen, uint8_t* dst, size_t ulen, uint32_t crc) {
@@ -104,59 +67,25 @@ bool inflate_block(const uint8_t* src, size_t clen, uint8_t* dst, size_t ulen, u
   return ok;
 }
 
-bool inflate_all(mcov_bam* b, int n_threads) {
-  std::vector<Block> blocks;
-  size_t total = 0;
-  if (!index_blocks(b->raw, blocks, total)) return false;
-  b->data.resize(total);
-  if (n_threads < 1) n_threads = 1;
-  n_threads = (int)std::min<size_t>((size_t)n_threads, std::max<size_t>(blocks.size(), 1));
+// Inflates every block from raw to dst + its uoff on n_threads host threads (at most one per block); false when a
+// block does not inflate to its ISIZE and CRC.
+bool inflate_blocks(const uint8_t* raw, const std::vector<BgzfBlock>& blocks, uint8_t* dst, int n_threads) {
+  const int nt = (int)std::max<size_t>(1, std::min<size_t>((size_t)std::max(n_threads, 1), blocks.size()));
   std::atomic<size_t> next(0);
   std::atomic<bool> good(true);
   auto work = [&]() {
     for (;;) {
-      size_t k = next.fetch_add(1);
+      const size_t k = next.fetch_add(1);
       if (k >= blocks.size() || !good.load()) break;
-      const Block& bl = blocks[k];
-      if (!inflate_block(b->raw.data() + bl.coff, bl.clen, b->data.data() + bl.uoff, bl.ulen, bl.crc)) good.store(false);
+      const BgzfBlock& bl = blocks[k];
+      if (!inflate_block(raw + bl.coff, bl.clen, dst + bl.uoff, bl.ulen, bl.crc)) good.store(false);
     }
   };
   std::vector<std::thread> th;
-  for (int t = 1; t < n_threads; ++t) th.emplace_back(work);
+  for (int t = 1; t < nt; ++t) th.emplace_back(work);
   work();
   for (auto& t : th) t.join();
   return good.load();
-}
-
-// parse the BAM header out of the inflated stream; returns false if malformed
-bool parse_header(mcov_bam* b) {
-  const std::vector<uint8_t>& d = b->data;
-  if (d.size() < 12 || std::memcmp(d.data(), "BAM\1", 4) != 0) return false;
-  uint32_t l_text = rd32(d.data() + 4);
-  size_t p = 8;
-  if (p + l_text + 4 > d.size()) return false;
-  b->text.assign(reinterpret_cast<const char*>(d.data() + p), strnlen(reinterpret_cast<const char*>(d.data() + p), l_text));
-  p += l_text;
-  uint32_t n_ref = rd32(d.data() + p);
-  p += 4;
-  b->ref_name.clear();
-  b->ref_len.clear();
-  for (uint32_t i = 0; i < n_ref; ++i) {
-    if (p + 4 > d.size()) return false;
-    uint32_t l_name = rd32(d.data() + p);
-    if (l_name == 0 || p + 4 + l_name + 4 > d.size()) return false;
-    b->ref_name.emplace_back(reinterpret_cast<const char*>(d.data() + p + 4), l_name - 1);
-    b->ref_len.push_back((int32_t)rd32(d.data() + p + 4 + l_name));
-    p += 8 + l_name;
-  }
-  b->rec_begin = p;
-  return true;
-}
-
-// fixed part + name + CIGAR + SEQ + QUAL of a record must fit its block_size (SAM spec 4.2)
-inline bool record_fits(const uint8_t* r, uint32_t bs) {
-  const uint64_t l_read_name = r[8], n_op = rd16(r + 12), l_seq = rd32(r + 16);
-  return 32ull + l_read_name + 4ull * n_op + (l_seq + 1) / 2 + l_seq <= (uint64_t)bs;
 }
 
 // nothing may throw across the C ABI: allocation failures and anything else become status codes
@@ -165,6 +94,22 @@ int guarded(F fn) {
   try { return fn(); }
   catch (const std::bad_alloc&) { return MCOV_ERR_NOMEM; }
   catch (...) { return MCOV_ERR_IO; }
+}
+
+// Calls f(i, r) for every record i of the inflated stream, r pointing behind its block_size; false when a record does
+// not fit its block_size or the stream does not end where the last record does.
+template <typename F>
+bool each_record(const mcov_bam* b, F f) {
+  const uint8_t* d = b->data.data();
+  const size_t n = b->data.size();
+  size_t p = b->rec_begin, i = 0;
+  while (p + 4 <= n) {
+    const uint32_t bs = rd32(d + p);
+    if (bs < 32 || p + 4 + bs > n || !record_fits(d + p + 4, bs)) return false;
+    f(i++, d + p + 4);
+    p += 4 + bs;
+  }
+  return p == n;
 }
 
 }  // namespace
@@ -181,9 +126,17 @@ static int read_inflate(mcov_bam* b) {
   size_t got = b->raw.empty() ? 0 : std::fread(b->raw.data(), 1, b->raw.size(), fh);
   std::fclose(fh);
   if (got != b->raw.size()) return 2;
+  std::vector<BgzfBlock> blocks;
+  uint64_t total = 0;
+  size_t used = 0;
+  if (!bgzf_index(b->raw.data(), b->raw.size(), 0, false, blocks, total, used)) return 3;
+  b->data.resize(total);
   unsigned hw = std::thread::hardware_concurrency();
-  if (!inflate_all(b, hw ? (int)hw : 4)) return 3;
-  if (!parse_header(b)) return 4;
+  if (!inflate_blocks(b->raw.data(), blocks, b->data.data(), hw ? (int)hw : 4)) return 3;
+  BamHeader h;
+  if (parse_bam_header(b->data.data(), b->data.size(), true, h) != HeaderParse::kOk) return 4;
+  b->text.swap(h.text); b->ref_name.swap(h.names); b->ref_len.swap(h.lens);
+  b->rec_begin = h.rec_begin;
   std::vector<uint8_t>().swap(b->raw);
   return 0;
 }
@@ -269,40 +222,14 @@ int mcov_bam_load(mcov_bam* b, int /*n_threads*/) {
   return guarded([&]() { return bam_load_impl(b); });
 }
 static int bam_load_impl(mcov_bam* b) {
-  const uint8_t* d = b->data.data();
-  const size_t n = b->data.size();
-  // pass 1: count records and ops
-  size_t p = b->rec_begin, n_rec = 0, n_cig = 0;
-  while (p + 4 <= n) {
-    uint32_t bs = rd32(d + p);
-    if (bs < 32 || p + 4 + bs > n || !record_fits(d + p + 4, bs)) return MCOV_ERR_IO;
-    n_cig += rd16(d + p + 4 + 12);
-    ++n_rec;
-    p += 4 + bs;
-  }
-  if (p != n) return MCOV_ERR_IO;
+  size_t n_rec = 0, n_cig = 0;
+  if (!each_record(b, [&](size_t, const uint8_t* r) { n_cig += record_n_op(r); ++n_rec; })) return MCOV_ERR_IO;
   if (n_cig > 0xFFFFFFFFull) return MCOV_ERR_RANGE;
   b->tid.resize(n_rec); b->pos.resize(n_rec); b->lseq.resize(n_rec); b->isize.resize(n_rec);
   b->flag.resize(n_rec); b->mapq.resize(n_rec); b->cig_off.resize(n_rec + 1); b->cig.resize(n_cig);
-  p = b->rec_begin;
+  const RecordCols c{b->tid.data(), b->pos.data(), b->lseq.data(), b->isize.data(), b->flag.data(), b->mapq.data()};
   size_t co = 0;
-  for (size_t i = 0; i < n_rec; ++i) {
-    uint32_t bs = rd32(d + p);
-    const uint8_t* r = d + p + 4;
-    b->tid[i] = (int32_t)rd32(r);
-    b->pos[i] = (int32_t)rd32(r + 4);
-    uint8_t l_read_name = r[8];
-    b->mapq[i] = r[9];
-    uint16_t n_op = rd16(r + 12);
-    b->flag[i] = rd16(r + 14);
-    b->lseq[i] = (int32_t)rd32(r + 16);
-    b->isize[i] = (int32_t)rd32(r + 28);
-    if (32u + l_read_name + 4u * n_op > bs) return MCOV_ERR_IO;
-    b->cig_off[i] = (uint32_t)co;
-    std::memcpy(b->cig.data() + co, r + 32 + l_read_name, 4u * n_op);
-    co += n_op;
-    p += 4 + bs;
-  }
+  each_record(b, [&](size_t i, const uint8_t* r) { b->cig_off[i] = (uint32_t)co; co += copy_record(r, c, i, b->cig.data() + co); });
   b->cig_off[n_rec] = (uint32_t)co;
   std::vector<uint8_t>().swap(b->data);   // the SoA arrays are all that is kept
   b->loaded = true;
@@ -330,38 +257,22 @@ int mcov_bam_load_seq(mcov_bam* b) {
 }
 static int bam_load_seq_impl(mcov_bam* b) {
   if (b->data.empty()) { if (read_inflate(b)) return MCOV_ERR_IO; }
-  const uint8_t* d = b->data.data();
-  const size_t n = b->data.size();
-  size_t p = b->rec_begin, n_rec = 0, bytes = 0;
-  while (p + 4 <= n) {
-    uint32_t bs = rd32(d + p);
-    if (bs < 32 || p + 4 + bs > n || !record_fits(d + p + 4, bs)) return MCOV_ERR_IO;
-    bytes += ((size_t)rd32(d + p + 4 + 16) + 1) / 2;
-    ++n_rec;
-    p += 4 + bs;
-  }
+  size_t n_rec = 0, bytes = 0;
+  if (!each_record(b, [&](size_t, const uint8_t* r) { bytes += ((size_t)rd32(r + 16) + 1) / 2; ++n_rec; })) return MCOV_ERR_IO;
   b->seq_off.resize(n_rec + 1);
   b->seq.resize(bytes);
   b->name_hash.resize(n_rec);
-  p = b->rec_begin;
   size_t so = 0;
-  for (size_t i = 0; i < n_rec; ++i) {
-    uint32_t bs = rd32(d + p);
-    const uint8_t* r = d + p + 4;
-    uint8_t l_read_name = r[8];
-    uint16_t n_op = rd16(r + 12);
-    size_t l_seq = rd32(r + 16), nb = (l_seq + 1) / 2;
-    if (32u + l_read_name + 4u * n_op + nb > bs) return MCOV_ERR_IO;
+  each_record(b, [&](size_t i, const uint8_t* r) {
+    const uint8_t l_read_name = r[8];
+    const size_t nb = ((size_t)rd32(r + 16) + 1) / 2;
     b->seq_off[i] = so;
-    {
-      uint64_t h = 1469598103934665603ull;                    // FNV-1a 64 over the name (without the NUL)
-      for (unsigned k = 0; k + 1 < l_read_name; ++k) { h ^= r[32 + k]; h *= 1099511628211ull; }
-      b->name_hash[i] = h == ~0ull ? h - 1 : h;               // ~0 is the "no entry" key of the pair sort
-    }
-    std::memcpy(b->seq.data() + so, r + 32 + l_read_name + 4u * n_op, nb);
+    uint64_t h = 1469598103934665603ull;                      // FNV-1a 64 over the name (without the NUL)
+    for (unsigned k = 0; k + 1 < l_read_name; ++k) { h ^= r[32 + k]; h *= 1099511628211ull; }
+    b->name_hash[i] = h == ~0ull ? h - 1 : h;                 // ~0 is the "no entry" key of the pair sort
+    std::memcpy(b->seq.data() + so, r + 32 + l_read_name + 4u * record_n_op(r), nb);
     so += nb;
-    p += 4 + bs;
-  }
+  });
   b->seq_off[n_rec] = so;
   b->has_seq = true;
   if (b->loaded) std::vector<uint8_t>().swap(b->data);
@@ -551,94 +462,29 @@ bool stream_refill(mcov_bam_stream* s) {
   const size_t got = std::fread(s->raw.data() + old, 1, want, s->fh);
   s->raw.resize(old + got);
   if (got < want) s->eof = true;
-  // index the complete blocks
-  std::vector<Block> blocks;
-  size_t off = 0, uoff = 0;
-  const size_t n = s->raw.size();
-  while (off + 18 <= n) {
-    const uint8_t* h = s->raw.data() + off;
-    if (h[0] != 0x1f || h[1] != 0x8b || h[2] != 8 || !(h[3] & 4)) return false;
-    const uint16_t xlen = rd16(h + 10);
-    if (off + 12 + xlen > n) break;
-    int bsize = -1;
-    size_t p = off + 12;
-    const size_t xend = off + 12 + xlen;
-    while (p + 4 <= xend) {
-      const uint16_t slen = rd16(s->raw.data() + p + 2);
-      if (s->raw[p] == 'B' && s->raw[p + 1] == 'C' && slen == 2 && p + 6 <= xend) bsize = rd16(s->raw.data() + p + 4);
-      p += 4 + slen;
-    }
-    if (bsize < 0) return false;
-    const size_t bend = off + (size_t)bsize + 1;
-    if (bend > n) break;                                   // incomplete block: wait for the next chunk
-    if ((size_t)bsize + 1 < (size_t)(12 + xlen + 8)) return false;
-    Block b;
-    b.coff = off + 12 + xlen; b.clen = bend - 8 - b.coff;
-    b.crc = rd32(s->raw.data() + bend - 8); b.ulen = rd32(s->raw.data() + bend - 4);
-    if (b.ulen > 65536) return false;
-    b.uoff = uoff; uoff += b.ulen;
-    blocks.push_back(b);
-    off = bend;
-  }
-  if (s->eof && off != n) return false;                    // trailing garbage / truncated block
-  const size_t base = s->data.size();
-  s->data.resize(base + uoff);
-  std::atomic<size_t> next(0);
-  std::atomic<bool> good(true);
-  auto work = [&]() {
-    for (;;) {
-      const size_t k = next.fetch_add(1);
-      if (k >= blocks.size() || !good.load()) break;
-      const Block& bl = blocks[k];
-      if (!inflate_block(s->raw.data() + bl.coff, bl.clen, s->data.data() + base + bl.uoff, bl.ulen, bl.crc)) good.store(false);
-    }
-  };
-  const int nt = (int)std::max<size_t>(1, std::min<size_t>((size_t)s->n_threads, blocks.size()));
-  std::vector<std::thread> th;
-  for (int t = 1; t < nt; ++t) th.emplace_back(work);
-  work();
-  for (auto& t : th) t.join();
-  if (!good.load()) return false;
-  s->raw.erase(s->raw.begin(), s->raw.begin() + (ptrdiff_t)off);
+  // inflate the complete blocks onto the end of `data`
+  std::vector<BgzfBlock> blocks;
+  uint64_t end = 0;
+  size_t used = 0;
+  if (!bgzf_index(s->raw.data(), s->raw.size(), s->data.size(), !s->eof, blocks, end, used)) return false;
+  s->data.resize(end);
+  if (!inflate_blocks(s->raw.data(), blocks, s->data.data(), s->n_threads)) return false;
+  s->raw.erase(s->raw.begin(), s->raw.begin() + (ptrdiff_t)used);
   return true;
 }
 
 // header: magic, text, reference table; may span several chunks
 int stream_parse_header(mcov_bam_stream* s) {
   for (;;) {
-    const std::vector<uint8_t>& d = s->data;
-    bool need = false;
-    size_t p = 0;
-    if (d.size() < 12) need = true;
-    else {
-      if (std::memcmp(d.data(), "BAM\1", 4) != 0) return 4;
-      const uint32_t l_text = rd32(d.data() + 4);
-      p = 8;
-      if (p + (size_t)l_text + 4 > d.size()) need = true;
-      else {
-        const uint32_t n_ref = rd32(d.data() + p + l_text);
-        size_t q = p + l_text + 4;
-        std::vector<std::string> names;
-        std::vector<int32_t> lens;
-        for (uint32_t i = 0; i < n_ref && !need; ++i) {
-          if (q + 4 > d.size()) { need = true; break; }
-          const uint32_t l_name = rd32(d.data() + q);
-          if (l_name == 0) return 4;
-          if (q + 4 + (size_t)l_name + 4 > d.size()) { need = true; break; }
-          names.emplace_back(reinterpret_cast<const char*>(d.data() + q + 4), l_name - 1);
-          lens.push_back((int32_t)rd32(d.data() + q + 4 + l_name));
-          q += 8 + l_name;
-        }
-        if (!need) {
-          s->text.assign(reinterpret_cast<const char*>(d.data() + p), strnlen(reinterpret_cast<const char*>(d.data() + p), l_text));
-          s->ref_name.swap(names); s->ref_len.swap(lens);
-          s->data_pos = q;
-          s->header_done = true;
-          return 0;
-        }
-      }
+    BamHeader h;
+    const HeaderParse r = parse_bam_header(s->data.data(), s->data.size(), true, h);
+    if (r == HeaderParse::kOk) {
+      s->text.swap(h.text); s->ref_name.swap(h.names); s->ref_len.swap(h.lens);
+      s->data_pos = h.rec_begin;
+      s->header_done = true;
+      return 0;
     }
-    if (s->eof) return 4;
+    if (r == HeaderParse::kBad || s->eof) return 4;
     if (!stream_refill(s)) return 3;
   }
 }
@@ -706,7 +552,7 @@ static int stream_next_impl(mcov_bam_stream* s, int32_t resend_tid, int32_t rese
       if (avail >= 4 + (size_t)bs) {
         if (!record_fits(s->data.data() + s->data_pos + 4, bs)) { s->err = "record fields exceed block_size"; return MCOV_ERR_IO; }
         s->rec_off.push_back(s->data_pos);
-        new_ops += rd16(s->data.data() + s->data_pos + 4 + 12);
+        new_ops += record_n_op(s->data.data() + s->data_pos + 4);
         s->data_pos += 4 + (size_t)bs;
         have = true;
       }
@@ -786,22 +632,16 @@ static int stream_next_impl(mcov_bam_stream* s, int32_t resend_tid, int32_t rese
   const int64_t nc = (int64_t)carry.size();
   // ---- new reads: offsets serially (a prefix sum over the op counts), fields and ops in parallel ----
   const uint8_t* d = s->data.data();
-  for (int64_t i = 0; i < n_new; ++i) { cur.cig_off[nc + i] = co; co += rd16(d + s->rec_off[(size_t)i] + 4 + 12); }
+  for (int64_t i = 0; i < n_new; ++i) { cur.cig_off[nc + i] = co; co += record_n_op(d + s->rec_off[(size_t)i] + 4); }
   cur.cig_off[n] = co;
   std::atomic<int32_t> mx(s->max_reflen);
+  const RecordCols cols{cur.tid, cur.pos, cur.lseq, cur.isize, cur.flag, cur.mapq};
   auto fill = [&](int64_t lo, int64_t hi) {
     int32_t local_max = 1;
     for (int64_t i = lo; i < hi; ++i) {
-      const uint8_t* r = d + s->rec_off[(size_t)i] + 4;
       const int64_t k = nc + i;
-      cur.tid[k] = (int32_t)rd32(r); cur.pos[k] = (int32_t)rd32(r + 4);
-      const uint8_t l_read_name = r[8];
-      cur.mapq[k] = r[9];
-      const uint16_t n_op = rd16(r + 12);
-      cur.flag[k] = rd16(r + 14);
-      cur.lseq[k] = (int32_t)rd32(r + 16); cur.isize[k] = (int32_t)rd32(r + 28);
       uint32_t* dst = cur.cig + cur.cig_off[k];
-      std::memcpy(dst, r + 32 + l_read_name, 4u * n_op);
+      const uint16_t n_op = copy_record(d + s->rec_off[(size_t)i] + 4, cols, (size_t)k, dst);
       int64_t rl = 0;
       for (uint16_t o = 0; o < n_op; ++o) { const uint32_t op = dst[o]; if ((0x18Du >> (op & 15u)) & 1u) rl += op >> 4; }
       const int32_t rl32 = rl > 0x7fffffff ? 0x7fffffff : (int32_t)rl;
