@@ -872,6 +872,65 @@ int  mcov_compare_sites(mcov_ctx* ctx, int32_t n_sig, const uint8_t* const* sig,
  * MCOV_ERR_ARG for a range outside it.  Synchronises. */
 int  mcov_compare_sites_read(mcov_ctx* ctx, int64_t first, int64_t n, mcov_compare_site* host_out);
 
+/* Linkage between nearby SNV sites from the reads and their mates
+ * (csrc/linkage.cu; the rules are restated in oracle/linkage.py).
+ *   sites   the SNV sites (kind bit 1) of the counts of the last
+ *           mcov_base_counts under sites.min_coverage / min_freq / min_count,
+ *           exactly those mcov_allele_sites lists with use_reference = 0.  At
+ *           a site the major allele is the consensus and the minor allele the
+ *           largest of the other three counts (ties to the first of A C G T).
+ *   units   the records mcov_base_counts counts, grouped by the FNV-1a 64 of
+ *           QNAME (~0 folded to ~0 - 1, the key of mcov_bam_gpu_names_seq):
+ *           mates and supplementary pieces are one unit; equal keys are one
+ *           unit, collisions included (two names collide with odds of about
+ *           2^-64 a pair).  A record whose QNAME is '*' is a unit of its own.
+ *   calls   a record gives a base at a site when the site's position is the
+ *           reference position of one of its M / = / X pairs, the base is A,
+ *           C, G or T and, with a non-zero quality_threshold, its quality is
+ *           at least the threshold: the bases the counts counted, under the
+ *           quality_threshold and mode the counts were made with.  A unit has
+ *           call 0 (major) or 1 (minor) at a site when all its bases there are
+ *           that allele; any disagreement, or a third allele, is no call.
+ *   pairs   sites s < t of one contig with 0 < pos_t - pos_s <= max_distance;
+ *           every unit with calls at both adds 1 to n[call_s][call_t].  A pair
+ *           is listed when n_AB + n_Ab + n_aB + n_ab >= min_reads, in (tid,
+ *           pos_a, pos_b) order (upper case: the major allele).
+ * path NULL reads the records of the last device decode (BAM or SAM); a path
+ * reads the BAM again through the streamed decoder (a second decode of the
+ * file), with chunk_bytes as in mcov_bam_gpu_stream_depth.  The counts must be
+ * those of the same records.  MCOV_ERR_ARG for bad parameters
+ * (sites.use_reference must be 0); MCOV_ERR_STATE without counts for the
+ * current contig table, or without a decoded file when path is NULL;
+ * MCOV_ERR_NOMEM, before the
+ * allocation, when a buffer does not fit the free device memory (the message
+ * holds both byte counts); MCOV_ERR_IO as mcov_base_counts reports it.  The
+ * depth store, its caches, the counts, the reference store and the allele and
+ * compare site lists are never written; after an error the context is
+ * usable.  Synchronises. */
+typedef struct mcov_linkage_params {
+  mcov_allele_params sites;      /* the SNV rules; sites.use_reference must be 0 */
+  int32_t  max_distance;         /* 1 .. 100000 */
+  uint32_t min_reads;            /* >= 1 */
+} mcov_linkage_params;
+/* One listed pair: the sites' 0-based positions, their alleles as 'A' 'C' 'G'
+ * 'T' and the four haplotype counts.  32 bytes. */
+typedef struct mcov_linkage_pair {
+  int32_t  tid, pos_a, pos_b;
+  uint8_t  major_a, minor_a, major_b, minor_b;
+  uint32_t n_AB, n_Ab, n_aB, n_ab;
+} mcov_linkage_pair;
+/* SNV sites; (record, site) bases; units with at least one such base;
+ * candidate pairs (site pairs within max_distance). */
+typedef struct mcov_linkage_info { int64_t n_sites, n_observations, n_units, n_candidates; } mcov_linkage_info;
+/* The pairs, into a list kept on the device; their number in *n_pairs_out,
+ * the totals above in *info (may be NULL). */
+int  mcov_linkage(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, const mcov_linkage_params* params,
+                  int64_t* n_pairs_out, mcov_linkage_info* info);
+/* The pairs [first, first + n) of the last mcov_linkage into host_out[n].
+ * MCOV_ERR_STATE without a list for the current contig table, MCOV_ERR_ARG for
+ * a range outside it.  Synchronises. */
+int  mcov_linkage_read(mcov_ctx* ctx, int64_t first, int64_t n, mcov_linkage_pair* host_out);
+
 /* Test hooks: the device inflate / CRC-32 code (csrc/inflate.cuh) compiled for the host, so that the CPU
  * suite can check it against zlib.  mcov_inflate_host returns 0 or a positive decoder status. */
 int  mcov_inflate_host(const uint8_t* src, uint32_t clen, uint8_t* dst, uint32_t ulen);

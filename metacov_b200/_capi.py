@@ -92,6 +92,24 @@ assert COMPARE_SITE_DTYPE.itemsize == 16      # mcov_compare_site
 COMPARE_CON_SNP, COMPARE_POP_SNP = 1, 2
 
 
+class LinkageParams(C.Structure):
+    """mcov_linkage_params."""
+    _fields_ = [("sites", AlleleParams), ("max_distance", C.c_int32), ("min_reads", C.c_uint32)]
+
+
+class LinkageInfo(C.Structure):
+    """mcov_linkage_info."""
+    _fields_ = [("n_sites", C.c_int64), ("n_observations", C.c_int64), ("n_units", C.c_int64), ("n_candidates", C.c_int64)]
+
+
+# mcov_linkage_pair: the two sites, their major / minor alleles as ASCII letters, the four haplotype counts (upper case
+# = the major allele)
+LINKAGE_PAIR_DTYPE = np.dtype([("tid", "<i4"), ("pos_a", "<i4"), ("pos_b", "<i4"), ("major_a", "S1"), ("minor_a", "S1"),
+                               ("major_b", "S1"), ("minor_b", "S1"), ("n_AB", "<u4"), ("n_Ab", "<u4"), ("n_aB", "<u4"),
+                               ("n_ab", "<u4")])
+assert LINKAGE_PAIR_DTYPE.itemsize == 32 and C.sizeof(LinkageParams) == 32      # mcov_linkage_pair, mcov_linkage_params
+
+
 class BamGpuStreamInfo(C.Structure):
     _fields_ = [("n_records", C.c_int64), ("n_chunks", C.c_int64), ("n_segments", C.c_int64), ("inflated_bytes", C.c_int64),
                 ("file_bytes", C.c_int64), ("max_carry", C.c_int64)]
@@ -203,6 +221,8 @@ SIGNATURES = {
     "mcov_compare_run": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i64, _vp, _vp, _vp, _vp]),
     "mcov_compare_sites": (C.c_int, [_vp, _i32, _vp, _i32, _vp, C.POINTER(_i64)]),
     "mcov_compare_sites_read": (C.c_int, [_vp, _i64, _i64, _vp]),
+    "mcov_linkage": (C.c_int, [_vp, C.c_char_p, _i64, C.POINTER(LinkageParams), C.POINTER(_i64), C.POINTER(LinkageInfo)]),
+    "mcov_linkage_read": (C.c_int, [_vp, _i64, _i64, _vp]),
     "mcov_sam_parse_host": (C.c_int, [_vp, C.c_int64, C.POINTER(SamHostCols), C.c_char_p, C.c_int]),
     "mcov_inflate_host": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint32]),
     "mcov_inflate_host_win": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint32, C.c_uint32]),

@@ -862,6 +862,32 @@ class AlignmentFile:
                                      min_coverage, min_freq, min_count)
         return eng.allele_signature(min_coverage, min_freq, min_count)
 
+    def linkage(self, quality_threshold=15, read_callback="all", min_coverage=5, min_freq=0.05, min_count=2,
+                max_distance=1000, min_reads=20):
+        """Linkage between nearby SNV sites (inStrain's linkage table with fixed allele calls): for every pair of SNV
+        sites of ``allele_sites`` (no reference) on one contig at most ``max_distance`` apart, the haplotype counts of
+        the units -- the records sharing a read name, so a read and its mate -- that call both sites, listed when at
+        least ``min_reads`` units do.  Returns (structured array ``_capi.LINKAGE_PAIR_DTYPE``: tid pos_a pos_b major_a
+        minor_a major_b minor_b n_AB n_Ab n_aB n_ab, in (tid, pos_a, pos_b) order; dict n_sites, n_observations,
+        n_units, n_candidates); ``alleles.derive_linkage`` gives distance, r2 and D'.  The rules are those of
+        ``mcov_linkage`` (include/metacov_b200.h).
+
+        The counts are those of ``count_coverage`` (same cache).  A file decoded on the device links from its resident
+        records; any other file is read again through the GPU decoder.  Bad parameters raise ValueError before any
+        work, a piped stream ValueError, device memory that does not fit MemoryError naming the file.  The depth, the
+        counts and the allele sites are left as they were."""
+        self._no_records("linkage()")
+        _check_read_callback(read_callback)
+        CoverageEngine._linkage_params(min_coverage, min_freq, min_count, max_distance, min_reads)   # (ValueError first)
+        eng = self._counted(quality_threshold, read_callback)
+        path = None if self._gpu is not None else self.filename
+        try:
+            return eng.linkage(min_coverage, min_freq, min_count, max_distance, min_reads, path=path,
+                               chunk_bytes=self._gpu_chunk_bytes)
+        except McovError as e:
+            self._raise_nomem(e)
+            raise
+
     def _allele_engine(self, what, fasta, quality_threshold, read_callback, min_coverage, min_freq, min_count):
         """The count engine with the counts of (threshold, read_callback) and, given a FASTA, its reference."""
         self._no_records(what)

@@ -41,3 +41,27 @@ def derive_compare(stats):
         "percent_compared": _ratio(s["compared"], s["length"]),
         "pop_ani": 1.0 - _ratio(s["pop_snp"], s["compared"]),
     }
+
+
+LINKAGE_DERIVED = ("distance", "r2", "d_prime")
+
+
+def derive_linkage(pairs):
+    """{name: float64 array} of the pair records of ``AlignmentFile.linkage`` / ``CoverageEngine.linkage``, with fixed
+    allele calls (upper case the major allele) and total = n_AB + n_Ab + n_aB + n_ab: p_A = (n_AB + n_Ab) / total,
+    p_B = (n_AB + n_aB) / total, D = n_AB / total - p_A p_B, r2 = D^2 / (p_A (1 - p_A) p_B (1 - p_B)) and
+    d_prime = |D| / D_max, D_max = min(p_A (1 - p_B), (1 - p_A) p_B) for D > 0, else min(p_A p_B, (1 - p_A)(1 - p_B));
+    distance = pos_b - pos_a.  These are inStrain's definitions of r2 and D', without its rarefied columns.  A division
+    by zero gives NaN."""
+    s = pairs
+    ab, a_b, ab_, ab2 = (np.asarray(s[k], dtype=np.float64) for k in ("n_AB", "n_Ab", "n_aB", "n_ab"))
+    total = ab + a_b + ab_ + ab2
+    p_a = _ratio(ab + a_b, total)
+    p_b = _ratio(ab + ab_, total)
+    d = _ratio(ab, total) - p_a * p_b
+    d_max = np.where(d > 0, np.minimum(p_a * (1.0 - p_b), (1.0 - p_a) * p_b), np.minimum(p_a * p_b, (1.0 - p_a) * (1.0 - p_b)))
+    return {
+        "distance": np.asarray(s["pos_b"], dtype=np.float64) - np.asarray(s["pos_a"], dtype=np.float64),
+        "r2": _ratio(d * d, p_a * (1.0 - p_a) * p_b * (1.0 - p_b)),
+        "d_prime": _ratio(np.abs(d), d_max),
+    }

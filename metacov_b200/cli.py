@@ -18,7 +18,7 @@ from . import pileup as _pileup
 from . import scan as _scan
 from . import util
 from .alignmentfile import AlignmentFile
-from .alleles import derive, derive_compare
+from .alleles import derive, derive_compare, derive_linkage
 from .compare import compare as _compare, read_references
 from .samstream import is_stream
 from .fasta import FastaFile
@@ -241,27 +241,37 @@ def scan(readfile, readfile_type, out_basehist, boffset, out_kmerhist, k, number
         n += 1
 
 
-def _allele_options(sites_help):
-    """The options `alleles` and `compare` share, in this order behind their own; ``sites_help``: --sites-out's help."""
+def _allele_rule_options():
+    """The allele rules' options (counts, present alleles, coverage) and --bam-decode, which `alleles`, `compare` and
+    `linkage` share, in this order behind their own."""
+    return [
+        click.option("--quality-threshold", "-q", type=int, default=15, show_default=True,
+                     help="Count a base only with a quality of at least this (0: every base)."),
+        click.option("--read-callback", type=click.Choice(["all", "nofilter"]), default="all", show_default=True,
+                     help="all: skip unmapped, secondary, QC-fail and duplicate reads; nofilter: count every "
+                          "placed read."),
+        click.option("--min-coverage", type=click.IntRange(1), default=5, show_default=True),
+        click.option("--min-freq", type=click.FloatRange(0, 1), default=0.05, show_default=True),
+        click.option("--min-count", type=click.IntRange(1), default=2, show_default=True),
+        click.option("--bam-decode", type=click.Choice(["host", "gpu", "gpu-stream", "auto"]), default="auto",
+                     show_default=True, help="Where the BAM file is inflated and parsed (see `pileup`).")]
+
+
+def _apply(options):
     def apply(f):
-        for option in reversed([
-                click.option("--regionfile-blast7", "-rb", type=click.File("r"), help="Input Region file in BLAST7 format"),
-                click.option("--regionfile-csv", "-rc", type=click.File("r"), help="Input Region file in CSV format"),
-                click.option("--outfile", "-o", type=click.File("w"), default="-", help="Output CSV (default STDOUT)"),
-                click.option("--sites-out", type=click.File("w"), metavar="FILE", help=sites_help),
-                click.option("--quality-threshold", "-q", type=int, default=15, show_default=True,
-                             help="Count a base only with a quality of at least this (0: every base)."),
-                click.option("--read-callback", type=click.Choice(["all", "nofilter"]), default="all", show_default=True,
-                             help="all: skip unmapped, secondary, QC-fail and duplicate reads; nofilter: count every "
-                                  "placed read."),
-                click.option("--min-coverage", type=click.IntRange(1), default=5, show_default=True),
-                click.option("--min-freq", type=click.FloatRange(0, 1), default=0.05, show_default=True),
-                click.option("--min-count", type=click.IntRange(1), default=2, show_default=True),
-                click.option("--bam-decode", type=click.Choice(["host", "gpu", "gpu-stream", "auto"]), default="auto",
-                             show_default=True, help="Where the BAM file is inflated and parsed (see `pileup`).")]):
+        for option in reversed(options):
             f = option(f)
         return f
     return apply
+
+
+def _allele_options(sites_help):
+    """The options `alleles` and `compare` share, in this order behind their own; ``sites_help``: --sites-out's help."""
+    return _apply([
+        click.option("--regionfile-blast7", "-rb", type=click.File("r"), help="Input Region file in BLAST7 format"),
+        click.option("--regionfile-csv", "-rc", type=click.File("r"), help="Input Region file in CSV format"),
+        click.option("--outfile", "-o", type=click.File("w"), default="-", help="Output CSV (default STDOUT)"),
+        click.option("--sites-out", type=click.File("w"), metavar="FILE", help=sites_help)] + _allele_rule_options())
 
 
 def _refuse_stream(path, option="-b/--bamfile"):
@@ -370,6 +380,47 @@ def compare(bamfiles, regionfile_blast7, regionfile_csv, outfile, sites_out, qua
             writer.writerow(row)
     if sites_out is not None:
         write_compare_sites(names, bamfiles, res.pairs, res.sites, sites_out)
+
+
+@main.command()
+@click.option("--bamfile", "-b", type=click.Path(dir_okay=False, allow_dash=True), required=True,
+              help="Input BAM or SAM file (any read order, no index needed; mates share a read name). Not a pipe: the "
+                   "linkage needs every record.")
+@click.option("--outfile", "-o", type=click.File("w"), default="-", help="Output TSV (default STDOUT)")
+@click.option("--max-distance", type=click.IntRange(1, 100000), default=1000, show_default=True,
+              help="Link SNV sites at most this many bases apart.")
+@click.option("--min-reads", type=click.IntRange(1), default=20, show_default=True,
+              help="List a pair of sites when at least this many read pairs (or reads) call both.")
+@_apply(_allele_rule_options())
+def linkage(bamfile, outfile, max_distance, min_reads, quality_threshold, read_callback, min_coverage, min_freq, min_count,
+            bam_decode):
+    """
+    Linkage between nearby SNV sites on the GPU: for each pair of SNV sites that enough reads and their mates span, the
+    four haplotype counts, r2 and D' (inStrain's linkage table with fixed allele calls).  Not in the reference:
+    additive.
+    """
+    _refuse_stream(bamfile)
+    with AlignmentFile(bamfile, decode=bam_decode) as bam:
+        pairs, _info = bam.linkage(quality_threshold=quality_threshold, read_callback=read_callback,
+                                   min_coverage=min_coverage, min_freq=min_freq, min_count=min_count,
+                                   max_distance=max_distance, min_reads=min_reads)
+        write_linkage(bam.references, pairs, outfile)
+
+
+def write_linkage(references, pairs, out):
+    """Linkage pairs as TSV lines: contig (first word of its name), both 0-based positions, their distance, the major
+    and minor allele of each site, the four haplotype counts (upper case = major), their total, r2 and D'."""
+    names = [ref.split()[0] for ref in references]
+    derived = derive_linkage(pairs)
+    out.write("contig\tpos_a\tpos_b\tdistance\tmajor_a\tminor_a\tmajor_b\tminor_b\tn_AB\tn_Ab\tn_aB\tn_ab\ttotal\tr2"
+              "\td_prime\n")
+    cols = [pairs[k].tolist() for k in ("tid", "pos_a", "pos_b", "major_a", "minor_a", "major_b", "minor_b", "n_AB", "n_Ab",
+                                        "n_aB", "n_ab")]
+    for (t, pa, pb, ma, na, mb, nb, c0, c1, c2, c3), r2, dp in zip(zip(*cols), derived["r2"].tolist(),
+                                                                  derived["d_prime"].tolist()):
+        out.write("%s\t%d\t%d\t%d\t%s\t%s\t%s\t%s\t%d\t%d\t%d\t%d\t%d\t%r\t%r\n" % (
+            names[t], pa, pb, pb - pa, ma.decode(), na.decode(), mb.decode(), nb.decode(), c0, c1, c2, c3,
+            c0 + c1 + c2 + c3, r2, dp))
 
 
 def _alleles_of(sig):

@@ -77,16 +77,25 @@ int upload_region_chunks(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int
   return MCOV_OK;
 }
 
-int size_site_list(mcov_ctx* ctx, SiteList& sl, int64_t items, size_t site_bytes, const char* who, int64_t* total) {
+int size_site_list(mcov_ctx* ctx, SiteList& sl, int64_t items, size_t site_bytes, const char* who, int64_t* total,
+                   const char* free_hook) {
   cudaStream_t s = ctx->stream;
   int64_t* tile_n = ctx->d_site_tiles.as<int64_t>();
   size_t tb = 0;
   CTX_CU(who, cub::DeviceScan::InclusiveSum(nullptr, tb, tile_n, tile_n + items, items, s));
-  CTX_CU(who, ctx->d_site_scan.ensure(tb));
+  if (!free_hook) {
+    CTX_CU(who, ctx->d_site_scan.ensure(tb));
+  } else if (int rc = ensure_fits_n(ctx, ctx->d_site_scan, tb, free_hook, who,
+                                    "the scan of %lld tile counts needs %zu bytes of device memory, %zu are free", items)) {
+    return rc;
+  }
   CTX_CU(who, cub::DeviceScan::InclusiveSum(ctx->d_site_scan.p, tb, tile_n, tile_n + items, items, s));
   CTX_CU(who, cudaMemcpyAsync(total, tile_n + 2 * items - 1, 8, cudaMemcpyDeviceToHost, s));
   CTX_CU(who, cudaStreamSynchronize(s));
   const size_t bytes = (size_t)*total * site_bytes;
+  if (*total > 0 && free_hook)
+    return ensure_fits_n(ctx, sl.list, bytes, free_hook, who, "a list of %lld records needs %zu bytes of device memory, %zu are free",
+                         (long long)*total);
   if (*total > 0 && sl.list.ensure(bytes) != cudaSuccess) {
     (void)cudaGetLastError();
     char msg[200];
@@ -165,18 +174,20 @@ extern "C" int mcov_allele_stats_run(mcov_ctx* ctx, int64_t g, const int32_t* ti
   return MCOV_OK;
 }
 
-extern "C" int mcov_allele_sites(mcov_ctx* ctx, const mcov_allele_params* params, int64_t* n_sites_out) {
-  const char* who = "mcov_allele_sites";
-  if (!ctx) return MCOV_ERR_ARG;
-  ctx->allele_sites.n = -1;
-  if (!n_sites_out) return ctx_fail(ctx, MCOV_ERR_ARG, "mcov_allele_sites: null n_sites_out");
-  AlleleParams P;
-  if (int rc = al_check(ctx, params, &P, who)) return rc;
-  CTX_CU(who, cudaSetDevice(ctx->device));
+namespace mcov {
+
+int allele_site_list(mcov_ctx* ctx, const AlleleParams& P, SiteList& sl, const char* who, int64_t* total_out,
+                     const char* free_hook) {
+  sl.n = -1;
   cudaStream_t s = ctx->stream;
   const int64_t n_tiles = (ctx->n_slots + kAlTile - 1) / kAlTile;
   // [n_tiles] site counts, then [n_tiles] their inclusive scan
-  CTX_CU(who, ctx->d_site_tiles.ensure((size_t)n_tiles * 16));
+  if (!free_hook) {
+    CTX_CU(who, ctx->d_site_tiles.ensure((size_t)n_tiles * 16));
+  } else if (int rc = ensure_fits_n(ctx, ctx->d_site_tiles, (size_t)n_tiles * 16, free_hook, who,
+                                    "the counts of %lld site tiles need %zu bytes of device memory, %zu are free", n_tiles)) {
+    return rc;
+  }
   AlSiteArgs a;
   a.cnt = ctx->d_bc.as<uint4>(); a.ref = ctx->d_ref.as<uint8_t>();
   a.n_slots = ctx->n_slots; a.n_tiles = n_tiles;
@@ -186,17 +197,30 @@ extern "C" int mcov_allele_sites(mcov_ctx* ctx, const mcov_allele_params* params
   MCOV_LAUNCH(ctx, kKAlleleSiteCount, (k_allele_site_count<<<al_grid(ctx, n_tiles, 1), kAlTileThreads, 0, s>>>(a)));
   CTX_CU(who, cudaGetLastError());
   int64_t total = 0;
-  if (int rc = size_site_list(ctx, ctx->allele_sites, n_tiles, sizeof(mcov_allele_site), who, &total)) return rc;
+  if (int rc = size_site_list(ctx, sl, n_tiles, sizeof(mcov_allele_site), who, &total, free_hook)) return rc;
   if (total > 0) {
-    a.sites = ctx->allele_sites.list.as<mcov_allele_site>();
+    a.sites = sl.list.as<mcov_allele_site>();
     MCOV_LAUNCH(ctx, kKAlleleSiteWrite, (k_allele_site_write<<<al_grid(ctx, n_tiles, 1), kAlTileThreads, 0, s>>>(a)));
     CTX_CU(who, cudaGetLastError());
     CTX_CU(who, cudaStreamSynchronize(s));
   }
-  ctx->allele_sites.n = total;
-  ctx->allele_sites.epoch = ctx->contig_epoch;
-  *n_sites_out = total;
+  sl.n = total;
+  sl.epoch = ctx->contig_epoch;
+  *total_out = total;
   return MCOV_OK;
+}
+
+}  // namespace mcov
+
+extern "C" int mcov_allele_sites(mcov_ctx* ctx, const mcov_allele_params* params, int64_t* n_sites_out) {
+  const char* who = "mcov_allele_sites";
+  if (!ctx) return MCOV_ERR_ARG;
+  ctx->allele_sites.n = -1;
+  if (!n_sites_out) return ctx_fail(ctx, MCOV_ERR_ARG, "mcov_allele_sites: null n_sites_out");
+  AlleleParams P;
+  if (int rc = al_check(ctx, params, &P, who)) return rc;
+  CTX_CU(who, cudaSetDevice(ctx->device));
+  return allele_site_list(ctx, P, ctx->allele_sites, who, n_sites_out);
 }
 
 extern "C" int mcov_allele_sites_read(mcov_ctx* ctx, int64_t first, int64_t n, mcov_allele_site* host_out) {

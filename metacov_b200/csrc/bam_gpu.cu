@@ -37,6 +37,7 @@
 #include "bamfmt.h"
 #include "ctx.cuh"
 #include "inflate.cuh"
+#include "k_sam.cuh"
 
 namespace mcov {
 
@@ -219,11 +220,7 @@ __global__ void k_bam_names_seq(const uint8_t* __restrict__ d, const uint64_t* _
   const uint8_t* cig = r + 32 + l_name;
   const uint8_t* sq = cig + 4ull * n_op;
   if (32ull + l_name + 4ull * n_op + (uint64_t)((l_seq + 1) / 2) > bs) { atomicExch(status + 2, 1); return; }   // SEQ leaves the record
-  if (name_hash) {
-    uint64_t h = 1469598103934665603ull;
-    for (uint32_t k = 0; k + 1 < l_name; ++k) { h ^= r[32 + k]; h *= 1099511628211ull; }
-    name_hash[i] = h == ~0ull ? h - 1 : h;                     // ~0 is the "no entry" key of the pair sort
-  }
+  if (name_hash) name_hash[i] = read_name_key<1>(r, 32, l_name);
   auto base = [&](int64_t a) -> uint32_t { const uint32_t b = sq[a >> 1]; return (a & 1) ? (b & 15u) : (b >> 4); };
   if (kmer_code) {
     int64_t lo = 0, hi = l_seq;

@@ -68,6 +68,8 @@ enum KernelId {
   kKBcAny,
   kKRefEncode, kKAlleleChunks, kKAlleleCombine, kKAlleleSiteCount, kKAlleleSiteWrite,
   kKAlleleSignature, kKCompareChunks, kKCompareCombine, kKCompareSiteCount, kKCompareSiteWrite,
+  kKLinkSites, kKLinkObsCount, kKLinkObsWrite, kKLinkSort, kKLinkUnitCalls, kKLinkSelect, kKLinkPairs, kKLinkPairCount,
+  kKLinkPairWrite,
   kKernelCount
 };
 
@@ -212,6 +214,12 @@ struct mcov_ctx {
   mcov::DevBuf d_chunks, d_chunk_meta, d_chunk_part, d_region_out, d_site_tiles, d_site_scan;
   // the site lists of the last mcov_allele_sites and mcov_compare_sites (both stay readable)
   mcov::SiteList allele_sites, compare_sites;
+  // Linkage (linkage.cu): its own SNV site list and pair list; per site the slot, contig, alleles, partner counts and
+  // their scan; per record of a batch its observation count and their scan; the observations (two buffers for the
+  // sort); the candidate pairs' counters; CUB scratch and the call / unit totals
+  mcov::SiteList link_sites, link_pairs;
+  mcov::DevBuf d_lk_slot, d_lk_tid, d_lk_allele, d_lk_partners, d_lk_base, d_lk_rec_n, d_lk_rec_off, d_lk_obs[2], d_lk_cnt,
+      d_lk_tmp, d_lk_word;
 
   // fused (sorted) path scratch
   mcov::DevBuf d_start_slot, d_far_list, d_tile_cnt, d_tile_off, d_far_sorted;
@@ -310,9 +318,10 @@ inline int ctx_fail(mcov_ctx* ctx, int code, const std::string& what, cudaError_
 }
 
 // buf.ensure(need), unless the allocation that takes (DevBuf::grown) exceeds the free device memory plus buf's own:
-// then MCOV_ERR_NOMEM, "who: " + msg, a format of (n_slots, bytes wanted, bytes free).  The environment variable
+// then MCOV_ERR_NOMEM, "who: " + msg, a format of (n, bytes wanted, bytes free); ensure_fits gives n_slots as n.  The environment variable
 // free_hook, when set, stands in for the free bytes (a test hook).
-inline int ensure_fits(mcov_ctx* ctx, DevBuf& buf, size_t need, const char* free_hook, const char* who, const char* msg) {
+inline int ensure_fits_n(mcov_ctx* ctx, DevBuf& buf, size_t need, const char* free_hook, const char* who, const char* msg,
+                         long long n) {
   if (buf.cap < need) {
     size_t free_b = 0, total_b = 0;
     CTX_CU(who, cudaMemGetInfo(&free_b, &total_b));
@@ -320,12 +329,15 @@ inline int ensure_fits(mcov_ctx* ctx, DevBuf& buf, size_t need, const char* free
     const size_t want = DevBuf::grown(need);
     if (want > free_b + buf.cap) {
       char text[256];
-      std::snprintf(text, sizeof(text), msg, (long long)ctx->n_slots, want, free_b + buf.cap);
+      std::snprintf(text, sizeof(text), msg, n, want, free_b + buf.cap);
       return ctx_fail(ctx, MCOV_ERR_NOMEM, std::string(who) + ": " + text);
     }
   }
   CTX_CU(who, buf.ensure(need));
   return MCOV_OK;
+}
+inline int ensure_fits(mcov_ctx* ctx, DevBuf& buf, size_t need, const char* free_hook, const char* who, const char* msg) {
+  return ensure_fits_n(ctx, buf, need, free_hook, who, msg, (long long)ctx->n_slots);
 }
 
 // g regions of the contig table, and where their records go
@@ -366,6 +378,14 @@ int upload_region_chunks(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int
 
 // alleles.cu: between a site list's count launch, which wrote `items` tile counts to ctx->d_site_tiles, and its write
 // launch: the counts' inclusive scan into the `items` words behind them, the total read back, sl.list sized for it.
-int size_site_list(mcov_ctx* ctx, SiteList& sl, int64_t items, size_t site_bytes, const char* who, int64_t* total);
+// With free_hook, the scan scratch and the list are checked against the free device memory first (ensure_fits_n, that
+// test hook); without, a list that does not fit is MCOV_ERR_NOMEM once its allocation has failed.
+int size_site_list(mcov_ctx* ctx, SiteList& sl, int64_t items, size_t site_bytes, const char* who, int64_t* total,
+                   const char* free_hook = nullptr);
+
+// alleles.cu: every site of the counts under P (mcov_allele_site records in slot order) into sl; *total their number.
+// free_hook as in size_site_list, for the tile counts as well.
+int allele_site_list(mcov_ctx* ctx, const AlleleParams& P, SiteList& sl, const char* who, int64_t* total,
+                     const char* free_hook = nullptr);
 
 }  // namespace mcov

@@ -71,6 +71,19 @@ MCOV_HD uint32_t sam_name_hash32(const uint8_t* p, uint32_t n) {
   return h;
 }
 
+// The key of a read name: FNV-1a 64 of the name's bytes, with ~0 folded to ~0 - 1 (~0 is the "no entry" key of the pair
+// sort of pileup.experimental).  The name is base[at, at + len - kNul): BAM's l_read_name counts a closing NUL that is
+// not hashed (kNul 1), a SAM QNAME is len bytes (kNul 0).  The one definition of the key that joins mates:
+// k_bam_names_seq, sam_names_seq_one and the linkage observations (k_linkage.cuh) all take it from here (the loop keeps
+// the form each of the first two had, so that they compile as before); the host reader's mcov_bam_name_hash computes
+// the same value.
+template <uint32_t kNul>
+MCOV_HD uint64_t read_name_key(const uint8_t* base, uint32_t at, uint32_t len) {
+  uint64_t h = 1469598103934665603ull;
+  for (uint32_t k = 0; k + kNul < len; ++k) { h ^= base[at + k]; h *= 1099511628211ull; }
+  return h == ~0ull ? h - 1 : h;
+}
+
 // The @SQ names as an open-addressing table: slot -> tid (-1 empty), names in one blob at name_off[tid].
 struct SamRefTable {
   const int32_t* slot; uint32_t mask;
@@ -115,11 +128,7 @@ MCOV_HD bool sam_field_value(int f, const uint8_t* p, uint32_t n, int64_t seq_le
 MCOV_HD void sam_names_seq_one(const uint8_t* qname, uint32_t l_qname, const uint8_t* seq, int64_t l_seq, uint32_t flag,
                                const uint32_t* cig, uint32_t n_op, int32_t k_len, int32_t win_bases, uint64_t* name_hash,
                                int32_t* kmer_code, uint8_t* win) {
-  if (name_hash) {
-    uint64_t h = 1469598103934665603ull;
-    for (uint32_t k = 0; k < l_qname; ++k) { h ^= qname[k]; h *= 1099511628211ull; }
-    *name_hash = h == ~0ull ? h - 1 : h;
-  }
+  if (name_hash) *name_hash = read_name_key<0>(qname, 0, l_qname);
   if (kmer_code) {
     int64_t lo = 0, hi = l_seq;
     for (uint32_t k = 0; k < n_op; ++k) {

@@ -607,7 +607,10 @@ void mcov_destroy(mcov_ctx* ctx) {
                     &ctx->d_out, &ctx->d_win_slot, &ctx->d_win_n, &ctx->d_win_out, &ctx->d_htasks, &ctx->d_tile_heavy, &ctx->d_run_tasks, &ctx->d_run_counts, &ctx->d_run_out,
                     &ctx->d_starts, &ctx->d_bc, &ctx->d_bc_word,
                     &ctx->d_ref, &ctx->d_ref_stage, &ctx->d_pair_sigs, &ctx->d_chunks, &ctx->d_chunk_meta, &ctx->d_chunk_part,
-                    &ctx->d_region_out, &ctx->d_site_tiles, &ctx->d_site_scan, &ctx->allele_sites.list, &ctx->compare_sites.list};
+                    &ctx->d_region_out, &ctx->d_site_tiles, &ctx->d_site_scan, &ctx->allele_sites.list, &ctx->compare_sites.list,
+                    &ctx->link_sites.list, &ctx->link_pairs.list, &ctx->d_lk_slot, &ctx->d_lk_tid, &ctx->d_lk_allele,
+                    &ctx->d_lk_partners, &ctx->d_lk_base, &ctx->d_lk_rec_n, &ctx->d_lk_rec_off, &ctx->d_lk_obs[0],
+                    &ctx->d_lk_obs[1], &ctx->d_lk_cnt, &ctx->d_lk_tmp, &ctx->d_lk_word};
   for (DevBuf* b : bufs) b->release();
   ctx->bam.release();
   ctx->h_pin.release();
@@ -1095,7 +1098,9 @@ static const char* kKernelNames[kKernelCount] = {
     "k_cap_exact", "k_sam_line_max",
     "k_bc_any",
     "k_ref_encode", "k_allele_chunks", "k_allele_combine", "k_allele_site_count", "k_allele_site_write",
-    "k_allele_signature", "k_compare_chunks", "k_compare_combine", "k_compare_site_count", "k_compare_site_write"};
+    "k_allele_signature", "k_compare_chunks", "k_compare_combine", "k_compare_site_count", "k_compare_site_write",
+    "k_link_sites", "k_link_obs_count", "k_link_obs_write", "cub_link_sort", "k_link_unit_calls", "cub_link_select",
+    "k_link_pairs", "k_link_pair_count", "k_link_pair_write"};
 
 int mcov_copy_to_host(mcov_ctx* ctx, const void* dev, void* host, int64_t n_bytes) {
   if (!ctx) return MCOV_ERR_ARG;

@@ -335,6 +335,33 @@ class CoverageEngine:
         self._check(lib.mcov_allele_sites_read(self._ctx, 0, n.value, _capi.ptr(out)))
         return out
 
+    # -- linkage (SNV sites of base_counts, then the records they were counted from) ---------------------------------
+    @staticmethod
+    def _linkage_params(min_coverage, min_freq, min_count, max_distance, min_reads):
+        p = _capi.LinkageParams()
+        p.sites = CoverageEngine._allele_params(min_coverage, min_freq, min_count, False)
+        if int(max_distance) != max_distance or not 1 <= int(max_distance) <= 100000:
+            raise ValueError("max_distance must be an integer in [1, 100000], got %r" % (max_distance,))
+        if int(min_reads) != min_reads or not 1 <= int(min_reads) < 2 ** 32:
+            raise ValueError("min_reads must be an integer >= 1, got %r" % (min_reads,))
+        p.max_distance, p.min_reads = int(max_distance), int(min_reads)
+        return p
+
+    def linkage(self, min_coverage=5, min_freq=0.05, min_count=2, max_distance=1000, min_reads=20, path=None,
+                chunk_bytes=0):
+        """Haplotype counts of every pair of SNV sites within ``max_distance`` that ``min_reads`` units span
+        (``mcov_linkage``) -> (structured array ``_capi.LINKAGE_PAIR_DTYPE``, dict n_sites / n_observations / n_units /
+        n_candidates).  Needs ``base_counts`` first; the records are those of the last decode on this engine, or of the
+        BAM at ``path`` read again through the streamed decoder."""
+        p = self._linkage_params(min_coverage, min_freq, min_count, max_distance, min_reads)
+        n = C.c_int64(0)
+        info = _capi.LinkageInfo()
+        path = os.fsencode(path) if path is not None else None
+        self._check(lib.mcov_linkage(self._ctx, path, int(chunk_bytes), C.byref(p), C.byref(n), C.byref(info)))
+        out = np.zeros(n.value, dtype=_capi.LINKAGE_PAIR_DTYPE)
+        self._check(lib.mcov_linkage_read(self._ctx, 0, n.value, _capi.ptr(out)))
+        return out, {name: int(getattr(info, name)) for name, _ in _capi.LinkageInfo._fields_}
+
     # -- comparisons (signatures of base_counts, then pairs of signatures) --------------------------------------------
     def allele_signature(self, min_coverage=5, min_freq=0.05, min_count=2):
         """The signature of every slot (``mcov_allele_signature``) -> CUDA ``torch.uint8`` tensor of ``n_slots``: 0x80

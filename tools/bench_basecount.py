@@ -48,8 +48,9 @@ def _bgzf(data, level=1, block=0xff00):
     return b"".join(blocks) + bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")
 
 
-def write_bam_fast(path, lengths, tid, pos, flag, mapq, cig_off, cig, seq_nt16, qual):
-    """A BAM of fixed-length reads (SEQ / QUAL [n, L_SEQ]) from columns, built with numpy (record layout SAM spec 4.2)."""
+def write_bam_fast(path, lengths, tid, pos, flag, mapq, cig_off, cig, seq_nt16, qual, names=None):
+    """A BAM of fixed-length reads (SEQ / QUAL [n, L_SEQ]) from columns, built with numpy (record layout SAM spec 4.2).
+    ``names``: per record a read name of exactly 11 bytes (default r0000000000, r0000000001, ...)."""
     n = len(tid)
     nop = np.diff(cig_off.astype(np.int64))
     fixed = np.zeros(n, dtype=[("bs", "<i4"), ("ref", "<i4"), ("pos", "<i4"), ("ln", "u1"), ("mq", "u1"), ("bin", "<u2"),
@@ -59,7 +60,7 @@ def write_bam_fast(path, lengths, tid, pos, flag, mapq, cig_off, cig, seq_nt16, 
     body = 32 + 12 + 4 * nop + sq + L_SEQ
     fixed["bs"] = body; fixed["ref"] = tid; fixed["pos"] = pos; fixed["ln"] = 12; fixed["mq"] = mapq; fixed["bin"] = 4680
     fixed["nc"] = nop; fixed["fl"] = flag; fixed["ls"] = L_SEQ; fixed["nr"] = -1; fixed["np"] = -1
-    fixed["name"] = np.char.mod("r%010d", np.arange(n)).astype("S12")
+    fixed["name"] = np.char.mod("r%010d", np.arange(n)).astype("S12") if names is None else np.asarray(names, "S12")
     text = ("@HD\tVN:1.4\tSO:coordinate\n" + "".join("@SQ\tSN:c%d\tLN:%d\n" % (c, l) for c, l in enumerate(lengths))).encode()
     head = b"BAM\x01" + struct.pack("<i", len(text)) + text + struct.pack("<i", len(lengths))
     for c, l in enumerate(lengths):
