@@ -931,6 +931,71 @@ int  mcov_linkage(mcov_ctx* ctx, const char* path, int64_t chunk_bytes, const mc
  * a range outside it.  Synchronises. */
 int  mcov_linkage_read(mcov_ctx* ctx, int64_t first, int64_t n, mcov_linkage_pair* host_out);
 
+/* Genes profiled codon by codon from the counts of the last mcov_base_counts
+ * and the reference (csrc/genes.cu; the rules are restated in oracle/genes.py).
+ *   gene     (tid, start, end, strand +1 / -1, phase 0-2), 0-based half-open,
+ *            0 <= start < end <= the contig's length.  Its codons are read
+ *            from its 5' end after phase bases (from start on +, back from end
+ *            on -): K = (end - start - phase) / 3 of them (0 if negative), a
+ *            trailing 1-2 bases belong to none; on - the bases are
+ *            complemented.  Codon index 0 is the 5'-most codon.
+ *   called   a codon whose three positions are covered (the allele rules
+ *            above) and whose three reference bases are known.  Everything
+ *            below counts over called codons only.
+ *   sites3   n3 + s3 = 9 a called codon: of its 3 positions x 3 other bases,
+ *            the changes that alter the amino acid (n3) or not (s3) under the
+ *            standard code, '*' counted as an amino acid (Nei-Gojobori in
+ *            thirds).
+ *   SNV      a position where two or more alleles are present; major = the
+ *            consensus, minor = the largest of the other three counts (ties
+ *            to the first of A C G T).  S when the codon with the major and
+ *            the codon with the minor at this position (reference bases at
+ *            the other two) translate alike, else N; M for every SNV position
+ *            of a codon that holds two or more.
+ *   SUB      a position whose consensus differs from the reference: the
+ *            reference codon against the codon with the consensus at this
+ *            position, S or N; M for a codon with two or more.
+ * The gene call takes the allele parameters with use_reference = 1 (else
+ * MCOV_ERR_ARG, as for bad parameters, a gene outside its contig, a strand
+ * other than +1 / -1 or a phase outside 0-2).  MCOV_ERR_STATE without counts
+ * for the current contig table or with a contig that has had no
+ * mcov_set_reference.  The depth store, its caches, the counts, the reference
+ * store and the allele, compare and linkage lists are never written; after an
+ * error the context is usable. */
+/* One gene: length = end - start, codons = K, codons_called, the expected
+ * sites in thirds (n_sites3 + s_sites3 = 9 codons_called), SNV and SUB
+ * positions by type.  96 bytes. */
+typedef struct mcov_gene_stats {
+  int64_t length, codons, codons_called, n_sites3, s_sites3;
+  int64_t snv_n, snv_s, snv_m, sub_n, sub_s, sub_m, pad;
+} mcov_gene_stats;
+/* One (gene, position) with kind SNV or SUB in a called codon: the gene's
+ * index, the contig and 0-based position, the codon index and the position in
+ * it (0-2 from the 5' end), the reference codon as three letters in gene
+ * orientation, the major (consensus) and minor allele in genomic orientation
+ * as allele_sites gives them, the amino acids of the reference codon and of
+ * the codon with the major / minor allele here, kind bits (1 SNV, 2 SUB) and
+ * the SNV and SUB types 'N' 'S' 'M'.  minor, aa_minor and snv_type are 0 off
+ * SNV positions, sub_type 0 off SUB positions.  32 bytes. */
+typedef struct mcov_gene_site {
+  int64_t  gene;
+  int32_t  tid, pos, codon;
+  uint8_t  codon_pos, ref_codon[3], major, minor, aa_ref, aa_major, aa_minor, kind, snv_type, sub_type;
+} mcov_gene_site;
+/* The records of g genes into host_out[g].  With n_sites_out, every site of
+ * every gene, in (gene, pos) order (pos ascending on both strands; a position
+ * in two genes is listed once for each), into a list kept on the device, and
+ * their number in *n_sites_out; NULL skips the list.  MCOV_ERR_NOMEM, with the
+ * byte count, when the list does not fit (test hook MCOV_GENE_FREE_BYTES).
+ * Synchronises. */
+int  mcov_gene_run(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int32_t* start, const int32_t* end,
+                   const int32_t* strand, const int32_t* phase, const mcov_allele_params* params,
+                   mcov_gene_stats* host_out, int64_t* n_sites_out);
+/* The sites [first, first + n) of the last mcov_gene_run with a list into
+ * host_out[n].  MCOV_ERR_STATE without a list for the current contig table,
+ * MCOV_ERR_ARG for a range outside it.  Synchronises. */
+int  mcov_gene_sites_read(mcov_ctx* ctx, int64_t first, int64_t n, mcov_gene_site* host_out);
+
 /* Test hooks: the device inflate / CRC-32 code (csrc/inflate.cuh) compiled for the host, so that the CPU
  * suite can check it against zlib.  mcov_inflate_host returns 0 or a positive decoder status. */
 int  mcov_inflate_host(const uint8_t* src, uint32_t clen, uint8_t* dst, uint32_t ulen);

@@ -18,7 +18,7 @@ INCLUDE = os.path.join(ROOT, "include")
 LIB = os.path.join(HERE, "libmetacov_b200.so")
 BUILD_DIR = os.path.join(ROOT, "build")
 
-CUDA_SOURCES = ["mcov_api.cu", "stats_sort.cu", "experimental.cu", "synth.cu", "bam_gpu.cu", "sam_gpu.cu", "basecount.cu", "alleles.cu", "compare.cu", "linkage.cu"]
+CUDA_SOURCES = ["mcov_api.cu", "stats_sort.cu", "experimental.cu", "synth.cu", "bam_gpu.cu", "sam_gpu.cu", "basecount.cu", "alleles.cu", "compare.cu", "linkage.cu", "genes.cu"]
 CXX_SOURCES = ["bamio.cpp", "transport.cpp"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -109,6 +109,20 @@ LINKAGE_PAIR_DTYPE = np.dtype([("tid", "<i4"), ("pos_a", "<i4"), ("pos_b", "<i4"
                                ("n_ab", "<u4")])
 assert LINKAGE_PAIR_DTYPE.itemsize == 32 and C.sizeof(LinkageParams) == 32      # mcov_linkage_pair, mcov_linkage_params
 
+GENE_STATS_DTYPE = np.dtype([(name, "<i8") for name in (
+    "length", "codons", "codons_called", "n_sites3", "s_sites3", "snv_n", "snv_s", "snv_m", "sub_n", "sub_s", "sub_m",
+    "pad")])
+assert GENE_STATS_DTYPE.itemsize == 96        # mcov_gene_stats
+
+# mcov_gene_site: the gene's index, the position, the codon and the position in it (0-2 from the 5' end), the reference
+# codon in gene orientation, major / minor allele in genomic orientation, the amino acids, kind bits (1 SNV, 2 SUB), the
+# types 'N' 'S' 'M' (b"" where a field does not apply)
+GENE_SITE_DTYPE = np.dtype([("gene", "<i8"), ("tid", "<i4"), ("pos", "<i4"), ("codon", "<i4"), ("codon_pos", "u1"),
+                            ("ref_codon", "S3"), ("major", "S1"), ("minor", "S1"), ("aa_ref", "S1"), ("aa_major", "S1"),
+                            ("aa_minor", "S1"), ("kind", "u1"), ("snv_type", "S1"), ("sub_type", "S1")])
+assert GENE_SITE_DTYPE.itemsize == 32         # mcov_gene_site
+GENE_SNV, GENE_SUB = 1, 2
+
 
 class BamGpuStreamInfo(C.Structure):
     _fields_ = [("n_records", C.c_int64), ("n_chunks", C.c_int64), ("n_segments", C.c_int64), ("inflated_bytes", C.c_int64),
@@ -223,6 +237,8 @@ SIGNATURES = {
     "mcov_compare_sites_read": (C.c_int, [_vp, _i64, _i64, _vp]),
     "mcov_linkage": (C.c_int, [_vp, C.c_char_p, _i64, C.POINTER(LinkageParams), C.POINTER(_i64), C.POINTER(LinkageInfo)]),
     "mcov_linkage_read": (C.c_int, [_vp, _i64, _i64, _vp]),
+    "mcov_gene_run": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, C.POINTER(AlleleParams), _vp, C.POINTER(_i64)]),
+    "mcov_gene_sites_read": (C.c_int, [_vp, _i64, _i64, _vp]),
     "mcov_sam_parse_host": (C.c_int, [_vp, C.c_int64, C.POINTER(SamHostCols), C.c_char_p, C.c_int]),
     "mcov_inflate_host": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint32]),
     "mcov_inflate_host_win": (C.c_int, [_vp, C.c_uint32, _vp, C.c_uint32, C.c_uint32]),

@@ -853,6 +853,49 @@ class AlignmentFile:
                                            min_coverage, min_freq, min_count)
         return eng.allele_sites(min_coverage, min_freq, min_count, use_reference=use_ref)
 
+    def gene_stats(self, genes, fasta, quality_threshold=15, read_callback="all", min_coverage=5, min_freq=0.05,
+                   min_count=2, sites=False):
+        """Genes profiled codon by codon (inStrain's gene_info with fixed allele calls) from the counts of
+        ``count_coverage`` (same counts, same cache) and the reference ``fasta`` (as in ``allele_stats``; required).
+        ``genes``: a ``genes.GeneTable`` (``genes.read_genes``) or anything with its columns contig, start, end (0-based
+        half-open), strand (+1 / -1) and phase (0-2); a contig is matched by the first word of its name.
+
+        Returns (records, stats, sites): ``_capi.GENE_STATS_DTYPE`` per gene (length, codons, codons_called, n_sites3,
+        s_sites3, snv_n / s / m, sub_n / s / m; ``alleles.derive_genes`` gives pN/pS and dN/dS), ``allele_stats`` over
+        the same intervals (``alleles.derive`` gives breadth, depth, pi ...), and with ``sites`` every SNV or SUB
+        position of a called codon in (gene, pos) order as ``_capi.GENE_SITE_DTYPE``, else None.  The rules are those
+        of ``mcov_gene_run`` (include/metacov_b200.h).  An unknown contig raises KeyError, a gene outside its contig or
+        bad parameters ValueError before any work, a piped stream ValueError, a site list that does not fit the device
+        MemoryError."""
+        if fasta is None:
+            raise ValueError("gene_stats() needs the reference FASTA")
+        first = {(name.split() or [name])[0]: tid for tid, name in enumerate(self.references)}
+        tid = np.array([first[(str(c).split() or [str(c)])[0]] for c in genes.contig], dtype=np.int64)
+        start = np.asarray(genes.start, dtype=np.int64).reshape(-1)
+        end = np.asarray(genes.end, dtype=np.int64).reshape(-1)
+        strand = np.asarray(genes.strand, dtype=np.int64).reshape(-1)
+        phase = np.asarray(genes.phase, dtype=np.int64).reshape(-1)
+        if not len(tid) == len(start) == len(end) == len(strand) == len(phase):
+            raise ValueError("the gene columns differ in length")
+        lengths = np.asarray(self.lengths, dtype=np.int64)
+        bad = np.nonzero((start < 0) | (end <= start) | (end > lengths[tid]) | ((strand != 1) & (strand != -1))
+                         | (phase < 0) | (phase > 2))[0]
+        if len(bad):
+            k = int(bad[0])
+            raise ValueError("gene %d (%s:%d-%d, strand %d, phase %d) needs 0 <= start < end <= the contig's length %d, "
+                             "strand +1 or -1 and phase 0-2" % (k, genes.contig[k], start[k], end[k], strand[k], phase[k],
+                                                                lengths[tid[k]]))
+        eng, _ = self._allele_engine("gene_stats()", fasta, quality_threshold, read_callback, min_coverage, min_freq,
+                                     min_count)
+        try:
+            records, listed = eng.gene_stats(tid, start, end, strand, phase, min_coverage, min_freq, min_count,
+                                             sites=sites)
+        except McovError as e:
+            self._raise_nomem(e)
+            raise
+        stats = eng.allele_stats(tid, start, end, min_coverage, min_freq, min_count, use_reference=True)
+        return records, stats, listed
+
     def allele_signature(self, quality_threshold=15, read_callback="all", min_coverage=5, min_freq=0.05, min_count=2):
         """The signature of every slot of the count engine's table from the counts of ``count_coverage`` (same counts,
         same cache): a CUDA ``torch.uint8`` tensor of ``n_slots`` bytes, 0x80 covered, bits 4-5 the consensus (0-3 =

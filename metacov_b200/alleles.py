@@ -65,3 +65,20 @@ def derive_linkage(pairs):
         "r2": _ratio(d * d, p_a * (1.0 - p_a) * p_b * (1.0 - p_b)),
         "d_prime": _ratio(np.abs(d), d_max),
     }
+
+
+GENE_DERIVED = ("N_sites", "S_sites", "pN", "pS", "pn_ps", "dN", "dS", "dn_ds")
+
+
+def derive_genes(records):
+    """{name: float64 array} of the gene records of ``AlignmentFile.gene_stats`` / ``CoverageEngine.gene_stats``:
+    N_sites = n_sites3 / 3, S_sites = s_sites3 / 3, pN = snv_n / N_sites, pS = snv_s / S_sites, pn_ps = pN / pS,
+    dN = sub_n / N_sites, dS = sub_s / S_sites, dn_ds = dN / dS; no Jukes-Cantor correction.  A division by zero gives
+    NaN."""
+    s = records
+    n_sites = np.asarray(s["n_sites3"], dtype=np.float64) / 3.0
+    s_sites = np.asarray(s["s_sites3"], dtype=np.float64) / 3.0
+    p_n, p_s = _ratio(s["snv_n"], n_sites), _ratio(s["snv_s"], s_sites)
+    d_n, d_s = _ratio(s["sub_n"], n_sites), _ratio(s["sub_s"], s_sites)
+    return {"N_sites": n_sites, "S_sites": s_sites, "pN": p_n, "pS": p_s, "pn_ps": _ratio(p_n, p_s),
+            "dN": d_n, "dS": d_s, "dn_ds": _ratio(d_n, d_s)}

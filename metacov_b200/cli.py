@@ -18,10 +18,11 @@ from . import pileup as _pileup
 from . import scan as _scan
 from . import util
 from .alignmentfile import AlignmentFile
-from .alleles import derive, derive_compare, derive_linkage
+from .alleles import derive, derive_compare, derive_genes, derive_linkage
 from .compare import compare as _compare, read_references
 from .samstream import is_stream
 from .fasta import FastaFile
+from .genes import read_genes
 
 logging.basicConfig(level=logging.INFO, format="[%(relativeCreated)6.1f %(funcName)s]  %(message)s",
                     datefmt="%I:%M:%S")
@@ -242,8 +243,8 @@ def scan(readfile, readfile_type, out_basehist, boffset, out_kmerhist, k, number
 
 
 def _allele_rule_options():
-    """The allele rules' options (counts, present alleles, coverage) and --bam-decode, which `alleles`, `compare` and
-    `linkage` share, in this order behind their own."""
+    """The allele rules' options (counts, present alleles, coverage) and --bam-decode, which `alleles`, `compare`,
+    `linkage` and `genes` share, in this order behind their own."""
     return [
         click.option("--quality-threshold", "-q", type=int, default=15, show_default=True,
                      help="Count a base only with a quality of at least this (0: every base)."),
@@ -421,6 +422,57 @@ def write_linkage(references, pairs, out):
         out.write("%s\t%d\t%d\t%d\t%s\t%s\t%s\t%s\t%d\t%d\t%d\t%d\t%d\t%r\t%r\n" % (
             names[t], pa, pb, pb - pa, ma.decode(), na.decode(), mb.decode(), nb.decode(), c0, c1, c2, c3,
             c0 + c1 + c2 + c3, r2, dp))
+
+
+@main.command()
+@click.option("--bamfile", "-b", type=click.Path(dir_okay=False, allow_dash=True), required=True,
+              help="Input BAM or SAM file (any read order, no index needed). Not a pipe: the counts need every record.")
+@click.option("--reference-fasta", "-f", type=click.Path(exists=True, dir_okay=False), required=True,
+              help="Reference the reads were mapped to.")
+@click.option("--genes", "-g", "gene_file", type=click.Path(exists=True, dir_okay=False), required=True,
+              help="Genes: Prodigal's nucleotide FASTA (genes.fna) or GFF3 (its CDS lines).")
+@click.option("--outfile", "-o", type=click.File("w"), default="-", help="Output CSV (default STDOUT)")
+@click.option("--sites-out", type=click.File("w"), metavar="FILE",
+              help="Also write every SNV / SUB position of a called codon as TSV (pos 0-based).")
+@_apply(_allele_rule_options())
+def genes(bamfile, reference_fasta, gene_file, outfile, sites_out, quality_threshold, read_callback, min_coverage,
+          min_freq, min_count, bam_decode):
+    """
+    Profile genes on the GPU: codons called, expected N and S sites, SNVs and substitutions typed synonymous (S),
+    nonsynonymous (N) or multiple (M), pN/pS and dN/dS, with the allele statistics of each gene (inStrain's gene_info
+    with fixed allele calls).  Not in the reference: additive.
+    """
+    _refuse_stream(bamfile)
+    table = read_genes(gene_file)
+    with AlignmentFile(bamfile, decode=bam_decode) as bam:
+        records, stats, sites = bam.gene_stats(
+            table, FastaFile(reference_fasta), quality_threshold=quality_threshold, read_callback=read_callback,
+            min_coverage=min_coverage, min_freq=min_freq, min_count=min_count, sites=sites_out is not None)
+    ints = [f for f in records.dtype.names if f != "pad"]
+    derived = derive(stats)
+    derived_genes = derive_genes(records)
+    writer = csv.writer(outfile)
+    writer.writerow(["name", "contig", "start", "end", "strand"] + ints + sorted(derived) + list(derived_genes))
+    for k in range(len(records)):
+        writer.writerow([table.name[k], table.contig[k], int(table.start[k]), int(table.end[k]),
+                         "+" if table.strand[k] > 0 else "-"] + [int(records[f][k]) for f in ints]
+                        + [float(derived[n][k]) for n in sorted(derived)] + [float(v[k]) for v in derived_genes.values()])
+    if sites is not None:
+        write_gene_sites(table, sites, sites_out)
+
+
+def write_gene_sites(table, sites, out):
+    """Gene sites as TSV lines: gene name, contig, 0-based position, codon index and position in it (from the 5' end),
+    the reference codon, major and minor allele (genomic orientation), the amino acids of the reference codon and with
+    the major / minor allele, the SNV / SUB flags as 0 / 1 and the SNV / SUB types N S M ('.' where none applies)."""
+    out.write("gene\tcontig\tpos\tcodon\tcodon_pos\tref_codon\tmajor\tminor\taa_ref\taa_major\taa_minor\tsnv\tsub"
+              "\tsnv_type\tsub_type\n")
+    cols = [sites[k].tolist() for k in ("gene", "pos", "codon", "codon_pos", "kind")]
+    letters = [[x.decode() or "." for x in sites[k].tolist()] for k in ("ref_codon", "major", "minor", "aa_ref", "aa_major",
+                                                                        "aa_minor", "snv_type", "sub_type")]
+    for (g, p, c, cp, k), (rc, ma, mi, ar, am, an, st, bt) in zip(zip(*cols), zip(*letters)):
+        out.write("%s\t%s\t%d\t%d\t%d\t%s\t%s\t%s\t%s\t%s\t%s\t%d\t%d\t%s\t%s\n" % (
+            table.name[g], table.contig[g], p, c, cp, rc, ma, mi, ar, am, an, k & 1, (k >> 1) & 1, st, bt))
 
 
 def _alleles_of(sig):

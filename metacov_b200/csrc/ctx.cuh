@@ -70,6 +70,7 @@ enum KernelId {
   kKAlleleSignature, kKCompareChunks, kKCompareCombine, kKCompareSiteCount, kKCompareSiteWrite,
   kKLinkSites, kKLinkObsCount, kKLinkObsWrite, kKLinkSort, kKLinkUnitCalls, kKLinkSelect, kKLinkPairs, kKLinkPairCount,
   kKLinkPairWrite,
+  kKGeneChunks, kKGeneCombine, kKGeneSiteWrite,
   kKernelCount
 };
 
@@ -208,8 +209,9 @@ struct mcov_ctx {
   mcov::DevBuf d_ref, d_ref_stage, d_pair_sigs;
   std::vector<uint8_t> ref_set;
   int64_t ref_epoch = -1;
-  // Scratch of the allele and compare region / site calls, one set for both: every such call synchronises before it
-  // returns.  Regions: the chunks (AlChunk), the meta [first[g + 1] | length[g]] (int64), a partial record per chunk,
+  // Scratch of the allele, compare and gene region / site calls, one set for all: every such call synchronises before
+  // it returns.  Regions: the chunks (AlChunk; GnChunk), the meta [first[g + 1] | length[g]] (int64; the gene call
+  // adds codons[g]), a partial record per chunk,
   // the region records.  Sites: the tile counts followed by their inclusive scan (int64), the scan's temporary storage.
   mcov::DevBuf d_chunks, d_chunk_meta, d_chunk_part, d_region_out, d_site_tiles, d_site_scan;
   // the site lists of the last mcov_allele_sites and mcov_compare_sites (both stay readable)
@@ -220,6 +222,8 @@ struct mcov_ctx {
   mcov::SiteList link_sites, link_pairs;
   mcov::DevBuf d_lk_slot, d_lk_tid, d_lk_allele, d_lk_partners, d_lk_base, d_lk_rec_n, d_lk_rec_off, d_lk_obs[2], d_lk_cnt,
       d_lk_tmp, d_lk_word;
+  // Genes (genes.cu): the site list of the last mcov_gene_run that asked for one (its scratch is the allele calls')
+  mcov::SiteList gene_sites;
 
   // fused (sorted) path scratch
   mcov::DevBuf d_start_slot, d_far_list, d_tile_cnt, d_tile_off, d_far_sorted;

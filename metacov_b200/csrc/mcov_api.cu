@@ -1100,7 +1100,8 @@ static const char* kKernelNames[kKernelCount] = {
     "k_ref_encode", "k_allele_chunks", "k_allele_combine", "k_allele_site_count", "k_allele_site_write",
     "k_allele_signature", "k_compare_chunks", "k_compare_combine", "k_compare_site_count", "k_compare_site_write",
     "k_link_sites", "k_link_obs_count", "k_link_obs_write", "cub_link_sort", "k_link_unit_calls", "cub_link_select",
-    "k_link_pairs", "k_link_pair_count", "k_link_pair_write"};
+    "k_link_pairs", "k_link_pair_count", "k_link_pair_write",
+    "k_gene_chunks", "k_gene_combine", "k_gene_site_write"};
 
 int mcov_copy_to_host(mcov_ctx* ctx, const void* dev, void* host, int64_t n_bytes) {
   if (!ctx) return MCOV_ERR_ARG;

@@ -335,6 +335,28 @@ class CoverageEngine:
         self._check(lib.mcov_allele_sites_read(self._ctx, 0, n.value, _capi.ptr(out)))
         return out
 
+    # -- genes (codons of base_counts and the reference) --------------------------------------------------------------
+    def gene_stats(self, tid, start, end, strand, phase, min_coverage=5, min_freq=0.05, min_count=2, sites=False):
+        """Codon-level records of g genes (``mcov_gene_run``) -> (structured array ``_capi.GENE_STATS_DTYPE``, and with
+        ``sites`` every site of every gene in (gene, pos) order as ``_capi.GENE_SITE_DTYPE``, else None).  Genes are
+        0-based half-open with strand +1 / -1 and phase 0-2.  Needs ``base_counts`` and a ``set_reference`` of every
+        contig first."""
+        tid, start, end, g = self._region_columns(tid, start, end)
+        strand = np.ascontiguousarray(strand, dtype=np.int32)
+        phase = np.ascontiguousarray(phase, dtype=np.int32)
+        if not len(strand) == len(phase) == g:
+            raise ValueError("tid/start/end/strand/phase lengths differ")
+        p = self._allele_params(min_coverage, min_freq, min_count, True)
+        out = np.zeros(g, dtype=_capi.GENE_STATS_DTYPE)
+        n = C.c_int64(0)
+        self._check(lib.mcov_gene_run(self._ctx, g, _capi.ptr(tid), _capi.ptr(start), _capi.ptr(end), _capi.ptr(strand),
+                                      _capi.ptr(phase), C.byref(p), _capi.ptr(out), C.byref(n) if sites else None))
+        if not sites:
+            return out, None
+        listed = np.zeros(n.value, dtype=_capi.GENE_SITE_DTYPE)
+        self._check(lib.mcov_gene_sites_read(self._ctx, 0, n.value, _capi.ptr(listed)))
+        return out, listed
+
     # -- linkage (SNV sites of base_counts, then the records they were counted from) ---------------------------------
     @staticmethod
     def _linkage_params(min_coverage, min_freq, min_count, max_distance, min_reads):
