@@ -426,6 +426,9 @@ int  mcov_copy_to_host(mcov_ctx* ctx, const void* dev, void* host, int64_t n_byt
 
 /* kernels (and clears) enqueued by this context since it was created */
 int64_t mcov_launch_count(const mcov_ctx* ctx);
+/* The cached statistics plan (the regions of the last mcov_region_stats_* call): CTAs of the large-region stream and
+ * regions it splits between CTAs (0 and 0 before any plan). */
+int  mcov_region_plan_info(const mcov_ctx* ctx, int32_t* stream_ctas, int32_t* split_regions);
 /* on=1: bracket every kernel launch with CUDA events and reset the totals; on=0: stop. */
 int  mcov_profile_enable(mcov_ctx* ctx, int on);
 /* Synchronises; fills up to cap entries; returns the number written (>=0) or an error. */

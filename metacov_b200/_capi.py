@@ -255,6 +255,7 @@ SIGNATURES = {
     "mcov_depth_ptr": (_vp, [_vp]),
     "mcov_pass_info_get": (C.c_int, [_vp, C.POINTER(PassInfo)]),
     "mcov_launch_count": (_i64, [_vp]),
+    "mcov_region_plan_info": (C.c_int, [_vp, _vp, _vp]),
     "mcov_profile_enable": (C.c_int, [_vp, C.c_int]),
     "mcov_profile_read": (C.c_int, [_vp, C.POINTER(KernelTime), C.c_int]),
     "mcov_isize_hist": (C.c_int, [_vp, _i64, _vp, _vp, C.c_int, _i32, _vp, _i32, _vp, _vp, _vp]),

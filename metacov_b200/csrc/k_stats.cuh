@@ -56,17 +56,20 @@ struct WalkOut {
 };
 
 // Walk the bins [lo, hi] of a counting histogram held in shared memory (bins outside the range are
-// not touched and may hold garbage); all THREADS threads participate, the result is valid on thread
-// 0.  n = number of values the histogram describes.
-// CONSUMERS_ONLY: the THREADS threads are the consumer warps of a warp-specialised CTA and meet at named barrier 1
-template <int THREADS, bool CONSUMERS_ONLY = false>
-__device__ __forceinline__ WalkOut hist_walk(const uint32_t* hist, long long n, int breadth_n, int lo, int hi,
+// not touched and may hold garbage); all THREADS threads participate, the result is valid on the
+// first of them.  n = number of values the histogram describes.
+// CONSUMERS_ONLY: the THREADS threads (an aligned group of threadIdx.x) are some of the warps of a warp-specialised CTA
+// and meet at named barrier BAR.
+// CLEAR: every thread zeroes the bins it walked, so [lo, hi] is zero again once all threads are past the walk's
+// second barrier (bins outside it must be zero on entry).
+template <int THREADS, bool CONSUMERS_ONLY = false, bool CLEAR = false, int BAR = 1>
+__device__ __forceinline__ WalkOut hist_walk(uint32_t* hist, long long n, int breadth_n, int lo, int hi,
                                              unsigned long long* s_u64 /* [6][THREADS/32] */,
                                              int* s_i32 /* [4][THREADS/32] */, int* s_med /* 2 */) {
   constexpr int kW = THREADS / 32;
   const long long k1 = n / 4, k2 = n - n / 4;                // interquartile ranks [k1, k2)
   const long long m1 = (n - 1) / 2, m2 = n / 2;              // median pair
-  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  const int t = threadIdx.x % THREADS, lane = t & 31, warp = t >> 5;
   const int per = (hi - lo + THREADS) / THREADS;             // bins per thread (>= 1)
   const int b0 = lo + t * per, b1 = min(b0 + per, hi + 1);   // this thread's bins [b0, b1)
   unsigned long long local = 0;
@@ -79,7 +82,7 @@ __device__ __forceinline__ WalkOut hist_walk(const uint32_t* hist, long long n, 
     if (lane >= o) x += y;
   }
   if (lane == 31) s_u64[warp] = x;
-  if (CONSUMERS_ONLY) named_bar_sync<1, THREADS>(); else __syncthreads();
+  if (CONSUMERS_ONLY) named_bar_sync<BAR, THREADS>(); else __syncthreads();
   unsigned long long before = 0;
 #pragma unroll
   for (int k = 0; k < kW; ++k) before += (k < warp) ? s_u64[k] : 0ull;
@@ -102,10 +105,11 @@ __device__ __forceinline__ WalkOut hist_walk(const uint32_t* hist, long long n, 
         if (c <= m1 && m1 < c + cn) s_med[0] = bb;
         if (c <= m2 && m2 < c + cn) s_med[1] = bb;
         c += cn;
+        if (CLEAR) hist[bb] = 0u;
       }
     }
   }
-  if (CONSUMERS_ONLY) named_bar_sync<1, THREADS>(); else __syncthreads();                                            // s_u64[0..kW) consumed, s_med written
+  if (CONSUMERS_ONLY) named_bar_sync<BAR, THREADS>(); else __syncthreads();                                            // s_u64[0..kW) consumed, s_med written
   sum = warp_sum(sum); iq = warp_sum(iq); ge1 = warp_sum(ge1); geN = warp_sum(geN); sumsq = warp_sum(sumsq);
   mn = warp_min(mn); mx = warp_max(mx);
   if (lane == 0) {
@@ -114,7 +118,7 @@ __device__ __forceinline__ WalkOut hist_walk(const uint32_t* hist, long long n, 
     s_u64[4 * kW + warp] = sumsq;
     s_i32[0 * kW + warp] = mn; s_i32[1 * kW + warp] = mx;
   }
-  if (CONSUMERS_ONLY) named_bar_sync<1, THREADS>(); else __syncthreads();
+  if (CONSUMERS_ONLY) named_bar_sync<BAR, THREADS>(); else __syncthreads();
   WalkOut w;
   w.sum = 0; w.iq_sum = 0; w.ge1 = 0; w.geN = 0; w.sumsq = 0; w.mn = INT_MAX; w.mx = INT_MIN;
   if (t == 0) {

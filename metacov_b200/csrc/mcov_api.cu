@@ -1123,6 +1123,13 @@ int mcov_sync(mcov_ctx* ctx) {
 
 int64_t mcov_launch_count(const mcov_ctx* ctx) { return ctx ? ctx->n_launches : 0; }
 
+int mcov_region_plan_info(const mcov_ctx* ctx, int32_t* stream_ctas, int32_t* split_regions) {
+  if (!ctx || !stream_ctas || !split_regions) return MCOV_ERR_ARG;
+  *stream_ctas = ctx->plan.valid ? ctx->plan.ss_grid : 0;
+  *split_regions = ctx->plan.valid ? ctx->plan.n_split : 0;
+  return MCOV_OK;
+}
+
 int mcov_profile_enable(mcov_ctx* ctx, int on) {
   if (!ctx) return MCOV_ERR_ARG;
   CU(cudaSetDevice(ctx->device));
@@ -1148,6 +1155,25 @@ int mcov_profile_read(mcov_ctx* ctx, mcov_kernel_time* out, int cap) {
   }
   return n;
 }
+
+#ifdef MCOV_SS_PROBE
+// Phase timer of k_stats_stream (tools/probe_stats_chain.py): copies [n_cta][kPrPhases] counters of the last launch to
+// out (clear != 0: zeroes them instead), returns the CTAs of the current plan's stream.
+int mcov_ss_probe(mcov_ctx* ctx, unsigned long long* out, int n_cta, int clear) {
+  if (!ctx || n_cta < 0 || n_cta > kPrMaxCtas) return MCOV_ERR_ARG;
+  CU(cudaSetDevice(ctx->device));
+  CU(cudaStreamSynchronize(ctx->stream));
+  const size_t bytes = (size_t)n_cta * kPrPhases * 8;
+  if (clear) {
+    void* p = nullptr;
+    CU(cudaGetSymbolAddress(&p, g_ss_probe));
+    CU(cudaMemset(p, 0, sizeof(g_ss_probe)));
+  } else if (bytes) {
+    CU(cudaMemcpyFromSymbol(out, g_ss_probe, bytes));
+  }
+  return ctx->plan.ss_grid;
+}
+#endif
 
 int32_t* mcov_depth_ptr(mcov_ctx* ctx) {
   if (!ctx || ctx->state != kDepthReady) return nullptr;
@@ -1197,39 +1223,81 @@ static int stats_launch(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int3
         small.push_back(t);
       }
     }
-    // The balanced stream over the large regions (k_stats_stream.cuh): their concatenation cut into equal slices,
-    // one per persistent CTA; a region cut by a slice border becomes a "split" region with a global histogram.
+    // The balanced stream over the large regions (k_stats_stream.cuh): one slice per persistent CTA, of equal cost.
+    // A piece costs the bytes k_stats_stream stages for it plus kSsPieceCost for its end and walk; a region cut by a
+    // slice border becomes a "split" region with a global histogram, whose merges cost kSsSplitCost more.  A border
+    // moves to the nearer region border when that unbalances the slices by less than a split costs.  The passes
+    // that follow count tile histograms when at least half of the tiles lie wholly inside a large region (the same
+    // test as mcov_depth_sorted's): only then does a tile inside a region cost 256 bytes rather than its depth.
     int64_t total_big = 0;
-    for (int64_t i = 0; i < g; ++i) if (rp.rlen[i] > kSmallRegion) total_big += rp.rlen[i];
+    int64_t region_tiles = 0;                // tiles that lie wholly inside a large region
+    std::vector<int64_t> big_slot((size_t)g, 0);
+    for (int64_t i = 0; i < g; ++i) {
+      if (rp.rlen[i] <= kSmallRegion) continue;
+      big_slot[i] = ctx->off[tid[i]] + clip_region(ctx, tid[i], start[i], end[i]).cs;
+      total_big += rp.rlen[i];
+      region_tiles += std::max<int64_t>(0, ((big_slot[i] + rp.rlen[i]) >> kTileShift) - ((big_slot[i] + kTile - 1) >> kTileShift));
+    }
+    const bool hist_gate = 2 * region_tiles >= (ctx->n_slots + kTile - 1) / kTile;
+    auto region_cost = [&](int64_t s0, int64_t n) -> double {
+      if (!hist_gate) return 4.0 * (double)n;
+      const int64_t t0 = (s0 + kTile - 1) >> kTileShift, t1 = (s0 + n) >> kTileShift;
+      if (t1 <= t0) return 4.0 * (double)n;
+      return 4.0 * (double)(n - ((t1 - t0) << kTileShift)) + (double)((t1 - t0) * kTileHistWords * 2) + (double)kSsPieceCost;
+    };
     std::vector<SsPiece> pieces;
     std::vector<int32_t> cta_start, split_npieces;
     const int32_t grid = (int32_t)std::min<int64_t>((int64_t)ctx->n_sm * MCOV_SS_CTAS, std::max<int64_t>(1, total_big / 16384));
-    const int64_t W = std::max<int64_t>(4, ((total_big + grid - 1) / grid + 3) & ~(int64_t)3);
-    int64_t room = W;
+    double total_cost = 0;
+    for (int64_t i = 0; i < g; ++i) if (rp.rlen[i] > kSmallRegion) total_cost += region_cost(big_slot[i], rp.rlen[i]);
+    const double T = total_cost / grid;
+    int32_t kb = 1;                          // next slice border: at cost kb * T
+    auto close_slice = [&]() { if (cta_start.back() != (int32_t)pieces.size()) cta_start.push_back((int32_t)pieces.size()); };
+    double cum = 0;
     cta_start.push_back(0);
     for (int64_t i = 0; i < g && total_big > 0; ++i) {
       if (rp.rlen[i] <= kSmallRegion) continue;
-      int64_t rem = rp.rlen[i];
-      int64_t slot = ctx->off[tid[i]] + clip_region(ctx, tid[i], start[i], end[i]).cs;
+      const double c = region_cost(big_slot[i], rp.rlen[i]), r0 = cum, r1 = cum + c;
+      const double per_slot = c / (double)rp.rlen[i];
+      int64_t slot = big_slot[i], rem = rp.rlen[i];
+      double at = r0;                        // cost up to `slot`
+      bool close_after = false;
       const size_t first_piece = pieces.size();
-      while (rem > 0) {
-        const int64_t take = std::min(rem, room);
+      auto piece = [&](int64_t n) {
         SsPiece pc;
-        pc.slot = slot; pc.n = (int32_t)take; pc.region = (int32_t)i; pc.pad = pieces.size() == first_piece ? rp.rpad[i] : 0; pc.split = -1;
+        pc.slot = slot; pc.n = (int32_t)n; pc.region = (int32_t)i; pc.pad = pieces.size() == first_piece ? rp.rpad[i] : 0;
+        pc.split = -1; pc.n_region = rp.rlen[i] + rp.rpad[i]; pc.reserved = 0;
         pieces.push_back(pc);
-        rem -= take; slot += take; room -= take;
-        if (room == 0) { cta_start.push_back((int32_t)pieces.size()); room = W; }
+        slot += n; rem -= n;
+      };
+      for (; kb < grid && kb * T < r1; ++kb) {
+        const double B = kb * T;
+        // (a border moves to the region's start only out of a slice that holds something: else every border up to the
+        // region's middle would collapse there and one slice would take the whole region)
+        if (slot == big_slot[i] && cta_start.back() != (int32_t)pieces.size() && B - r0 <= r1 - B && B - r0 <= kSsSplitCost) {
+          close_slice();
+          continue;
+        }
+        if (r1 - B <= kSsSplitCost) { close_after = true; continue; }
+        const int64_t take = std::min<int64_t>(rem - 1, std::max<int64_t>(1, (int64_t)((B - at) / per_slot)));
+        if (take <= 0) { close_after = true; continue; }
+        piece(take);
+        at = B;
+        close_slice();
       }
+      piece(rem);
+      if (close_after) close_slice();
+      cum = r1;
       if (pieces.size() - first_piece > 1) {
         const int32_t id = (int32_t)split_npieces.size();
         split_npieces.push_back((int32_t)(pieces.size() - first_piece));
         for (size_t k = first_piece; k < pieces.size(); ++k) pieces[k].split = id;
       }
     }
-    if (cta_start.back() != (int32_t)pieces.size()) cta_start.push_back((int32_t)pieces.size());
+    close_slice();
     rp.ss_grid = total_big > 0 ? (int32_t)cta_start.size() - 1 : 0;
     rp.n_split = (int32_t)split_npieces.size();
-    // tiles that lie wholly inside a large region (overlapping regions may count a tile twice): decide whether the fused
+    // tiles that lie wholly inside a piece (overlapping regions may count a tile twice): decide whether the fused
     // passes that follow count depth histograms
     rp.hist_tiles = 0;
     for (const SsPiece& pc : pieces) rp.hist_tiles += std::max<int64_t>(0, ((pc.slot + pc.n) >> kTileShift) - ((pc.slot + kTile - 1) >> kTileShift));
@@ -1265,9 +1333,7 @@ static int stats_launch(mcov_ctx* ctx, int64_t g, const int32_t* tid, const int3
   if (g > 0) {
     if (rp.ss_grid > 0) {
       SsArgs a;
-      int32_t* d_rlen = ctx->d_rlen.as<int32_t>();
       a.depth = ctx->depth; a.pieces = ctx->d_ss_pieces.as<SsPiece>(); a.cta_piece_start = ctx->d_ss_cta.as<int32_t>();
-      a.region_len = d_rlen; a.region_pad = d_rlen + g;
       a.split_scratch = ctx->d_ss_pool.as<RegionScratch>();
       a.split_hist = reinterpret_cast<uint32_t*>(ctx->d_ss_pool.as<char>() + (size_t)rp.n_split * sizeof(RegionScratch));
       a.split_pieces = ctx->d_ss_split.as<int32_t>();

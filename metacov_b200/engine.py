@@ -443,6 +443,12 @@ class CoverageEngine:
     def launch_count(self):
         return lib.mcov_launch_count(self._ctx)
 
+    def region_plan_info(self):
+        """(CTAs of the large-region stream, regions split between them) of the cached statistics plan."""
+        ctas, splits = C.c_int32(), C.c_int32()
+        self._check(lib.mcov_region_plan_info(self._ctx, C.byref(ctas), C.byref(splits)))
+        return ctas.value, splits.value
+
     def profile(self, on=True):
         self._check(lib.mcov_profile_enable(self._ctx, 1 if on else 0))
 
